@@ -11,10 +11,11 @@ slam_mapping; the Adam pose fit and the EKF stay on the host in the reference an
 the metric (the whole step with pose feedback is reported beside it as `e2e_closed_loop`).
 
   value : frames/s with the sequence resident in HBM (nav_frontend_sequence_dev: one launch per frame,
-          consecutive launches overlapped by programmatic dependent launch).  The K timed steps are
-          repeated on different frames of the resident set until >= --min-timed-ms of device time has
-          been measured; every repetition is bracketed by its own CUDA events and `ms_per_step` is the
-          median repetition (min / median / max per rank are reported too).
+          consecutive launches overlapped by programmatic dependent launch).  Exactly K = --steps steps
+          are timed, after W = --warmup untimed ones, between one pair of CUDA events (three untimed
+          passes over the same frames come first, so that their first device touch is not timed);
+          `ms_per_step` is that time / K.  --dump-outputs DIR writes what the last timed step computed
+          (labels, NN indices and distances, mapped cloud, map masks) as DIR/<name>.npy.
   e2e   : frames/s through the host-buffer C ABI call (nav_frontend_submit): every step copies the frame
           from pinned host memory to the device and copies the step's results -- labels, NN indices, NN
           distances -- back; uploads, kernels and downloads of consecutive frames overlap.
@@ -409,6 +410,32 @@ def bind_near_gpu(torch, local):
 
 
 # ------------------------------------------------------------------ GPU arm ---------------------
+class Raw:
+    """n elements of a device buffer the library owns, for torch.as_tensor(..., device="cuda")."""
+    def __init__(self, ptr, n, typestr):
+        self.__cuda_array_interface__ = {"shape": (n,), "typestr": typestr, "data": (ptr, False), "version": 2}
+
+
+def dump_outputs(out_dir, res, torch):
+    """What the timed path hands its caller for the last timed frame (nav_frame_results_dev), copied to the
+    host: int32 labels as float32, indices and bit masks as float64 (exact), distances and the mapped cloud
+    as float64.  5.8 MB in all."""
+    n_chunks = (COLS + 15) // 16
+    arrays = {"labels": (res.labels, (ROWS, COLS), "<i4", np.float32),
+              "nn_idx": (res.nn_idx, (ROWS, COLS), "<i4", np.float64),
+              "nn_dist": (res.nn_dist, (ROWS, COLS), "<f8", np.float64),
+              "global_cloud": (res.global_, (ROWS, COLS, 3), "<f8", np.float64),
+              "map_mask": (res.map_mask, (ROWS, n_chunks), "<i4", np.float64)}
+    torch.cuda.synchronize()
+    os.makedirs(out_dir, exist_ok=True)
+    for name, (ptr, shape, typestr, np_dtype) in arrays.items():
+        n = int(np.prod(shape))
+        host = torch.as_tensor(Raw(ptr, n, typestr), device="cuda").cpu().numpy().reshape(shape)
+        if name == "map_mask":
+            host = host.view(np.uint32)        # 32-bit masks: read as unsigned
+        np.save(os.path.join(out_dir, name + ".npy"), host.astype(np_dtype))
+
+
 def run_gpu_arm(args):
     import torch
     import torch.distributed as dist
@@ -487,56 +514,38 @@ def run_gpu_arm(args):
                 a[i] = pos_c(p)
         return arrs
 
-    # ---------------- value: device resident, K steps per repetition, repeated on different frames
-    span = W + K                       # frames one repetition consumes after its initial frame
-    n_starts = max(1, (n_res - 1 - span) // max(1, K) + 1)
+    # ---------------- value: device resident, the K timed steps on frames F0 + W .. F0 + W + K - 1
+    F0 = 1
+    p_init, wp, kp = pos_c(pose_of(F0 - 1)), pose_block(F0, W), pose_block(F0 + W, K)
 
-    def rep_first_frame(r):
-        return 1 + (r % n_starts) * K if n_res - 1 - span > 0 else 1
-
-    def run_reps(n_reps):
-        """Queue n_reps repetitions back to back (no host synchronisation in between): re-initialise the map
-        on the frame before the window, W untimed steps, then K steps between two events."""
-        evs = []
-        blocks = {}
-        for r in range(n_reps):
-            f0 = rep_first_frame(r)
-            if f0 not in blocks:
-                blocks[f0] = (pos_c(pose_of(f0 - 1)), pose_block(f0, W), pose_block(f0 + W, K))
+    def run_window():
+        """Re-initialise the map on frame F0 - 1, W untimed steps, then the K steps between two events.
+        Returns their device ms and the launches of the whole window (re-init and warm-up included)."""
         barrier()
         l0 = ctx.launch_count()
-        for r in range(n_reps):
-            f0 = rep_first_frame(r)
-            p_init, wp, kp = blocks[f0]
-            check(L.nav_slam_init_dev(ctx.h, d_base + (f0 - 1) * FRAME_BYTES, C.byref(p_init)))
-            check(L.nav_frontend_sequence_dev(ctx.h, d_base + f0 * FRAME_BYTES, W, *wp))
-            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            e0.record(stream)
-            check(L.nav_frontend_sequence_dev(ctx.h, d_base + (f0 + W) * FRAME_BYTES, K, *kp))
-            e1.record(stream)
-            evs.append((e0, e1))
+        check(L.nav_slam_init_dev(ctx.h, d_base + (F0 - 1) * FRAME_BYTES, C.byref(p_init)))
+        check(L.nav_frontend_sequence_dev(ctx.h, d_base + F0 * FRAME_BYTES, W, *wp))
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record(stream)
+        check(L.nav_frontend_sequence_dev(ctx.h, d_base + (F0 + W) * FRAME_BYTES, K, *kp))
+        e1.record(stream)
         barrier()
-        ms = [a.elapsed_time(b) for a, b in evs]
-        return ms, ctx.launch_count() - l0
+        return e0.elapsed_time(e1), ctx.launch_count() - l0
 
     clocks = ClockSampler(local)
     clocks.start()
     spin_up()
-    cal, _ = run_reps(3)
-    est = max(float(np.median(cal)), 1e-3)
-    n_reps = int(min(2000, max(5, np.ceil(args.min_timed_ms / est))))
+    for _ in range(3):     # untimed passes over the same frames: their first device touch is not timed
+        run_window()
     spin_up()
-    rep_ms, rep_launches = run_reps(n_reps)
-    rep_ms = np.array(rep_ms)
-    dev_ms = float(np.median(rep_ms))                       # K steps
-    timed_ms_total = float(rep_ms.sum())
-    launches_per_rep = rep_launches / n_reps                # K fused launches + W warm-up + 2 for the re-init
-    my_stats = [float(rep_ms.min()) / K, dev_ms / K, float(rep_ms.max()) / K]
+    dev_ms, window_launches = run_window()       # --steps is the number of timed steps
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, ctx.frame_results_dev(), torch)
     if world > 1:
-        gathered = [None] * world
-        dist.all_gather_object(gathered, my_stats)
+        per_rank = [None] * world
+        dist.all_gather_object(per_rank, dev_ms / K)
     else:
-        gathered = [my_stats]
+        per_rank = [dev_ms / K]
     dev_ms = reduce_max([dev_ms])[0]
 
     # ---------------- per-kernel durations (CUDA events on the launching stream, one pair per launch)
@@ -725,10 +734,6 @@ def run_gpu_arm(args):
     # ---------------- dominant kernel roofline (SURVEY 8d algorithmic bytes)
     torch.cuda.synchronize()
     res = ctx.frame_results_dev()
-
-    class Raw:
-        def __init__(self, ptr, n, typestr):
-            self.__cuda_array_interface__ = {"shape": (n,), "typestr": typestr, "data": (ptr, False), "version": 2}
     nq = int((torch.as_tensor(Raw(res.labels, NPX, "<i4"), device="cuda") == 1).sum())
     n_map = nq  # consecutive frames label ~the same number of points
     n_leaf, n_sup = COLS // 16, COLS // 256
@@ -741,7 +746,7 @@ def run_gpu_arm(args):
         "map": NPX * (24 + 4 + 24) + side,
     }
     peak, tc_peak, peak_src = measured_peaks()
-    seq_mode = launches_per_rep < K          # the library ran the timed steps as one sequence launch
+    seq_mode = window_launches < K          # the library ran the timed steps as one sequence launch
     dom_kernel = "k_frame_seq" if seq_mode else "k_frame_match"
     kernels = {}
     for name, (ms, n) in prof.items():
@@ -749,16 +754,16 @@ def run_gpu_arm(args):
             us = 1e3 * ms / n
             extra = {}
             if name == "frame_fused":
-                # the timed region of `value` is K launches of this kernel per repetition: its average launch
+                # the timed region of `value` is K launches of this kernel: its average launch
                 # duration there (consecutive launches overlap through programmatic dependent launch) is the
                 # step time; the event-bracketed single launch is kept beside it
                 extra = {"us_per_launch_isolated": us}
-                us, n = 1e3 * dev_ms / K, K * n_reps
+                us, n = 1e3 * dev_ms / K, K
                 if seq_mode:
                     # the K timed steps are ONE launch of k_frame_seq (a thread-block cluster per image row walks
                     # through the frames): K frames of algorithmic bytes per launch over that launch's duration
                     extra.update({"frames_per_launch": K, "us_per_frame": us})
-                    us, n = 1e3 * dev_ms, n_reps
+                    us, n = 1e3 * dev_ms, 1
             ab = alg_bytes[name] * (K if (seq_mode and name == "frame_fused") else 1)
             ach = ab / (us * 1e-6) / 1e9
             kernels[name] = {"us_per_launch": us, "launches": n, "alg_bytes_per_launch": ab,
@@ -868,12 +873,11 @@ def run_gpu_arm(args):
                                     "resident sequence (L2 is 0.13 GB); the previous frame's row map (5 MB) is "
                                     "legitimately L2-warm; the clock spin-up between regions runs on a buffer of its own"
                                     % (n_res * FRAME_BYTES / 1e9),
-                       "timing": "%d repetitions of the K = %d timed steps, each on its own frames and between its own "
-                                 "CUDA events (queued back to back); ms_per_step = median repetition / K, MAX over ranks"
-                                 % (n_reps, K)},
-            "timed_region": {"repetitions": n_reps, "device_ms_total": timed_ms_total,
-                             "launches_per_repetition": launches_per_rep,
-                             "ms_per_step_min_median_max_per_rank": gathered},
+                       "timing": "the K = %d timed steps (frames %d..%d) between one pair of CUDA events, after 3 untimed "
+                                 "passes over the same frames and %d untimed warm-up steps; ms_per_step = that time / K, "
+                                 "MAX over ranks" % (K, F0 + W, F0 + W + K - 1, W)},
+            "timed_region": {"steps": K, "device_ms": dev_ms, "launches": window_launches,
+                             "ms_per_step_per_rank": per_rank},
             # headline e2e: pinned cloud in, the step's results (labels as bit masks + NN index + NN distance) out,
             # per frame, pipelined.  The mapped global cloud is persistent state (the next frame's search structure
             # and the source of the GPU CSV writer) and stays in HBM; the other variants are reported beside it.
@@ -900,12 +904,12 @@ def run_gpu_arm(args):
                                       "wall_ms_per_step": 1e3 * blk_wall / n_block}},
             "e2e_closed_loop": closed, "e2e_shim": shim,
             "gpu_launches": 1 if seq_mode else int(round(K)),
-            "gpu_launches_note": ("ONE launch of k_frame_seq covers the K timed steps of a repetition (a thread-block cluster "
-                                  "per image row walks through the frames; %.0f launches per repetition including the untimed "
+            "gpu_launches_note": ("ONE launch of k_frame_seq covers the K timed steps (a thread-block cluster "
+                                  "per image row walks through the frames; %.0f launches in the window including the untimed "
                                   "re-init and warm-up; NAV_SEQ_LAUNCHES=1 gives one k_frame_match launch per step)"
                                   if seq_mode else
-                                  "K launches of k_frame_match per timed repetition (%.0f launches per repetition including the "
-                                  "untimed re-init and warm-up)") % launches_per_rep,
+                                  "K launches of k_frame_match in the timed region (%.0f launches in the window including the "
+                                  "untimed re-init and warm-up)") % window_launches,
             "clocks": clk, "cpu_cores_bound_near_gpu": bound_cores,
             "roofline": None if dom is None else {
                 "kernel": {"frame_fused": ("k_frame_seq (labels + match + next map, K frames per launch)" if seq_mode else
@@ -1111,7 +1115,9 @@ def main():
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--frames", type=int, default=256, help="frames of the resident sequence (805 MB at 256)")
-    ap.add_argument("--min-timed-ms", type=float, default=60.0, help="device time to accumulate in the timed region")
+    ap.add_argument("--min-timed-ms", type=float, default=60.0, help="device time to accumulate in the e2e legs")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the results of the last timed step (rank 0) as DIR/<name>.npy")
     ap.add_argument("--stencil-images", type=int, default=512)
     ap.add_argument("--cpu-frames", type=int, default=60)
     ap.add_argument("--cpu-whole-frames", type=int, default=3)

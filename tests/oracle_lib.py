@@ -10,6 +10,8 @@ Nothing in nav-slam_b200/ imports this module.
 from __future__ import annotations
 
 import ctypes as C
+import hashlib
+import json
 import os
 import subprocess
 from contextlib import contextmanager
@@ -278,6 +280,66 @@ class OracleSlam:
 
 def ref_available(shape: str) -> bool:
     return os.path.exists(os.path.join(REF_DIR, f"libnavref_{shape}.so"))
+
+
+# ------------------------------------------------------------------ stored reference answers
+# The reference's sources are not part of this repository, so oracle/_ref is usually absent.  Every
+# comparison with it goes through check_ref(): against RefLib where oracle/_ref is built, otherwise against
+# the sha256 digest of the same answer stored in tests/golden/ref_digests.json.  Where oracle/_ref is built,
+# check_ref() also holds the stored digest to the live answer, so every such run validates the file.  The
+# file says what its answers were recorded from ("recorded_from") and lists the keys that were never
+# compared with the reference ("never_compared_with_the_reference"); tests/test_golden.py ties the keys it
+# shares with the reference-generated tests/golden/ref_*.npz to those vectors.
+# tests/golden/make_ref_digests.py re-records the file.
+REF_DIGESTS = os.path.join(ROOT, "tests", "golden", "ref_digests.json")
+_RECORD_TO = os.environ.get("NAVSLAM_RECORD_REF_DIGESTS")
+_digests = None
+_recorded = {}
+
+
+def digest(a) -> str:
+    """sha256 over dtype, shape and bytes: equal digests mean bit-identical arrays."""
+    a = np.ascontiguousarray(a)
+    h = hashlib.sha256(f"{a.dtype.str}{a.shape}".encode())
+    h.update(a.tobytes())
+    return h.hexdigest()
+
+
+def stored_answers() -> dict:
+    global _digests
+    if _digests is None:
+        with open(REF_DIGESTS) as f:
+            _digests = json.load(f)["answers"]
+    return _digests
+
+
+def check_ref(key: str, got, ref_fn=None, also=()):
+    """Assert that `got` is bit-identical to the reference's answer for `key`: ref_fn() (the live reference)
+    when it is given, else the stored digest.  `also` lists other forms of our answer that the reference may
+    equally give (the first one that matches counts).  With NAVSLAM_RECORD_REF_DIGESTS set the answer is
+    recorded instead of checked against the file."""
+    mine = [digest(x) for x in (got, *also)]
+    if ref_fn is not None:
+        want = digest(ref_fn())
+        assert want in mine, key
+    else:
+        want = mine[0]
+    if _RECORD_TO:
+        _recorded[key] = want
+        return
+    stored = stored_answers().get(key)
+    if ref_fn is None:
+        assert stored is not None, f"no stored reference answer for {key}"
+        assert stored in mine, key
+    elif stored is not None:
+        assert stored == want, f"{key}: tests/golden/ref_digests.json differs from the reference"
+
+
+def write_recorded(header: dict):
+    """Write what check_ref() recorded, under `header`, to the file NAVSLAM_RECORD_REF_DIGESTS names."""
+    with open(_RECORD_TO, "w") as f:
+        json.dump({**header, "answers": dict(sorted(_recorded.items()))}, f, indent=0)
+        f.write("\n")
 
 
 class RefLib:

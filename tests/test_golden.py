@@ -159,6 +159,27 @@ def test_oracle_kdtree_golden(oracle):
         oracle.tree_free(h)
 
 
+def test_stored_reference_answers_match_golden():
+    """tests/golden/ref_digests.json against these reference-generated vectors wherever both hold the
+    reference's answer to the same input: the whole step at 8x8 (same clouds, start pose and predictions as
+    test_whole_step_bit_exact, frames 0-4), its first step at 5x33 (later 5x33 golden frames carry invalid
+    returns) and the labels of the first 5x33 frame."""
+    from oracle_lib import digest, stored_answers
+    stored = stored_answers()
+    pairs = []
+    g = gold((8, 8))
+    for f in range(5):
+        pairs.append((f"whole_step/8x8/global{f}", g["globals"][f]))
+        if f:
+            pairs += [(f"whole_step/8x8/pose{f}", g["poses"][f]), (f"whole_step/8x8/error{f}", g["errors"][f])]
+    g = gold((5, 33))
+    pairs += [("whole_step/5x33/global0", g["globals"][0]), ("whole_step/5x33/global1", g["globals"][1]),
+              ("whole_step/5x33/pose1", g["poses"][1]), ("whole_step/5x33/error1", g["errors"][1]),
+              ("extract_feature/5x33/0", g["labels"][0])]
+    for key, want in pairs:
+        assert stored[key] == digest(want), key
+
+
 # ------------------------------------------------------------------------------ GPU ----------
 @pytest.mark.gpu
 @pytest.mark.parametrize("shape", [(8, 8), (5, 33)])

@@ -1,6 +1,7 @@
 """The data formats either side of the path (SURVEY 8f #3, #4): the L9 CSV reader (src/main.c:77-128)
 and the 25-column CSV row writer (src/main.c:243,320-352).  Host code of the C-ABI library, so these
-run without a GPU.  Checkers: the reference's own L9_LidarProcessData (oracle/_ref), the oracle's
+run without a GPU.  Checkers: the reference's own readers (oracle/_ref where built, else their stored
+answers, oracle_lib.check_ref), the oracle's
 fscanf / snprintf restatements, and Python's correctly rounded '%.2f'."""
 import importlib
 import os
@@ -8,7 +9,7 @@ import os
 import numpy as np
 import pytest
 
-from oracle_lib import Oracle, RefLib, ref_available
+from oracle_lib import Oracle, RefLib, check_ref, ref_available
 
 nav = importlib.import_module("nav-slam_b200")
 synth = importlib.import_module("nav-slam_b200.synth")
@@ -118,11 +119,10 @@ def test_reader_matches_reference_and_oracle(tmp_path, oracle, shape):
     assert rc == 0 and len(frames) == 6
     assert np.array_equal(ts, ots) and list(ts) == [10, 13, 16, 19, 22, 25]
     assert frames.tobytes() == oframes.tobytes()
-    if not ref_available(f"{rows}x{cols}"):
-        pytest.skip("oracle/_ref not built")
-    rframes, rts, _ = RefLib(rows, cols).l9_csv_read(path, 10)
-    assert np.array_equal(rts, ts)
-    assert rframes.tobytes() == frames.tobytes()
+    ref = RefLib(rows, cols) if ref_available(f"{rows}x{cols}") else None
+    rd = ref.l9_csv_read(path, 10) if ref is not None else None
+    check_ref(f"l9_csv_read/{rows}x{cols}/timestamps", ts, rd and (lambda: rd[1]))
+    check_ref(f"l9_csv_read/{rows}x{cols}/frames", frames, rd and (lambda: rd[0]))
 
 
 def test_reader_integer_frames_config2(tmp_path, oracle):
@@ -132,9 +132,9 @@ def test_reader_integer_frames_config2(tmp_path, oracle):
     frames, ts = nav.l9_csv_read(path, 16, 1800, 10)
     assert list(ts) == [0, 1, 2]
     assert np.array_equal(frames, np.trunc(seq))
-    if ref_available("16x1800"):
-        rframes, rts, _ = RefLib(16, 1800).l9_csv_read(path, 10)
-        assert rframes.tobytes() == frames.tobytes() and np.array_equal(rts, ts)
+    rd = RefLib(16, 1800).l9_csv_read(path, 10) if ref_available("16x1800") else None
+    check_ref("l9_csv_read/16x1800/timestamps", ts, rd and (lambda: rd[1]))
+    check_ref("l9_csv_read/16x1800/frames", frames, rd and (lambda: rd[0]))
 
 
 def test_reader_edge_cases(tmp_path, oracle):
@@ -225,15 +225,14 @@ def test_json_readers_match_reference(tmp_path):
             assert d[2].ravel()[:64].tolist() == list(range(64))
             assert d[3].ravel()[:3].tolist() == [7, 8, -77] and ts[3] == 9
             assert prm[0].tolist() == [0.0, 2.0, 3.5, 4.25, 0.5, 6.0] and prm[1].tolist() == [0.0] * 6
-        if not ref_available("8x8"):
-            continue
-        ref = RefLib(8, 8)
-        rd, rts = ref.l5_json_read(p, 100, fill=-77)
-        rprm, rits = ref.imu_json_read(p, 100)
-        assert np.array_equal(d, rd) and np.array_equal(prm, rprm)
+        ref = RefLib(8, 8) if ref_available("8x8") else None
+        rd, rts = ref.l5_json_read(p, 100, fill=-77) if ref is not None else (None, None)
+        rprm, rits = ref.imu_json_read(p, 100) if ref is not None else (None, None)
+        check_ref(f"l5_json_read/{name}/distances", d, ref and (lambda: rd))
+        check_ref(f"imu_json_read/{name}/params", prm, ref and (lambda: rprm))
+        check_ref(f"imu_json_read/{name}/timestamps", its, ref and (lambda: rits))
         # a frame without an integer "time_main" keeps whatever the caller's buffer held: both start from 0 / -77
-        assert np.array_equal(np.where(ts == 0, -77, ts), np.where(rts == -77, -77, rts)) or np.array_equal(ts, rts)
-        assert np.array_equal(its, rits)
+        check_ref(f"l5_json_read/{name}/timestamps", ts, ref and (lambda: rts), also=(np.where(ts == 0, -77, ts),))
 
 
 def test_json_invalid_documents_read_nothing(tmp_path):

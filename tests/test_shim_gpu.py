@@ -1,6 +1,7 @@
 """GPU tests of the drop-in shim: the reference's own symbols (init_slam, slam_localization,
 slam_mapping, ...) served by libnavslam_shim_<RxC>.so, and the reference's UNMODIFIED main.c +
-ekf.c linked against it (oracle/_ref/navshim_main_*), compared with the reference itself."""
+ekf.c linked against it (oracle/_ref/navshim_main_*), compared with the reference itself.  The two
+whole-program tests need the reference's sources at build time and skip without them."""
 import ctypes as C
 import os
 import subprocess
@@ -9,7 +10,7 @@ import numpy as np
 import pytest
 
 from conftest import big_stack
-from oracle_lib import Pos, REF_DIR, RefLib, quiet_stdout, ref_available
+from oracle_lib import Pos, REF_DIR, RefLib, check_ref, quiet_stdout, ref_available
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -55,37 +56,67 @@ class Shim:
         return int(np.frombuffer(self.attr[off:off + 4].tobytes(), dtype=np.int32)[0])
 
 
-@pytest.mark.parametrize("shape,frames", [((8, 8), 8), ((5, 33), 6), ((64, 2048), 3)])
-def test_shim_slam_step_matches_reference(pkg, oracle, synth, shape, frames):
+SLAM_STEP_CASES = [((8, 8), 8), ((5, 33), 6), ((64, 2048), 3)]
+
+
+def reference_slam_steps(oracle, synth, shape, frames):
+    """The reference's init_slam / slam_localization / slam_mapping on the shim test's inputs: the oracle in
+    the reference's tie mode, checked against the reference (live where oracle/_ref is built, else its stored
+    answers).  Returns the clouds, the start pose and per frame (pose, error, global cloud)."""
     r, c = shape
-    if not ref_available(f"{r}x{c}"):
-        pytest.skip("reference library not built")
-    ref = RefLib(r, c)
-    shim = Shim(pkg, r, c)
+    key = f"shim_slam_step/{r}x{c}"
+    ref = RefLib(r, c) if ref_available(f"{r}x{c}") else None
     if shape == (8, 8):
         clouds = [oracle.convert(synth.l5_depth_frame(f)) for f in range(frames)]
     else:
         clouds = [synth.room_frame(r, c, f) for f in range(frames)]
-    attr = ref.new_attr()
+    attr = ref.new_attr() if ref is not None else None
+    slam = oracle.slam(r, c, 0)
     pos = np.array([10.0, -20.0, 5.0, 1.0, -2.0, 30.0])
-    big_stack(ref.init_slam, attr, pos, clouds[0])
-    pc = shim.pack(clouds[0], 7)
-    shim.lib.init_slam(shim.attr.ctypes.data, Pos.of(pos), pc.ctypes.data)
-    assert np.array_equal(shim.global_cloud(0), ref.attr_global(attr, 0))
-    assert shim.frame_count() == 1
+    if ref is not None:
+        big_stack(ref.init_slam, attr, pos, clouds[0])
+    g = slam.init(pos, clouds[0])
+    check_ref(f"{key}/global0", g, ref and (lambda: ref.attr_global(attr, 0)))
+    steps = [(pos, 0.0, g)]
     last = pos
     for f in range(1, frames):
         pred = last + np.array([45.0, 3.0, -1.0, 0.0, 0.0, 0.0])
-        p_ref = big_stack(ref.slam_localization, attr, clouds[f], pred, last)
+        p, _, err, _ = slam.localize(clouds[f], pred, last)
+        if ref is not None:
+            p_ref = big_stack(ref.slam_localization, attr, clouds[f], pred, last)
+            big_stack(ref.slam_mapping, attr, p_ref, clouds[f])
+            assert ref.attr_frame_count(attr) == f + 1
+        check_ref(f"{key}/pose{f}", p, ref and (lambda: p_ref))
+        check_ref(f"{key}/error{f}", np.float64(err), ref and (lambda: np.float64(ref.attr_error(attr))))
+        g = slam.map(p, clouds[f])
+        check_ref(f"{key}/global{f}", g, ref and (lambda: ref.attr_global(attr, f)))
+        steps.append((p, err, g))
+        last = p
+    slam.close()
+    return clouds, pos, steps
+
+
+@pytest.mark.parametrize("shape,frames", SLAM_STEP_CASES)
+def test_shim_slam_step_matches_reference(pkg, oracle, synth, shape, frames):
+    r, c = shape
+    clouds, pos, steps = reference_slam_steps(oracle, synth, shape, frames)
+    shim = Shim(pkg, r, c)
+    pc = shim.pack(clouds[0], 7)
+    shim.lib.init_slam(shim.attr.ctypes.data, Pos.of(pos), pc.ctypes.data)
+    assert np.array_equal(shim.global_cloud(0), steps[0][2])
+    assert shim.frame_count() == 1
+    last = pos
+    for f in range(1, frames):
+        p_ref, err_ref, g_ref = steps[f]
+        pred = last + np.array([45.0, 3.0, -1.0, 0.0, 0.0, 0.0])
         pc = shim.pack(clouds[f], 7 + f)
         with quiet_stdout():
             p = shim.lib.slam_localization(shim.attr.ctypes.data, pc.ctypes.data, Pos.of(pred), Pos.of(last)).arr()
         assert np.array_equal(p, p_ref), (f, p - p_ref)
-        assert shim.error() == ref.attr_error(attr)
-        big_stack(ref.slam_mapping, attr, p_ref, clouds[f])
+        assert shim.error() == err_ref
         shim.lib.slam_mapping(shim.attr.ctypes.data, Pos.of(p), pc.ctypes.data)
-        assert np.array_equal(shim.global_cloud(f), ref.attr_global(attr, f))
-        assert shim.frame_count() == f + 1 == ref.attr_frame_count(attr)
+        assert np.array_equal(shim.global_cloud(f), g_ref)
+        assert shim.frame_count() == f + 1
         last = p_ref
 
 
