@@ -165,6 +165,10 @@ int nav_slam_localization(nav_ctx *ctx, const nav_point *cloud, const nav_pos *p
  * for the oldest prefetched frame. */
 int nav_slam_localization_fast(nav_ctx *ctx, const nav_point *cloud, const nav_pos *pos_predict,
                                const nav_pos *pos_last, nav_pos *pos_out, double *error_out, size_t *n_corr_out);
+/* the five totals {N, sum rx, sum ry, sum rz, sum |r|^2} the last nav_slam_localization_fast call, or the last
+ * frame of nav_slam_run, was fitted from (r = ori - nearest of each dedupe winner).  Fails if no such fit has
+ * completed on this context. */
+int nav_slam_fit_stats(nav_ctx *ctx, double out[5]);
 /* slam_mapping (src/slam.c:393): global_out = pose(cloud), per-row map for the next frame.
  * cloud == NULL reuses the cloud (and labels) of the preceding nav_slam_match/localization call; with
  * global_out == NULL as well the call only queues the map kernel and does not synchronise. */
@@ -225,9 +229,11 @@ int nav_frontend_frame_depth_async(nav_ctx *ctx, const int *distances, const nav
  * nav_slam_prefetch queues both on a copy stream and returns at once; a later
  * nav_slam_localization_fast(ctx, cloud, ...) with the same `cloud` pointer (or NULL = the oldest prefetched
  * frame) finds the frame resident and labelled and only runs match + dedupe + statistics (2.5 KB come back).
- * nav_slam_mapping(ctx, pos, NULL, NULL) then maps that frame without synchronising.  Up to three frames may
- * be prefetched ahead.  The host buffer must be pinned and stay untouched until the localization call
- * that consumes it returns.
+ * nav_slam_mapping(ctx, pos, NULL, NULL) then maps that frame without synchronising.  There are three prefetch
+ * slots, and the frame a localization call consumed keeps its slot until nav_slam_mapping has queued its
+ * map: up to three frames may wait ahead of the next localization call, two while a consumed frame still
+ * waits for its mapping (a prefetch into that slot is refused).  The host buffer must be pinned and stay
+ * untouched until the localization call that consumes it returns.
  *     nav_slam_prefetch(ctx, frame[1]);
  *     for (t = 1; t < n; ++t) {
  *         if (t + 1 < n) nav_slam_prefetch(ctx, frame[t + 1]);

@@ -54,7 +54,7 @@ EXPORTS = [
     "nav_l9_csv_read", "nav_csv_header", "nav_csv_format_frame", "nav_csv_format_frame_gpu",
     "nav_csv_format_frame_dev", "nav_l5_json_read", "nav_imu_json_read",
     "nav_frontend_submit", "nav_frontend_frame_depth_async", "nav_slam_prefetch", "nav_slam_prefetch_depth",
-    "nav_host_register", "nav_host_unregister", "nav_slam_run",
+    "nav_host_register", "nav_host_unregister", "nav_slam_run", "nav_slam_fit_stats",
     "nav_peer_create", "nav_peer_connect", "nav_kdtree_nn_allgather_dev", "nav_kdtree_nn_sharded_map_dev", "nav_peer_check",
     "nav_peer_destroy", "nav_shard_range", "nav_shard_owner",
 ]
@@ -122,6 +122,7 @@ def load_library(build_if_missing: bool = True):
     L.nav_slam_localization_fast.argtypes = [vp, vp, C.POINTER(NavPos), C.POINTER(NavPos), C.POINTER(NavPos),
                                              c_double_p, C.POINTER(C.c_size_t)]
     L.nav_slam_mapping.argtypes = [vp, C.POINTER(NavPos), vp, vp]
+    L.nav_slam_fit_stats.argtypes = [vp, c_double_p]
     L.nav_frontend_frame.argtypes = [vp, vp, C.POINTER(NavPos), C.POINTER(NavPos), C.POINTER(NavPos),
                                      vp, vp, vp, vp]
     L.nav_frontend_frame_async.argtypes = [vp, vp, C.POINTER(NavPos), C.POINTER(NavPos), C.POINTER(NavPos),
@@ -376,6 +377,12 @@ class Context:
         _check(self.L.nav_slam_localization_fast(self.h, cloud_ptr, _pos_array(pos_predict), _pos_array(pos_last),
                                                  C.byref(out), C.byref(err), C.byref(n)), self.L)
         return np.array([out.x, out.y, out.z, out.roll, out.pitch, out.yaw]), err.value, int(n.value)
+
+    def slam_fit_stats(self):
+        """nav_slam_fit_stats: [N, sum rx, sum ry, sum rz, sum |r|^2] of the last closed-loop fit."""
+        out = (C.c_double * 5)()
+        _check(self.L.nav_slam_fit_stats(self.h, out), self.L)
+        return np.array(out[:])
 
     def slam_run(self, frame_ptrs, deltas, pos_start, depth_input=False):
         """nav_slam_run: the closed loop over pinned host frames (raw pointers) with dead-reckoning increments

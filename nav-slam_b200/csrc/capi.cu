@@ -216,7 +216,6 @@ struct nav_ctx {
     size_t npx = 0, ntot = 0;
     cudaStream_t stream = nullptr, own_stream = nullptr;
     double *d_cloud = nullptr, *d_global = nullptr, *d_curv = nullptr, *d_nn_dist = nullptr;
-    double *d_stats = nullptr;      // [n_seq][5] sufficient statistics of the translation fit
     unsigned *d_n_exact = nullptr;  // labels the fp32 filter could not decide (exact re-evaluations)
     int *d_labels = nullptr, *d_nn_idx = nullptr;
     RowMap map = {};      // the map the next match searches (frame mapped last)
@@ -354,7 +353,7 @@ extern "C" void nav_destroy(nav_ctx *c) {
     cudaSetDevice(c->device);
     if (c->stream) cudaStreamSynchronize(c->stream);
     void *ptrs[] = {c->d_cloud, c->d_global, c->d_curv, c->d_nn_dist, c->d_labels, c->d_nn_idx, c->map.pts,
-                    c->map.mask, c->d_n_exact, c->d_stats, c->map.box, c->map.sbox, c->map_alt.pts, c->map_alt.mask,
+                    c->map.mask, c->d_n_exact, c->map.box, c->map.sbox, c->map_alt.pts, c->map_alt.mask,
                     c->map_alt.box, c->map_alt.sbox, c->d_corr_rows, c->d_corr,
                     c->d_corr_row_count, c->d_corr_total, c->d_dist, c->d_tan_col, c->d_tan_row, c->d_flat,
                     c->d_flat_count};
@@ -449,7 +448,6 @@ extern "C" nav_ctx *nav_create(int rows, int cols, int device, int n_seq) {
     ALLOC(c->map.pts, nt * 24);
     ALLOC(c->map.mask, nr * c->map.n_chunks * 4);
     ALLOC(c->d_n_exact, 4);
-    ALLOC(c->d_stats, (size_t)n_seq * 5 * 8);
     ALLOC(c->d_row_stats, nr * 5 * 8);
     ALLOC(c->d_tile_stats, nr * (size_t)div_up(cols, 256) * 5 * 8);
     ALLOC(c->map.box, nr * c->map.n_chunks * 32);
@@ -480,6 +478,8 @@ extern "C" nav_ctx *nav_create(int rows, int cols, int device, int n_seq) {
         nav_destroy(c);
         return nullptr;
     }
+    // the mailbox flag (h_fit[5]) must not hold a sequence number the host will wait for before any post
+    memset(c->h_fit, 0, 64);
     // tan tables of utils/pointcloud.c:10-41, evaluated with the host libm exactly as the reference
     {
         std::vector<double> tc(cols), tr(rows);
@@ -874,9 +874,16 @@ static int prefetch_common(nav_ctx *c, const char *name, const nav_point *cloud,
     if (pre_setup(c)) return 1;
     nav_ctx::PreSlot &ps = c->pre[c->pre_next];
     if (ps.pending) return fail("%s: three prefetched frames are already waiting for nav_slam_localization_fast", name);
-    // the slot's buffers were last used by the frame before the current one: its map kernel is the last
-    // reader and is already queued on the context's stream (nav_slam_run records the event right behind that
-    // kernel, so that a prefetch issued later -- under the next frame's match -- does not wait for more)
+    // the frame the last localization call matched stays in its slot until its map kernel is queued:
+    // nav_slam_mapping(pos, NULL, ...) maps it from there
+    const bool holds_resident = c->cloud_resident && c->cur_cloud == ps.d_cloud;
+    if (holds_resident && !ps.release_recorded)
+        return fail("%s: the slot still holds the frame matched last; call nav_slam_mapping before prefetching "
+                    "another frame", name);
+    if (holds_resident) c->cloud_resident = false;  // overwritten below: nothing is left for mapping(NULL)
+    // otherwise the slot's last reader is already queued on the context's stream: the match of a frame that
+    // was not mapped from the slot, or the map kernel after which nav_slam_mapping / nav_slam_run recorded
+    // `released` (right behind that kernel, so that a prefetch issued later does not wait for more)
     if (!ps.release_recorded) CU(cudaEventRecord(ps.released, c->stream));
     ps.release_recorded = false;
     CU(cudaStreamWaitEvent(c->s_in, ps.released, 0));
@@ -1052,6 +1059,19 @@ extern "C" int nav_slam_localization_fast(nav_ctx *c, const nav_point *cloud, co
     return loc_fast_finish(c, pos_predict, pos_last, pos_out, error_out, n_corr_out);
 }
 
+extern "C" int nav_slam_fit_stats(nav_ctx *c, double out[5]) {
+    CTX_ENTER(c, "nav_slam_fit_stats");
+    if (!out) return fail("nav_slam_fit_stats: null argument");
+    if (c->fit_seq == 0) return fail("nav_slam_fit_stats: no closed-loop fit has run on this context");
+    // the localization call that launched the fit waited for this post before it returned (wait_fit_mail);
+    // a different number means that call failed
+    if (*(volatile unsigned long long *)(c->h_fit + 5) != c->fit_seq)
+        return fail("nav_slam_fit_stats: the last closed-loop fit did not complete");
+    __atomic_thread_fence(__ATOMIC_ACQUIRE);
+    memcpy(out, c->h_fit, 5 * sizeof(double));
+    return 0;
+}
+
 // The closed loop of a whole sequence in one call: the loop of src/main.c:300-318 with the EKF prediction
 // supplied by the caller -- a callback, or an array of dead-reckoning increments (pred = last + delta[t]).
 // Frame t+1 is prefetched (upload + labels on the copy-in stream) while frame t is matched and fitted.
@@ -1069,6 +1089,9 @@ extern "C" int nav_slam_run(nav_ctx *c, const void *const *frames, int n_frames,
                            : prefetch_common(c, "nav_slam_run", (const nav_point *)frames[t], nullptr);
     };
     for (auto &ps : c->pre) ps.pending = false;
+    // the loop maps its own frames: a frame an earlier localization call left unmapped in a prefetch slot is
+    // given up, so that the slot can be refilled
+    if (n_frames > 0) c->cloud_resident = false;
     // NAV_RUN_UNFUSED=1 keeps the three launches per frame (match, statistics dedupe, map) of the separate calls
     static const bool unfused = getenv("NAV_RUN_UNFUSED") != nullptr;
     const bool fused = !unfused && dedupe_stats_supported(c->cols);
@@ -1132,10 +1155,6 @@ extern "C" int nav_slam_run(nav_ctx *c, const void *const *frames, int n_frames,
         const double tm = c->trace ? now_us() : 0.0;
         if (!fused || t + 1 == n_frames) {  // fused: only the last frame is mapped by a launch of its own
             if (nav_slam_mapping(c, &poses_out[t], nullptr, nullptr)) return 1;
-            if (c->cur_pre) {  // the map kernel just queued is the last reader of the frame's prefetch slot
-                CU(cudaEventRecord(c->cur_pre->released, c->stream));
-                c->cur_pre->release_recorded = true;
-            }
         }
         if (c->trace) c->trace_us[4] += now_us() - tm;
         last = poses_out[t];
@@ -1163,6 +1182,11 @@ extern "C" int nav_slam_mapping(nav_ctx *c, const nav_pos *pos, const nav_point 
         return fail("nav_slam_mapping: cloud == NULL but no cloud is resident from a preceding match");
     }
     run_map(c, c->cur_cloud, c->cur_labels, pose_batch(c, pos, nullptr));
+    if (c->cur_pre && c->cur_cloud == c->cur_pre->d_cloud) {
+        // the map kernel just queued is the last reader of the frame's prefetch slot: the slot is free behind it
+        CU(cudaEventRecord(c->cur_pre->released, c->stream));
+        c->cur_pre->release_recorded = true;
+    }
     if (!cloud && !global_out) {  // nothing to wait for: the map kernel is queued, errors surface at the next call
         CU(cudaGetLastError());
         return 0;
@@ -1351,9 +1375,10 @@ extern "C" int nav_csv_format_frame_gpu(nav_ctx *c, unsigned long long timestamp
 // device slots for the per-frame buffers.  All host pointers must be pinned.  Outputs of frame t
 // are valid after nav_frontend_wait() (or after two further submissions).
 static int async_setup(nav_ctx *c) {
-    if (c->s_in) return 0;
-    CU(cudaStreamCreateWithFlags(&c->s_in, cudaStreamNonBlocking));
-    CU(cudaStreamCreateWithFlags(&c->s_out, cudaStreamNonBlocking));
+    if (c->slots[0].d_cloud) return 0;
+    // the closed-loop prefetch (pre_setup) may have created the copy-in stream already
+    if (!c->s_in) CU(cudaStreamCreateWithFlags(&c->s_in, cudaStreamNonBlocking));
+    if (!c->s_out) CU(cudaStreamCreateWithFlags(&c->s_out, cudaStreamNonBlocking));
     for (auto &sl : c->slots) {
         CU(cudaMalloc((void **)&sl.d_cloud, c->ntot * 24));
         // labels, NN index and NN distance of a slot are one allocation [labels | nn_idx | nn_dist], so

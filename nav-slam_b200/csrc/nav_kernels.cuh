@@ -78,8 +78,6 @@ int launch_loop_step(const double *cloud, const int *labels, const RowMap &map, 
                      double *part, const FitMailbox &mail);
 void launch_gather_corr(const nav_corr *corr_rows, const int *corr_row_count, nav_corr *corr_out,
                         int *corr_total, int n_seq, int rows, int cols, cudaStream_t stream);
-void launch_corr_stats(const nav_corr *corr, const int *corr_total, double *stats_out, int n_seq, int rows, int cols,
-                       int sm_count, cudaStream_t stream);
 void launch_flatten_row(const double *row_pts, const int *row_feature, const unsigned *row_mask, double *out,
                         int *col_out, int *count, int cols, cudaStream_t stream);
 

@@ -813,9 +813,11 @@ __device__ __forceinline__ void post_fit_totals(const double *__restrict__ part,
         for (int w = 0; w < T / 32; ++w) a = dadd(a, s_tot[w][threadIdx.x]);
         mail.host[threadIdx.x] = a;
     }
-    __threadfence_system();
     __syncthreads();
     if (threadIdx.x == 0) {
+        // cumulative, by the thread that writes the flag: the five totals (ordered before it by the barrier)
+        // reach the host before the sequence number does
+        __threadfence_system();
         *mail.ticket = 0u;
         *(volatile unsigned long long *)(mail.host + 5) = mail.seq;
     }
@@ -952,29 +954,51 @@ k_dedupe_rows(const double *__restrict__ cloud, const int *__restrict__ labels, 
 // Phases 1-3 of the cluster dedupe.  Called by ALL threads of every CTA of the row's cluster (four cluster
 // barriers inside).  key = matched map column of this thread's query (or -1), dbits = bits of its distance,
 // c = the query's column.  Returns whether this query is the one kept for its map point.
+// The slots are reached with shared::cluster addresses, and the smallest distance is posted with a 64-bit
+// compare-and-swap loop.  The hardware has no 64-bit atomic min on shared memory: for atomicMin(u64) on a generic
+// address the compiler falls back, for shared addresses, to an LDS + ATOMS compare-and-swap loop, and ATOMS
+// only reaches the issuing CTA's own shared memory.  Posts to another CTA of the cluster through a `mapa.u64`
+// pointer were lost that way, and rows whose matches crossed tiles kept wrong (and run-to-run varying) dedupe
+// winners.  64-bit compare-and-swap and 32-bit min on distributed shared memory are single ATOM instructions.
+__device__ __forceinline__ unsigned cluster_slot(const void *local, unsigned rank) {
+    unsigned r;
+    asm("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"((unsigned)__cvta_generic_to_shared(local)), "r"(rank));
+    return r;
+}
+
 __device__ __forceinline__ bool cluster_dedupe_winner(unsigned long long *s_best, int *s_win, int key,
                                                       unsigned long long dbits, int c) {
     s_best[threadIdx.x] = ~0ull;
     s_win[threadIdx.x] = INT_MAX;
-    unsigned long long *r_best = nullptr;
-    int *r_win = nullptr;
+    unsigned r_best = 0, r_win = 0;
     if (key >= 0) {  // the slots of map column `key` live in the CTA of its tile (rank = tile index in the cluster)
         const unsigned owner = (unsigned)(key / kTile);
-        unsigned long long *b0;
-        int *w0;
-        asm("mapa.u64 %0, %1, %2;" : "=l"(b0) : "l"(s_best), "r"(owner));
-        asm("mapa.u64 %0, %1, %2;" : "=l"(w0) : "l"(s_win), "r"(owner));
-        r_best = b0 + key % kTile;
-        r_win = w0 + key % kTile;
+        r_best = cluster_slot(s_best + key % kTile, owner);
+        r_win = cluster_slot(s_win + key % kTile, owner);
     }
     cluster_sync_all();  // every CTA of the row has initialised its slots
-    if (key >= 0) atomicMin(r_best, dbits);
+    if (key >= 0) {
+        unsigned long long cur;
+        asm volatile("ld.shared::cluster.u64 %0, [%1];" : "=l"(cur) : "r"(r_best) : "memory");
+        while (dbits < cur) {
+            unsigned long long seen;
+            asm volatile("atom.shared::cluster.cas.b64 %0, [%1], %2, %3;"
+                         : "=l"(seen) : "r"(r_best), "l"(cur), "l"(dbits) : "memory");
+            if (seen == cur) break;
+            cur = seen;
+        }
+    }
     cluster_sync_all();
-    if (key >= 0 && *(volatile unsigned long long *)r_best == dbits) atomicMin(r_win, c);
+    if (key >= 0) {
+        unsigned long long best;
+        asm volatile("ld.shared::cluster.u64 %0, [%1];" : "=l"(best) : "r"(r_best) : "memory");
+        if (best == dbits) asm volatile("red.shared::cluster.min.s32 [%0], %1;" ::"r"(r_win), "r"(c) : "memory");
+    }
     cluster_sync_all();
-    const bool winner = key >= 0 && *(volatile int *)r_win == c;
+    int win = -1;
+    if (key >= 0) asm volatile("ld.shared::cluster.s32 %0, [%1];" : "=r"(win) : "r"(r_win) : "memory");
     cluster_sync_all();  // nobody leaves (or reuses its slots) while a neighbour may still read them
-    return winner;
+    return key >= 0 && win == c;
 }
 
 struct StatsSmem {
@@ -1235,52 +1259,6 @@ __global__ void k_gather_corr(const nav_corr *__restrict__ corr_rows, const int 
 void launch_gather_corr(const nav_corr *corr_rows, const int *corr_row_count, nav_corr *corr_out,
                         int *corr_total, int n_seq, int rows, int cols, cudaStream_t stream) {
     k_gather_corr<<<n_seq * rows, 256, 0, stream>>>(corr_rows, corr_row_count, corr_out, corr_total, rows, cols);
-}
-
-// ---------------------------------------------------------------------------------------------
-// Sufficient statistics of the translation-only fit (SURVEY 8f #2).  With r_i = ori_i - nearest_i
-// every iteration of src/slam.c:319-338 only needs N, sum r (3) and sum |r|^2:
-//   totalError(t) = sum|r|^2 - 2 t.sum r + N|t|^2,   gradient = -(sum r - N t)/N.
-// stats_out[0..4] = {N, sum rx, sum ry, sum rz, sum |r|^2} per sequence, accumulated with fp64
-// atomics (the summation order differs from the reference's sequential loop: tolerance parity).
-__global__ void __launch_bounds__(256)
-k_corr_stats(const nav_corr *__restrict__ corr, const int *__restrict__ corr_total, double *__restrict__ stats_out,
-             int rows, int cols) {
-    __shared__ double s_part[8][4];
-    const int seq = blockIdx.y;
-    const int n = corr_total[seq];
-    const nav_corr *list = corr + (long long)seq * rows * cols;
-    double a[4] = {0, 0, 0, 0};
-    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-        const double rx = list[i].ori.x - list[i].nearest.x, ry = list[i].ori.y - list[i].nearest.y,
-                     rz = list[i].ori.z - list[i].nearest.z;
-        a[0] += rx;
-        a[1] += ry;
-        a[2] += rz;
-        a[3] += rx * rx + ry * ry + rz * rz;
-    }
-#pragma unroll
-    for (int k = 0; k < 4; ++k)
-#pragma unroll
-        for (int d = 16; d >= 1; d >>= 1) a[k] += __shfl_xor_sync(kFull, a[k], d);
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    if (lane == 0)
-#pragma unroll
-        for (int k = 0; k < 4; ++k) s_part[warp][k] = a[k];
-    __syncthreads();
-    if (threadIdx.x < 4) {
-        double t = 0;
-        for (int w = 0; w < 8; ++w) t += s_part[w][threadIdx.x];
-        atomicAdd(&stats_out[seq * 5 + 1 + threadIdx.x], t);
-    }
-    if (threadIdx.x == 0 && blockIdx.x == 0) stats_out[seq * 5] = (double)n;
-}
-
-void launch_corr_stats(const nav_corr *corr, const int *corr_total, double *stats_out, int n_seq, int rows, int cols,
-                       int sm_count, cudaStream_t stream) {
-    cudaMemsetAsync(stats_out, 0, sizeof(double) * 5 * n_seq, stream);
-    dim3 grid(sm_count, n_seq);
-    k_corr_stats<<<grid, 256, 0, stream>>>(corr, corr_total, stats_out, rows, cols);
 }
 
 // ---------------------------------------------------------------------------------------------
