@@ -135,8 +135,9 @@ void nav_peer_destroy(nav_peer *p);
 /* exact brute force on the same contract.  use_tensor_cores == 0: plain binary64 scan.
  * use_tensor_cores != 0: tcgen05 candidate tiles (bf16 hi/mid/lo splits, fp32 accumulate in TMEM) flag
  * every 32-point group that can contain the nearest neighbour, then an exact binary64 re-rank of the
- * flagged groups; same answers for any input.  Measured on B200 it beats the fp64 scan from ~4 K
- * points but never the kd-tree (profiles/README.md), so nothing selects it automatically. */
+ * flagged groups; same answers for any input.  Inputs whose centred coordinates could overflow the fp32
+ * operands are answered by the binary64 re-rank of every group.  Measured on B200 it beats the fp64
+ * scan from ~4 K points but never the kd-tree (profiles/README.md), so nothing selects it automatically. */
 int nav_bruteforce_nn_batch_dev(int device, const void *dev_points, size_t n, const void *dev_queries,
                                 size_t nq, void *dev_idx_out, void *dev_dist_out,
                                 int use_tensor_cores, void *cuda_stream);
@@ -176,7 +177,9 @@ int nav_slam_mapping(nav_ctx *ctx, const nav_pos *pos, const nav_point *cloud, n
 /* one front-end frame with raw per-pixel outputs (SURVEY 8d "one frame of work"): labels, queries,
  * NN vs the previous frame, then mapping with pos_final.  nn_idx = flat pixel (row*cols+col) of the
  * match in the previous frame, -1 if unlabelled or the row's map is empty; nn_dist = -1 if
- * unlabelled, +inf if the map is empty.  Any output pointer may be NULL. */
+ * unlabelled, +inf if the map is empty.  A labelled point whose dsq to every map point of its row is
+ * +inf or NaN (a diverged pose) gets the outcome of an empty row: nn_idx = -1, nn_dist = +inf, and the
+ * closed loop makes no correspondence for it.  Any output pointer may be NULL. */
 int nav_frontend_frame(nav_ctx *ctx, const nav_point *cloud, const nav_pos *pos_predict,
                        const nav_pos *pos_last, const nav_pos *pos_final, int *feature_out,
                        int32_t *nn_idx_out, double *nn_dist_out, nav_point *global_out);

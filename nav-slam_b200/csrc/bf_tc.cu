@@ -367,11 +367,14 @@ k_tc_rerank(const double *__restrict__ pts, long long n, const double *__restric
     double best = INFINITY;
     int bidx = INT_MAX;
     unsigned evals = 0;
-    // infinite coordinates make the centred operands meaningless: then every group is re-ranked
+    // The bf16 operands of the tiles are bounded by Qmax, Pmax and 1.5 Pmax^2, every fp32 product and partial sum
+    // by 3 Qmax Pmax + 1.5 Pmax^2 (times a factor near 1).  Beyond 2^90 -- or with an infinite centre -- some of
+    // them may have overflowed to inf / NaN and the flags mean nothing: then every group is re-ranked.
     double c[3], pmax;
     centre_of(stats, c, pmax);
     const double qmax = stats[6] ? okey_inv(stats[6]) : 0.0;
-    const bool scan_all = !(pmax < INFINITY) || !(qmax < INFINITY) || !(fabs(c[0]) + fabs(c[1]) + fabs(c[2]) < INFINITY);
+    const double bound = fmax(fmax(qmax, pmax), 3.0 * qmax * pmax + 1.5 * pmax * pmax);
+    const bool scan_all = !(bound < 0x1p90) || !(fabs(c[0]) + fabs(c[1]) + fabs(c[2]) < INFINITY);
     for (int t0 = 0; t0 < n_tiles; t0 += 32) {
         const int tl = t0 + lane;
         unsigned mine = 0;
@@ -406,9 +409,10 @@ k_tc_rerank(const double *__restrict__ pts, long long n, const double *__restric
         }
     }
     if (lane == 0) {
-        const bool found = best < INFINITY || bidx != INT_MAX;
-        idx_out[qi] = found && bidx != INT_MAX ? bidx : -1;
-        dist_out[qi] = found && bidx != INT_MAX ? __dsqrt_rn(best) : INFINITY;
+        // no point at a finite dsq (every dsq +inf or NaN): no answer, as in k_bf_nn
+        const bool found = best < INFINITY;
+        idx_out[qi] = found ? bidx : -1;
+        dist_out[qi] = found ? __dsqrt_rn(best) : INFINITY;
         if (n_evals) atomicAdd(n_evals, (unsigned long long)evals * kTcGroup);
     }
 }

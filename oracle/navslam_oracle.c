@@ -352,7 +352,9 @@ void nso_slam_map(nso_slam *s, const nso_pos *pos, const nso_point *cloud, nso_p
 
 /* one query against row r's map.  Returns the column of the match in the previous frame
  * (-1 if the row's map is empty: the reference reads an uninitialised Point there,
- * utils/kdtree.c:112 + src/slam.c:242 -- undefined, so no correspondence is produced). */
+ * utils/kdtree.c:112 + src/slam.c:242 -- undefined, so no correspondence is produced).
+ * A query whose dsq to every map point of the row is +inf or NaN has no nearest point either:
+ * -1 with *dist = +inf, as for an empty row. */
 static int32_t row_query(const nso_slam *s, int r, const nso_point *q, nso_point *nearest, double *dist) {
     size_t base = (size_t)r * s->cols, n = s->map_n[r];
     if (n == 0) return -1;
@@ -360,6 +362,7 @@ static int32_t row_query(const nso_slam *s, int r, const nso_point *q, nso_point
         double best = INFINITY;
         nso_tree_nn(s->trees[r], q, nearest, &best, 0);
         *dist = best;
+        if (!(best < INFINITY)) return -1;
         for (size_t j = 0; j < n; ++j) {
             const nso_point *p = &s->map_pts[base + j];
             if (p->x == nearest->x && p->y == nearest->y && p->z == nearest->z) return s->map_col[base + j];
@@ -368,6 +371,7 @@ static int32_t row_query(const nso_slam *s, int r, const nso_point *q, nso_point
     }
     int32_t bi;
     nso_nn_brute(s->map_pts + base, n, q, 1, &bi, dist);
+    if (bi < 0) return -1;
     *nearest = s->map_pts[base + bi];
     return s->map_col[base + bi];
 }

@@ -935,18 +935,24 @@ def test_slam_run_with_a_prediction_callback_and_registered_memory(pkg, synth):
     ptrs = (C.c_void_p * (n - 1))(*[own[f].ctypes.data for f in range(1, n)])
     out = (NavPos * (n - 1))()
     start = NavPos(0, 0, 0, 0, 0, 0)
+    # the library handle is shared by the whole process: the callback signature is restored afterwards, so that
+    # later Context.slam_run calls (predict = NULL) keep the binding's own argument types
+    saved = L.nav_slam_run.argtypes
     L.nav_slam_run.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.c_int, C.c_int, PRED, C.c_void_p, C.c_void_p,
                                C.POINTER(NavPos), C.POINTER(NavPos), C.c_void_p, C.c_void_p]
-    rc = L.nav_slam_run(ctx.h, ptrs, n - 1, 0, cb, None, None, C.byref(start), out, None, None)
-    assert rc == 0, L.nav_last_error()
-    assert calls == list(range(n - 1))
-    got = np.array([[p.x, p.y, p.z, p.roll, p.pitch, p.yaw] for p in out])
-    assert np.array_equal(got, want)
-    assert L.nav_host_unregister(own.ctypes.data) == 0
-    # pageable frames: refused with a message, nothing queued
-    ctx.slam_init(np.zeros(6), clouds[0], want_global=False)
-    rc = L.nav_slam_run(ctx.h, ptrs, n - 1, 0, cb, None, None, C.byref(start), out, None, None)
-    assert rc != 0 and b"pinned" in L.nav_last_error()
+    try:
+        rc = L.nav_slam_run(ctx.h, ptrs, n - 1, 0, cb, None, None, C.byref(start), out, None, None)
+        assert rc == 0, L.nav_last_error()
+        assert calls == list(range(n - 1))
+        got = np.array([[p.x, p.y, p.z, p.roll, p.pitch, p.yaw] for p in out])
+        assert np.array_equal(got, want)
+        assert L.nav_host_unregister(own.ctypes.data) == 0
+        # pageable frames: refused with a message, nothing queued
+        ctx.slam_init(np.zeros(6), clouds[0], want_global=False)
+        rc = L.nav_slam_run(ctx.h, ptrs, n - 1, 0, cb, None, None, C.byref(start), out, None, None)
+        assert rc != 0 and b"pinned" in L.nav_last_error()
+    finally:
+        L.nav_slam_run.argtypes = saved
     ctx.close()
 
 
