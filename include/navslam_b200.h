@@ -170,6 +170,12 @@ int nav_slam_localization_fast(nav_ctx *ctx, const nav_point *cloud, const nav_p
  * frame of nav_slam_run, was fitted from (r = ori - nearest of each dedupe winner).  Fails if no such fit has
  * completed on this context. */
 int nav_slam_fit_stats(nav_ctx *ctx, double out[5]);
+/* the host fit nav_slam_localization_fast runs on the five totals above (200 Adam iterations on the translation,
+ * rotation kept at the prediction), exposed: pos_out = pos_last + the fitted change, *error_out (may be NULL) =
+ * sqrt(residual / N).  N = 0 (no correspondence): the translation stays at the prediction, pos_out = pos_last +
+ * (pos_predict - pos_last) component by component, and the error is 0.  Host only, no device involved. */
+int nav_slam_fit_from_stats(const double stats[5], const nav_pos *pos_predict, const nav_pos *pos_last,
+                            nav_pos *pos_out, double *error_out);
 /* slam_mapping (src/slam.c:393): global_out = pose(cloud), per-row map for the next frame.
  * cloud == NULL reuses the cloud (and labels) of the preceding nav_slam_match/localization call; with
  * global_out == NULL as well the call only queues the map kernel and does not synchronise. */
@@ -328,6 +334,37 @@ typedef struct {
     void *map_mask; /* uint32 [n_seq][rows][ceil(cols/16)] edge-point bit masks of the frame just mapped */
 } nav_frame_results;
 int nav_frame_results_dev(nav_ctx *ctx, nav_frame_results *out);
+
+/* Per-frame results of a sequence replay.  Device pointers on the context's device; every field is optional.
+ * Frame f of the call (0-based) fills slot f. */
+typedef struct {
+    void *label_mask;  /* uint32 [n_frames][n_seq][rows][ceil(cols/16)], the mask_out format of nav_frame_io */
+    void *nn_idx;      /* int32  [n_frames][n_seq][rows][cols]  (-1 where unlabelled / no match)          */
+    void *nn_dist;     /* double [n_frames][n_seq][rows][cols]  (-1.0 unlabelled, +inf no match)          */
+    void *fit_stats;   /* double [n_frames][n_seq][5] = {N, sum rx, sum ry, sum rz, sum |r|^2} of the frame's
+                          dedupe winners, r = ori - nearest: what nav_slam_localization_fast would fit from */
+} nav_sequence_out;
+/* nav_frontend_sequence_dev that keeps every frame's results instead of only the last one's.
+ *   - Frame contents: slot f holds exactly what the context holds after nav_frontend_sequence_dev is stopped
+ *     after frame f -- nav_frame_results_dev's map_mask, nn_idx and nn_dist, for every pixel, labelled or not.
+ *   - Fit totals: fit_stats slot f equals, bit for bit, what nav_slam_fit_stats reports after
+ *     nav_slam_localization_fast on frame f with pos_predict[f] and pos_last[f], on a context of the same shape
+ *     that holds the map of frame f-1 at pos_final[f-1].  For n_seq > 1 the totals of sequence s are those of a
+ *     single-sequence context replaying sequence s.  nav_slam_fit_from_stats turns them into the pose.
+ *   - Context state: afterwards the context (result buffers, maps) is exactly as after nav_frontend_sequence_dev
+ *     with the same arguments; the two calls and the closed loop mix freely.
+ *   - out == NULL, or every field NULL: the call is nav_frontend_sequence_dev (same kernels, same launch count).
+ *     n_frames == 0 returns 0 and writes nothing.
+ *   - A field that is not device or managed memory on the context's device fails the call before anything is
+ *     queued; the error names the field.
+ *   - The work goes on the context's stream: the outputs are complete once the stream has passed the call.  No
+ *     host synchronisation is added to what nav_frontend_sequence_dev does, except a one-time one when the
+ *     statistics scratch (about 20 KB per 64x2048 frame) has to grow.
+ * One sequence of rows up to 2048 columns runs as one launch (two with fit_stats); otherwise every frame is a
+ * launch of its own, followed by the copies into its slots and, with fit_stats, its dedupe. */
+int nav_frontend_sequence_out_dev(nav_ctx *ctx, const void *dev_frames, size_t n_frames,
+                                  const nav_pos *pos_predict, const nav_pos *pos_last, const nav_pos *pos_final,
+                                  const nav_sequence_out *out);
 
 /* copy out the map the context holds for one (sequence,row): the labelled global points of the
  * frame mapped last, compacted in column order (= the flattenedPoints array of src/slam.c:170-171),

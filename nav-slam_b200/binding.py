@@ -32,6 +32,11 @@ class NavFrameIO(C.Structure):
                                           "nn_idx_out", "nn_dist_out", "global_out")]
 
 
+class NavSequenceOut(C.Structure):
+    """nav_sequence_out of include/navslam_b200.h (device pointers, any field may be None)."""
+    _fields_ = [(n, C.c_void_p) for n in ("label_mask", "nn_idx", "nn_dist", "fit_stats")]
+
+
 class NavError(RuntimeError):
     pass
 
@@ -55,6 +60,7 @@ EXPORTS = [
     "nav_csv_format_frame_dev", "nav_l5_json_read", "nav_imu_json_read",
     "nav_frontend_submit", "nav_frontend_frame_depth_async", "nav_slam_prefetch", "nav_slam_prefetch_depth",
     "nav_host_register", "nav_host_unregister", "nav_slam_run", "nav_slam_fit_stats",
+    "nav_frontend_sequence_out_dev", "nav_slam_fit_from_stats",
     "nav_peer_create", "nav_peer_connect", "nav_kdtree_nn_allgather_dev", "nav_kdtree_nn_sharded_map_dev", "nav_peer_check",
     "nav_peer_destroy", "nav_shard_range", "nav_shard_owner",
 ]
@@ -123,6 +129,8 @@ def load_library(build_if_missing: bool = True):
                                              c_double_p, C.POINTER(C.c_size_t)]
     L.nav_slam_mapping.argtypes = [vp, C.POINTER(NavPos), vp, vp]
     L.nav_slam_fit_stats.argtypes = [vp, c_double_p]
+    L.nav_slam_fit_from_stats.argtypes = [c_double_p, C.POINTER(NavPos), C.POINTER(NavPos), C.POINTER(NavPos),
+                                          c_double_p]
     L.nav_frontend_frame.argtypes = [vp, vp, C.POINTER(NavPos), C.POINTER(NavPos), C.POINTER(NavPos),
                                      vp, vp, vp, vp]
     L.nav_frontend_frame_async.argtypes = [vp, vp, C.POINTER(NavPos), C.POINTER(NavPos), C.POINTER(NavPos),
@@ -164,6 +172,8 @@ def load_library(build_if_missing: bool = True):
     L.nav_frontend_frame_dev.argtypes = [vp, vp, C.POINTER(NavPos), C.POINTER(NavPos), C.POINTER(NavPos)]
     L.nav_frontend_sequence_dev.argtypes = [vp, vp, C.c_size_t, C.POINTER(NavPos), C.POINTER(NavPos),
                                             C.POINTER(NavPos)]
+    L.nav_frontend_sequence_out_dev.argtypes = [vp, vp, C.c_size_t, C.POINTER(NavPos), C.POINTER(NavPos),
+                                                C.POINTER(NavPos), C.POINTER(NavSequenceOut)]
     L.nav_frame_results_dev.argtypes = [vp, C.POINTER(NavFrameResults)]
     L.nav_row_map_export.argtypes = [vp, C.c_int, C.c_int, vp, vp, C.POINTER(C.c_size_t)]
     L.nav_exact_fallback_count.restype = C.c_uint64
@@ -428,6 +438,16 @@ class Context:
         _check(self.L.nav_frontend_sequence_dev(self.h, dev_frames_ptr, n_frames, _pos_array(pos_predict, n),
                                                 _pos_array(pos_last, n), _pos_array(pos_final, n)), self.L)
 
+    def frontend_sequence_out_dev(self, dev_frames_ptr, n_frames, pos_predict, pos_last, pos_final, label_mask=None,
+                                  nn_idx=None, nn_dist=None, fit_stats=None):
+        """nav_frontend_sequence_out_dev: the replay of frontend_sequence_dev keeping every frame's results in the
+        given device buffers (ints; None = not wanted).  With all four None the call passes out = NULL."""
+        n = n_frames * self.n_seq
+        fields = (label_mask, nn_idx, nn_dist, fit_stats)
+        out = None if all(v is None for v in fields) else C.byref(NavSequenceOut(*fields))
+        _check(self.L.nav_frontend_sequence_out_dev(self.h, dev_frames_ptr, n_frames, _pos_array(pos_predict, n),
+                                                    _pos_array(pos_last, n), _pos_array(pos_final, n), out), self.L)
+
     def frame_results_dev(self) -> NavFrameResults:
         r = NavFrameResults()
         _check(self.L.nav_frame_results_dev(self.h, C.byref(r)), self.L)
@@ -570,6 +590,17 @@ def csv_format_frame(timestamp, global_cloud, lidar_pos, distances=None, imu=Non
     if n == 0:
         raise NavError("nav_csv_format_frame: buffer too small")
     return buf.raw[:n]
+
+
+def fit_from_stats(stats, pos_predict, pos_last):
+    """nav_slam_fit_from_stats: the closed loop's host fit on five totals [N, sum rx, sum ry, sum rz, sum |r|^2].
+    Returns (pose [6], rms error)."""
+    L = load_library()
+    st = (C.c_double * 5)(*[float(v) for v in np.asarray(stats, dtype=np.float64).reshape(5)])
+    out = NavPos()
+    err = C.c_double(0)
+    _check(L.nav_slam_fit_from_stats(st, _pos_array(pos_predict), _pos_array(pos_last), C.byref(out), C.byref(err)), L)
+    return np.array([out.x, out.y, out.z, out.roll, out.pitch, out.yaw]), err.value
 
 
 def device_count() -> int:

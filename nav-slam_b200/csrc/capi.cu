@@ -278,6 +278,9 @@ struct nav_ctx {
     int pose_ring_next = 0;
     void *d_pose = nullptr;
     size_t d_pose_cap = 0;
+    // per-frame partials of the fit statistics of nav_frontend_sequence_out_dev (grows like d_pose)
+    double *d_seq_part = nullptr;
+    size_t d_seq_part_cap = 0;
     // NAV_RUN_TRACE=1: nav_slam_run prints where the host side of the closed loop spends its time
     // [prefetch call, launches of match + dedupe, wait for the statistics, fit, mapping call]
     bool trace = false;
@@ -382,6 +385,7 @@ extern "C" void nav_destroy(nav_ctx *c) {
         if (pr.done) cudaEventDestroy(pr.done);
     }
     if (c->d_pose) cudaFree(c->d_pose);
+    if (c->d_seq_part) cudaFree(c->d_seq_part);
     if (c->d_fit_ticket) cudaFree(c->d_fit_ticket);
     if (c->s_in) cudaStreamDestroy(c->s_in);
     if (c->s_out) cudaStreamDestroy(c->s_out);
@@ -950,7 +954,7 @@ static int wait_fit_mail(nav_ctx *c, const char *name) {
     return 0;
 }
 
-// the O(1)-per-iteration Adam loop on the five totals; bias corrections 1 - beta^t from tables computed once
+// the O(1)-per-iteration Adam loop on the five totals (also exported as nav_slam_fit_from_stats); bias corrections 1 - beta^t from tables computed once
 // with the same pow() calls the loop used to make
 static void fit_from_stats(const double st[5], const nav_pos *pos_predict, const nav_pos *pos_last, nav_pos *pos_out,
                            double *error_out, size_t *n_corr_out) {
@@ -1057,6 +1061,13 @@ extern "C" int nav_slam_localization_fast(nav_ctx *c, const nav_point *cloud, co
     if (!pos_out) return fail("nav_slam_localization_fast: null argument");
     if (loc_fast_launch(c, cloud, pos_predict, pos_last)) return 1;
     return loc_fast_finish(c, pos_predict, pos_last, pos_out, error_out, n_corr_out);
+}
+
+extern "C" int nav_slam_fit_from_stats(const double stats[5], const nav_pos *pos_predict, const nav_pos *pos_last,
+                                       nav_pos *pos_out, double *error_out) {
+    if (!stats || !pos_predict || !pos_last || !pos_out) return fail("nav_slam_fit_from_stats: null argument");
+    fit_from_stats(stats, pos_predict, pos_last, pos_out, error_out, nullptr);
+    return 0;
 }
 
 extern "C" int nav_slam_fit_stats(nav_ctx *c, double out[5]) {
@@ -1524,12 +1535,30 @@ extern "C" int nav_frontend_frame_dev(nav_ctx *c, const void *dev_cloud, const n
     return 0;
 }
 
-extern "C" int nav_frontend_sequence_dev(nav_ctx *c, const void *dev_frames, size_t n_frames,
-                                         const nav_pos *pos_predict, const nav_pos *pos_last,
-                                         const nav_pos *pos_final) {
-    CTX_ENTER(c, "nav_frontend_sequence_dev");
-    if (!dev_frames || !pos_predict || !pos_last || !pos_final) return fail("nav_frontend_sequence_dev: null argument");
-    if (!c->have_map) return fail("nav_frontend_sequence_dev: call nav_slam_init_dev first");
+// device (or managed) memory of the context's device?
+static bool on_ctx_device(const nav_ctx *c, const void *p) {
+    cudaPointerAttributes a;
+    if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
+        cudaGetLastError();  // not a sticky error: clear it
+        return false;
+    }
+    return (a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged) && a.device == c->device;
+}
+
+// nav_frontend_sequence_dev, and with per-frame outputs (so != null) nav_frontend_sequence_out_dev
+static int frontend_sequence(nav_ctx *c, const char *name, const void *dev_frames, size_t n_frames,
+                             const nav_pos *pos_predict, const nav_pos *pos_last, const nav_pos *pos_final,
+                             const nav_sequence_out *so) {
+    if (!dev_frames || !pos_predict || !pos_last || !pos_final) return fail("%s: null argument", name);
+    if (!c->have_map) return fail("%s: call nav_slam_init_dev first", name);
+    if (so) {
+        const std::pair<const void *, const char *> fields[] = {
+            {so->label_mask, "label_mask"}, {so->nn_idx, "nn_idx"}, {so->nn_dist, "nn_dist"}, {so->fit_stats, "fit_stats"}};
+        for (const auto &fd : fields)
+            if (fd.first && !on_ctx_device(c, fd.first))
+                return fail("%s: out->%s is not device or managed memory on device %d", name, fd.second, c->device);
+        if (!so->label_mask && !so->nn_idx && !so->nn_dist && !so->fit_stats) so = nullptr;
+    }
     const double *base = (const double *)dev_frames;
     order_after_async(c);
     // One launch for the whole sequence (k_frame_seq: a thread-block cluster per image row walks through the
@@ -1539,71 +1568,135 @@ extern "C" int nav_frontend_sequence_dev(nav_ctx *c, const void *dev_frames, siz
     // sequence -- the chain of one row is what takes that long -- with one launch instead of n_frames for the
     // host to issue; several sequences side by side (n_seq > 1) fill the machine better as separate launches.
     static const bool per_frame = getenv("NAV_SEQ_LAUNCHES") != nullptr;
-    if (!per_frame && !c->prof && c->n_seq == 1 && n_frames > 1 && frame_seq_supported(c->cols) && n_frames <= 0x7fffffff) {
+    const bool fused =
+        !per_frame && !c->prof && c->n_seq == 1 && n_frames > 1 && frame_seq_supported(c->cols) && n_frames <= 0x7fffffff;
+    // fit statistics: CTA partials per frame in scratch -- one per (row, tile) from k_frame_seq or k_dedupe_stats
+    // (rows up to 2048 columns), one per row from k_dedupe_rows (wider rows) -- then one totals launch
+    const size_t nr = (size_t)c->n_seq * c->rows;
+    const bool tile_parts = dedupe_stats_supported(c->cols);
+    const size_t part_frame = tile_parts ? nr * div_up(c->cols, 256) : nr;  // partials per frame
+    double *part = nullptr;
+    if (so && so->fit_stats && n_frames > 0) {
+        const size_t bytes = n_frames * part_frame * 5 * sizeof(double);
+        if (c->d_seq_part_cap < bytes) {
+            CU(cudaStreamSynchronize(c->stream));
+            if (c->d_seq_part) cudaFree(c->d_seq_part);
+            c->d_seq_part = nullptr;
+            c->d_seq_part_cap = 0;
+            CU(cudaMalloc((void **)&c->d_seq_part, bytes));
+            c->d_seq_part_cap = bytes;
+        }
+        part = c->d_seq_part;
+    }
+    const SeqOut seq_out = {so ? (unsigned *)so->label_mask : nullptr, so ? (int *)so->nn_idx : nullptr,
+                            so ? (double *)so->nn_dist : nullptr, part};
+    if (fused) {
         const size_t n_pose = n_frames * (size_t)c->n_seq, bytes = n_pose * 2 * sizeof(PoseXf);
         const MatchOut out = {c->d_nn_idx, c->d_nn_dist, c->d_corr_rows, c->d_corr_row_count};
         if ((int)n_frames <= frame_seq_inline_frames()) {  // short sequence: poses as kernel parameters
             PoseXf loc[64], fin[64];
             static_assert(sizeof(loc) / sizeof(loc[0]) >= 64, "");
-            if (frame_seq_inline_frames() > 64) return fail("nav_frontend_sequence_dev: inline pose capacity");
+            if (frame_seq_inline_frames() > 64) return fail("%s: inline pose capacity", name);
             for (size_t i = 0; i < n_pose; ++i) {
                 loc[i] = make_pose(&pos_predict[i], &pos_last[i]);
                 fin[i] = make_pose(&pos_final[i], nullptr);
             }
             CU((cudaError_t)launch_frame_seq(base, (long long)c->ntot * 3, (int)n_frames, c->d_labels, c->map, c->map_alt, out,
-                                             nullptr, nullptr, c->n_seq, c->rows, c->cols, c->d_n_exact, c->stream, loc, fin));
-            c->launches++;
-            if (n_frames & 1) std::swap(c->map, c->map_alt);
-            c->cloud_resident = false;
-            CU(cudaGetLastError());
-            return 0;
+                                             nullptr, nullptr, c->n_seq, c->rows, c->cols, c->d_n_exact, c->stream, loc, fin,
+                                             so ? &seq_out : nullptr));
+        } else {
+            nav_ctx::PoseRing &pr = c->pose_ring[c->pose_ring_next];
+            c->pose_ring_next = (c->pose_ring_next + 1) % nav_ctx::kPoseRing;
+            if (pr.done) CU(cudaEventSynchronize(pr.done));  // the staging buffer's previous upload (several sequences ago)
+            if (pr.cap < bytes) {
+                if (pr.host) cudaFreeHost(pr.host);
+                pr.host = nullptr;
+                pr.cap = 0;
+                CU(cudaHostAlloc((void **)&pr.host, bytes, cudaHostAllocDefault));
+                pr.cap = bytes;
+            }
+            if (!pr.done) CU(cudaEventCreateWithFlags(&pr.done, cudaEventDisableTiming));
+            if (c->d_pose_cap < bytes) {
+                CU(cudaStreamSynchronize(c->stream));
+                if (c->d_pose) cudaFree(c->d_pose);
+                c->d_pose = nullptr;
+                c->d_pose_cap = 0;
+                CU(cudaMalloc((void **)&c->d_pose, bytes));
+                c->d_pose_cap = bytes;
+            }
+            PoseXf *loc = (PoseXf *)pr.host, *fin = loc + n_pose;
+            for (size_t i = 0; i < n_pose; ++i) {
+                loc[i] = make_pose(&pos_predict[i], &pos_last[i]);
+                fin[i] = make_pose(&pos_final[i], nullptr);
+            }
+            CU(cudaMemcpyAsync(c->d_pose, pr.host, bytes, cudaMemcpyHostToDevice, c->stream));
+            CU(cudaEventRecord(pr.done, c->stream));
+            CU((cudaError_t)launch_frame_seq(base, (long long)c->ntot * 3, (int)n_frames, c->d_labels, c->map, c->map_alt, out,
+                                             (const PoseXf *)c->d_pose, (const PoseXf *)c->d_pose + n_pose, c->n_seq, c->rows,
+                                             c->cols, c->d_n_exact, c->stream, nullptr, nullptr, so ? &seq_out : nullptr));
         }
-        nav_ctx::PoseRing &pr = c->pose_ring[c->pose_ring_next];
-        c->pose_ring_next = (c->pose_ring_next + 1) % nav_ctx::kPoseRing;
-        if (pr.done) CU(cudaEventSynchronize(pr.done));  // the staging buffer's previous upload (several sequences ago)
-        if (pr.cap < bytes) {
-            if (pr.host) cudaFreeHost(pr.host);
-            pr.host = nullptr;
-            pr.cap = 0;
-            CU(cudaHostAlloc((void **)&pr.host, bytes, cudaHostAllocDefault));
-            pr.cap = bytes;
-        }
-        if (!pr.done) CU(cudaEventCreateWithFlags(&pr.done, cudaEventDisableTiming));
-        if (c->d_pose_cap < bytes) {
-            CU(cudaStreamSynchronize(c->stream));
-            if (c->d_pose) cudaFree(c->d_pose);
-            c->d_pose = nullptr;
-            c->d_pose_cap = 0;
-            CU(cudaMalloc((void **)&c->d_pose, bytes));
-            c->d_pose_cap = bytes;
-        }
-        PoseXf *loc = (PoseXf *)pr.host, *fin = loc + n_pose;
-        for (size_t i = 0; i < n_pose; ++i) {
-            loc[i] = make_pose(&pos_predict[i], &pos_last[i]);
-            fin[i] = make_pose(&pos_final[i], nullptr);
-        }
-        CU(cudaMemcpyAsync(c->d_pose, pr.host, bytes, cudaMemcpyHostToDevice, c->stream));
-        CU(cudaEventRecord(pr.done, c->stream));
-        CU((cudaError_t)launch_frame_seq(base, (long long)c->ntot * 3, (int)n_frames, c->d_labels, c->map, c->map_alt, out,
-                                         (const PoseXf *)c->d_pose, (const PoseXf *)c->d_pose + n_pose, c->n_seq, c->rows,
-                                         c->cols, c->d_n_exact, c->stream));
         c->launches++;
         if (n_frames & 1) std::swap(c->map, c->map_alt);
-        c->cloud_resident = false;
-        CU(cudaGetLastError());
-        return 0;
+    } else {
+        const size_t n_chunks = (size_t)c->map.n_chunks;
+        for (size_t f = 0; f < n_frames; ++f) {
+            const double *cl = base + f * c->ntot * 3;
+            const size_t o = f * (size_t)c->n_seq;
+            // consecutive launches overlap (programmatic dependent launch): frame f+1 computes its labels
+            // while frame f finishes its searches.  With per-frame outputs the copies and the dedupe of frame f
+            // come between them, and the launches are ordinary.
+            run_frame_fused(c, cl, c->d_labels, c->d_nn_idx, c->d_nn_dist, pos_predict + o, pos_last + o, pos_final + o,
+                            /*pdl=*/!so);
+            if (!so) continue;
+            // frame f's results while the context holds them: the map just built carries its label masks, and
+            // the map it searched (now map_alt) is intact until the next frame's kernel
+            if (seq_out.nn_idx)
+                CU(cudaMemcpyAsync(seq_out.nn_idx + f * c->ntot, c->d_nn_idx, c->ntot * 4, cudaMemcpyDeviceToDevice, c->stream));
+            if (seq_out.nn_dist)
+                CU(cudaMemcpyAsync(seq_out.nn_dist + f * c->ntot, c->d_nn_dist, c->ntot * 8, cudaMemcpyDeviceToDevice,
+                                   c->stream));
+            if (seq_out.mask)
+                CU(cudaMemcpyAsync(seq_out.mask + f * nr * n_chunks, c->map.mask, nr * n_chunks * 4, cudaMemcpyDeviceToDevice,
+                                   c->stream));
+            if (part) {
+                const MatchOut out = {c->d_nn_idx, c->d_nn_dist, c->d_corr_rows, c->d_corr_row_count};
+                const PoseBatch loc = pose_batch(c, pos_predict + o, pos_last + o);
+                double *pf = part + f * part_frame * 5;
+                if (tile_parts) {
+                    const FitMailbox no_mail = {nullptr, nullptr, 0ull};
+                    CU((cudaError_t)launch_dedupe_stats(cl, c->d_labels, c->map_alt, out, loc, c->n_seq, c->rows, c->cols,
+                                                        c->stream, pf, no_mail));
+                } else {
+                    launch_dedupe(cl, c->d_labels, c->map_alt, out, loc, c->n_seq, c->rows, c->cols, c->stream, pf, false);
+                }
+                c->launches++;
+            }
+        }
     }
-    for (size_t f = 0; f < n_frames; ++f) {
-        const double *cl = base + f * c->ntot * 3;
-        const size_t o = f * (size_t)c->n_seq;
-        // consecutive launches overlap (programmatic dependent launch): frame f+1 computes its labels
-        // while frame f finishes its searches
-        run_frame_fused(c, cl, c->d_labels, c->d_nn_idx, c->d_nn_dist, pos_predict + o, pos_last + o, pos_final + o,
-                        /*pdl=*/true);
+    if (part) {
+        launch_seq_fit_totals(part, !tile_parts, (int)(part_frame / c->n_seq), (int)n_frames, c->n_seq,
+                              (double *)so->fit_stats, c->stream);
+        c->launches++;
     }
     c->cloud_resident = false;
     CU(cudaGetLastError());
     return 0;
+}
+
+extern "C" int nav_frontend_sequence_dev(nav_ctx *c, const void *dev_frames, size_t n_frames,
+                                         const nav_pos *pos_predict, const nav_pos *pos_last,
+                                         const nav_pos *pos_final) {
+    CTX_ENTER(c, "nav_frontend_sequence_dev");
+    return frontend_sequence(c, "nav_frontend_sequence_dev", dev_frames, n_frames, pos_predict, pos_last, pos_final,
+                             nullptr);
+}
+
+extern "C" int nav_frontend_sequence_out_dev(nav_ctx *c, const void *dev_frames, size_t n_frames,
+                                             const nav_pos *pos_predict, const nav_pos *pos_last,
+                                             const nav_pos *pos_final, const nav_sequence_out *out) {
+    CTX_ENTER(c, "nav_frontend_sequence_out_dev");
+    return frontend_sequence(c, "nav_frontend_sequence_out_dev", dev_frames, n_frames, pos_predict, pos_last, pos_final,
+                             out);
 }
 
 extern "C" int nav_frame_results_dev(nav_ctx *c, nav_frame_results *out) {

@@ -42,12 +42,25 @@ struct FitMailbox {
 // a whole sequence of frames with known poses in one launch (one thread-block cluster per image row walks
 // through the frames); map0 is searched by frame 0, frame f builds the map for frame f+1 in the other buffer.
 // d_pose_loc / d_pose_fin: device arrays [n_frames][n_seq].  Needs frame_seq_supported(cols).
+// seq_out (optional): per-frame outputs -- slot f of every non-null ring receives frame f (nav_sequence_out), and
+// part != null adds the statistics dedupe, CTA partials [n_frames][n_seq*rows*tiles][5] for launch_seq_fit_totals.
 bool frame_seq_supported(int cols);
 int frame_seq_inline_frames();  // sequences up to this length (one sequence) carry their poses as kernel parameters
+struct SeqOut {
+    unsigned *mask;   // [n_frames][n_seq*rows][n_chunks]
+    int *nn_idx;      // [n_frames][n_seq*rows][cols]
+    double *nn_dist;  // [n_frames][n_seq*rows][cols]
+    double *part;     // [n_frames][n_seq*rows*tiles][5]
+};
 int launch_frame_seq(const double *frames, long long frame_stride, int n_frames, int *labels, const RowMap &map0,
                      const RowMap &map1, const MatchOut &out, const PoseXf *d_pose_loc, const PoseXf *d_pose_fin,
                      int n_seq, int rows, int cols, unsigned *n_exact, cudaStream_t stream,
-                     const PoseXf *h_pose_loc = nullptr, const PoseXf *h_pose_fin = nullptr);
+                     const PoseXf *h_pose_loc = nullptr, const PoseXf *h_pose_fin = nullptr,
+                     const SeqOut *seq_out = nullptr);
+// fit totals stats[f][s][0..4] of the partials part[f][s][n_part][5], in the closed loop's summation order:
+// row_partials = false for tile partials (k_frame_seq, k_dedupe_stats), true for row totals (k_dedupe_rows)
+void launch_seq_fit_totals(const double *part, bool row_partials, int n_part, int n_frames, int n_seq, double *stats,
+                           cudaStream_t stream);
 
 size_t dedupe_smem_bytes(int cols);
 int configure_row_kernels(int cols);  // opt in to large dynamic shared memory; 0 on success

@@ -73,9 +73,11 @@ __device__ __forceinline__ float half_max(float v, unsigned half_mask) {
 // ---------------------------------------------------------------------------------------------
 // One (row, 256-column tile) of the map: transform the thread's own column, write the global
 // cloud, the 16-bit label masks, the leaf boxes and the tile's super box.  Called by all kTile
-// threads of the CTA (contains one __syncthreads).
+// threads of the CTA (contains one __syncthreads).  mask_out (optional): a second copy of the label masks,
+// laid out as map.mask ([n_seq*rows][n_chunks]).
 __device__ __forceinline__ void map_tile(bool lab, bool valid, const P3 &p, const PoseXf &pose, const RowMap &map,
-                                         int rid, int tile, int c, long long base, float4 *s_lo, float4 *s_hi) {
+                                         int rid, int tile, int c, long long base, float4 *s_lo, float4 *s_hi,
+                                         unsigned *__restrict__ mask_out = nullptr) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, half = lane >> 4, l16 = lane & 15;
     P3 g = {0, 0, 0};
     if (valid) {
@@ -101,6 +103,7 @@ __device__ __forceinline__ void map_tile(bool lab, bool valid, const P3 &p, cons
         s_hi[leaf_in_tile] = fhi;
         if (leaf < map.n_chunks) {
             map.mask[(long long)rid * map.n_chunks + leaf] = mask16;
+            if (mask_out) mask_out[(long long)rid * map.n_chunks + leaf] = mask16;
             float4 *b = map.box + ((long long)rid * map.n_chunks + leaf) * 2;
             b[0] = flo;
             b[1] = fhi;
@@ -560,177 +563,6 @@ __device__ __forceinline__ void cluster_sync_all() {
     asm volatile("barrier.cluster.arrive.release;\n\tbarrier.cluster.wait.acquire;" ::: "memory");
 }
 
-// ---------------------------------------------------------------------------------------------
-// A whole SEQUENCE of frames with known poses in ONE launch (nav_frontend_sequence_dev).  Frame t+1 of an image
-// row only depends on the map the eight tiles of the SAME row built from frame t, so the CTAs of a row form a
-// thread-block cluster that walks through the frames on its own, with a cluster barrier per frame where
-// separate launches had a grid-wide dependency: no launch latency between frames, and rows that are ahead are
-// not held back by rows that are behind.  Per frame the body is that of k_frame_match<fused labels, fused map>:
-// labels (a3), query transform (a7), exact search of the row map of the previous frame (a6), the next map from
-// the frame's final pose into the other map buffer (a7, a4/a5).  labels / nn_idx / nn_dist hold the results of
-// the last frame, as after the same number of separate launches.
-#ifdef NAV_SEQ_TIMING
-// developer instrumentation (profiles/prof_seq_phases.py; build rowmap.cu with -DNAV_SEQ_TIMING): thread 0 of every
-// CTA stamps %globaltimer at seven points of every frame of k_frame_seq
-__device__ unsigned long long *g_seq_stamps;   // [frames][ctas][8]
-#define NAV_STAMP(k)                                                                                              \
-    do {                                                                                                          \
-        if (threadIdx.x == 0 && g_seq_stamps) {                                                                   \
-            unsigned long long t_;                                                                                \
-            asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t_));                                               \
-            const int cta_ = (blockIdx.z * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x;                      \
-            g_seq_stamps[((long long)f * gridDim.x * gridDim.y * gridDim.z + cta_) * 8 + (k)] = t_;               \
-        }                                                                                                         \
-    } while (0)
-extern "C" int nav_debug_set_seq_stamps(void *dev_ptr) {
-    return (int)cudaMemcpyToSymbol(g_seq_stamps, &dev_ptr, sizeof(void *));
-}
-#else
-#define NAV_STAMP(k)
-#endif
-
-constexpr int kSeqInlineFrames = 64;
-struct SeqArgs {
-    const double *frames;     // [n_frames][n_seq*rows][cols][3]
-    long long frame_stride;   // doubles between consecutive frames
-    int n_frames, n_seq;
-    const PoseXf *pose_loc;   // [n_frames][n_seq] predicted pose + shift (queries)
-    const PoseXf *pose_fin;   // [n_frames][n_seq] final pose (map)
-};
-// poses of a short sequence travel as kernel parameters (CUDA 12.1+: up to 32 764 bytes): no upload to queue
-// in front of the launch, no staging buffer to guard
-struct SeqInlinePoses {
-    PoseXf loc[kSeqInlineFrames], fin[kSeqInlineFrames];
-};
-static_assert(sizeof(SeqInlinePoses) + 256 < 32764, "inline poses must fit the kernel parameter space");
-
-template <bool kInline>
-__global__ void __launch_bounds__(kTile, NAV_MATCH_MIN_CTAS)
-k_frame_seq(SeqArgs a, int *__restrict__ labels, RowMap map0, RowMap map1, MatchOut out, int rows, int cols,
-            unsigned *__restrict__ n_exact, const __grid_constant__ SeqInlinePoses ip) {
-    __shared__ __align__(16) double s_pts[2][kTilePts * 3];  // the tile of this frame / of the next one (in flight)
-    __shared__ float s_f1[kTile + kHalo], s_f2[kTile + kHalo];
-    __shared__ int s_warp[65];
-    __shared__ int s_qcol[kTile];
-    __shared__ MapSmem sm;
-    __shared__ float4 s_lo[kChunksPerSuper], s_hi[kChunksPerSuper];
-    const int tile = blockIdx.x, row = blockIdx.y, seq = blockIdx.z;
-    const int rid = seq * rows + row;
-    const long long base = (long long)rid * cols;
-    const int c0 = tile * kTile;
-    const int c = c0 + threadIdx.x;
-    tile_stage_async(s_pts[0], a.frames + base * 3, c0, cols);
-    cp_async_commit();
-    for (int f = 0; f < a.n_frames; ++f) {
-        NAV_STAMP(0);
-        const double *pts = s_pts[f & 1];
-        const RowMap &map = (f & 1) ? map1 : map0;
-        const RowMap &map_next = (f & 1) ? map0 : map1;
-        const RowView rv = {map.pts + base * 3, map.mask + (long long)rid * map.n_chunks,
-                            map.box + (long long)rid * map.n_chunks * 2, map.sbox + (long long)rid * map.n_super * 2,
-                            map.n_chunks, map.n_super, tile * kChunksPerSuper - 1};
-        cp_async_wait_group<0>();  // this frame's tile has landed
-        __syncthreads();
-        NAV_STAMP(1);
-        // the labels need nothing from the row's other tiles: they are computed BEFORE waiting for the cluster
-        // (the barrier was only signalled at the end of the previous frame), which turns the wait for the row's
-        // slowest tile into useful time
-        const int label = tile_labels_filtered(pts, s_f1, s_f2, c0, cols, n_exact);
-        NAV_STAMP(2);
-        if (f > 0) cluster_wait_all();  // the row's map of the previous frame is complete (also a CTA barrier)
-        NAV_STAMP(3);
-        prefetch_neighbourhood<true>(sm, rv, cols);
-        cp_async_commit();
-        // the next frame's tile starts its way from HBM now and has the whole search to arrive
-        if (f + 1 < a.n_frames)
-            tile_stage_async(s_pts[(f + 1) & 1], a.frames + (long long)(f + 1) * a.frame_stride + base * 3, c0, cols);
-        cp_async_commit();
-        if (c < cols) {
-            labels[base + c] = label;
-            if (label != 1) {
-                out.nn_idx[base + c] = -1;
-                out.nn_dist[base + c] = -1.0;
-            }
-        }
-        {
-            P3 own = {0, 0, 0};
-            if (c < cols) {
-                const double *sp = pts + (threadIdx.x + kHalo) * 3;
-                own.x = sp[0];
-                own.y = sp[1];
-                own.z = sp[2];
-            }
-            map_tile(label == 1, c < cols, own, kInline ? ip.fin[f] : a.pose_fin[(long long)f * a.n_seq + seq], map_next, rid,
-                     tile, c, base, s_lo, s_hi);
-        }
-        NAV_STAMP(4);
-        cp_async_wait_group<1>();  // the neighbourhood of the map; the next tile may still be in flight
-        int nq;
-        const int slot = block_excl_count(label == 1, s_warp, nq);  // its barriers also publish the prefetch
-        if (label == 1) s_qcol[slot] = threadIdx.x;
-        __syncthreads();
-        NAV_STAMP(5);
-        if ((int)(threadIdx.x & ~31u) < nq) {  // warps with at least one query; spare lanes repeat the last one
-            const int t = s_qcol[min((int)threadIdx.x, nq - 1)];
-            const int qc = c0 + t;
-            const double *sp = pts + (t + kHalo) * 3;
-            const P3 p = {sp[0], sp[1], sp[2]};
-            const PoseXf &pose = kInline ? ip.loc[f] : a.pose_loc[(long long)f * a.n_seq + seq];
-            const P3 q = shift_point(pose, xf_point(pose, p));
-            double best;
-            int bcol;
-            search_row<true>(sm, rv, qc, q, best, bcol, kFull);
-            if ((int)threadIdx.x < nq) {
-                out.nn_idx[base + qc] = bcol >= 0 ? row * cols + bcol : -1;
-                out.nn_dist[base + qc] = bcol >= 0 ? __dsqrt_rn(best) : INFINITY;
-            }
-        }
-        // this CTA's part of the row's next map is written and it no longer reads the current one: signal the
-        // cluster (release) and go on; the matching wait sits in front of the next frame's map prefetch
-        NAV_STAMP(6);
-        cluster_arrive_all();
-    }
-    cluster_wait_all();  // every arrive has its wait
-}
-
-bool frame_seq_supported(int cols) { return div_up(cols, kTile) <= 8; }
-
-int frame_seq_inline_frames() { return kSeqInlineFrames; }
-
-// h_pose_loc / h_pose_fin != null (n_seq == 1, n_frames <= frame_seq_inline_frames()): the poses are passed as
-// kernel parameters and the device arrays are not read
-int launch_frame_seq(const double *frames, long long frame_stride, int n_frames, int *labels, const RowMap &map0,
-                     const RowMap &map1, const MatchOut &out, const PoseXf *d_pose_loc, const PoseXf *d_pose_fin,
-                     int n_seq, int rows, int cols, unsigned *n_exact, cudaStream_t stream, const PoseXf *h_pose_loc,
-                     const PoseXf *h_pose_fin) {
-    const int tiles = div_up(cols, kTile);
-    const SeqArgs a = {frames, frame_stride, n_frames, n_seq, d_pose_loc, d_pose_fin};
-    const bool inl = h_pose_loc && h_pose_fin && n_seq == 1 && n_frames <= kSeqInlineFrames;
-
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)tiles, (unsigned)rows, (unsigned)n_seq);
-    cfg.blockDim = dim3(kTile);
-    cfg.stream = stream;
-    cudaLaunchAttribute attr;
-    attr.id = cudaLaunchAttributeClusterDimension;
-    attr.val.clusterDim.x = (unsigned)tiles;
-    attr.val.clusterDim.y = 1;
-    attr.val.clusterDim.z = 1;
-    cfg.attrs = &attr;
-    cfg.numAttrs = 1;
-    if (inl) {
-        SeqInlinePoses ip;  // the launch copies its parameters at the call
-        for (int f = 0; f < n_frames; ++f) {
-            ip.loc[f] = h_pose_loc[f];
-            ip.fin[f] = h_pose_fin[f];
-        }
-        for (int f = n_frames; f < kSeqInlineFrames; ++f) ip.loc[f] = ip.fin[f] = h_pose_loc[0];
-        return (int)cudaLaunchKernelEx(&cfg, k_frame_seq<true>, a, labels, map0, map1, out, rows, cols, n_exact, ip);
-    }
-    static const SeqInlinePoses none = {};
-    return (int)cudaLaunchKernelEx(&cfg, k_frame_seq<false>, a, labels, map0, map1, out, rows, cols, n_exact, none);
-}
-
 void launch_frame_map(const double *cloud, const int *labels, const RowMap &map, const PoseBatch &poses,
                       int n_seq, int rows, int cols, cudaStream_t stream) {
     const int tiles = div_up(cols, kTile);
@@ -785,12 +617,13 @@ void launch_frame_match(const double *cloud, int *labels, bool fused_labels, con
 
 constexpr int kRowThreads = 512;
 
-// Called by every thread of the CTA that finished last: adds the five partial sums of all `n_part` CTAs
-// (part[i*5 + k]) in a fixed order -- thread-strided with independent loads, a shuffle tree, then warp by
-// warp -- and posts the totals followed by the sequence number to the host mailbox.  T = blockDim.x.
+// The fixed summation order of the fit totals: adds the five partial sums of `n_part` CTAs or rows
+// (part[i*5 + k]) thread-strided with independent loads, then a shuffle tree, then warp by warp, and writes
+// them to dst[0..4].  Called by all T = blockDim.x threads.  Every kernel that reports totals of the same
+// partials uses this, so they are the same bits whichever kernel formed them.
 template <int T>
-__device__ __forceinline__ void post_fit_totals(const double *__restrict__ part, int n_part, const FitMailbox &mail,
-                                                double (*s_tot)[5]) {
+__device__ __forceinline__ void sum_fit_partials(const double *__restrict__ part, int n_part, double (*s_tot)[5],
+                                                 double *dst) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     double t[5] = {0.0, 0.0, 0.0, 0.0, 0.0};
     for (int i = threadIdx.x; i < n_part; i += T) {
@@ -811,8 +644,16 @@ __device__ __forceinline__ void post_fit_totals(const double *__restrict__ part,
     if (threadIdx.x < 5) {
         double a = 0.0;
         for (int w = 0; w < T / 32; ++w) a = dadd(a, s_tot[w][threadIdx.x]);
-        mail.host[threadIdx.x] = a;
+        dst[threadIdx.x] = a;
     }
+}
+
+// Called by every thread of the CTA that finished last: adds the partials of all `n_part` CTAs
+// (sum_fit_partials) and posts the totals followed by the sequence number to the host mailbox.  T = blockDim.x.
+template <int T>
+__device__ __forceinline__ void post_fit_totals(const double *__restrict__ part, int n_part, const FitMailbox &mail,
+                                                double (*s_tot)[5]) {
+    sum_fit_partials<T>(part, n_part, s_tot, mail.host);
     __syncthreads();
     if (threadIdx.x == 0) {
         // cumulative, by the thread that writes the flag: the five totals (ordered before it by the barrier)
@@ -1213,6 +1054,261 @@ int launch_loop_step(const double *cloud, const int *labels, const RowMap &map, 
     cfg.numAttrs = 1;
     return (int)cudaLaunchKernelEx(&cfg, k_loop_step, cloud, labels, map, out, poses, rows, cols, tiles, prev_cloud,
                                    prev_labels, prev_poses, do_map ? 1 : 0, part, mail);
+}
+
+// ---------------------------------------------------------------------------------------------
+// A whole SEQUENCE of frames with known poses in ONE launch (nav_frontend_sequence_dev).  Frame t+1 of an image
+// row only depends on the map the eight tiles of the SAME row built from frame t, so the CTAs of a row form a
+// thread-block cluster that walks through the frames on its own, with a cluster barrier per frame where
+// separate launches had a grid-wide dependency: no launch latency between frames, and rows that are ahead are
+// not held back by rows that are behind.  Per frame the body is that of k_frame_match<fused labels, fused map>:
+// labels (a3), query transform (a7), exact search of the row map of the previous frame (a6), the next map from
+// the frame's final pose into the other map buffer (a7, a4/a5).  labels / nn_idx / nn_dist hold the results of
+// the last frame, as after the same number of separate launches.
+// kOut (nav_frontend_sequence_out_dev): every frame also stores its label masks, nn_idx and nn_dist into slot f of
+// the caller's rings (SeqOut), and -- when o.part is set -- runs the statistics dedupe of k_loop_step on the search
+// results still in registers, writing the CTA partials of frame f to o.part (k_seq_fit_totals adds them up).  The
+// four cluster barriers of the dedupe sit between the frame's cluster wait and its arrive, so arrive and wait
+// still alternate; the dedupe reads the map the frame searched, which frame f+1 overwrites only after its
+// cluster wait, i.e. after every CTA of the row has finished its dedupe.
+#ifdef NAV_SEQ_TIMING
+// developer instrumentation (profiles/prof_seq_phases.py; build rowmap.cu with -DNAV_SEQ_TIMING): thread 0 of every
+// CTA stamps %globaltimer at seven points of every frame of k_frame_seq
+__device__ unsigned long long *g_seq_stamps;   // [frames][ctas][8]
+#define NAV_STAMP(k)                                                                                              \
+    do {                                                                                                          \
+        if (threadIdx.x == 0 && g_seq_stamps) {                                                                   \
+            unsigned long long t_;                                                                                \
+            asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t_));                                               \
+            const int cta_ = (blockIdx.z * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x;                      \
+            g_seq_stamps[((long long)f * gridDim.x * gridDim.y * gridDim.z + cta_) * 8 + (k)] = t_;               \
+        }                                                                                                         \
+    } while (0)
+extern "C" int nav_debug_set_seq_stamps(void *dev_ptr) {
+    return (int)cudaMemcpyToSymbol(g_seq_stamps, &dev_ptr, sizeof(void *));
+}
+#else
+#define NAV_STAMP(k)
+#endif
+
+constexpr int kSeqInlineFrames = 64;
+struct SeqArgs {
+    const double *frames;     // [n_frames][n_seq*rows][cols][3]
+    long long frame_stride;   // doubles between consecutive frames
+    int n_frames, n_seq;
+    const PoseXf *pose_loc;   // [n_frames][n_seq] predicted pose + shift (queries)
+    const PoseXf *pose_fin;   // [n_frames][n_seq] final pose (map)
+};
+// poses of a short sequence travel as kernel parameters (CUDA 12.1+: up to 32 764 bytes): no upload to queue
+// in front of the launch, no staging buffer to guard
+struct SeqInlinePoses {
+    PoseXf loc[kSeqInlineFrames], fin[kSeqInlineFrames];
+};
+static_assert(sizeof(SeqInlinePoses) + 256 < 32764, "inline poses must fit the kernel parameter space");
+
+template <bool kInline, bool kOut>
+__global__ void __launch_bounds__(kTile, NAV_MATCH_MIN_CTAS)
+k_frame_seq(SeqArgs a, int *__restrict__ labels, RowMap map0, RowMap map1, MatchOut out, int rows, int cols,
+            unsigned *__restrict__ n_exact, const __grid_constant__ SeqInlinePoses ip, SeqOut o) {
+    __shared__ __align__(16) double s_pts[2][kTilePts * 3];  // the tile of this frame / of the next one (in flight)
+    __shared__ float s_f1[kTile + kHalo], s_f2[kTile + kHalo];
+    __shared__ int s_warp[65];
+    __shared__ int s_qcol[kTile];
+    __shared__ MapSmem sm;
+    __shared__ float4 s_lo[kChunksPerSuper], s_hi[kChunksPerSuper];
+    const int tile = blockIdx.x, row = blockIdx.y, seq = blockIdx.z;
+    const int rid = seq * rows + row;
+    const long long base = (long long)rid * cols;
+    const int c0 = tile * kTile;
+    const int c = c0 + threadIdx.x;
+    // ring slots: per frame n_seq*rows rows of cols pixels / n_chunks mask words / `tiles` CTA partials
+    const long long px_frame = (long long)a.n_seq * rows * cols, cta_frame = (long long)a.n_seq * rows * gridDim.x;
+    tile_stage_async(s_pts[0], a.frames + base * 3, c0, cols);
+    cp_async_commit();
+    for (int f = 0; f < a.n_frames; ++f) {
+        NAV_STAMP(0);
+        const double *pts = s_pts[f & 1];
+        const RowMap &map = (f & 1) ? map1 : map0;
+        const RowMap &map_next = (f & 1) ? map0 : map1;
+        const RowView rv = {map.pts + base * 3, map.mask + (long long)rid * map.n_chunks,
+                            map.box + (long long)rid * map.n_chunks * 2, map.sbox + (long long)rid * map.n_super * 2,
+                            map.n_chunks, map.n_super, tile * kChunksPerSuper - 1};
+        cp_async_wait_group<0>();  // this frame's tile has landed
+        __syncthreads();
+        NAV_STAMP(1);
+        // the labels need nothing from the row's other tiles: they are computed BEFORE waiting for the cluster
+        // (the barrier was only signalled at the end of the previous frame), which turns the wait for the row's
+        // slowest tile into useful time
+        const int label = tile_labels_filtered(pts, s_f1, s_f2, c0, cols, n_exact);
+        NAV_STAMP(2);
+        if (f > 0) cluster_wait_all();  // the row's map of the previous frame is complete (also a CTA barrier)
+        NAV_STAMP(3);
+        prefetch_neighbourhood<true>(sm, rv, cols);
+        cp_async_commit();
+        // the next frame's tile starts its way from HBM now and has the whole search to arrive
+        if (f + 1 < a.n_frames)
+            tile_stage_async(s_pts[(f + 1) & 1], a.frames + (long long)(f + 1) * a.frame_stride + base * 3, c0, cols);
+        cp_async_commit();
+        if (c < cols) {
+            labels[base + c] = label;
+            if (label != 1) {
+                out.nn_idx[base + c] = -1;
+                out.nn_dist[base + c] = -1.0;
+                if (kOut && o.nn_idx) o.nn_idx[f * px_frame + base + c] = -1;
+                if (kOut && o.nn_dist) o.nn_dist[f * px_frame + base + c] = -1.0;
+            }
+        }
+        {
+            P3 own = {0, 0, 0};
+            if (c < cols) {
+                const double *sp = pts + (threadIdx.x + kHalo) * 3;
+                own.x = sp[0];
+                own.y = sp[1];
+                own.z = sp[2];
+            }
+            unsigned *mask_out = nullptr;
+            if (kOut && o.mask) mask_out = o.mask + f * (long long)a.n_seq * rows * map_next.n_chunks;
+            map_tile(label == 1, c < cols, own, kInline ? ip.fin[f] : a.pose_fin[(long long)f * a.n_seq + seq], map_next, rid,
+                     tile, c, base, s_lo, s_hi, mask_out);
+        }
+        NAV_STAMP(4);
+        cp_async_wait_group<1>();  // the neighbourhood of the map; the next tile may still be in flight
+        int nq;
+        const int slot = block_excl_count(label == 1, s_warp, nq);  // its barriers also publish the prefetch
+        if (label == 1) s_qcol[slot] = threadIdx.x;
+        __syncthreads();
+        NAV_STAMP(5);
+        int key = -1, qc_won = -1;  // kOut: the query's match (map column) and column, for the dedupe
+        unsigned long long dbits = 0;
+        if ((int)(threadIdx.x & ~31u) < nq) {  // warps with at least one query; spare lanes repeat the last one
+            const int t = s_qcol[min((int)threadIdx.x, nq - 1)];
+            const int qc = c0 + t;
+            const double *sp = pts + (t + kHalo) * 3;
+            const P3 p = {sp[0], sp[1], sp[2]};
+            const PoseXf &pose = kInline ? ip.loc[f] : a.pose_loc[(long long)f * a.n_seq + seq];
+            const P3 q = shift_point(pose, xf_point(pose, p));
+            double best;
+            int bcol;
+            search_row<true>(sm, rv, qc, q, best, bcol, kFull);
+            if ((int)threadIdx.x < nq) {
+                out.nn_idx[base + qc] = bcol >= 0 ? row * cols + bcol : -1;
+                out.nn_dist[base + qc] = bcol >= 0 ? __dsqrt_rn(best) : INFINITY;
+                if (kOut) {
+                    const int idx = bcol >= 0 ? row * cols + bcol : -1;
+                    const double dist = bcol >= 0 ? __dsqrt_rn(best) : INFINITY;
+                    if (o.nn_idx) o.nn_idx[f * px_frame + base + qc] = idx;
+                    if (o.nn_dist) o.nn_dist[f * px_frame + base + qc] = dist;
+                    if (bcol >= 0) {
+                        key = bcol;
+                        qc_won = qc;
+                        dbits = (unsigned long long)__double_as_longlong(dist);
+                    }
+                }
+            }
+        }
+        if (kOut && o.part) {  // uniform over the grid: every CTA of the cluster takes it
+            __shared__ unsigned long long s_best[kTile];
+            __shared__ int s_win[kTile];
+            __shared__ StatsSmem ss;
+            const bool winner = cluster_dedupe_winner(s_best, s_win, key, dbits, qc_won);
+            // residuals back into column order through shared memory, as k_loop_step does (the search is over and
+            // the cluster barriers were CTA barriers too: the map neighbourhood and the query list are free).  The
+            // winner's ori is transformed again from the tile, the same bits as during the search.
+            double *s_r = sm.pts;
+            int *s_flag = s_qcol;
+            s_flag[threadIdx.x] = 0;
+            __syncthreads();
+            if (winner) {
+                const int t = qc_won - c0;
+                const double *sp = pts + (t + kHalo) * 3;
+                const P3 p = {sp[0], sp[1], sp[2]};
+                const P3 ori = xf_point(kInline ? ip.loc[f] : a.pose_loc[(long long)f * a.n_seq + seq], p);
+                const double *np = map.pts + (base + key) * 3;
+                s_r[t * 3] = dsub(ori.x, np[0]);
+                s_r[t * 3 + 1] = dsub(ori.y, np[1]);
+                s_r[t * 3 + 2] = dsub(ori.z, np[2]);
+                s_flag[t] = 1;
+            }
+            __syncthreads();
+            const bool mine = s_flag[threadIdx.x] != 0;
+            const double rx = mine ? s_r[threadIdx.x * 3] : 0.0, ry = mine ? s_r[threadIdx.x * 3 + 1] : 0.0,
+                         rz = mine ? s_r[threadIdx.x * 3 + 2] : 0.0;
+            // part + (rid * tiles + tile) * 5: the CTA order of k_dedupe_stats
+            const FitMailbox no_mail = {nullptr, nullptr, 0ull};
+            block_post_stats(ss, mine, rx, ry, rz, o.part + (f * cta_frame + (long long)rid * gridDim.x) * 5, no_mail);
+        }
+        // this CTA's part of the row's next map is written and it no longer reads the current one: signal the
+        // cluster (release) and go on; the matching wait sits in front of the next frame's map prefetch
+        NAV_STAMP(6);
+        cluster_arrive_all();
+    }
+    cluster_wait_all();  // every arrive has its wait
+}
+
+bool frame_seq_supported(int cols) { return div_up(cols, kTile) <= 8; }
+
+int frame_seq_inline_frames() { return kSeqInlineFrames; }
+
+// h_pose_loc / h_pose_fin != null (n_seq == 1, n_frames <= frame_seq_inline_frames()): the poses are passed as
+// kernel parameters and the device arrays are not read.  seq_out != null: the output mode of k_frame_seq.
+int launch_frame_seq(const double *frames, long long frame_stride, int n_frames, int *labels, const RowMap &map0,
+                     const RowMap &map1, const MatchOut &out, const PoseXf *d_pose_loc, const PoseXf *d_pose_fin,
+                     int n_seq, int rows, int cols, unsigned *n_exact, cudaStream_t stream, const PoseXf *h_pose_loc,
+                     const PoseXf *h_pose_fin, const SeqOut *seq_out) {
+    const int tiles = div_up(cols, kTile);
+    const SeqArgs a = {frames, frame_stride, n_frames, n_seq, d_pose_loc, d_pose_fin};
+    const bool inl = h_pose_loc && h_pose_fin && n_seq == 1 && n_frames <= kSeqInlineFrames;
+
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3((unsigned)tiles, (unsigned)rows, (unsigned)n_seq);
+    cfg.blockDim = dim3(kTile);
+    cfg.stream = stream;
+    cudaLaunchAttribute attr;
+    attr.id = cudaLaunchAttributeClusterDimension;
+    attr.val.clusterDim.x = (unsigned)tiles;
+    attr.val.clusterDim.y = 1;
+    attr.val.clusterDim.z = 1;
+    cfg.attrs = &attr;
+    cfg.numAttrs = 1;
+    const SeqOut no_out = {nullptr, nullptr, nullptr, nullptr};
+    if (inl) {
+        SeqInlinePoses ip;  // the launch copies its parameters at the call
+        for (int f = 0; f < n_frames; ++f) {
+            ip.loc[f] = h_pose_loc[f];
+            ip.fin[f] = h_pose_fin[f];
+        }
+        for (int f = n_frames; f < kSeqInlineFrames; ++f) ip.loc[f] = ip.fin[f] = h_pose_loc[0];
+        if (seq_out)
+            return (int)cudaLaunchKernelEx(&cfg, k_frame_seq<true, true>, a, labels, map0, map1, out, rows, cols, n_exact,
+                                           ip, *seq_out);
+        return (int)cudaLaunchKernelEx(&cfg, k_frame_seq<true, false>, a, labels, map0, map1, out, rows, cols, n_exact, ip,
+                                       no_out);
+    }
+    static const SeqInlinePoses none = {};
+    if (seq_out)
+        return (int)cudaLaunchKernelEx(&cfg, k_frame_seq<false, true>, a, labels, map0, map1, out, rows, cols, n_exact,
+                                       none, *seq_out);
+    return (int)cudaLaunchKernelEx(&cfg, k_frame_seq<false, false>, a, labels, map0, map1, out, rows, cols, n_exact, none,
+                                   no_out);
+}
+
+// Fit totals of frame blockIdx.x, sequence blockIdx.y: part = [n_frames][n_seq][n_part][5] partials, stats =
+// [n_frames][n_seq][5].  T = kTile adds the tile partials of k_frame_seq / k_dedupe_stats, T = kRowThreads the row
+// totals of k_dedupe_rows -- each in the order the closed loop's post uses for them (sum_fit_partials<T>).
+template <int T>
+__global__ void __launch_bounds__(T) k_seq_fit_totals(const double *__restrict__ part, int n_part, double *stats) {
+    __shared__ double s_tot[T / 32][5];
+    const long long fs = (long long)blockIdx.x * gridDim.y + blockIdx.y;
+    sum_fit_partials<T>(part + fs * n_part * 5, n_part, s_tot, stats + fs * 5);
+}
+
+void launch_seq_fit_totals(const double *part, bool row_partials, int n_part, int n_frames, int n_seq, double *stats,
+                           cudaStream_t stream) {
+    const dim3 grid((unsigned)n_frames, (unsigned)n_seq);
+    if (row_partials)
+        k_seq_fit_totals<kRowThreads><<<grid, kRowThreads, 0, stream>>>(part, n_part, stats);
+    else
+        k_seq_fit_totals<kTile><<<grid, kTile, 0, stream>>>(part, n_part, stats);
 }
 
 size_t dedupe_smem_bytes(int cols) { return (size_t)cols * 16; }
