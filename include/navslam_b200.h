@@ -70,6 +70,31 @@ int nav_synchronize(nav_ctx *ctx);
 /* number of kernels this library has launched on behalf of ctx since creation */
 uint64_t nav_launch_count(const nav_ctx *ctx);
 
+/* Tie rule of the per-row nearest-neighbour matches.  The two rules differ only where at least two map points of
+ * the row share the query's smallest rounded distance sqrt(dsq) (integer-valued data, e.g. whole millimetres).
+ *   NAV_TIE_LOWEST_INDEX (default): the lowest column among the points of smallest dsq (see Conventions).
+ *   NAV_TIE_REFERENCE: the reference's answer -- the first point of smallest rounded distance that the depth-first
+ *     search of its per-row tree reaches (utils/kdtree.c:20-82 build, 110-152 search).  The match kernel lists the
+ *     tied queries; the call copies the list and the rows it names back, builds the reference's tree of each such
+ *     row on the host and re-answers the listed queries with the reference's search before anything reads nn_idx.
+ *     nn_dist is the same under both rules.  Costs one extra stream synchronisation per call, two more plus the
+ *     copies when a query is tied.  Supported by the blocking calls: nav_slam_match and nav_slam_localization
+ *     (the correspondence list, and so the pose, is the reference's bit for bit), nav_frontend_frame and
+ *     nav_frontend_frame_depth (any n_seq).  Refused -- non-zero return, an error naming the tie rule, nothing
+ *     queued, the context unchanged -- by the calls that search the row map without a host round trip:
+ *     nav_frontend_frame_dev, nav_frontend_sequence_dev, nav_frontend_sequence_out_dev, nav_frontend_submit,
+ *     nav_frontend_frame_async, nav_frontend_frame_depth_async, nav_slam_localization_fast and nav_slam_run.
+ *     Calls that only label or map (nav_slam_init[_dev], nav_slam_mapping, nav_slam_prefetch, ...) and the
+ *     kd-tree calls work as before.
+ * The first switch to NAV_TIE_REFERENCE allocates a list of one 32-byte record per pixel of the context.
+ * Note: these constants are the inverse of the CPU oracle's tie_mode numbering (tie_mode 0 = reference). */
+#define NAV_TIE_LOWEST_INDEX 0
+#define NAV_TIE_REFERENCE 1
+int nav_set_tie_rule(nav_ctx *ctx, int rule);
+int nav_tie_rule(const nav_ctx *ctx);
+/* number of tied queries the host has re-answered under NAV_TIE_REFERENCE since the context was created */
+uint64_t nav_tie_resolve_count(const nav_ctx *ctx);
+
 /* ---- function-level mirrors, HOST buffers (one image each) ------------------------ */
 /* replaces convertToPointCloud, utils/pointcloud.c:8 (utils/pointcloud.h:55) */
 int nav_convert_to_pointcloud(nav_ctx *ctx, const int *distances, nav_point *cloud_out);
@@ -377,7 +402,10 @@ uint64_t nav_exact_fallback_count(nav_ctx *ctx);
 
 /* per-kernel device time accumulated with CUDA events on the context's stream (enable first) */
 int nav_profile_enable(nav_ctx *ctx, int on);
-/* name = "labels" | "match" | "map"; returns accumulated ms and launches since the last reset */
+/* name = "labels" | "match" | "map"; returns accumulated ms and launches since the last reset.
+ * Under NAV_TIE_REFERENCE also the host wall-clock time of the tie resolution, per step, with the number of matches
+ * that listed a tied query in place of launches: "tie_copies" (list and rows back to the host), "tie_search" (the
+ * reference's trees and searches), "tie_upload" (answers back and the scatter launch). */
 int nav_profile_read(nav_ctx *ctx, const char *name, double *ms_out, uint64_t *launches_out, int reset);
 
 #ifdef __cplusplus

@@ -61,6 +61,7 @@ EXPORTS = [
     "nav_frontend_submit", "nav_frontend_frame_depth_async", "nav_slam_prefetch", "nav_slam_prefetch_depth",
     "nav_host_register", "nav_host_unregister", "nav_slam_run", "nav_slam_fit_stats",
     "nav_frontend_sequence_out_dev", "nav_slam_fit_from_stats",
+    "nav_set_tie_rule", "nav_tie_rule", "nav_tie_resolve_count",
     "nav_peer_create", "nav_peer_connect", "nav_kdtree_nn_allgather_dev", "nav_kdtree_nn_sharded_map_dev", "nav_peer_check",
     "nav_peer_destroy", "nav_shard_range", "nav_shard_owner",
 ]
@@ -178,6 +179,10 @@ def load_library(build_if_missing: bool = True):
     L.nav_row_map_export.argtypes = [vp, C.c_int, C.c_int, vp, vp, C.POINTER(C.c_size_t)]
     L.nav_exact_fallback_count.restype = C.c_uint64
     L.nav_exact_fallback_count.argtypes = [vp]
+    L.nav_set_tie_rule.argtypes = [vp, C.c_int]
+    L.nav_tie_rule.argtypes = [vp]
+    L.nav_tie_resolve_count.restype = C.c_uint64
+    L.nav_tie_resolve_count.argtypes = [vp]
     L.nav_profile_enable.argtypes = [vp, C.c_int]
     L.nav_profile_read.argtypes = [vp, C.c_char_p, c_double_p, C.POINTER(C.c_uint64), C.c_int]
     _LIB = L
@@ -462,6 +467,24 @@ class Context:
 
     def exact_fallback_count(self) -> int:
         return int(self.L.nav_exact_fallback_count(self.h))
+
+    TIE_RULES = {"lowest_index": 0, "reference": 1}  # NAV_TIE_* of include/navslam_b200.h
+
+    def set_tie_rule(self, rule: str):
+        """nav_set_tie_rule: "lowest_index" (default) or "reference" (the reference's nearest point on exact
+        distance ties; blocking calls only, see include/navslam_b200.h)."""
+        if rule not in self.TIE_RULES:
+            raise ValueError(f"unknown tie rule {rule!r}; expected one of {sorted(self.TIE_RULES)}")
+        _check(self.L.nav_set_tie_rule(self.h, self.TIE_RULES[rule]), self.L)
+
+    @property
+    def tie_rule(self) -> str:
+        v = int(self.L.nav_tie_rule(self.h))
+        return {n: k for k, n in self.TIE_RULES.items()}[v]
+
+    def tie_resolve_count(self) -> int:
+        """tied queries re-answered by the host under the "reference" rule since the context was created"""
+        return int(self.L.nav_tie_resolve_count(self.h))
 
     def launch_count(self) -> int:
         return int(self.L.nav_launch_count(self.h))

@@ -1,6 +1,7 @@
 // capi.cu -- the C ABI of libnavslam_b200.so (include/navslam_b200.h): contexts, host<->device
 // staging, and the host-side scalar pieces the reference keeps on the CPU (rotation matrix from
 // libm sin/cos, tan tables, the translation-only Adam fit of src/slam.c:218-379).
+#include <assert.h>
 #include <math.h>
 #include <stdarg.h>
 #include <stdio.h>
@@ -8,6 +9,7 @@
 #include <time.h>
 #include <string.h>
 
+#include <algorithm>
 #include <string>
 #include <utility>
 #include <vector>
@@ -287,6 +289,15 @@ struct nav_ctx {
     double trace_us[5] = {0, 0, 0, 0, 0};
     bool prof = false;
     ProfSlot prof_labels, prof_match, prof_map;
+    // tie rule (nav_set_tie_rule).  NAV_TIE_REFERENCE: the match kernel lists its tied queries here (one record per
+    // pixel at most), and the blocking calls re-answer them on the host with the reference's own search
+    int tie_rule = NAV_TIE_LOWEST_INDEX;
+    TieRec *d_tie_rec = nullptr;
+    unsigned *d_tie_count = nullptr;
+    int2 *d_tie_fix = nullptr;  // (pixel, nn_idx) answers of the host, one per record
+    uint64_t tie_resolved = 0;
+    double tie_ms[3] = {0, 0, 0};  // profiler (c->prof): host ms of the copies, the searches, the upload
+    uint64_t tie_calls = 0;
 };
 
 static void rotation_from_pos(const nav_pos *pos, double R[9]) {
@@ -359,7 +370,7 @@ extern "C" void nav_destroy(nav_ctx *c) {
                     c->map.mask, c->d_n_exact, c->map.box, c->map.sbox, c->map_alt.pts, c->map_alt.mask,
                     c->map_alt.box, c->map_alt.sbox, c->d_corr_rows, c->d_corr,
                     c->d_corr_row_count, c->d_corr_total, c->d_dist, c->d_tan_col, c->d_tan_row, c->d_flat,
-                    c->d_flat_count};
+                    c->d_flat_count, c->d_tie_rec, c->d_tie_count, c->d_tie_fix};
     for (void *p : ptrs)
         if (p) cudaFree(p);
     if (c->h_small) cudaFreeHost(c->h_small);
@@ -542,6 +553,17 @@ extern "C" int nav_profile_enable(nav_ctx *c, int on) {
 
 extern "C" int nav_profile_read(nav_ctx *c, const char *name, double *ms, uint64_t *launches, int reset) {
     if (!c || !name) return fail("nav_profile_read: null argument");
+    const char *tie_names[3] = {"tie_copies", "tie_search", "tie_upload"};
+    for (int i = 0; i < 3; ++i)
+        if (!strcmp(name, tie_names[i])) {
+            if (ms) *ms = c->tie_ms[i];
+            if (launches) *launches = c->tie_calls;
+            if (reset) {
+                c->tie_ms[i] = 0;
+                if (i == 2) c->tie_calls = 0;
+            }
+            return 0;
+        }
     ProfSlot *s = !strcmp(name, "labels") ? &c->prof_labels
                   : !strcmp(name, "match") ? &c->prof_match
                   : !strcmp(name, "map")   ? &c->prof_map
@@ -596,19 +618,181 @@ static void run_map(nav_ctx *c, const double *d_cloud, const int *d_labels, cons
     c->have_map = true;
 }
 
+// ---- the reference tie rule (NAV_TIE_REFERENCE) ------------------------------------------------------------------
+// The device search keeps the lowest column among equal dsq.  The reference keeps the first point of the smallest
+// rounded distance sqrt(dsq) that the depth-first search of its per-row tree reaches.  The two differ only where two
+// map points of the row share that smallest rounded distance; the match kernel's kRefTies variant lists exactly those
+// queries, and resolve_ties re-answers them here with the reference's own tree and search, built per call for the
+// rows the list names (no tree outlives the call, so no map update can leave a stale one behind).
+// Host code compiled with -ffp-contract=off, like adam_fit: every operation rounds as the reference's does.
+static double ref_key(const nav_point &p, int axis) { return axis == 0 ? p.x : (axis == 1 ? p.y : p.z); }
+
+// utils/kdtree.c:20-62: Lomuto partition with the last element as pivot, (key - pivot) <= 0 to the front
+static void ref_select(nav_point *p, size_t first, size_t last, size_t nth, int axis) {
+    while (first < last) {
+        const double pivot = ref_key(p[last], axis);
+        size_t store = first;
+        for (size_t j = first; j < last; ++j) {
+            const double cmp = ref_key(p[j], axis) - pivot;
+            if (cmp <= 0) {
+                std::swap(p[store], p[j]);
+                ++store;
+            }
+        }
+        std::swap(p[store], p[last]);
+        if (store == nth) return;
+        if (store < nth)
+            first = store + 1;
+        else
+            last = store - 1;
+    }
+}
+
+// utils/kdtree.c:65-82 in place: the node of p[0..n) is p[n/2] (axis depth % 3), its children are p[0..m) and
+// p[m+1..n) -- the pointer tree of the reference, laid out as the array it was selected in
+static void ref_build(nav_point *p, size_t n, int depth) {
+    if (n == 0) return;
+    const size_t m = n / 2;
+    ref_select(p, 0, n - 1, m, depth % 3);
+    ref_build(p, m, depth + 1);
+    ref_build(p + m + 1, n - m - 1, depth + 1);
+}
+
+// utils/kdtree.c:110-152: dist = sqrt((dx*dx + dy*dy) + dz*dz) with root - target, update on strict '<', near side
+// first, far side iff fabs(delta) < best
+static void ref_nn(const nav_point *p, size_t n, int depth, const nav_point &q, nav_point &best, double &best_dist) {
+    if (n == 0) return;
+    const size_t m = n / 2;
+    const nav_point &r = p[m];
+    const double dx = r.x - q.x, dy = r.y - q.y, dz = r.z - q.z;
+    const double d = sqrt(dx * dx + dy * dy + dz * dz);
+    if (d < best_dist) {
+        best_dist = d;
+        best = r;
+    }
+    const int axis = depth % 3;
+    const double delta = ref_key(q, axis) - ref_key(r, axis);
+    const nav_point *lo = p, *hi = p + m + 1;
+    const size_t n_lo = m, n_hi = n - m - 1;
+    if (delta < 0) {
+        ref_nn(lo, n_lo, depth + 1, q, best, best_dist);
+        if (fabs(delta) < best_dist) ref_nn(hi, n_hi, depth + 1, q, best, best_dist);
+    } else {
+        ref_nn(hi, n_hi, depth + 1, q, best, best_dist);
+        if (fabs(delta) < best_dist) ref_nn(lo, n_lo, depth + 1, q, best, best_dist);
+    }
+}
+
+// After a match launched with the tie list: re-answers the listed queries against `map` (the map that launch searched)
+// and rewrites their entries of d_nn_idx on the context's stream.  nn_dist needs no change: the reference's minimum is
+// the device's.  Synchronises the stream once (twice when something is listed).
+static double now_us();
+static int resolve_ties(nav_ctx *c, const RowMap &map, int *d_nn_idx, const char *name) {
+    CU(cudaMemcpyAsync(c->h_small, c->d_tie_count, 4, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    const size_t n = (size_t)(unsigned)c->h_small[0];
+    if (n == 0) return 0;
+    if (n > c->ntot) return fail("%s: tie list overflow (%zu records for %zu pixels)", name, n, c->ntot);
+    double t[4] = {c->prof ? now_us() : 0.0, 0.0, 0.0, 0.0};
+    const size_t cols = (size_t)c->cols, n_chunks = (size_t)map.n_chunks;
+    std::vector<TieRec> rec(n);
+    CU(cudaMemcpyAsync(rec.data(), c->d_tie_rec, n * sizeof(TieRec), cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    // the searched rows the list names, in order; records grouped by row (stable: the list order is the device's)
+    std::stable_sort(rec.begin(), rec.end(), [&](const TieRec &a, const TieRec &b) {
+        return a.px / (long long)cols < b.px / (long long)cols;
+    });
+    std::vector<long long> rids;
+    for (const TieRec &r : rec)
+        if (rids.empty() || rids.back() != r.px / (long long)cols) rids.push_back(r.px / (long long)cols);
+    std::vector<nav_point> row_pts(rids.size() * cols);
+    std::vector<unsigned> row_mask(rids.size() * n_chunks);
+    for (size_t i = 0; i < rids.size(); ++i) {
+        CU(cudaMemcpyAsync(&row_pts[i * cols], map.pts + rids[i] * cols * 3, cols * 24, cudaMemcpyDeviceToHost, c->stream));
+        CU(cudaMemcpyAsync(&row_mask[i * n_chunks], map.mask + rids[i] * n_chunks, n_chunks * 4, cudaMemcpyDeviceToHost,
+                           c->stream));
+    }
+    CU(cudaStreamSynchronize(c->stream));
+    if (c->prof) t[1] = now_us();
+    std::vector<int2> fix(n);
+    std::vector<nav_point> flat(cols), tree(cols);
+    std::vector<int> flat_col(cols);
+    size_t k = 0;
+    for (size_t i = 0; i < rids.size(); ++i) {
+        // flattenedPoints (src/slam.c:170-171): the row's labelled map points in column order, as k_flatten_row
+        // compacts them for nav_row_map_export
+        size_t m = 0;
+        for (size_t col = 0; col < cols; ++col)
+            if ((row_mask[i * n_chunks + col / kChunk] >> (col % kChunk)) & 1u) {
+                flat[m] = row_pts[i * cols + col];
+                flat_col[m++] = (int)col;
+            }
+        std::copy(flat.begin(), flat.begin() + m, tree.begin());  // the reference builds on a copy of the row
+        ref_build(tree.data(), m, 0);
+        const int row = (int)(rids[i] % c->rows);
+        for (; k < n && rec[k].px / (long long)cols == rids[i]; ++k) {
+            const nav_point q = {rec[k].q[0], rec[k].q[1], rec[k].q[2]};
+            nav_point near = {0.0, 0.0, 0.0};
+            double best = INFINITY;
+            ref_nn(tree.data(), m, 0, q, near, best);
+            // the new match: the lowest column whose map point is the returned xyz (as the oracle's row_query)
+            int col = -1;
+            for (size_t j = 0; j < m && col < 0; ++j)
+                if (flat[j].x == near.x && flat[j].y == near.y && flat[j].z == near.z) col = flat_col[j];
+            if (!(best < INFINITY) || col < 0)
+                return fail("%s: a tied query of row %lld found no map point in the reference search", name, rids[i]);
+#ifndef NDEBUG
+            // the reference's minimum is the device's sqrt(best), the smallest rounded distance of the row
+            double brute = INFINITY;
+            for (size_t j = 0; j < m; ++j) {
+                const double dx = flat[j].x - q.x, dy = flat[j].y - q.y, dz = flat[j].z - q.z;
+                brute = fmin(brute, sqrt(dx * dx + dy * dy + dz * dz));
+            }
+            assert(best == brute);
+#endif
+            fix[k] = make_int2((int)(rec[k].px), row * c->cols + col);
+        }
+    }
+    c->tie_resolved += n;
+    if (c->prof) t[2] = now_us();
+    // a pageable source: the copy has left `fix` when the call returns
+    CU(cudaMemcpyAsync(c->d_tie_fix, fix.data(), n * sizeof(int2), cudaMemcpyHostToDevice, c->stream));
+    launch_apply_tie_fix(c->d_tie_fix, (int)n, d_nn_idx, c->stream);
+    c->launches++;
+    if (c->prof) {
+        t[3] = now_us();
+        for (int i = 0; i < 3; ++i) c->tie_ms[i] += (t[i + 1] - t[i]) * 1e-3;
+        c->tie_calls++;
+    }
+    return 0;
+}
+
+static int refuse_ref_ties(const char *name) {
+    return fail("%s: not available under the reference tie rule (NAV_TIE_REFERENCE): this call runs without a host "
+                "round trip, and the rule resolves ties on the host; use the blocking calls, or the lowest-index rule",
+                name);
+}
+#define REFUSE_UNDER_REF_TIES(c, name) \
+    if ((c) && (c)->tie_rule == NAV_TIE_REFERENCE) return refuse_ref_ties(name);
+
 // labels (a3: fused into the match kernel, or already in d_labels) + queries (a7) + exact per-row NN (a6),
-// then the per-row dedupe (a8) producing the correspondence list and/or the per-row fit statistics
+// then the per-row dedupe (a8) producing the correspondence list and/or the per-row fit statistics.
+// ref_ties (fused labels only): the reference tie rule -- the tied queries are re-answered on the host before the
+// dedupe reads nn_idx (a blocking step).
 enum { kDedupeNone = 0, kDedupeCorr = 1, kDedupeStats = 2 };
-static void run_match(nav_ctx *c, const double *d_cloud, int *d_labels, bool fused_labels, const PoseBatch &poses,
-                      int dedupe, const FitMailbox *mail = nullptr) {
+static int run_match(nav_ctx *c, const double *d_cloud, int *d_labels, bool fused_labels, const PoseBatch &poses,
+                     int dedupe, const FitMailbox *mail = nullptr, const char *ref_ties = nullptr) {
     order_after_async(c);
     MatchOut out = {c->d_nn_idx, c->d_nn_dist, c->d_corr_rows, c->d_corr_row_count};
+    const TieList ties = {c->d_tie_rec, c->d_tie_count};
+    if (ref_ties) CU(cudaMemsetAsync(c->d_tie_count, 0, 4, c->stream));
     {
         ProfScope ps(c, &c->prof_match);
         launch_frame_match(d_cloud, d_labels, fused_labels, c->map, out, poses, c->n_seq, c->rows, c->cols,
-                           c->d_n_exact, c->stream);
+                           c->d_n_exact, c->stream, nullptr, nullptr, false, ref_ties ? &ties : nullptr);
         c->launches++;
     }
+    if (ref_ties && resolve_ties(c, c->map, c->d_nn_idx, ref_ties)) return 1;
     if (dedupe & kDedupeCorr) {
         launch_dedupe(d_cloud, d_labels, c->map, out, poses, c->n_seq, c->rows, c->cols, c->stream,
                       (dedupe & kDedupeStats) ? c->d_row_stats : nullptr, true);
@@ -624,24 +808,31 @@ static void run_match(nav_ctx *c, const double *d_cloud, int *d_labels, bool fus
                           false, mail);
         c->launches += 1;
     }
+    return 0;
 }
 
 static PoseBatch pose_batch(const nav_ctx *c, const nav_pos *pos, const nav_pos *last);
 
 // the whole front-end frame in ONE launch: labels (a3) + queries (a7) + exact per-row NN against the
 // current map (a6) + the next map from the final pose (a7, a4/a5) into the other map buffer
-static void run_frame_fused(nav_ctx *c, const double *d_cloud, int *d_labels, int *d_nn_idx, double *d_nn_dist,
-                            const nav_pos *pos_predict, const nav_pos *pos_last, const nav_pos *pos_final,
-                            bool pdl = false) {
+// ref_ties: the reference tie rule (blocking; see run_match)
+static int run_frame_fused(nav_ctx *c, const double *d_cloud, int *d_labels, int *d_nn_idx, double *d_nn_dist,
+                           const nav_pos *pos_predict, const nav_pos *pos_last, const nav_pos *pos_final,
+                           bool pdl = false, const char *ref_ties = nullptr) {
     MatchOut out = {d_nn_idx, d_nn_dist, c->d_corr_rows, c->d_corr_row_count};
     const PoseBatch loc = pose_batch(c, pos_predict, pos_last), fin = pose_batch(c, pos_final, nullptr);
+    const TieList ties = {c->d_tie_rec, c->d_tie_count};
+    if (ref_ties) CU(cudaMemsetAsync(c->d_tie_count, 0, 4, c->stream));
     {
         ProfScope ps(c, &c->prof_match);
         launch_frame_match(d_cloud, d_labels, true, c->map, out, loc, c->n_seq, c->rows, c->cols, c->d_n_exact,
-                           c->stream, &c->map_alt, &fin, pdl && !c->prof);
+                           c->stream, &c->map_alt, &fin, pdl && !c->prof, ref_ties ? &ties : nullptr);
     }
     c->launches++;
     std::swap(c->map, c->map_alt);
+    // the search read the map that is map_alt now
+    if (ref_ties && resolve_ties(c, c->map_alt, d_nn_idx, ref_ties)) return 1;
+    return 0;
 }
 
 static PoseBatch pose_batch(const nav_ctx *c, const nav_pos *pos, const nav_pos *last) {
@@ -772,7 +963,9 @@ extern "C" int nav_slam_match(nav_ctx *c, const nav_point *cloud, const nav_pos 
     if (c->stage.reserve(c->ntot * 24 + c->ntot * sizeof(nav_corr) + 1024, c->stream))
         return fail("nav_slam_match: staging");
     if (upload_cloud(c, cloud, "nav_slam_match")) return 1;
-    run_match(c, c->d_cloud, c->d_labels, true, pose_batch(c, pos_predict, pos_last), kDedupeCorr);
+    if (run_match(c, c->d_cloud, c->d_labels, true, pose_batch(c, pos_predict, pos_last), kDedupeCorr, nullptr,
+                  c->tie_rule == NAV_TIE_REFERENCE ? "nav_slam_match" : nullptr))
+        return 1;
     c->cloud_resident = true;
     c->cur_cloud = c->d_cloud;
     c->cur_labels = c->d_labels;
@@ -1020,7 +1213,7 @@ static int loc_fast_launch(nav_ctx *c, const nav_point *cloud, const nav_pos *po
     const FitMailbox mail = {c->h_fit, c->d_fit_ticket, ++c->fit_seq};
     if (ps) {
         CU(cudaStreamWaitEvent(c->stream, ps->ready, 0));
-        run_match(c, ps->d_cloud, ps->d_labels, false, poses, kDedupeStats, &mail);
+        if (run_match(c, ps->d_cloud, ps->d_labels, false, poses, kDedupeStats, &mail)) return 1;
         ps->pending = false;
         c->cur_pre = ps;
         c->cur_cloud = ps->d_cloud;
@@ -1029,7 +1222,7 @@ static int loc_fast_launch(nav_ctx *c, const nav_point *cloud, const nav_pos *po
         c->cur_pre = nullptr;
         if (c->stage.reserve(c->ntot * 24 + 1024, c->stream)) return fail("nav_slam_localization_fast: staging");
         if (upload_cloud(c, cloud, "nav_slam_localization_fast")) return 1;
-        run_match(c, c->d_cloud, c->d_labels, true, poses, kDedupeStats, &mail);
+        if (run_match(c, c->d_cloud, c->d_labels, true, poses, kDedupeStats, &mail)) return 1;
         c->cur_cloud = c->d_cloud;
         c->cur_labels = c->d_labels;
     }
@@ -1058,6 +1251,7 @@ extern "C" int nav_slam_localization_fast(nav_ctx *c, const nav_point *cloud, co
                                           const nav_pos *pos_last, nav_pos *pos_out, double *error_out,
                                           size_t *n_corr_out) {
     CTX_ENTER(c, "nav_slam_localization_fast");
+    REFUSE_UNDER_REF_TIES(c, "nav_slam_localization_fast");
     if (!pos_out) return fail("nav_slam_localization_fast: null argument");
     if (loc_fast_launch(c, cloud, pos_predict, pos_last)) return 1;
     return loc_fast_finish(c, pos_predict, pos_last, pos_out, error_out, n_corr_out);
@@ -1090,6 +1284,7 @@ extern "C" int nav_slam_run(nav_ctx *c, const void *const *frames, int n_frames,
                             nav_predict_fn predict, void *user, const nav_pos *deltas, const nav_pos *pos_start,
                             nav_pos *poses_out, double *error_out, size_t *n_corr_out) {
     CTX_ENTER(c, "nav_slam_run");
+    REFUSE_UNDER_REF_TIES(c, "nav_slam_run");
     if (!frames || n_frames < 0 || !pos_start || !poses_out || (!predict && !deltas))
         return fail("nav_slam_run: null argument");
     if (c->n_seq != 1) return fail("nav_slam_run: needs n_seq == 1");
@@ -1216,7 +1411,9 @@ extern "C" int nav_frontend_frame(nav_ctx *c, const nav_point *cloud, const nav_
     if (c->stage.reserve(c->ntot * (24 + 24 + 4 + 4 + 8) + 4096, c->stream)) return fail("nav_frontend_frame: staging");
     if (upload_cloud(c, cloud, "nav_frontend_frame")) return 1;
     order_after_async(c);
-    run_frame_fused(c, c->d_cloud, c->d_labels, c->d_nn_idx, c->d_nn_dist, pos_predict, pos_last, pos_final);
+    if (run_frame_fused(c, c->d_cloud, c->d_labels, c->d_nn_idx, c->d_nn_dist, pos_predict, pos_last, pos_final, false,
+                        c->tie_rule == NAV_TIE_REFERENCE ? "nav_frontend_frame" : nullptr))
+        return 1;
     c->cloud_resident = true;
     c->cur_cloud = c->d_cloud;
     c->cur_labels = c->d_labels;
@@ -1243,7 +1440,9 @@ extern "C" int nav_frontend_frame_depth(nav_ctx *c, const int *distances, const 
     launch_convert(c->d_dist, c->d_tan_col, c->d_tan_row, c->d_cloud, c->rows, c->cols, c->sm_count, c->stream);
     c->launches++;
     order_after_async(c);
-    run_frame_fused(c, c->d_cloud, c->d_labels, c->d_nn_idx, c->d_nn_dist, pos_predict, pos_last, pos_final);
+    if (run_frame_fused(c, c->d_cloud, c->d_labels, c->d_nn_idx, c->d_nn_dist, pos_predict, pos_last, pos_final, false,
+                        c->tie_rule == NAV_TIE_REFERENCE ? "nav_frontend_frame_depth" : nullptr))
+        return 1;
     c->cloud_resident = true;
     c->cur_cloud = c->d_cloud;
     c->cur_labels = c->d_labels;
@@ -1407,6 +1606,7 @@ static int async_setup(nav_ctx *c) {
 extern "C" int nav_frontend_submit(nav_ctx *c, const nav_frame_io *io, const nav_pos *pos_predict,
                                    const nav_pos *pos_last, const nav_pos *pos_final) {
     CTX_ENTER(c, "nav_frontend_submit");
+    REFUSE_UNDER_REF_TIES(c, "nav_frontend_submit");
     if (!io || !pos_predict || !pos_last || !pos_final) return fail("nav_frontend_submit: null argument");
     if (!io->cloud == !io->distances) return fail("nav_frontend_submit: give exactly one of cloud and distances");
     if (io->distances && c->n_seq != 1) return fail("nav_frontend_submit: depth input needs n_seq == 1");
@@ -1437,7 +1637,7 @@ extern "C" int nav_frontend_submit(nav_ctx *c, const nav_frame_io *io, const nav
         launch_convert(sl.d_depth, c->d_tan_col, c->d_tan_row, sl.d_cloud, c->rows, c->cols, c->sm_count, c->stream);
         c->launches++;
     }
-    run_frame_fused(c, sl.d_cloud, sl.d_labels, sl.d_nn_idx, sl.d_nn_dist, pos_predict, pos_last, pos_final);
+    if (run_frame_fused(c, sl.d_cloud, sl.d_labels, sl.d_nn_idx, sl.d_nn_dist, pos_predict, pos_last, pos_final)) return 1;
     CU(cudaEventRecord(sl.compute_done, c->stream));
     c->cloud_resident = false;
     c->async_synced = false;
@@ -1470,6 +1670,7 @@ extern "C" int nav_frontend_submit(nav_ctx *c, const nav_frame_io *io, const nav
 extern "C" int nav_frontend_frame_async(nav_ctx *c, const nav_point *cloud, const nav_pos *pos_predict,
                                         const nav_pos *pos_last, const nav_pos *pos_final, int *feature_out,
                                         int32_t *nn_idx_out, double *nn_dist_out, nav_point *global_out) {
+    REFUSE_UNDER_REF_TIES(c, "nav_frontend_frame_async");
     if (!cloud) return fail("nav_frontend_frame_async: null argument");
     nav_frame_io io = {};
     io.cloud = cloud;
@@ -1484,6 +1685,7 @@ extern "C" int nav_frontend_frame_depth_async(nav_ctx *c, const int *distances, 
                                               const nav_pos *pos_last, const nav_pos *pos_final, nav_point *cloud_out,
                                               int *feature_out, int32_t *nn_idx_out, double *nn_dist_out,
                                               nav_point *global_out) {
+    REFUSE_UNDER_REF_TIES(c, "nav_frontend_frame_depth_async");
     if (!distances) return fail("nav_frontend_frame_depth_async: null argument");
     nav_frame_io io = {};
     io.distances = distances;
@@ -1525,11 +1727,13 @@ extern "C" int nav_extract_feature_batch_dev(nav_ctx *c, const void *dev_clouds,
 extern "C" int nav_frontend_frame_dev(nav_ctx *c, const void *dev_cloud, const nav_pos *pos_predict,
                                       const nav_pos *pos_last, const nav_pos *pos_final) {
     CTX_ENTER(c, "nav_frontend_frame_dev");
+    REFUSE_UNDER_REF_TIES(c, "nav_frontend_frame_dev");
     if (!dev_cloud || !pos_predict || !pos_last || !pos_final) return fail("nav_frontend_frame_dev: null argument");
     if (!c->have_map) return fail("nav_frontend_frame_dev: call nav_slam_init_dev first");
     order_after_async(c);
-    run_frame_fused(c, (const double *)dev_cloud, c->d_labels, c->d_nn_idx, c->d_nn_dist, pos_predict, pos_last,
-                    pos_final);
+    if (run_frame_fused(c, (const double *)dev_cloud, c->d_labels, c->d_nn_idx, c->d_nn_dist, pos_predict, pos_last,
+                        pos_final))
+        return 1;
     c->cloud_resident = false;
     CU(cudaGetLastError());
     return 0;
@@ -1645,8 +1849,9 @@ static int frontend_sequence(nav_ctx *c, const char *name, const void *dev_frame
             // consecutive launches overlap (programmatic dependent launch): frame f+1 computes its labels
             // while frame f finishes its searches.  With per-frame outputs the copies and the dedupe of frame f
             // come between them, and the launches are ordinary.
-            run_frame_fused(c, cl, c->d_labels, c->d_nn_idx, c->d_nn_dist, pos_predict + o, pos_last + o, pos_final + o,
-                            /*pdl=*/!so);
+            if (run_frame_fused(c, cl, c->d_labels, c->d_nn_idx, c->d_nn_dist, pos_predict + o, pos_last + o, pos_final + o,
+                                /*pdl=*/!so))
+                return 1;
             if (!so) continue;
             // frame f's results while the context holds them: the map just built carries its label masks, and
             // the map it searched (now map_alt) is intact until the next frame's kernel
@@ -1687,6 +1892,7 @@ extern "C" int nav_frontend_sequence_dev(nav_ctx *c, const void *dev_frames, siz
                                          const nav_pos *pos_predict, const nav_pos *pos_last,
                                          const nav_pos *pos_final) {
     CTX_ENTER(c, "nav_frontend_sequence_dev");
+    REFUSE_UNDER_REF_TIES(c, "nav_frontend_sequence_dev");
     return frontend_sequence(c, "nav_frontend_sequence_dev", dev_frames, n_frames, pos_predict, pos_last, pos_final,
                              nullptr);
 }
@@ -1695,6 +1901,7 @@ extern "C" int nav_frontend_sequence_out_dev(nav_ctx *c, const void *dev_frames,
                                              const nav_pos *pos_predict, const nav_pos *pos_last,
                                              const nav_pos *pos_final, const nav_sequence_out *out) {
     CTX_ENTER(c, "nav_frontend_sequence_out_dev");
+    REFUSE_UNDER_REF_TIES(c, "nav_frontend_sequence_out_dev");
     return frontend_sequence(c, "nav_frontend_sequence_out_dev", dev_frames, n_frames, pos_predict, pos_last, pos_final,
                              out);
 }
@@ -1731,6 +1938,33 @@ extern "C" int nav_row_map_export(nav_ctx *c, int seq, int row, nav_point *pts_o
     *n_out = (size_t)n;
     return 0;
 }
+
+extern "C" int nav_set_tie_rule(nav_ctx *c, int rule) {
+    CTX_ENTER(c, "nav_set_tie_rule");
+    if (rule != NAV_TIE_LOWEST_INDEX && rule != NAV_TIE_REFERENCE)
+        return fail("nav_set_tie_rule: unknown tie rule %d (NAV_TIE_LOWEST_INDEX = 0, NAV_TIE_REFERENCE = 1)", rule);
+    if (rule == NAV_TIE_REFERENCE && !c->d_tie_rec) {  // one record per pixel: the list cannot overflow
+        TieRec *rec = nullptr;
+        unsigned *count = nullptr;
+        int2 *fix = nullptr;
+        if (cudaMalloc((void **)&rec, c->ntot * sizeof(TieRec)) != cudaSuccess ||
+            cudaMalloc((void **)&count, 4) != cudaSuccess || cudaMalloc((void **)&fix, c->ntot * sizeof(int2)) != cudaSuccess) {
+            cudaGetLastError();
+            for (void *p : {(void *)rec, (void *)count, (void *)fix})
+                if (p) cudaFree(p);
+            return fail("nav_set_tie_rule: cudaMalloc of the tie list (%zu records) failed", c->ntot);
+        }
+        c->d_tie_rec = rec;
+        c->d_tie_count = count;
+        c->d_tie_fix = fix;
+    }
+    c->tie_rule = rule;
+    return 0;
+}
+
+extern "C" int nav_tie_rule(const nav_ctx *c) { return c ? c->tie_rule : NAV_TIE_LOWEST_INDEX; }
+
+extern "C" uint64_t nav_tie_resolve_count(const nav_ctx *c) { return c ? c->tie_resolved : 0; }
 
 extern "C" uint64_t nav_exact_fallback_count(nav_ctx *c) {
     if (!c) return 0;

@@ -67,12 +67,26 @@ int configure_row_kernels(int cols);  // opt in to large dynamic shared memory; 
 
 void launch_frame_map(const double *cloud, const int *labels, const RowMap &map, const PoseBatch &poses,
                       int n_seq, int rows, int cols, cudaStream_t stream);
+// The queries of a frame search whose smallest rounded distance sqrt(dsq) is reached by at least two map points
+// of the row (the reference tie rule resolves them on the host): one record per query, appended in any order.
+struct TieRec {
+    long long px;  // flat pixel (sequence * rows + row) * cols + column
+    double q[3];   // the query exactly as the search used it
+};
+struct TieList {
+    TieRec *rec;      // capacity: one record per pixel of the context
+    unsigned *count;  // zeroed before the launch
+};
+
 // map_next/final_poses non-null: the kernel also builds the next map (frame transformed with its final
-// pose) into *map_next, which must be a different buffer than `map`
+// pose) into *map_next, which must be a different buffer than `map`.  ties non-null (fused labels only): the
+// search also lists its tied queries there.
 void launch_frame_match(const double *cloud, int *labels, bool fused_labels, const RowMap &map,
                         const MatchOut &out, const PoseBatch &poses, int n_seq, int rows, int cols,
                         unsigned *n_exact, cudaStream_t stream, const RowMap *map_next = nullptr,
-                        const PoseBatch *final_poses = nullptr, bool pdl = false);
+                        const PoseBatch *final_poses = nullptr, bool pdl = false, const TieList *ties = nullptr);
+// nn_idx[fix[i].x] = fix[i].y for i < n (the host's answers for tied queries)
+void launch_apply_tie_fix(const int2 *fix, int n, int *nn_idx, cudaStream_t stream);
 // row_stats (optional): [n_seq*rows][5] per-row {n, sum r (3), sum |r|^2} of the deduped correspondences;
 // write_corr = false skips the correspondence entries themselves
 void launch_dedupe(const double *cloud, const int *labels, const RowMap &map, const MatchOut &out,

@@ -177,14 +177,20 @@ __device__ __forceinline__ int block_excl_count(bool pred, int *s_warp, int &tot
 // the block (shared-memory copy for the CTA's own neighbourhood, global memory otherwise).  Four
 // candidates are loaded before any arithmetic so that their load latencies overlap; a short last
 // group repeats its final candidate, which the lexicographic compare ignores.
+// kRefTies: best2 also tracks the second smallest dsq over the scanned columns (each column counts once, so two
+// columns with the same xyz both count; the repeated padding candidate does not).
+template <bool kRefTies = false>
 __device__ __forceinline__ void scan_leaf(const double *pts, unsigned mask, int col0, const P3 &q, double &best,
-                                          int &bcol) {
+                                          int &bcol, double &best2) {
     while (mask) {
         int b[4];
+        bool real[4];  // kRefTies: false for the padding repeats of a short last group
         b[0] = __ffs(mask) - 1;
+        real[0] = true;
         mask &= mask - 1;
 #pragma unroll
         for (int i = 1; i < 4; ++i) {
+            real[i] = mask != 0;
             b[i] = mask ? __ffs(mask) - 1 : b[i - 1];
             mask &= mask - 1;  // 0 & anything stays 0
         }
@@ -202,8 +208,11 @@ __device__ __forceinline__ void scan_leaf(const double *pts, unsigned mask, int 
             const double d = dsq3(dsub(x[i], q.x), dsub(y[i], q.y), dsub(z[i], q.z));
             const int col = col0 + b[i];
             if (d < best || (d == best && col < bcol)) {
+                if (kRefTies) best2 = best;
                 best = d;
                 bcol = col;
+            } else if (kRefTies && real[i]) {
+                best2 = fmin(best2, d);
             }
         }
     }
@@ -295,9 +304,17 @@ __device__ __forceinline__ void prefetch_neighbourhood(MapSmem &sm, const RowVie
 
 // exact nearest labelled map point of the row for query q of column qc: seed leaf, its neighbours, then the
 // box hierarchy.  best = smallest dsq (INFINITY if the row map is empty), bcol = its column (lowest on ties).
-template <bool kCoherent>
+// kRefTies: *best2_out = the second smallest dsq over the scanned columns (scan_leaf).  The pruning needs no change
+// for it to see every column whose rounded distance sqrt(dsq) equals sqrt(best): two doubles with the same correctly
+// rounded square root differ by a factor of at most (1 + 2^-51), so such a column has dsq <= (1 + 2^-51) * best, and
+// no float lies strictly between best_up = float_round_up(best) and that dsq.  A leaf's fp32 lower bound is a float
+// <= the dsq of each of its points (box_lower_bound32), hence <= best_up, and the leaf is scanned.  best_up only
+// decreases towards its final value, so this holds for every test made along the way: the warp-cooperative cull
+// (wbest >= the lane's best_up, and the warp's bound is below the lane's), the per-lane super-box path of rows wider
+// than 2048 columns and the neighbour leaves alike; while best_up is +inf nothing is pruned.
+template <bool kCoherent, bool kRefTies = false>
 __device__ __forceinline__ void search_row(const MapSmem &sm, const RowView &rv, int qc, const P3 &q, double &best,
-                                           int &bcol, unsigned wmask) {
+                                           int &bcol, unsigned wmask, double *best2_out = nullptr) {
     const double *m_pts = rv.pts;
     const unsigned *m_mask = rv.mask;
     const float4 *m_box = rv.box, *m_sbox = rv.sbox;
@@ -308,8 +325,10 @@ __device__ __forceinline__ void search_row(const MapSmem &sm, const RowView &rv,
     best = INFINITY;
     float best_up = INFINITY;  // float(best) rounded up
     bcol = -1;
+    double &b2 = kRefTies ? *best2_out : best;  // kRefTies only (scan_leaf<false> never touches it)
+    if (kRefTies) b2 = INFINITY;
     const int seed = qc / kChunk;
-    scan_leaf(sm.pts + (seed - leaf0) * kChunk * 3, sm.mask[seed - leaf0], seed * kChunk, q, best, bcol);
+    scan_leaf<kRefTies>(sm.pts + (seed - leaf0) * kChunk * 3, sm.mask[seed - leaf0], seed * kChunk, q, best, bcol, b2);
     best_up = __double2float_ru(best);
     // The leaves next to the seed come first, addressed RELATIVE to the seed: the lanes of a warp hold
     // queries of neighbouring columns with different seeds, and stepping through "seed-1, seed+1, ..."
@@ -333,9 +352,9 @@ __device__ __forceinline__ void search_row(const MapSmem &sm, const RowView &rv,
             const float4 bhi = row_in_smem ? sm.rbox[lf * 2 + 1] : (near_leaf ? sm.box[j * 2 + 1] : ld_map<kCoherent>(m_box + lf * 2 + 1));
             if (box_lower_bound32(blo, bhi, q32) > best_up) continue;
             if (near_leaf)
-                scan_leaf(sm.pts + j * kChunk * 3, sm.mask[j], lf * kChunk, q, best, bcol);
+                scan_leaf<kRefTies>(sm.pts + j * kChunk * 3, sm.mask[j], lf * kChunk, q, best, bcol, b2);
             else
-                scan_leaf(m_pts + (long long)lf * kChunk * 3, ld_map<kCoherent>(m_mask + lf), lf * kChunk, q, best, bcol);
+                scan_leaf<kRefTies>(m_pts + (long long)lf * kChunk * 3, ld_map<kCoherent>(m_mask + lf), lf * kChunk, q, best, bcol, b2);
             best_up = __double2float_ru(best);
         }
     }
@@ -391,13 +410,13 @@ __device__ __forceinline__ void search_row(const MapSmem &sm, const RowView &rv,
                 own &= own - 1;
                 if (box_lower_bound32(sm.rbox[lf * 2], sm.rbox[lf * 2 + 1], q32) > best_up) continue;
                 if (j >= 0 && j < kNbLeaves)
-                    scan_leaf(sm.pts + j * kChunk * 3, sm.mask[j], lf * kChunk, q, best, bcol);
+                    scan_leaf<kRefTies>(sm.pts + j * kChunk * 3, sm.mask[j], lf * kChunk, q, best, bcol, b2);
                 else
-                    scan_leaf(m_pts + (long long)lf * kChunk * 3, ld_map<kCoherent>(m_mask + lf), lf * kChunk, q, best, bcol);
+                    scan_leaf<kRefTies>(m_pts + (long long)lf * kChunk * 3, ld_map<kCoherent>(m_mask + lf), lf * kChunk, q, best, bcol, b2);
                 best_up = __double2float_ru(best);
             }
         }
-        return;
+        return;  // b2 lives in *best2_out
     }
     for (int sc = 0; sc < n_sup; ++sc) {
         const float4 slo = sup_in_smem ? sm.sbox[sc * 2] : ld_map<kCoherent>(m_sbox + sc * 2);
@@ -433,9 +452,9 @@ __device__ __forceinline__ void search_row(const MapSmem &sm, const RowView &rv,
                 pass &= pass - 1;
                 if (box_lower_bound32(sm.rbox[lf * 2], sm.rbox[lf * 2 + 1], q32) > best_up) continue;
                 if (j >= 0 && j < kNbLeaves)
-                    scan_leaf(sm.pts + j * kChunk * 3, sm.mask[j], lf * kChunk, q, best, bcol);
+                    scan_leaf<kRefTies>(sm.pts + j * kChunk * 3, sm.mask[j], lf * kChunk, q, best, bcol, b2);
                 else
-                    scan_leaf(m_pts + (long long)lf * kChunk * 3, ld_map<kCoherent>(m_mask + lf), lf * kChunk, q, best, bcol);
+                    scan_leaf<kRefTies>(m_pts + (long long)lf * kChunk * 3, ld_map<kCoherent>(m_mask + lf), lf * kChunk, q, best, bcol, b2);
                 best_up = __double2float_ru(best);
             }
             continue;
@@ -448,9 +467,9 @@ __device__ __forceinline__ void search_row(const MapSmem &sm, const RowView &rv,
             const float4 bhi = near_leaf ? sm.box[j * 2 + 1] : ld_map<kCoherent>(m_box + lf * 2 + 1);
             if (box_lower_bound32(blo, bhi, q32) > best_up) continue;
             if (near_leaf)
-                scan_leaf(sm.pts + j * kChunk * 3, sm.mask[j], lf * kChunk, q, best, bcol);
+                scan_leaf<kRefTies>(sm.pts + j * kChunk * 3, sm.mask[j], lf * kChunk, q, best, bcol, b2);
             else
-                scan_leaf(m_pts + (long long)lf * kChunk * 3, ld_map<kCoherent>(m_mask + lf), lf * kChunk, q, best, bcol);
+                scan_leaf<kRefTies>(m_pts + (long long)lf * kChunk * 3, ld_map<kCoherent>(m_mask + lf), lf * kChunk, q, best, bcol, b2);
             best_up = __double2float_ru(best);
         }
     }
@@ -460,12 +479,14 @@ __device__ __forceinline__ void search_row(const MapSmem &sm, const RowView &rv,
 // otherwise read them from `labels`.  kFuseMap: also build the NEXT map (this frame transformed with
 // its final pose) into map_next -- a second buffer, because neighbouring CTAs are still searching the
 // current one -- which makes the whole front-end frame a single launch.
-template <bool kFusedLabels, bool kFuseMap>
+// kRefTies: the reference tie rule's variant -- every query whose smallest rounded distance is reached by at least
+// two map points of the row is appended to `ties` (the host re-answers it with the reference's own search).
+template <bool kFusedLabels, bool kFuseMap, bool kRefTies = false>
 __global__ void __launch_bounds__(kTile, NAV_MATCH_MIN_CTAS)
 k_frame_match(const double *__restrict__ cloud, int *__restrict__ labels, RowMap map, MatchOut out,
               const __grid_constant__ PoseBatch poses, int rows, int cols, int tiles_per_row,
               unsigned *__restrict__ n_exact, RowMap map_next, const __grid_constant__ PoseBatch final_poses,
-              int pdl) {
+              int pdl, TieList ties) {
     __shared__ StencilSmem s;
     // grid = (tiles per row, rows, sequences): no integer divisions to find the tile
     const int tile = blockIdx.x, row = blockIdx.y, seq = blockIdx.z;
@@ -549,9 +570,28 @@ k_frame_match(const double *__restrict__ cloud, int *__restrict__ labels, RowMap
     }
     const PoseXf &pose = poses.p[seq];
     const P3 q = shift_point(pose, xf_point(pose, p));
-    double best;
+    double best, best2;
     int bcol;
-    search_row<false>(sm, rv, qc, q, best, bcol, kFull);
+    search_row<false, kRefTies>(sm, rv, qc, q, best, bcol, kFull, kRefTies ? &best2 : nullptr);
+    if (kRefTies) {
+        // tied: at least two map columns at the smallest rounded distance (exact duplicates included: they resolve
+        // to the same answer).  The spare lanes repeat a query and append nothing; one atomic per warp.
+        const bool tied = has_query && bcol >= 0 && __dsqrt_rn(best2) == __dsqrt_rn(best);
+        const unsigned m = __ballot_sync(kFull, tied);
+        if (m) {
+            const unsigned lane = threadIdx.x & 31u;
+            unsigned first = 0;
+            if (lane == 0) first = atomicAdd(ties.count, (unsigned)__popc(m));
+            first = __shfl_sync(kFull, first, 0);
+            if (tied) {
+                TieRec *r = ties.rec + first + __popc(m & ((1u << lane) - 1u));
+                r->px = base + qc;
+                r->q[0] = q.x;
+                r->q[1] = q.y;
+                r->q[2] = q.z;
+            }
+        }
+    }
     if (!has_query) return;
     out.nn_idx[base + qc] = bcol >= 0 ? row * cols + bcol : -1;
     out.nn_dist[base + qc] = bcol >= 0 ? __dsqrt_rn(best) : INFINITY;
@@ -569,10 +609,11 @@ void launch_frame_map(const double *cloud, const int *labels, const RowMap &map,
     k_frame_map<<<n_seq * rows * tiles, kTile, 0, stream>>>(cloud, labels, map, poses, rows, cols, tiles);
 }
 
-template <bool kFusedLabels, bool kFuseMap>
+template <bool kFusedLabels, bool kFuseMap, bool kRefTies = false>
 static void launch_match_variant(int grid, cudaStream_t stream, bool pdl, const double *cloud, int *labels,
                                  const RowMap &map, const MatchOut &out, const PoseBatch &poses, int rows, int cols,
-                                 int tiles, unsigned *n_exact, const RowMap &map_next, const PoseBatch &final_poses) {
+                                 int tiles, unsigned *n_exact, const RowMap &map_next, const PoseBatch &final_poses,
+                                 const TieList &ties = TieList{nullptr, nullptr}) {
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)tiles, (unsigned)rows, (unsigned)(grid / (tiles * rows)));
     cfg.blockDim = dim3(kTile);
@@ -582,8 +623,8 @@ static void launch_match_variant(int grid, cudaStream_t stream, bool pdl, const 
     attr.val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = &attr;
     cfg.numAttrs = pdl ? 1 : 0;
-    cudaLaunchKernelEx(&cfg, k_frame_match<kFusedLabels, kFuseMap>, cloud, labels, map, out, poses, rows, cols, tiles,
-                       n_exact, map_next, final_poses, pdl ? 1 : 0);
+    cudaLaunchKernelEx(&cfg, k_frame_match<kFusedLabels, kFuseMap, kRefTies>, cloud, labels, map, out, poses, rows, cols,
+                       tiles, n_exact, map_next, final_poses, pdl ? 1 : 0, ties);
 }
 
 // pdl: launch with programmatic stream serialisation, so that consecutive frame launches on one stream
@@ -593,11 +634,20 @@ static void launch_match_variant(int grid, cudaStream_t stream, bool pdl, const 
 void launch_frame_match(const double *cloud, int *labels, bool fused_labels, const RowMap &map,
                         const MatchOut &out, const PoseBatch &poses, int n_seq, int rows, int cols,
                         unsigned *n_exact, cudaStream_t stream, const RowMap *map_next,
-                        const PoseBatch *final_poses, bool pdl) {
+                        const PoseBatch *final_poses, bool pdl, const TieList *ties) {
     const int tiles = div_up(cols, kTile);
     const int grid = n_seq * rows * tiles;
     // programmatic serialisation only on ordinary streams (not the legacy / per-thread default streams)
     pdl = pdl && stream != nullptr && stream != cudaStreamLegacy && stream != cudaStreamPerThread;
+    if (ties) {  // the reference tie rule: the two forms of the blocking calls (labels fused, map fused or not)
+        if (map_next && final_poses)
+            launch_match_variant<true, true, true>(grid, stream, pdl, cloud, labels, map, out, poses, rows, cols, tiles,
+                                                   n_exact, *map_next, *final_poses, *ties);
+        else
+            launch_match_variant<true, false, true>(grid, stream, pdl, cloud, labels, map, out, poses, rows, cols, tiles,
+                                                    n_exact, map, poses, *ties);
+        return;
+    }
     if (map_next && final_poses) {
         if (fused_labels)
             launch_match_variant<true, true>(grid, stream, pdl, cloud, labels, map, out, poses, rows, cols, tiles,
@@ -1350,6 +1400,15 @@ __global__ void k_gather_corr(const nav_corr *__restrict__ corr_rows, const int 
     const double *src = (const double *)(corr_rows + (long long)rid * cols);
     double *dst = (double *)(corr_out + (long long)seq * rows * cols + s_off);
     for (int i = threadIdx.x; i < n * 7; i += blockDim.x) dst[i] = src[i];
+}
+
+__global__ void k_apply_tie_fix(const int2 *__restrict__ fix, int n, int *__restrict__ nn_idx) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) nn_idx[fix[i].x] = fix[i].y;
+}
+
+void launch_apply_tie_fix(const int2 *fix, int n, int *nn_idx, cudaStream_t stream) {
+    k_apply_tie_fix<<<div_up(n, 256), 256, 0, stream>>>(fix, n, nn_idx);
 }
 
 void launch_gather_corr(const nav_corr *corr_rows, const int *corr_row_count, nav_corr *corr_out,

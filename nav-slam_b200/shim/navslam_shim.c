@@ -88,11 +88,28 @@ static void die(const char *what) {
     abort();
 }
 
-static nav_ctx *default_ctx(void) {
-    if (!g_default_ctx) {
-        g_default_ctx = nav_create(MAX_ROWS, MAX_COLS, 0, 1);
-        if (!g_default_ctx) die("nav_create");
+/* NAVSLAM_TIES=reference: every context the shim creates resolves exact distance ties as the reference does (the
+ * first tied point its per-row tree search reaches, NAV_TIE_REFERENCE) instead of by lowest index, so that
+ * integer-valued data gives the reference's correspondences, poses and CSV bit for bit.  Opt-in: it costs a host
+ * round trip per slam_localization, and the default output stays as it was. */
+static int ties_reference(void) {
+    static int v = -1;
+    if (v < 0) {
+        const char *e = getenv("NAVSLAM_TIES");
+        v = e && strcmp(e, "reference") == 0;
     }
+    return v;
+}
+
+static nav_ctx *new_ctx(void) {
+    nav_ctx *c = nav_create(MAX_ROWS, MAX_COLS, 0, 1);
+    if (!c) die("nav_create");
+    if (ties_reference() && nav_set_tie_rule(c, NAV_TIE_REFERENCE)) die("NAVSLAM_TIES=reference");
+    return c;
+}
+
+static nav_ctx *default_ctx(void) {
+    if (!g_default_ctx) g_default_ctx = new_ctx();
     return g_default_ctx;
 }
 
@@ -110,8 +127,7 @@ static int slot_of(SLAM_attr *attr, int create) {
         abort();
     }
     g_slots[free_slot].attr = attr;
-    g_slots[free_slot].ctx = nav_create(MAX_ROWS, MAX_COLS, 0, 1);
-    if (!g_slots[free_slot].ctx) die("nav_create");
+    g_slots[free_slot].ctx = new_ctx();
     static int at_exit_registered;
     if (!at_exit_registered) { /* after the first CUDA call, so that it runs before the runtime's own teardown */
         at_exit_registered = 1;
@@ -203,6 +219,12 @@ Pos slam_localization(SLAM_attr *attr, PointCloud *lidarPointCloud, Pos pos_pred
     if (fast < 0) {
         const char *e = getenv("NAVSLAM_ADAM");
         fast = e && strcmp(e, "stats") == 0;
+    }
+    if (fast && ties_reference()) {
+        fprintf(stderr, "navslam_shim(%dx%d): NAVSLAM_ADAM=stats cannot be combined with NAVSLAM_TIES=reference: the "
+                        "fit from device-reduced sums deduplicates on the device, the reference tie rule needs the "
+                        "host round trip of the default fit\n", MAX_ROWS, MAX_COLS);
+        abort();
     }
     if (fast) {
         if (nav_slam_localization_fast(g_slots[s].ctx, (const nav_point *)&lidarPointCloud->ToF_position[0][0],
