@@ -775,24 +775,32 @@ static int refuse_ref_ties(const char *name) {
 #define REFUSE_UNDER_REF_TIES(c, name) \
     if ((c) && (c)->tie_rule == NAV_TIE_REFERENCE) return refuse_ref_ties(name);
 
-// labels (a3: fused into the match kernel, or already in d_labels) + queries (a7) + exact per-row NN (a6),
-// then the per-row dedupe (a8) producing the correspondence list and/or the per-row fit statistics.
-// ref_ties (fused labels only): the reference tie rule -- the tied queries are re-answered on the host before the
-// dedupe reads nn_idx (a blocking step).
-enum { kDedupeNone = 0, kDedupeCorr = 1, kDedupeStats = 2 };
-static int run_match(nav_ctx *c, const double *d_cloud, int *d_labels, bool fused_labels, const PoseBatch &poses,
-                     int dedupe, const FitMailbox *mail = nullptr, const char *ref_ties = nullptr) {
-    order_after_async(c);
-    MatchOut out = {c->d_nn_idx, c->d_nn_dist, c->d_corr_rows, c->d_corr_row_count};
+// one match launch against c->map: labels (a3: fused into the match kernel, or already in d_labels) + queries (a7) +
+// exact per-row NN (a6).  fin != null: the next map from the final poses (a7, a4/a5) into c->map_alt, after which the
+// two maps change places.  ref_ties (the calling API's name; fused labels only): the reference tie rule -- the tied
+// queries are re-answered on the host against the map that was searched (a blocking step).
+static int run_frame_match(nav_ctx *c, const double *d_cloud, int *d_labels, bool fused_labels, const MatchOut &out,
+                           const PoseBatch &poses, const PoseBatch *fin, bool pdl, const char *ref_ties) {
     const TieList ties = {c->d_tie_rec, c->d_tie_count};
     if (ref_ties) CU(cudaMemsetAsync(c->d_tie_count, 0, 4, c->stream));
     {
         ProfScope ps(c, &c->prof_match);
         launch_frame_match(d_cloud, d_labels, fused_labels, c->map, out, poses, c->n_seq, c->rows, c->cols,
-                           c->d_n_exact, c->stream, nullptr, nullptr, false, ref_ties ? &ties : nullptr);
-        c->launches++;
+                           c->d_n_exact, c->stream, fin ? &c->map_alt : nullptr, fin, pdl, ref_ties ? &ties : nullptr);
     }
-    if (ref_ties && resolve_ties(c, c->map, c->d_nn_idx, ref_ties)) return 1;
+    c->launches++;
+    if (fin) std::swap(c->map, c->map_alt);  // the search read the map that is map_alt now
+    return ref_ties ? resolve_ties(c, fin ? c->map_alt : c->map, out.nn_idx, ref_ties) : 0;
+}
+
+// the match (run_frame_match), then the per-row dedupe (a8) producing the correspondence list and/or the per-row fit
+// statistics; under the reference tie rule the dedupe reads the host's answers
+enum { kDedupeNone = 0, kDedupeCorr = 1, kDedupeStats = 2 };
+static int run_match(nav_ctx *c, const double *d_cloud, int *d_labels, bool fused_labels, const PoseBatch &poses,
+                     int dedupe, const FitMailbox *mail = nullptr, const char *ref_ties = nullptr) {
+    order_after_async(c);
+    MatchOut out = {c->d_nn_idx, c->d_nn_dist, c->d_corr_rows, c->d_corr_row_count};
+    if (run_frame_match(c, d_cloud, d_labels, fused_labels, out, poses, nullptr, false, ref_ties)) return 1;
     if (dedupe & kDedupeCorr) {
         launch_dedupe(d_cloud, d_labels, c->map, out, poses, c->n_seq, c->rows, c->cols, c->stream,
                       (dedupe & kDedupeStats) ? c->d_row_stats : nullptr, true);
@@ -800,7 +808,7 @@ static int run_match(nav_ctx *c, const double *d_cloud, int *d_labels, bool fuse
                            c->cols, c->stream);
         c->launches += 2;
     } else if (dedupe & kDedupeStats) {
-        if (mail && c->n_seq == 1 && dedupe_stats_supported(c->cols))
+        if (mail && c->n_seq == 1 && row_cluster_supported(c->cols))
             launch_dedupe_stats(d_cloud, d_labels, c->map, out, poses, c->n_seq, c->rows, c->cols, c->stream,
                                 c->d_tile_stats, *mail);
         else
@@ -819,20 +827,9 @@ static PoseBatch pose_batch(const nav_ctx *c, const nav_pos *pos, const nav_pos 
 static int run_frame_fused(nav_ctx *c, const double *d_cloud, int *d_labels, int *d_nn_idx, double *d_nn_dist,
                            const nav_pos *pos_predict, const nav_pos *pos_last, const nav_pos *pos_final,
                            bool pdl = false, const char *ref_ties = nullptr) {
-    MatchOut out = {d_nn_idx, d_nn_dist, c->d_corr_rows, c->d_corr_row_count};
+    const MatchOut out = {d_nn_idx, d_nn_dist, c->d_corr_rows, c->d_corr_row_count};
     const PoseBatch loc = pose_batch(c, pos_predict, pos_last), fin = pose_batch(c, pos_final, nullptr);
-    const TieList ties = {c->d_tie_rec, c->d_tie_count};
-    if (ref_ties) CU(cudaMemsetAsync(c->d_tie_count, 0, 4, c->stream));
-    {
-        ProfScope ps(c, &c->prof_match);
-        launch_frame_match(d_cloud, d_labels, true, c->map, out, loc, c->n_seq, c->rows, c->cols, c->d_n_exact,
-                           c->stream, &c->map_alt, &fin, pdl && !c->prof, ref_ties ? &ties : nullptr);
-    }
-    c->launches++;
-    std::swap(c->map, c->map_alt);
-    // the search read the map that is map_alt now
-    if (ref_ties && resolve_ties(c, c->map_alt, d_nn_idx, ref_ties)) return 1;
-    return 0;
+    return run_frame_match(c, d_cloud, d_labels, true, out, loc, &fin, pdl && !c->prof, ref_ties);
 }
 
 static PoseBatch pose_batch(const nav_ctx *c, const nav_pos *pos, const nav_pos *last) {
@@ -922,6 +919,16 @@ extern "C" int nav_transform_cloud(nav_ctx *c, const nav_point *cloud, const nav
 }
 
 // ------------------------------------------------------------------ SLAM step ----------------
+// the frame nav_slam_mapping(pos, NULL, ...) maps from now on: the one in the context's own buffers, or (pre != null)
+// the prefetched frame of slot `pre`, which is then no longer waiting
+static void set_current_frame(nav_ctx *c, nav_ctx::PreSlot *pre = nullptr) {
+    if (pre) pre->pending = false;
+    c->cur_pre = pre;
+    c->cur_cloud = pre ? pre->d_cloud : c->d_cloud;
+    c->cur_labels = pre ? pre->d_labels : c->d_labels;
+    c->cloud_resident = true;
+}
+
 static int upload_cloud(nav_ctx *c, const nav_point *cloud, const char *name) {
     if (c->stage.h2d(c->d_cloud, cloud, c->ntot * 24, c->stream)) return fail("%s: H2D of the cloud failed", name);
     return 0;
@@ -935,9 +942,7 @@ extern "C" int nav_slam_init(nav_ctx *c, const nav_pos *pos, const nav_point *cl
     if (upload_cloud(c, cloud, "nav_slam_init")) return 1;
     run_labels(c, c->d_cloud, c->d_labels, nullptr, c->n_seq);
     run_map(c, c->d_cloud, c->d_labels, pose_batch(c, pos, nullptr));
-    c->cloud_resident = true;
-    c->cur_cloud = c->d_cloud;
-    c->cur_labels = c->d_labels;
+    set_current_frame(c);
     if (global_out && c->stage.d2h(global_out, c->map.pts, c->ntot * 24, c->stream))
         return fail("nav_slam_init: D2H");
     return finish_call(c, "nav_slam_init");
@@ -966,9 +971,7 @@ extern "C" int nav_slam_match(nav_ctx *c, const nav_point *cloud, const nav_pos 
     if (run_match(c, c->d_cloud, c->d_labels, true, pose_batch(c, pos_predict, pos_last), kDedupeCorr, nullptr,
                   c->tie_rule == NAV_TIE_REFERENCE ? "nav_slam_match" : nullptr))
         return 1;
-    c->cloud_resident = true;
-    c->cur_cloud = c->d_cloud;
-    c->cur_labels = c->d_labels;
+    set_current_frame(c);
     CU(cudaMemcpyAsync(c->h_small, c->d_corr_total, 4, cudaMemcpyDeviceToHost, c->stream));
     CU(cudaStreamSynchronize(c->stream));
     const size_t n = (size_t)c->h_small[0];
@@ -1214,19 +1217,12 @@ static int loc_fast_launch(nav_ctx *c, const nav_point *cloud, const nav_pos *po
     if (ps) {
         CU(cudaStreamWaitEvent(c->stream, ps->ready, 0));
         if (run_match(c, ps->d_cloud, ps->d_labels, false, poses, kDedupeStats, &mail)) return 1;
-        ps->pending = false;
-        c->cur_pre = ps;
-        c->cur_cloud = ps->d_cloud;
-        c->cur_labels = ps->d_labels;
     } else {
-        c->cur_pre = nullptr;
         if (c->stage.reserve(c->ntot * 24 + 1024, c->stream)) return fail("nav_slam_localization_fast: staging");
         if (upload_cloud(c, cloud, "nav_slam_localization_fast")) return 1;
         if (run_match(c, c->d_cloud, c->d_labels, true, poses, kDedupeStats, &mail)) return 1;
-        c->cur_cloud = c->d_cloud;
-        c->cur_labels = c->d_labels;
     }
-    c->cloud_resident = true;
+    set_current_frame(c, ps);
     CU(cudaGetLastError());
     if (c->trace) c->trace_us[1] += now_us() - t0;
     return 0;
@@ -1298,9 +1294,9 @@ extern "C" int nav_slam_run(nav_ctx *c, const void *const *frames, int n_frames,
     // the loop maps its own frames: a frame an earlier localization call left unmapped in a prefetch slot is
     // given up, so that the slot can be refilled
     if (n_frames > 0) c->cloud_resident = false;
-    // NAV_RUN_UNFUSED=1 keeps the three launches per frame (match, statistics dedupe, map) of the separate calls
-    static const bool unfused = getenv("NAV_RUN_UNFUSED") != nullptr;
-    const bool fused = !unfused && dedupe_stats_supported(c->cols);
+    // one launch per frame (k_loop_step) where a row fits one thread-block cluster; wider rows keep the three launches
+    // per frame (match, statistics dedupe, map) of the separate calls
+    const bool fused = row_cluster_supported(c->cols);
     nav_ctx::PreSlot *deferred = nullptr;  // fused: the frame whose map the next launch builds first
     static const bool want_trace = getenv("NAV_RUN_TRACE") != nullptr;
     c->trace = want_trace;
@@ -1342,11 +1338,7 @@ extern "C" int nav_slam_run(nav_ctx *c, const void *const *frames, int n_frames,
                 CU(cudaEventRecord(deferred->released, c->stream));
                 deferred->release_recorded = true;
             }
-            ps->pending = false;
-            c->cur_pre = ps;
-            c->cur_cloud = ps->d_cloud;
-            c->cur_labels = ps->d_labels;
-            c->cloud_resident = true;
+            set_current_frame(c, ps);
             deferred = ps;
             if (c->trace) c->trace_us[1] += now_us() - t0;
         } else if (loc_fast_launch(c, depth_input ? nullptr : (const nav_point *)frames[t], &pred, &last)) {
@@ -1381,9 +1373,7 @@ extern "C" int nav_slam_mapping(nav_ctx *c, const nav_pos *pos, const nav_point 
     if (cloud) {
         if (upload_cloud(c, cloud, "nav_slam_mapping")) return 1;
         run_labels(c, c->d_cloud, c->d_labels, nullptr, c->n_seq);
-        c->cloud_resident = true;
-        c->cur_cloud = c->d_cloud;
-        c->cur_labels = c->d_labels;
+        set_current_frame(c);
     } else if (!c->cloud_resident || !c->cur_cloud) {
         return fail("nav_slam_mapping: cloud == NULL but no cloud is resident from a preceding match");
     }
@@ -1402,58 +1392,55 @@ extern "C" int nav_slam_mapping(nav_ctx *c, const nav_pos *pos, const nav_point 
     return finish_call(c, "nav_slam_mapping");
 }
 
+// the blocking front-end frame from a host cloud, or (distances != null) from a depth matrix: L5 ingest fused with
+// the frame (SURVEY 8f #3, device part) -- the depth matrix (4 B/pixel instead of the 24 B/pixel cloud) is uploaded,
+// converted on the device (a2) and fed straight to the frame kernel; the converted lidar-frame cloud is returned only
+// if the caller asks for it (cloud_out)
+static int frontend_frame(nav_ctx *c, const char *name, const nav_point *cloud, const int *distances,
+                          const nav_pos *pos_predict, const nav_pos *pos_last, const nav_pos *pos_final,
+                          nav_point *cloud_out, int *feature_out, int32_t *nn_idx_out, double *nn_dist_out,
+                          nav_point *global_out) {
+    if ((!cloud && !distances) || !pos_predict || !pos_last || !pos_final) return fail("%s: null argument", name);
+    if (distances && c->n_seq != 1) return fail("%s: needs n_seq == 1", name);
+    if (!c->have_map) return fail("%s: call nav_slam_init first", name);
+    if (c->stage.reserve(c->ntot * ((distances ? 4 : 0) + 24 + 24 + 4 + 4 + 8) + 4096, c->stream))
+        return fail("%s: staging", name);
+    if (distances) {
+        if (c->stage.h2d(c->d_dist, distances, c->npx * 4, c->stream)) return fail("%s: H2D", name);
+        launch_convert(c->d_dist, c->d_tan_col, c->d_tan_row, c->d_cloud, c->rows, c->cols, c->sm_count, c->stream);
+        c->launches++;
+    } else if (upload_cloud(c, cloud, name)) {
+        return 1;
+    }
+    order_after_async(c);
+    if (run_frame_fused(c, c->d_cloud, c->d_labels, c->d_nn_idx, c->d_nn_dist, pos_predict, pos_last, pos_final, false,
+                        c->tie_rule == NAV_TIE_REFERENCE ? name : nullptr))
+        return 1;
+    set_current_frame(c);
+    if (cloud_out && c->stage.d2h(cloud_out, c->d_cloud, c->ntot * 24, c->stream)) return fail("%s: D2H", name);
+    if (feature_out && c->stage.d2h(feature_out, c->d_labels, c->ntot * 4, c->stream)) return fail("%s: D2H", name);
+    if (nn_idx_out && c->stage.d2h(nn_idx_out, c->d_nn_idx, c->ntot * 4, c->stream)) return fail("%s: D2H", name);
+    if (nn_dist_out && c->stage.d2h(nn_dist_out, c->d_nn_dist, c->ntot * 8, c->stream)) return fail("%s: D2H", name);
+    if (global_out && c->stage.d2h(global_out, c->map.pts, c->ntot * 24, c->stream)) return fail("%s: D2H", name);
+    return finish_call(c, name);
+}
+
 extern "C" int nav_frontend_frame(nav_ctx *c, const nav_point *cloud, const nav_pos *pos_predict,
                                   const nav_pos *pos_last, const nav_pos *pos_final, int *feature_out,
                                   int32_t *nn_idx_out, double *nn_dist_out, nav_point *global_out) {
     CTX_ENTER(c, "nav_frontend_frame");
-    if (!cloud || !pos_predict || !pos_last || !pos_final) return fail("nav_frontend_frame: null argument");
-    if (!c->have_map) return fail("nav_frontend_frame: call nav_slam_init first");
-    if (c->stage.reserve(c->ntot * (24 + 24 + 4 + 4 + 8) + 4096, c->stream)) return fail("nav_frontend_frame: staging");
-    if (upload_cloud(c, cloud, "nav_frontend_frame")) return 1;
-    order_after_async(c);
-    if (run_frame_fused(c, c->d_cloud, c->d_labels, c->d_nn_idx, c->d_nn_dist, pos_predict, pos_last, pos_final, false,
-                        c->tie_rule == NAV_TIE_REFERENCE ? "nav_frontend_frame" : nullptr))
-        return 1;
-    c->cloud_resident = true;
-    c->cur_cloud = c->d_cloud;
-    c->cur_labels = c->d_labels;
-    if (feature_out && c->stage.d2h(feature_out, c->d_labels, c->ntot * 4, c->stream)) return fail("nav_frontend_frame: D2H");
-    if (nn_idx_out && c->stage.d2h(nn_idx_out, c->d_nn_idx, c->ntot * 4, c->stream)) return fail("nav_frontend_frame: D2H");
-    if (nn_dist_out && c->stage.d2h(nn_dist_out, c->d_nn_dist, c->ntot * 8, c->stream)) return fail("nav_frontend_frame: D2H");
-    if (global_out && c->stage.d2h(global_out, c->map.pts, c->ntot * 24, c->stream)) return fail("nav_frontend_frame: D2H");
-    return finish_call(c, "nav_frontend_frame");
+    return frontend_frame(c, "nav_frontend_frame", cloud, nullptr, pos_predict, pos_last, pos_final, nullptr, feature_out,
+                          nn_idx_out, nn_dist_out, global_out);
 }
 
-// L5 ingest fused with the frame (SURVEY 8f #3, device part): the depth matrix (4 B/pixel instead of the
-// 24 B/pixel cloud) is uploaded, converted on the device (a2) and fed straight to the frame kernel;
-// the converted lidar-frame cloud is returned only if the caller asks for it.
 extern "C" int nav_frontend_frame_depth(nav_ctx *c, const int *distances, const nav_pos *pos_predict,
                                         const nav_pos *pos_last, const nav_pos *pos_final, nav_point *cloud_out,
                                         int *feature_out, int32_t *nn_idx_out, double *nn_dist_out,
                                         nav_point *global_out) {
     CTX_ENTER(c, "nav_frontend_frame_depth");
-    if (!distances || !pos_predict || !pos_last || !pos_final) return fail("nav_frontend_frame_depth: null argument");
-    if (c->n_seq != 1) return fail("nav_frontend_frame_depth: needs n_seq == 1");
-    if (!c->have_map) return fail("nav_frontend_frame_depth: call nav_slam_init first");
-    if (c->stage.reserve(c->ntot * (4 + 24 + 24 + 4 + 4 + 8) + 4096, c->stream)) return fail("nav_frontend_frame_depth: staging");
-    if (c->stage.h2d(c->d_dist, distances, c->npx * 4, c->stream)) return fail("nav_frontend_frame_depth: H2D");
-    launch_convert(c->d_dist, c->d_tan_col, c->d_tan_row, c->d_cloud, c->rows, c->cols, c->sm_count, c->stream);
-    c->launches++;
-    order_after_async(c);
-    if (run_frame_fused(c, c->d_cloud, c->d_labels, c->d_nn_idx, c->d_nn_dist, pos_predict, pos_last, pos_final, false,
-                        c->tie_rule == NAV_TIE_REFERENCE ? "nav_frontend_frame_depth" : nullptr))
-        return 1;
-    c->cloud_resident = true;
-    c->cur_cloud = c->d_cloud;
-    c->cur_labels = c->d_labels;
-    if (cloud_out && c->stage.d2h(cloud_out, c->d_cloud, c->ntot * 24, c->stream)) return fail("nav_frontend_frame_depth: D2H");
-    if (feature_out && c->stage.d2h(feature_out, c->d_labels, c->ntot * 4, c->stream)) return fail("nav_frontend_frame_depth: D2H");
-    if (nn_idx_out && c->stage.d2h(nn_idx_out, c->d_nn_idx, c->ntot * 4, c->stream)) return fail("nav_frontend_frame_depth: D2H");
-    if (nn_dist_out && c->stage.d2h(nn_dist_out, c->d_nn_dist, c->ntot * 8, c->stream)) return fail("nav_frontend_frame_depth: D2H");
-    if (global_out && c->stage.d2h(global_out, c->map.pts, c->ntot * 24, c->stream)) return fail("nav_frontend_frame_depth: D2H");
-    return finish_call(c, "nav_frontend_frame_depth");
+    return frontend_frame(c, "nav_frontend_frame_depth", nullptr, distances, pos_predict, pos_last, pos_final, cloud_out,
+                          feature_out, nn_idx_out, nn_dist_out, global_out);
 }
-
 
 // ------------------------------------------------------------------ CSV rows on the device ---
 // SURVEY 8f #4: the text of src/main.c:320-352 for one frame, produced where the global cloud lives.
@@ -1773,11 +1760,11 @@ static int frontend_sequence(nav_ctx *c, const char *name, const void *dev_frame
     // host to issue; several sequences side by side (n_seq > 1) fill the machine better as separate launches.
     static const bool per_frame = getenv("NAV_SEQ_LAUNCHES") != nullptr;
     const bool fused =
-        !per_frame && !c->prof && c->n_seq == 1 && n_frames > 1 && frame_seq_supported(c->cols) && n_frames <= 0x7fffffff;
+        !per_frame && !c->prof && c->n_seq == 1 && n_frames > 1 && row_cluster_supported(c->cols) && n_frames <= 0x7fffffff;
     // fit statistics: CTA partials per frame in scratch -- one per (row, tile) from k_frame_seq or k_dedupe_stats
     // (rows up to 2048 columns), one per row from k_dedupe_rows (wider rows) -- then one totals launch
     const size_t nr = (size_t)c->n_seq * c->rows;
-    const bool tile_parts = dedupe_stats_supported(c->cols);
+    const bool tile_parts = row_cluster_supported(c->cols);
     const size_t part_frame = tile_parts ? nr * div_up(c->cols, 256) : nr;  // partials per frame
     double *part = nullptr;
     if (so && so->fit_stats && n_frames > 0) {

@@ -41,10 +41,9 @@ struct FitMailbox {
 
 // a whole sequence of frames with known poses in one launch (one thread-block cluster per image row walks
 // through the frames); map0 is searched by frame 0, frame f builds the map for frame f+1 in the other buffer.
-// d_pose_loc / d_pose_fin: device arrays [n_frames][n_seq].  Needs frame_seq_supported(cols).
+// d_pose_loc / d_pose_fin: device arrays [n_frames][n_seq].  Needs row_cluster_supported(cols).
 // seq_out (optional): per-frame outputs -- slot f of every non-null ring receives frame f (nav_sequence_out), and
 // part != null adds the statistics dedupe, CTA partials [n_frames][n_seq*rows*tiles][5] for launch_seq_fit_totals.
-bool frame_seq_supported(int cols);
 int frame_seq_inline_frames();  // sequences up to this length (one sequence) carry their poses as kernel parameters
 struct SeqOut {
     unsigned *mask;   // [n_frames][n_seq*rows][n_chunks]
@@ -92,13 +91,15 @@ void launch_apply_tie_fix(const int2 *fix, int n, int *nn_idx, cudaStream_t stre
 void launch_dedupe(const double *cloud, const int *labels, const RowMap &map, const MatchOut &out,
                    const PoseBatch &poses, int n_seq, int rows, int cols, cudaStream_t stream,
                    double *row_stats = nullptr, bool write_corr = true, const FitMailbox *mail = nullptr);
+// whether the tiles of a row fit one thread-block cluster, as launch_frame_seq, launch_dedupe_stats and
+// launch_loop_step need (rows up to 2048 columns)
+bool row_cluster_supported(int cols);
 // statistics-only dedupe spread over the tiles of a row (thread-block cluster per row); part: [n_seq*rows*tiles][5]
-bool dedupe_stats_supported(int cols);
 int launch_dedupe_stats(const double *cloud, const int *labels, const RowMap &map, const MatchOut &out,
                         const PoseBatch &poses, int n_seq, int rows, int cols, cudaStream_t stream, double *part,
                         const FitMailbox &mail);
 // the closed-loop step in one launch: (do_map) map of the previous frame from prev_cloud / prev_labels /
-// prev_poses, match of this frame against it, statistics dedupe, mailbox post.  Needs dedupe_stats_supported(cols).
+// prev_poses, match of this frame against it, statistics dedupe, mailbox post.  Needs row_cluster_supported(cols).
 int launch_loop_step(const double *cloud, const int *labels, const RowMap &map, const MatchOut &out,
                      const PoseBatch &poses, int n_seq, int rows, int cols, cudaStream_t stream,
                      const double *prev_cloud, const int *prev_labels, const PoseBatch &prev_poses, bool do_map,

@@ -29,6 +29,8 @@
 #include <math.h>
 #include <stdlib.h>
 
+#include <utility>
+
 #include "nav_kernels.cuh"
 #include "stencil_tile.cuh"
 
@@ -270,6 +272,12 @@ struct RowView {
     int n_leaf, n_sup, leaf0;  // leaf0: first leaf of the CTA's shared-memory neighbourhood (may be -1)
 };
 
+// row rid (first pixel base = rid * cols) of `map`, as seen by the CTA of 256-column tile `tile`
+__device__ __forceinline__ RowView row_view(const RowMap &map, int rid, long long base, int tile) {
+    return {map.pts + base * 3, map.mask + (long long)rid * map.n_chunks, map.box + (long long)rid * map.n_chunks * 2,
+            map.sbox + (long long)rid * map.n_super * 2, map.n_chunks, map.n_super, tile * kChunksPerSuper - 1};
+}
+
 // map data outside the shared-memory neighbourhood: through the read-only path when the map was written by
 // an earlier launch, with ordinary (coherent) loads when this launch wrote it (k_loop_step)
 template <bool kCoherent, typename T>
@@ -475,6 +483,81 @@ __device__ __forceinline__ void search_row(const MapSmem &sm, const RowView &rv,
     }
 }
 
+// what the query of a thread found (the statistics dedupe of k_loop_step and k_frame_seq<kOut> starts from it)
+struct TileQuery {
+    int qc;                    // the query's column; -1 for a thread without a query
+    int key;                   // the column of its nearest map point; -1 for none (empty map row)
+    unsigned long long dbits;  // the bits of its nn_dist as stored (INFINITY when key is -1)
+    P3 ori;                    // the query point in the global frame, xf_point(pose, p), before the shift
+};
+
+// The match of one (row, 256-column tile) once its labels are known and the cp.async group of the map neighbourhood
+// has been waited for: nn_idx / nn_dist = -1 / -1.0 for the unlabelled columns; the labelled columns are compacted so
+// that the search runs on densely populated warps; each query -- point_at(t) of its column-in-tile t, transformed
+// with the pose pose_at() returns -- is searched in the row (search_row) and its nn_idx / nn_dist stored.  The pose
+// is taken where it is used: a reference passed in from the caller kept its parameter offset in a per-thread
+// register, and the pose reads of k_frame_match<fused labels, fused map> became per-thread constant loads (measured
+// 2.7 % slower per-frame launches on a B200).  Called by all kTile threads
+// (contains barriers).  Whole warps without a query skip the search; in the last warp with queries the spare lanes
+// repeat its last query, so that the warp-cooperative part of the search always runs with 32 lanes (they store
+// nothing).  kRefTies: every query whose smallest rounded distance is reached by at least two map points of the row
+// is also appended to `ties`.
+template <bool kCoherent, bool kRefTies, typename PointAt, typename PoseAt>
+__device__ __forceinline__ TileQuery match_tile(const MapSmem &sm, const RowView &rv, int *s_warp, int *s_qcol,
+                                                int label, PointAt point_at, PoseAt pose_at, const MatchOut &out,
+                                                long long base, int row, int cols, int c0, const TieList &ties) {
+    const int c = c0 + threadIdx.x;
+    if (c < cols && label != 1) {
+        out.nn_idx[base + c] = -1;
+        out.nn_dist[base + c] = -1.0;
+    }
+    int nq;
+    const int slot = block_excl_count(label == 1, s_warp, nq);  // its barriers also publish the prefetch
+    if (label == 1) s_qcol[slot] = threadIdx.x;
+    __syncthreads();
+    TileQuery m = {-1, -1, 0ull, {0, 0, 0}};
+    if ((int)(threadIdx.x & ~31u) < nq) {
+        const bool has_query = (int)threadIdx.x < nq;
+        const int t = s_qcol[min((int)threadIdx.x, nq - 1)];  // column-in-tile handled by this thread
+        const int qc = c0 + t;
+        const PoseXf &pose = pose_at();
+        const P3 ori = xf_point(pose, point_at(t));
+        const P3 q = shift_point(pose, ori);
+        double best, best2;
+        int bcol;
+        search_row<kCoherent, kRefTies>(sm, rv, qc, q, best, bcol, kFull, kRefTies ? &best2 : nullptr);
+        if (kRefTies) {
+            // tied: at least two map columns at the smallest rounded distance (exact duplicates included: they
+            // resolve to the same answer).  The spare lanes repeat a query and append nothing; one atomic per warp.
+            const bool tied = has_query && bcol >= 0 && __dsqrt_rn(best2) == __dsqrt_rn(best);
+            const unsigned tm = __ballot_sync(kFull, tied);
+            if (tm) {
+                const unsigned lane = threadIdx.x & 31u;
+                unsigned first = 0;
+                if (lane == 0) first = atomicAdd(ties.count, (unsigned)__popc(tm));
+                first = __shfl_sync(kFull, first, 0);
+                if (tied) {
+                    TieRec *r = ties.rec + first + __popc(tm & ((1u << lane) - 1u));
+                    r->px = base + qc;
+                    r->q[0] = q.x;
+                    r->q[1] = q.y;
+                    r->q[2] = q.z;
+                }
+            }
+        }
+        if (has_query) {
+            const double dist = bcol >= 0 ? __dsqrt_rn(best) : INFINITY;
+            out.nn_idx[base + qc] = bcol >= 0 ? row * cols + bcol : -1;
+            out.nn_dist[base + qc] = dist;
+            m.qc = qc;
+            m.key = bcol;
+            m.dbits = (unsigned long long)__double_as_longlong(dist);
+            m.ori = ori;
+        }
+    }
+    return m;
+}
+
 // grid as k_frame_map.  kFusedLabels: compute the labels of the tile here (and store them);
 // otherwise read them from `labels`.  kFuseMap: also build the NEXT map (this frame transformed with
 // its final pose) into map_next -- a second buffer, because neighbouring CTAs are still searching the
@@ -498,13 +581,7 @@ k_frame_match(const double *__restrict__ cloud, int *__restrict__ labels, RowMap
     __shared__ int s_warp[65];
     __shared__ int s_qcol[kTile];
     __shared__ MapSmem sm;
-    const double *m_pts = map.pts + base * 3;
-    const unsigned *m_mask = map.mask + (long long)rid * map.n_chunks;
-    const float4 *m_box = map.box + (long long)rid * map.n_chunks * 2;
-    const float4 *m_sbox = map.sbox + (long long)rid * map.n_super * 2;
-    const int n_leaf = map.n_chunks, n_sup = map.n_super;
-    const int leaf0 = tile * kChunksPerSuper - 1;  // first leaf of the prefetched neighbourhood (may be -1)
-    const RowView rv = {m_pts, m_mask, m_box, m_sbox, n_leaf, n_sup, leaf0};
+    const RowView rv = row_view(map, rid, base, tile);
     // asynchronous prefetch (cp.async) of the neighbourhood; consumed after the compaction
     auto prefetch_map = [&]() { prefetch_neighbourhood<false>(sm, rv, cols); };
     // Programmatic dependent launch (pdl != 0, kernel launched with the stream-serialisation attribute):
@@ -528,73 +605,21 @@ k_frame_match(const double *__restrict__ cloud, int *__restrict__ labels, RowMap
     } else {
         label = c < cols ? labels[base + c] : 0;
     }
-    if (c < cols && label != 1) {
-        out.nn_idx[base + c] = -1;
-        out.nn_dist[base + c] = -1.0;
-    }
+    // the lidar-frame point of column-in-tile t
+    auto point_at = [&](int t) {
+        if (kFusedLabels) {
+            const double *sp = s.pts + (t + kHalo) * 3;
+            return P3{sp[0], sp[1], sp[2]};
+        }
+        return ldg_p3(cloud + (base + (c0 + t)) * 3);
+    };
     if (kFuseMap) {  // a7 + a4/a5 for the next frame's search, into the other map buffer
         __shared__ float4 s_lo[kChunksPerSuper], s_hi[kChunksPerSuper];
-        P3 own = {0, 0, 0};
-        if (c < cols) {
-            if (kFusedLabels) {
-                const double *sp = s.pts + (threadIdx.x + kHalo) * 3;
-                own.x = sp[0];
-                own.y = sp[1];
-                own.z = sp[2];
-            } else {
-                own = ldg_p3(cloud + (base + c) * 3);
-            }
-        }
+        const P3 own = c < cols ? point_at(threadIdx.x) : P3{0, 0, 0};
         map_tile(label == 1, c < cols, own, final_poses.p[seq], map_next, rid, tile, c, base, s_lo, s_hi);
     }
-    // compact the labelled columns of the tile so that the search runs on densely populated warps
     cp_async_wait_all();
-    int nq;
-    const int slot = block_excl_count(label == 1, s_warp, nq);  // its barriers also publish the prefetch
-    if (label == 1) s_qcol[slot] = threadIdx.x;
-    __syncthreads();
-    // whole warps without a query leave; in the last warp with queries the spare lanes repeat its last query,
-    // so that the warp-cooperative part of the search always runs with 32 lanes (they store nothing)
-    if ((int)(threadIdx.x & ~31u) >= nq) return;
-    const bool has_query = (int)threadIdx.x < nq;
-    const int t = s_qcol[min((int)threadIdx.x, nq - 1)];  // column-in-tile handled by this thread
-    const int qc = c0 + t;
-    P3 p;
-    if (kFusedLabels) {
-        const double *sp = s.pts + (t + kHalo) * 3;
-        p.x = sp[0];
-        p.y = sp[1];
-        p.z = sp[2];
-    } else {
-        p = ldg_p3(cloud + (base + qc) * 3);
-    }
-    const PoseXf &pose = poses.p[seq];
-    const P3 q = shift_point(pose, xf_point(pose, p));
-    double best, best2;
-    int bcol;
-    search_row<false, kRefTies>(sm, rv, qc, q, best, bcol, kFull, kRefTies ? &best2 : nullptr);
-    if (kRefTies) {
-        // tied: at least two map columns at the smallest rounded distance (exact duplicates included: they resolve
-        // to the same answer).  The spare lanes repeat a query and append nothing; one atomic per warp.
-        const bool tied = has_query && bcol >= 0 && __dsqrt_rn(best2) == __dsqrt_rn(best);
-        const unsigned m = __ballot_sync(kFull, tied);
-        if (m) {
-            const unsigned lane = threadIdx.x & 31u;
-            unsigned first = 0;
-            if (lane == 0) first = atomicAdd(ties.count, (unsigned)__popc(m));
-            first = __shfl_sync(kFull, first, 0);
-            if (tied) {
-                TieRec *r = ties.rec + first + __popc(m & ((1u << lane) - 1u));
-                r->px = base + qc;
-                r->q[0] = q.x;
-                r->q[1] = q.y;
-                r->q[2] = q.z;
-            }
-        }
-    }
-    if (!has_query) return;
-    out.nn_idx[base + qc] = bcol >= 0 ? row * cols + bcol : -1;
-    out.nn_dist[base + qc] = bcol >= 0 ? __dsqrt_rn(best) : INFINITY;
+    match_tile<false, kRefTies>(sm, rv, s_warp, s_qcol, label, point_at, [&]() -> const PoseXf & { return poses.p[seq]; }, out, base, row, cols, c0, ties);
 }
 
 __device__ __forceinline__ void cluster_arrive_all() { asm volatile("barrier.cluster.arrive.release;" ::: "memory"); }
@@ -938,6 +963,38 @@ __device__ __forceinline__ void block_post_stats(StatsSmem &ss, bool winner, dou
     post_fit_totals<kTile>(part, (int)gridDim.x, mail, ss.tot);
 }
 
+// The statistics dedupe of a tile's search results (k_loop_step, k_frame_seq<kOut>): the winners of the cluster
+// dedupe, their residuals ori - nearest back into COLUMN order (thread = column, as in k_dedupe_stats) so that the
+// partial sums are formed in the same order and the totals are the same bits whichever kernel produced them, then
+// block_post_stats.  ori_at(t): the winner's ori, t = its column in the tile.  Called by all kTile threads of every
+// CTA of the row's cluster once the search is over; its point buffer sm.pts and the query list s_qcol are reused
+// (the cluster barriers are CTA barriers too).
+template <typename OriAt>
+__device__ __forceinline__ void tile_fit_stats(const TileQuery &m, OriAt ori_at, const double *__restrict__ map_pts,
+                                               long long base, int c0, MapSmem &sm, int *s_qcol,
+                                               unsigned long long *s_best, int *s_win, StatsSmem &ss,
+                                               double *__restrict__ part, const FitMailbox &mail) {
+    const bool winner = cluster_dedupe_winner(s_best, s_win, m.key, m.dbits, m.qc);
+    double *s_r = sm.pts;
+    int *s_flag = s_qcol;
+    s_flag[threadIdx.x] = 0;
+    __syncthreads();
+    if (winner) {
+        const int t = m.qc - c0;
+        const P3 ori = ori_at(t);
+        const double *np = map_pts + (base + m.key) * 3;
+        s_r[t * 3] = dsub(ori.x, np[0]);
+        s_r[t * 3 + 1] = dsub(ori.y, np[1]);
+        s_r[t * 3 + 2] = dsub(ori.z, np[2]);
+        s_flag[t] = 1;
+    }
+    __syncthreads();
+    const bool mine = s_flag[threadIdx.x] != 0;
+    const double rx = mine ? s_r[threadIdx.x * 3] : 0.0, ry = mine ? s_r[threadIdx.x * 3 + 1] : 0.0,
+                 rz = mine ? s_r[threadIdx.x * 3 + 2] : 0.0;
+    block_post_stats(ss, mine, rx, ry, rz, part, mail);
+}
+
 __global__ void __launch_bounds__(kTile)
 k_dedupe_stats(const double *__restrict__ cloud, const int *__restrict__ labels, RowMap map, MatchOut out,
                const __grid_constant__ PoseBatch poses, int rows, int cols, int tiles_per_row,
@@ -1006,74 +1063,23 @@ k_loop_step(const double *__restrict__ cloud, const int *__restrict__ labels, Ro
         map_tile(lab, c < cols, p, prev_poses.p[seq], map, rid, tile, c, base, s_lo, s_hi);
         cluster_sync_all();  // release / acquire: the row's new map is visible to all CTAs of its cluster
     }
-    const RowView rv = {map.pts + base * 3, map.mask + (long long)rid * map.n_chunks,
-                        map.box + (long long)rid * map.n_chunks * 2, map.sbox + (long long)rid * map.n_super * 2,
-                        map.n_chunks, map.n_super, tile * kChunksPerSuper - 1};
+    const RowView rv = row_view(map, rid, base, tile);
     prefetch_neighbourhood<true>(sm, rv, cols);
-    if (c < cols && label != 1) {
-        out.nn_idx[base + c] = -1;
-        out.nn_dist[base + c] = -1.0;
-    }
     cp_async_wait_all();
-    int nq;
-    const int slot = block_excl_count(label == 1, s_warp, nq);  // its barriers also publish the prefetch
-    if (label == 1) s_qcol[slot] = threadIdx.x;
-    __syncthreads();
-    int key = -1, qc = -1;
-    unsigned long long dbits = 0;
-    P3 ori = {0, 0, 0};
-    if ((int)(threadIdx.x & ~31u) < nq) {  // warps with at least one query; spare lanes repeat the last one
-        const bool has_query = (int)threadIdx.x < nq;
-        const int my_qc = c0 + s_qcol[min((int)threadIdx.x, nq - 1)];
-        const PoseXf &pose = poses.p[seq];
-        const P3 my_ori = xf_point(pose, load_p3(cloud + (base + my_qc) * 3));
-        const P3 q = shift_point(pose, my_ori);
-        double best;
-        int bcol;
-        search_row<true>(sm, rv, my_qc, q, best, bcol, kFull);
-        if (has_query) {
-            qc = my_qc;
-            ori = my_ori;
-            const double dist = bcol >= 0 ? __dsqrt_rn(best) : INFINITY;
-            out.nn_idx[base + qc] = bcol >= 0 ? row * cols + bcol : -1;
-            out.nn_dist[base + qc] = dist;
-            if (bcol >= 0) {
-                key = bcol;
-                dbits = (unsigned long long)__double_as_longlong(dist);
-            }
-        }
-    }
-    const bool winner = cluster_dedupe_winner(s_best, s_win, key, dbits, qc);
-    // residuals back into COLUMN order (thread = column, as in k_dedupe_stats), so that the partial sums are
-    // formed in the same order and the totals are the same bits whichever kernel produced them.  The search
-    // is over (the cluster barriers above were CTA barriers too): its point buffer is free.
-    double *s_r = sm.pts;
-    int *s_flag = s_qcol;
-    s_flag[threadIdx.x] = 0;
-    __syncthreads();
-    if (winner) {
-        const double *np = map.pts + (base + key) * 3;
-        const int t = qc - c0;
-        s_r[t * 3] = dsub(ori.x, np[0]);
-        s_r[t * 3 + 1] = dsub(ori.y, np[1]);
-        s_r[t * 3 + 2] = dsub(ori.z, np[2]);
-        s_flag[t] = 1;
-    }
-    __syncthreads();
-    const bool mine = s_flag[threadIdx.x] != 0;
-    const double rx = mine ? s_r[threadIdx.x * 3] : 0.0, ry = mine ? s_r[threadIdx.x * 3 + 1] : 0.0,
-                 rz = mine ? s_r[threadIdx.x * 3 + 2] : 0.0;
-    block_post_stats(ss, mine, rx, ry, rz, part, mail);
+    const TileQuery m = match_tile<true, false>(sm, rv, s_warp, s_qcol, label,
+                                                [&](int t) { return load_p3(cloud + (base + (c0 + t)) * 3); },
+                                                [&]() -> const PoseXf & { return poses.p[seq]; }, out, base, row, cols, c0,
+                                                TieList{nullptr, nullptr});
+    tile_fit_stats(m, [&](int) { return m.ori; }, map.pts, base, c0, sm, s_qcol, s_best, s_win, ss, part, mail);
 }
 
-bool dedupe_stats_supported(int cols) { return div_up(cols, kTile) <= 8; }  // portable cluster size
+bool row_cluster_supported(int cols) { return div_up(cols, kTile) <= 8; }  // portable cluster size
 
-int launch_dedupe_stats(const double *cloud, const int *labels, const RowMap &map, const MatchOut &out,
-                        const PoseBatch &poses, int n_seq, int rows, int cols, cudaStream_t stream, double *part,
-                        const FitMailbox &mail) {
-    const int tiles = div_up(cols, kTile);
+// a launch of kTile-thread CTAs in which the `tiles` CTAs of an image row form one thread-block cluster
+template <typename... Params, typename... Args>
+static int launch_row_clusters(void (*kernel)(Params...), dim3 grid, int tiles, cudaStream_t stream, Args &&...args) {
     cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)(n_seq * rows * tiles));
+    cfg.gridDim = grid;
     cfg.blockDim = dim3(kTile);
     cfg.stream = stream;
     cudaLaunchAttribute attr;
@@ -1083,7 +1089,15 @@ int launch_dedupe_stats(const double *cloud, const int *labels, const RowMap &ma
     attr.val.clusterDim.z = 1;
     cfg.attrs = &attr;
     cfg.numAttrs = 1;
-    return (int)cudaLaunchKernelEx(&cfg, k_dedupe_stats, cloud, labels, map, out, poses, rows, cols, tiles, part, mail);
+    return (int)cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
+}
+
+int launch_dedupe_stats(const double *cloud, const int *labels, const RowMap &map, const MatchOut &out,
+                        const PoseBatch &poses, int n_seq, int rows, int cols, cudaStream_t stream, double *part,
+                        const FitMailbox &mail) {
+    const int tiles = div_up(cols, kTile);
+    return launch_row_clusters(k_dedupe_stats, dim3((unsigned)(n_seq * rows * tiles)), tiles, stream, cloud, labels, map,
+                               out, poses, rows, cols, tiles, part, mail);
 }
 
 int launch_loop_step(const double *cloud, const int *labels, const RowMap &map, const MatchOut &out,
@@ -1091,19 +1105,9 @@ int launch_loop_step(const double *cloud, const int *labels, const RowMap &map, 
                      const double *prev_cloud, const int *prev_labels, const PoseBatch &prev_poses, bool do_map,
                      double *part, const FitMailbox &mail) {
     const int tiles = div_up(cols, kTile);
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)(n_seq * rows * tiles));
-    cfg.blockDim = dim3(kTile);
-    cfg.stream = stream;
-    cudaLaunchAttribute attr;
-    attr.id = cudaLaunchAttributeClusterDimension;
-    attr.val.clusterDim.x = (unsigned)tiles;
-    attr.val.clusterDim.y = 1;
-    attr.val.clusterDim.z = 1;
-    cfg.attrs = &attr;
-    cfg.numAttrs = 1;
-    return (int)cudaLaunchKernelEx(&cfg, k_loop_step, cloud, labels, map, out, poses, rows, cols, tiles, prev_cloud,
-                                   prev_labels, prev_poses, do_map ? 1 : 0, part, mail);
+    return launch_row_clusters(k_loop_step, dim3((unsigned)(n_seq * rows * tiles)), tiles, stream, cloud, labels, map,
+                               out, poses, rows, cols, tiles, prev_cloud, prev_labels, prev_poses, do_map ? 1 : 0, part,
+                               mail);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1180,9 +1184,7 @@ k_frame_seq(SeqArgs a, int *__restrict__ labels, RowMap map0, RowMap map1, Match
         const double *pts = s_pts[f & 1];
         const RowMap &map = (f & 1) ? map1 : map0;
         const RowMap &map_next = (f & 1) ? map0 : map1;
-        const RowView rv = {map.pts + base * 3, map.mask + (long long)rid * map.n_chunks,
-                            map.box + (long long)rid * map.n_chunks * 2, map.sbox + (long long)rid * map.n_super * 2,
-                            map.n_chunks, map.n_super, tile * kChunksPerSuper - 1};
+        const RowView rv = row_view(map, rid, base, tile);
         cp_async_wait_group<0>();  // this frame's tile has landed
         __syncthreads();
         NAV_STAMP(1);
@@ -1201,21 +1203,18 @@ k_frame_seq(SeqArgs a, int *__restrict__ labels, RowMap map0, RowMap map1, Match
         cp_async_commit();
         if (c < cols) {
             labels[base + c] = label;
-            if (label != 1) {
-                out.nn_idx[base + c] = -1;
-                out.nn_dist[base + c] = -1.0;
-                if (kOut && o.nn_idx) o.nn_idx[f * px_frame + base + c] = -1;
-                if (kOut && o.nn_dist) o.nn_dist[f * px_frame + base + c] = -1.0;
+            if (kOut && label != 1) {
+                if (o.nn_idx) o.nn_idx[f * px_frame + base + c] = -1;
+                if (o.nn_dist) o.nn_dist[f * px_frame + base + c] = -1.0;
             }
         }
+        const PoseXf &pose = kInline ? ip.loc[f] : a.pose_loc[(long long)f * a.n_seq + seq];
+        auto point_at = [&](int t) {  // the lidar-frame point of column-in-tile t
+            const double *sp = pts + (t + kHalo) * 3;
+            return P3{sp[0], sp[1], sp[2]};
+        };
         {
-            P3 own = {0, 0, 0};
-            if (c < cols) {
-                const double *sp = pts + (threadIdx.x + kHalo) * 3;
-                own.x = sp[0];
-                own.y = sp[1];
-                own.z = sp[2];
-            }
+            const P3 own = c < cols ? point_at(threadIdx.x) : P3{0, 0, 0};
             unsigned *mask_out = nullptr;
             if (kOut && o.mask) mask_out = o.mask + f * (long long)a.n_seq * rows * map_next.n_chunks;
             map_tile(label == 1, c < cols, own, kInline ? ip.fin[f] : a.pose_fin[(long long)f * a.n_seq + seq], map_next, rid,
@@ -1223,69 +1222,22 @@ k_frame_seq(SeqArgs a, int *__restrict__ labels, RowMap map0, RowMap map1, Match
         }
         NAV_STAMP(4);
         cp_async_wait_group<1>();  // the neighbourhood of the map; the next tile may still be in flight
-        int nq;
-        const int slot = block_excl_count(label == 1, s_warp, nq);  // its barriers also publish the prefetch
-        if (label == 1) s_qcol[slot] = threadIdx.x;
-        __syncthreads();
         NAV_STAMP(5);
-        int key = -1, qc_won = -1;  // kOut: the query's match (map column) and column, for the dedupe
-        unsigned long long dbits = 0;
-        if ((int)(threadIdx.x & ~31u) < nq) {  // warps with at least one query; spare lanes repeat the last one
-            const int t = s_qcol[min((int)threadIdx.x, nq - 1)];
-            const int qc = c0 + t;
-            const double *sp = pts + (t + kHalo) * 3;
-            const P3 p = {sp[0], sp[1], sp[2]};
-            const PoseXf &pose = kInline ? ip.loc[f] : a.pose_loc[(long long)f * a.n_seq + seq];
-            const P3 q = shift_point(pose, xf_point(pose, p));
-            double best;
-            int bcol;
-            search_row<true>(sm, rv, qc, q, best, bcol, kFull);
-            if ((int)threadIdx.x < nq) {
-                out.nn_idx[base + qc] = bcol >= 0 ? row * cols + bcol : -1;
-                out.nn_dist[base + qc] = bcol >= 0 ? __dsqrt_rn(best) : INFINITY;
-                if (kOut) {
-                    const int idx = bcol >= 0 ? row * cols + bcol : -1;
-                    const double dist = bcol >= 0 ? __dsqrt_rn(best) : INFINITY;
-                    if (o.nn_idx) o.nn_idx[f * px_frame + base + qc] = idx;
-                    if (o.nn_dist) o.nn_dist[f * px_frame + base + qc] = dist;
-                    if (bcol >= 0) {
-                        key = bcol;
-                        qc_won = qc;
-                        dbits = (unsigned long long)__double_as_longlong(dist);
-                    }
-                }
-            }
+        const TileQuery m = match_tile<true, false>(sm, rv, s_warp, s_qcol, label, point_at, [&]() -> const PoseXf & { return pose; }, out, base, row, cols,
+                                                    c0, TieList{nullptr, nullptr});
+        if (kOut && m.qc >= 0) {
+            if (o.nn_idx) o.nn_idx[f * px_frame + base + m.qc] = m.key >= 0 ? row * cols + m.key : -1;
+            if (o.nn_dist) o.nn_dist[f * px_frame + base + m.qc] = __longlong_as_double((long long)m.dbits);
         }
         if (kOut && o.part) {  // uniform over the grid: every CTA of the cluster takes it
             __shared__ unsigned long long s_best[kTile];
             __shared__ int s_win[kTile];
             __shared__ StatsSmem ss;
-            const bool winner = cluster_dedupe_winner(s_best, s_win, key, dbits, qc_won);
-            // residuals back into column order through shared memory, as k_loop_step does (the search is over and
-            // the cluster barriers were CTA barriers too: the map neighbourhood and the query list are free).  The
-            // winner's ori is transformed again from the tile, the same bits as during the search.
-            double *s_r = sm.pts;
-            int *s_flag = s_qcol;
-            s_flag[threadIdx.x] = 0;
-            __syncthreads();
-            if (winner) {
-                const int t = qc_won - c0;
-                const double *sp = pts + (t + kHalo) * 3;
-                const P3 p = {sp[0], sp[1], sp[2]};
-                const P3 ori = xf_point(kInline ? ip.loc[f] : a.pose_loc[(long long)f * a.n_seq + seq], p);
-                const double *np = map.pts + (base + key) * 3;
-                s_r[t * 3] = dsub(ori.x, np[0]);
-                s_r[t * 3 + 1] = dsub(ori.y, np[1]);
-                s_r[t * 3 + 2] = dsub(ori.z, np[2]);
-                s_flag[t] = 1;
-            }
-            __syncthreads();
-            const bool mine = s_flag[threadIdx.x] != 0;
-            const double rx = mine ? s_r[threadIdx.x * 3] : 0.0, ry = mine ? s_r[threadIdx.x * 3 + 1] : 0.0,
-                         rz = mine ? s_r[threadIdx.x * 3 + 2] : 0.0;
-            // part + (rid * tiles + tile) * 5: the CTA order of k_dedupe_stats
+            // part + (rid * tiles + tile) * 5: the CTA order of k_dedupe_stats.  The winner's ori is transformed
+            // again from the tile, the same bits as during the search.
             const FitMailbox no_mail = {nullptr, nullptr, 0ull};
-            block_post_stats(ss, mine, rx, ry, rz, o.part + (f * cta_frame + (long long)rid * gridDim.x) * 5, no_mail);
+            tile_fit_stats(m, [&](int t) { return xf_point(pose, point_at(t)); }, map.pts, base, c0, sm, s_qcol, s_best,
+                           s_win, ss, o.part + (f * cta_frame + (long long)rid * gridDim.x) * 5, no_mail);
         }
         // this CTA's part of the row's next map is written and it no longer reads the current one: signal the
         // cluster (release) and go on; the matching wait sits in front of the next frame's map prefetch
@@ -1294,8 +1246,6 @@ k_frame_seq(SeqArgs a, int *__restrict__ labels, RowMap map0, RowMap map1, Match
     }
     cluster_wait_all();  // every arrive has its wait
 }
-
-bool frame_seq_supported(int cols) { return div_up(cols, kTile) <= 8; }
 
 int frame_seq_inline_frames() { return kSeqInlineFrames; }
 
@@ -1308,18 +1258,7 @@ int launch_frame_seq(const double *frames, long long frame_stride, int n_frames,
     const int tiles = div_up(cols, kTile);
     const SeqArgs a = {frames, frame_stride, n_frames, n_seq, d_pose_loc, d_pose_fin};
     const bool inl = h_pose_loc && h_pose_fin && n_seq == 1 && n_frames <= kSeqInlineFrames;
-
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)tiles, (unsigned)rows, (unsigned)n_seq);
-    cfg.blockDim = dim3(kTile);
-    cfg.stream = stream;
-    cudaLaunchAttribute attr;
-    attr.id = cudaLaunchAttributeClusterDimension;
-    attr.val.clusterDim.x = (unsigned)tiles;
-    attr.val.clusterDim.y = 1;
-    attr.val.clusterDim.z = 1;
-    cfg.attrs = &attr;
-    cfg.numAttrs = 1;
+    const dim3 grid((unsigned)tiles, (unsigned)rows, (unsigned)n_seq);
     const SeqOut no_out = {nullptr, nullptr, nullptr, nullptr};
     if (inl) {
         SeqInlinePoses ip;  // the launch copies its parameters at the call
@@ -1329,17 +1268,17 @@ int launch_frame_seq(const double *frames, long long frame_stride, int n_frames,
         }
         for (int f = n_frames; f < kSeqInlineFrames; ++f) ip.loc[f] = ip.fin[f] = h_pose_loc[0];
         if (seq_out)
-            return (int)cudaLaunchKernelEx(&cfg, k_frame_seq<true, true>, a, labels, map0, map1, out, rows, cols, n_exact,
-                                           ip, *seq_out);
-        return (int)cudaLaunchKernelEx(&cfg, k_frame_seq<true, false>, a, labels, map0, map1, out, rows, cols, n_exact, ip,
-                                       no_out);
+            return launch_row_clusters(k_frame_seq<true, true>, grid, tiles, stream, a, labels, map0, map1, out, rows,
+                                       cols, n_exact, ip, *seq_out);
+        return launch_row_clusters(k_frame_seq<true, false>, grid, tiles, stream, a, labels, map0, map1, out, rows, cols,
+                                   n_exact, ip, no_out);
     }
     static const SeqInlinePoses none = {};
     if (seq_out)
-        return (int)cudaLaunchKernelEx(&cfg, k_frame_seq<false, true>, a, labels, map0, map1, out, rows, cols, n_exact,
-                                       none, *seq_out);
-    return (int)cudaLaunchKernelEx(&cfg, k_frame_seq<false, false>, a, labels, map0, map1, out, rows, cols, n_exact, none,
-                                   no_out);
+        return launch_row_clusters(k_frame_seq<false, true>, grid, tiles, stream, a, labels, map0, map1, out, rows, cols,
+                                   n_exact, none, *seq_out);
+    return launch_row_clusters(k_frame_seq<false, false>, grid, tiles, stream, a, labels, map0, map1, out, rows, cols,
+                               n_exact, none, no_out);
 }
 
 // Fit totals of frame blockIdx.x, sequence blockIdx.y: part = [n_frames][n_seq][n_part][5] partials, stats =

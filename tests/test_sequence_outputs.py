@@ -23,7 +23,8 @@ CANARY = 0xA5
 # ------------------------------------------------------------------ helpers ----------------------------------
 def seq_frames(synth, shape, n_seq, n, motion):
     """[n][n_seq][rows][cols][3]; 'scrambled' permutes every frame's columns, so a query's neighbour sits in an
-    arbitrary tile of the row."""
+    arbitrary tile of the row; 'empty_row' zeroes the middle row of every even frame, so the labelled queries of
+    that row in the next frame search an empty map row (nn_idx -1, nn_dist +inf)."""
     r, c = shape
     fr = np.stack([np.stack([synth.room_frame(r, c, f, seq=s) for s in range(n_seq)]) for f in range(n)])
     if motion == "scrambled":
@@ -31,6 +32,8 @@ def seq_frames(synth, shape, n_seq, n, motion):
         for f in range(n):
             for s in range(n_seq):
                 fr[f, s] = fr[f, s][:, rng.permutation(c)]
+    if motion == "empty_row":
+        fr[::2, :, r // 2] = 0.0
     return np.ascontiguousarray(fr)
 
 
@@ -150,7 +153,7 @@ CASES = [((64, 2048), 1, 12), ((64, 2048), 1, 70), ((16, 1800), 1, 9), ((5, 33),
 
 @gpu
 @pytest.mark.parametrize("shape,n_seq,k", CASES)
-@pytest.mark.parametrize("motion", ["small", "large", "scrambled"])
+@pytest.mark.parametrize("motion", ["small", "large", "scrambled", "empty_row"])
 def test_every_frame_matches_oracle_and_closed_loop(pkg, oracle, synth, shape, n_seq, k, motion):
     """Slot f against the oracle's frontend_frame of frame f (labels from the mask, nn_idx / nn_dist bit for bit
     on labelled pixels, -1 / -1.0 elsewhere); fit totals against a second single-sequence context stepped with
@@ -183,6 +186,10 @@ def test_every_frame_matches_oracle_and_closed_loop(pkg, oracle, synth, shape, n
                 assert np.array_equal(idx[f, s][lab], oidx[lab]), (f, s)
                 assert dist[f, s][lab].tobytes() == odist[lab].tobytes(), (f, s)
                 assert (idx[f, s][~lab] == -1).all() and (dist[f, s][~lab] == -1.0).all(), (f, s)
+                if motion == "empty_row" and f % 2 == 0:  # frame f + 1 searched the empty row of frame f's map
+                    q = lab[r // 2]
+                    assert q.any() and (idx[f, s][r // 2][q] == -1).all(), (f, s)
+                    assert (dist[f, s][r // 2][q] == np.inf).all(), (f, s)
                 # the closed loop on the same map: localization_fast, then the map of the frame at final[f]
                 p, err, nc = loop.slam_localization_fast(cloud, pred[f, s], last[f, s])
                 st = stats[f, s]
