@@ -79,13 +79,13 @@ uint64_t nav_launch_count(const nav_ctx *ctx);
  *     row on the host and re-answers the listed queries with the reference's search before anything reads nn_idx.
  *     nn_dist is the same under both rules.  Costs one extra stream synchronisation per call, two more plus the
  *     copies when a query is tied.  Supported by the blocking calls: nav_slam_match and nav_slam_localization
- *     (the correspondence list, and so the pose, is the reference's bit for bit), nav_frontend_frame and
- *     nav_frontend_frame_depth (any n_seq).  Refused -- non-zero return, an error naming the tie rule, nothing
- *     queued, the context unchanged -- by the calls that search the row map without a host round trip:
- *     nav_frontend_frame_dev, nav_frontend_sequence_dev, nav_frontend_sequence_out_dev, nav_frontend_submit,
- *     nav_frontend_frame_async, nav_frontend_frame_depth_async, nav_slam_localization_fast and nav_slam_run.
- *     Calls that only label or map (nav_slam_init[_dev], nav_slam_mapping, nav_slam_prefetch, ...) and the
- *     kd-tree calls work as before.
+ *     (the correspondence list, and so the pose, is the reference's bit for bit), nav_frontend_frame,
+ *     nav_frontend_frame_depth and nav_frontend_frame_mm (any n_seq).  Refused -- non-zero return, an error naming
+ *     the tie rule, nothing queued, the context unchanged -- by the calls that search the row map without a host
+ *     round trip: nav_frontend_frame_dev, nav_frontend_sequence_dev, nav_frontend_sequence_out_dev,
+ *     nav_frontend_submit, nav_frontend_submit_mm, nav_frontend_frame_async, nav_frontend_frame_depth_async,
+ *     nav_slam_localization_fast and nav_slam_run.  Calls that only label or map (nav_slam_init[_dev],
+ *     nav_slam_mapping, nav_slam_prefetch[_depth|_mm], ...) and the kd-tree calls work as before.
  * The first switch to NAV_TIE_REFERENCE allocates a list of one 32-byte record per pixel of the context.
  * Note: these constants are the inverse of the CPU oracle's tie_mode numbering (tie_mode 0 = reference). */
 #define NAV_TIE_LOWEST_INDEX 0
@@ -223,6 +223,18 @@ int nav_frontend_frame_depth(nav_ctx *ctx, const int *distances, const nav_pos *
                              const nav_pos *pos_last, const nav_pos *pos_final, nav_point *cloud_out,
                              int *feature_out, int32_t *nn_idx_out, double *nn_dist_out, nav_point *global_out);
 
+/* ---- integer-millimetre input (the reference's L9 sensor, src/main.c:77-128) -----------------------------------
+ * cloud_mm: int32 [n_seq][rows][cols][3], x y z of every point in whole millimetres -- 12 B/point cross PCIe
+ * instead of the 24 of a nav_point cloud.  Every int32 is exactly representable in binary64, so the device widens
+ * the frame into the very cloud an upload of (double)v would have given, and every later kernel is the cloud
+ * path's: all outputs equal, bit for bit, those of the same call on the cloud {(double)x, (double)y, (double)z}.
+ * (A -0.0 coordinate of a double cloud widens back as +0.0: nav_l9_csv_read_mm refuses "-0" for that reason.)
+ * Host buffers may be pageable unless a call says "pinned". */
+/* nav_frontend_frame on integer-mm input: any n_seq; supports NAV_TIE_REFERENCE as nav_frontend_frame does. */
+int nav_frontend_frame_mm(nav_ctx *ctx, const int32_t *cloud_mm, const nav_pos *pos_predict, const nav_pos *pos_last,
+                          const nav_pos *pos_final, int *feature_out, int32_t *nn_idx_out, double *nn_dist_out,
+                          nav_point *global_out);
+
 /* Pipelined variant of nav_frontend_frame for streams of frames: returns immediately; the upload of
  * this frame, the kernels of the previous one and the downloads of the one before overlap on three
  * CUDA streams.  All host pointers must be pinned (nav_host_alloc / cudaHostRegister).  The outputs
@@ -253,6 +265,12 @@ typedef struct {
 } nav_frame_io;
 int nav_frontend_submit(nav_ctx *ctx, const nav_frame_io *io, const nav_pos *pos_predict,
                         const nav_pos *pos_last, const nav_pos *pos_final);
+/* nav_frontend_submit on integer-mm input (see nav_frontend_frame_mm): cloud_mm (pinned) is the frame, any n_seq;
+ * io carries outputs only -- io->cloud, io->distances and io->cloud_out must be NULL, else the call fails and
+ * queues nothing.  The upload goes on the copy-in stream, the widening runs in front of the frame kernel.  Refused
+ * under NAV_TIE_REFERENCE like nav_frontend_submit. */
+int nav_frontend_submit_mm(nav_ctx *ctx, const int32_t *cloud_mm, const nav_frame_io *io, const nav_pos *pos_predict,
+                           const nav_pos *pos_last, const nav_pos *pos_final);
 /* nav_frontend_frame_depth, pipelined (src/main.c:194-197,308: depth -> xyz -> SLAM step per frame) */
 int nav_frontend_frame_depth_async(nav_ctx *ctx, const int *distances, const nav_pos *pos_predict,
                                    const nav_pos *pos_last, const nav_pos *pos_final, nav_point *cloud_out,
@@ -279,15 +297,24 @@ int nav_slam_prefetch(nav_ctx *ctx, const nav_point *cloud);
 /* the same for L5 input: uploads the depth matrix and converts it on the device; consume it with
  * nav_slam_localization_fast(ctx, NULL, ...) */
 int nav_slam_prefetch_depth(nav_ctx *ctx, const int *distances);
+/* the same for integer-mm input (see nav_frontend_frame_mm): uploads int32 [n_seq][rows][cols][3] and widens it on
+ * the device; consume it with nav_slam_localization_fast(ctx, NULL, ...).  Prefetches of the three kinds may be
+ * mixed; the slots are filled and consumed in order. */
+int nav_slam_prefetch_mm(nav_ctx *ctx, const int32_t *cloud_mm);
 /* The loop above as one call (src/main.c:300-318 with the EKF's prediction supplied by the caller): for
  * t = 0 .. n_frames-1: pred = predict(user, t, &last) -- or last + deltas[t] when predict is NULL --,
  * poses_out[t] = nav_slam_localization_fast(frames[t], pred, last), nav_slam_mapping(poses_out[t]),
  * last = poses_out[t]; `last` starts as *pos_start (the pose nav_slam_init mapped frame -1 with).
- * frames[t]: pinned nav_point[rows*cols] clouds, or pinned int[rows*cols] depth matrices when depth_input != 0.
- * error_out / n_corr_out: optional per-frame RMS residual and correspondence count.  Same poses as the
- * separate calls. */
+ * frames[t] (pinned), by input_kind: NAV_RUN_INPUT_XYZ nav_point[rows*cols] clouds, NAV_RUN_INPUT_DEPTH
+ * int[rows*cols] depth matrices, NAV_RUN_INPUT_MM int32[rows*cols][3] integer-mm clouds (see nav_frontend_frame_mm:
+ * the same poses, errors and correspondence counts as the clouds {(double)v}).  Every other non-zero value also
+ * selects depth matrices.  error_out / n_corr_out: optional per-frame RMS residual and correspondence count.  Same
+ * poses as the separate calls.  Refused under NAV_TIE_REFERENCE. */
+#define NAV_RUN_INPUT_XYZ 0
+#define NAV_RUN_INPUT_DEPTH 1
+#define NAV_RUN_INPUT_MM 2
 typedef void (*nav_predict_fn)(void *user, int t, const nav_pos *last, nav_pos *pred_out);
-int nav_slam_run(nav_ctx *ctx, const void *const *frames, int n_frames, int depth_input, nav_predict_fn predict,
+int nav_slam_run(nav_ctx *ctx, const void *const *frames, int n_frames, int input_kind, nav_predict_fn predict,
                  void *user, const nav_pos *deltas, const nav_pos *pos_start, nav_pos *poses_out, double *error_out,
                  size_t *n_corr_out);
 
@@ -299,6 +326,14 @@ int nav_slam_run(nav_ctx *ctx, const void *const *frames, int n_frames, int dept
  * array uninitialised there).  Same values as fscanf("%lf") bit for bit. */
 int nav_l9_csv_read(const char *path, int rows, int cols, size_t max_frames, nav_point *frames_out,
                     int *timestamps_out, size_t *n_frames_out);
+/* nav_l9_csv_read into integer-mm frames int32 [max_frames][rows][cols][3] (the input of nav_frontend_frame_mm,
+ * nav_frontend_submit_mm, nav_slam_prefetch_mm, NAV_RUN_INPUT_MM): the same parsing, records, frames, timestamps
+ * and failures.  A value v is stored as int32(v) only where (double)int32(v) has the same bits as v, so widening
+ * the frames gives exactly what nav_l9_csv_read stores.  Any other value -- a fraction, |v| > 2^31-1, inf, nan, or
+ * -0 (which reads as -0.0 and would widen back to +0.0) -- fails the call with an error naming the line and the
+ * value; *n_frames_out is then 0 and frames_out partly written. */
+int nav_l9_csv_read_mm(const char *path, int rows, int cols, size_t max_frames, int32_t *frames_out,
+                       int *timestamps_out, size_t *n_frames_out);
 /* replaces LidarProcessData (src/main.c:12-75): `parsed_data.json`, a top-level array whose elements are
  * objects {"time_main": integer, "distance": [integers, row-major], ...}.  Every array element is one
  * frame; integer distances with index < rows*cols are stored, everything else of distances_out keeps

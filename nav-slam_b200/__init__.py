@@ -12,4 +12,5 @@ The directory name has a hyphen, so import it with importlib.import_module("nav-
 """
 from . import build, synth  # noqa: F401
 from .binding import (Context, KdTree, NavError, bruteforce_nn_dev, csv_format_frame,  # noqa: F401
-                      device_count, fit_from_stats, imu_json_read, l5_json_read, l9_csv_read, load_library)
+                      device_count, fit_from_stats, imu_json_read, l5_json_read, l9_csv_read, l9_csv_read_mm,
+                      load_library, to_mm)

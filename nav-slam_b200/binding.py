@@ -64,6 +64,7 @@ EXPORTS = [
     "nav_set_tie_rule", "nav_tie_rule", "nav_tie_resolve_count",
     "nav_peer_create", "nav_peer_connect", "nav_kdtree_nn_allgather_dev", "nav_kdtree_nn_sharded_map_dev", "nav_peer_check",
     "nav_peer_destroy", "nav_shard_range", "nav_shard_owner",
+    "nav_frontend_frame_mm", "nav_frontend_submit_mm", "nav_slam_prefetch_mm", "nav_l9_csv_read_mm",
 ]
 
 
@@ -157,6 +158,12 @@ def load_library(build_if_missing: bool = True):
     L.nav_peer_destroy.argtypes = [vp]
     L.nav_slam_prefetch.argtypes = [vp, vp]
     L.nav_slam_prefetch_depth.argtypes = [vp, vp]
+    L.nav_slam_prefetch_mm.argtypes = [vp, vp]
+    L.nav_frontend_frame_mm.argtypes = [vp, vp, C.POINTER(NavPos), C.POINTER(NavPos), C.POINTER(NavPos),
+                                        vp, vp, vp, vp]
+    L.nav_frontend_submit_mm.argtypes = [vp, vp, C.POINTER(NavFrameIO), C.POINTER(NavPos), C.POINTER(NavPos),
+                                         C.POINTER(NavPos)]
+    L.nav_l9_csv_read_mm.argtypes = [C.c_char_p, C.c_int, C.c_int, C.c_size_t, vp, vp, C.POINTER(C.c_size_t)]
     L.nav_l9_csv_read.argtypes = [C.c_char_p, C.c_int, C.c_int, C.c_size_t, vp, vp, C.POINTER(C.c_size_t)]
     L.nav_csv_format_frame_gpu.argtypes = [vp, C.c_ulonglong, vp, vp, vp, C.POINTER(NavPos), C.POINTER(NavPos), vp,
                                            C.c_size_t, C.POINTER(C.c_size_t)]
@@ -208,6 +215,29 @@ def _pts(a):
     a = np.ascontiguousarray(a, dtype=np.float64)
     assert a.shape[-1] == 3
     return a
+
+
+def _mm(a):
+    """an integer-mm cloud as the C ABI takes it: C-contiguous int32 [..., 3] (no implicit conversion: see to_mm)"""
+    if not isinstance(a, np.ndarray) or a.dtype != np.int32:
+        raise TypeError("integer-mm clouds are int32 arrays; convert with to_mm()")
+    assert a.shape[-1] == 3
+    return np.ascontiguousarray(a)
+
+
+def to_mm(cloud) -> np.ndarray:
+    """int32 copy of an xyz cloud in whole millimetres, for the *_mm calls.  Raises ValueError unless every value v
+    comes back bit for bit as float64(int32(v)) -- the rule of nav_l9_csv_read_mm: fractions, |v| > 2^31-1, inf, nan
+    and -0.0 (whose int32 widens to +0.0) are refused."""
+    a = np.ascontiguousarray(cloud, dtype=np.float64)
+    in_range = (a >= -2.0 ** 31) & (a <= 2.0 ** 31 - 1)  # False for nan
+    m = np.where(in_range, a, 0.0).astype(np.int32)
+    bad = ~in_range | (m.astype(np.float64).view(np.uint64) != a.view(np.uint64))
+    if bad.any():
+        i = np.unravel_index(int(np.argmax(bad)), a.shape)
+        raise ValueError(f"to_mm: value {a[i]!r} at index {tuple(int(k) for k in i)} is not a whole number of "
+                         f"millimetres that int32 holds with the same float64 bits ({int(bad.sum())} such values)")
+    return m
 
 
 class Context:
@@ -340,6 +370,20 @@ class Context:
                                                idx.ctypes.data, dist.ctypes.data, g.ctypes.data), self.L)
         return cloud, feat, idx, dist, g
 
+    def frontend_frame_mm(self, cloud_mm, pos_predict, pos_last, pos_final):
+        """nav_frontend_frame_mm: cloud_mm int32 [..., rows, cols, 3]; returns (labels, nn_idx, nn_dist, global)."""
+        m = _mm(cloud_mm)
+        shp = m.shape[:-1]
+        feat = np.empty(shp, dtype=np.int32)
+        idx = np.empty(shp, dtype=np.int32)
+        dist = np.empty(shp)
+        g = np.empty(shp + (3,))
+        n = self.n_seq
+        _check(self.L.nav_frontend_frame_mm(self.h, m.ctypes.data, _pos_array(pos_predict, n),
+                                            _pos_array(pos_last, n), _pos_array(pos_final, n), feat.ctypes.data,
+                                            idx.ctypes.data, dist.ctypes.data, g.ctypes.data), self.L)
+        return feat, idx, dist, g
+
     def csv_rows(self, timestamp, lidar_pos, global_cloud=None, distances=None, imu=None, ekf_pos=None,
                  out_ptr=None, out_cap=0) -> bytes:
         """nav_csv_format_frame_gpu: the frame's CSV lines (src/main.c:320-352) formatted on the GPU.
@@ -377,9 +421,19 @@ class Context:
         _check(self.L.nav_frontend_submit(self.h, C.byref(io), _pos_array(pos_predict, n), _pos_array(pos_last, n),
                                           _pos_array(pos_final, n)), self.L)
 
-    def slam_prefetch(self, cloud_ptr=None, depth_ptr=None):
-        """nav_slam_prefetch / nav_slam_prefetch_depth with a pinned host pointer (int)."""
-        if depth_ptr is not None:
+    def frontend_submit_mm(self, cloud_mm_ptr, pos_predict, pos_last, pos_final, **outputs):
+        """nav_frontend_submit_mm: cloud_mm_ptr is a pinned int32 [..., 3] frame (int); keyword arguments are the
+        output fields of nav_frame_io (pinned host pointers as ints)."""
+        io = NavFrameIO(**outputs)
+        n = self.n_seq
+        _check(self.L.nav_frontend_submit_mm(self.h, cloud_mm_ptr, C.byref(io), _pos_array(pos_predict, n),
+                                             _pos_array(pos_last, n), _pos_array(pos_final, n)), self.L)
+
+    def slam_prefetch(self, cloud_ptr=None, depth_ptr=None, mm_ptr=None):
+        """nav_slam_prefetch / nav_slam_prefetch_depth / nav_slam_prefetch_mm with a pinned host pointer (int)."""
+        if mm_ptr is not None:
+            _check(self.L.nav_slam_prefetch_mm(self.h, mm_ptr), self.L)
+        elif depth_ptr is not None:
             _check(self.L.nav_slam_prefetch_depth(self.h, depth_ptr), self.L)
         else:
             _check(self.L.nav_slam_prefetch(self.h, cloud_ptr), self.L)
@@ -399,16 +453,22 @@ class Context:
         _check(self.L.nav_slam_fit_stats(self.h, out), self.L)
         return np.array(out[:])
 
-    def slam_run(self, frame_ptrs, deltas, pos_start, depth_input=False):
+    RUN_INPUT_XYZ, RUN_INPUT_DEPTH, RUN_INPUT_MM = 0, 1, 2  # NAV_RUN_INPUT_* of include/navslam_b200.h
+
+    def slam_run(self, frame_ptrs, deltas, pos_start, depth_input=False, mm_input=False):
         """nav_slam_run: the closed loop over pinned host frames (raw pointers) with dead-reckoning increments
-        deltas[t] (prediction = last pose + deltas[t]).  Returns (poses [n,6], rms [n], n_corr [n])."""
+        deltas[t] (prediction = last pose + deltas[t]).  Frames are clouds, depth matrices (depth_input) or int32
+        integer-mm clouds (mm_input).  Returns (poses [n,6], rms [n], n_corr [n])."""
+        if depth_input and mm_input:
+            raise ValueError("slam_run: depth_input and mm_input exclude each other")
+        kind = self.RUN_INPUT_DEPTH if depth_input else self.RUN_INPUT_MM if mm_input else self.RUN_INPUT_XYZ
         n = len(frame_ptrs)
         ptrs = (C.c_void_p * n)(*[int(p) for p in frame_ptrs])
         d = (NavPos * n)(*[NavPos(*[float(v) for v in row]) for row in np.asarray(deltas, dtype=np.float64).reshape(n, 6)])
         out = (NavPos * n)()
         err = (C.c_double * n)()
         nc = (C.c_size_t * n)()
-        _check(self.L.nav_slam_run(self.h, ptrs, n, 1 if depth_input else 0, None, None, d, _pos_array(pos_start),
+        _check(self.L.nav_slam_run(self.h, ptrs, n, kind, None, None, d, _pos_array(pos_start),
                                    out, err, nc), self.L)
         poses = np.array([[p.x, p.y, p.z, p.roll, p.pitch, p.yaw] for p in out]).reshape(n, 6)
         return poses, np.array(err[:]), np.array(nc[:], dtype=np.int64)
@@ -576,6 +636,18 @@ def l9_csv_read(path, rows, cols, max_frames):
     ts = np.zeros(max_frames, dtype=np.int32)
     n = C.c_size_t(0)
     _check(L.nav_l9_csv_read(path.encode(), rows, cols, max_frames, frames.ctypes.data, ts.ctypes.data, C.byref(n)), L)
+    return frames[:n.value], ts[:n.value]
+
+
+def l9_csv_read_mm(path, rows, cols, max_frames):
+    """nav_l9_csv_read_mm: returns (frames [n,rows,cols,3] int32, timestamps [n] int32); fails on any value that is
+    not an exact int32 (see to_mm)."""
+    L = load_library()
+    frames = np.zeros((max_frames, rows, cols, 3), dtype=np.int32)
+    ts = np.zeros(max_frames, dtype=np.int32)
+    n = C.c_size_t(0)
+    _check(L.nav_l9_csv_read_mm(path.encode(), rows, cols, max_frames, frames.ctypes.data, ts.ctypes.data,
+                                C.byref(n)), L)
     return frames[:n.value], ts[:n.value]
 
 

@@ -55,7 +55,7 @@ int nav_io_fail(const char *fmt, ...) {
         }                                                                                     \
     } while (0)
 
-extern "C" const char *nav_version(void) { return "navslam_b200 0.1 (sm_100a)"; }
+extern "C" const char *nav_version(void) { return "navslam_b200 0.2 (sm_100a)"; }
 extern "C" const char *nav_last_error(void) { return g_err; }
 
 extern "C" int nav_device_count(void) {
@@ -225,6 +225,7 @@ struct nav_ctx {
     nav_corr *d_corr_rows = nullptr, *d_corr = nullptr;
     int *d_corr_row_count = nullptr, *d_corr_total = nullptr;
     int *d_dist = nullptr;
+    int *d_mm = nullptr;  // integer-mm cloud of the blocking call, int32 [ntot][3] (lazy)
     double *d_tan_col = nullptr, *d_tan_row = nullptr;
     double *d_flat = nullptr;
     int *d_flat_count = nullptr;
@@ -242,7 +243,7 @@ struct nav_ctx {
     static constexpr int kSlots = 2;
     struct AsyncSlot {
         double *d_cloud = nullptr, *d_nn_dist = nullptr;
-        int *d_labels = nullptr, *d_nn_idx = nullptr, *d_depth = nullptr;
+        int *d_labels = nullptr, *d_nn_idx = nullptr, *d_depth = nullptr, *d_mm = nullptr;
         cudaEvent_t in_done = nullptr, compute_done = nullptr, out_done = nullptr;
     } slots[kSlots];
     cudaStream_t s_in = nullptr, s_out = nullptr;
@@ -252,7 +253,7 @@ struct nav_ctx {
     // stream while the current one is matched and fitted
     struct PreSlot {
         double *d_cloud = nullptr;
-        int *d_labels = nullptr, *d_depth = nullptr;
+        int *d_labels = nullptr, *d_depth = nullptr, *d_mm = nullptr;
         cudaEvent_t ready = nullptr, released = nullptr;
         const void *host_src = nullptr;  // identity of the prefetched frame
         bool pending = false;
@@ -370,20 +371,20 @@ extern "C" void nav_destroy(nav_ctx *c) {
                     c->map.mask, c->d_n_exact, c->map.box, c->map.sbox, c->map_alt.pts, c->map_alt.mask,
                     c->map_alt.box, c->map_alt.sbox, c->d_corr_rows, c->d_corr,
                     c->d_corr_row_count, c->d_corr_total, c->d_dist, c->d_tan_col, c->d_tan_row, c->d_flat,
-                    c->d_flat_count, c->d_tie_rec, c->d_tie_count, c->d_tie_fix};
+                    c->d_flat_count, c->d_tie_rec, c->d_tie_count, c->d_tie_fix, c->d_mm};
     for (void *p : ptrs)
         if (p) cudaFree(p);
     if (c->h_small) cudaFreeHost(c->h_small);
     if (c->d_csv) cudaFree(c->d_csv);
     if (c->d_csv_scratch) cudaFree(c->d_csv_scratch);
     for (auto &sl : c->slots) {
-        for (void *p : {(void *)sl.d_cloud, (void *)sl.d_labels, (void *)sl.d_depth})  // the other outputs live inside d_labels
+        for (void *p : {(void *)sl.d_cloud, (void *)sl.d_labels, (void *)sl.d_depth, (void *)sl.d_mm})  // the other outputs live inside d_labels
             if (p) cudaFree(p);
         for (cudaEvent_t e : {sl.in_done, sl.compute_done, sl.out_done})
             if (e) cudaEventDestroy(e);
     }
     for (auto &ps : c->pre) {
-        for (void *p : {(void *)ps.d_cloud, (void *)ps.d_labels, (void *)ps.d_depth})
+        for (void *p : {(void *)ps.d_cloud, (void *)ps.d_labels, (void *)ps.d_depth, (void *)ps.d_mm})
             if (p) cudaFree(p);
         for (cudaEvent_t e : {ps.ready, ps.released})
             if (e) cudaEventDestroy(e);
@@ -1054,6 +1055,11 @@ extern "C" int nav_slam_localization(nav_ctx *c, const nav_point *cloud, const n
 // needs pose(t)), but uploading frame t+1 and labelling it (a3 is pose independent) need neither.
 // nav_slam_prefetch queues both on the copy-in stream, so they run under frame t's match, download and
 // host fit; nav_slam_localization_fast then finds the frame resident and labelled.
+
+// What a host frame holds: the cloud itself (nav_point, 24 B/point), the L5 depth matrix (int mm per pixel, converted
+// on the device, n_seq == 1) or integer-mm xyz (int32 [n][3], widened on the device).
+enum InputKind { kInputCloud, kInputDepth, kInputMm };
+
 static int pre_setup(nav_ctx *c) {
     if (c->pre[0].d_cloud) return 0;
     if (!c->s_in) CU(cudaStreamCreateWithFlags(&c->s_in, cudaStreamNonBlocking));
@@ -1066,10 +1072,9 @@ static int pre_setup(nav_ctx *c) {
     return 0;
 }
 
-static int prefetch_common(nav_ctx *c, const char *name, const nav_point *cloud, const int *distances) {
-    const void *src = cloud ? (const void *)cloud : (const void *)distances;
+static int prefetch_common(nav_ctx *c, const char *name, InputKind kind, const void *src) {
     if (!src) return fail("%s: null argument", name);
-    if (distances && c->n_seq != 1) return fail("%s: depth input needs n_seq == 1", name);
+    if (kind == kInputDepth && c->n_seq != 1) return fail("%s: depth input needs n_seq == 1", name);
     if (!Stager::is_pinned(src)) return fail("%s: the host buffer must be pinned (nav_host_alloc / cudaHostRegister)", name);
     if (pre_setup(c)) return 1;
     nav_ctx::PreSlot &ps = c->pre[c->pre_next];
@@ -1087,13 +1092,18 @@ static int prefetch_common(nav_ctx *c, const char *name, const nav_point *cloud,
     if (!ps.release_recorded) CU(cudaEventRecord(ps.released, c->stream));
     ps.release_recorded = false;
     CU(cudaStreamWaitEvent(c->s_in, ps.released, 0));
-    if (distances) {
+    if (kind == kInputDepth) {
         if (!ps.d_depth) CU(cudaMalloc((void **)&ps.d_depth, c->npx * 4));
-        CU(cudaMemcpyAsync(ps.d_depth, distances, c->npx * 4, cudaMemcpyHostToDevice, c->s_in));
+        CU(cudaMemcpyAsync(ps.d_depth, src, c->npx * 4, cudaMemcpyHostToDevice, c->s_in));
         launch_convert(ps.d_depth, c->d_tan_col, c->d_tan_row, ps.d_cloud, c->rows, c->cols, c->sm_count, c->s_in);
         c->launches++;
+    } else if (kind == kInputMm) {
+        if (!ps.d_mm) CU(cudaMalloc((void **)&ps.d_mm, c->ntot * 12));
+        CU(cudaMemcpyAsync(ps.d_mm, src, c->ntot * 12, cudaMemcpyHostToDevice, c->s_in));
+        launch_widen_mm(ps.d_mm, ps.d_cloud, (long long)c->ntot, c->sm_count, c->s_in);
+        c->launches++;
     } else {
-        CU(cudaMemcpyAsync(ps.d_cloud, cloud, c->ntot * 24, cudaMemcpyHostToDevice, c->s_in));
+        CU(cudaMemcpyAsync(ps.d_cloud, src, c->ntot * 24, cudaMemcpyHostToDevice, c->s_in));
     }
     launch_labels(ps.d_cloud, ps.d_labels, nullptr, (long long)c->n_seq * c->rows, c->cols, c->sm_count, c->d_n_exact,
                   c->s_in);
@@ -1107,12 +1117,17 @@ static int prefetch_common(nav_ctx *c, const char *name, const nav_point *cloud,
 
 extern "C" int nav_slam_prefetch(nav_ctx *c, const nav_point *cloud) {
     CTX_ENTER(c, "nav_slam_prefetch");
-    return prefetch_common(c, "nav_slam_prefetch", cloud, nullptr);
+    return prefetch_common(c, "nav_slam_prefetch", kInputCloud, cloud);
 }
 
 extern "C" int nav_slam_prefetch_depth(nav_ctx *c, const int *distances) {
     CTX_ENTER(c, "nav_slam_prefetch_depth");
-    return prefetch_common(c, "nav_slam_prefetch_depth", nullptr, distances);
+    return prefetch_common(c, "nav_slam_prefetch_depth", kInputDepth, distances);
+}
+
+extern "C" int nav_slam_prefetch_mm(nav_ctx *c, const int32_t *cloud_mm) {
+    CTX_ENTER(c, "nav_slam_prefetch_mm");
+    return prefetch_common(c, "nav_slam_prefetch_mm", kInputMm, cloud_mm);
 }
 
 // slam_localization with the fit driven by five sufficient statistics reduced on the device
@@ -1276,7 +1291,7 @@ extern "C" int nav_slam_fit_stats(nav_ctx *c, double out[5]) {
 // The closed loop of a whole sequence in one call: the loop of src/main.c:300-318 with the EKF prediction
 // supplied by the caller -- a callback, or an array of dead-reckoning increments (pred = last + delta[t]).
 // Frame t+1 is prefetched (upload + labels on the copy-in stream) while frame t is matched and fitted.
-extern "C" int nav_slam_run(nav_ctx *c, const void *const *frames, int n_frames, int depth_input,
+extern "C" int nav_slam_run(nav_ctx *c, const void *const *frames, int n_frames, int input_kind,
                             nav_predict_fn predict, void *user, const nav_pos *deltas, const nav_pos *pos_start,
                             nav_pos *poses_out, double *error_out, size_t *n_corr_out) {
     CTX_ENTER(c, "nav_slam_run");
@@ -1286,10 +1301,13 @@ extern "C" int nav_slam_run(nav_ctx *c, const void *const *frames, int n_frames,
     if (c->n_seq != 1) return fail("nav_slam_run: needs n_seq == 1");
     if (!c->have_map) return fail("nav_slam_run: call nav_slam_init first");
     nav_pos last = *pos_start;
-    auto prefetch = [&](int t) {
-        return depth_input ? prefetch_common(c, "nav_slam_run", nullptr, (const int *)frames[t])
-                           : prefetch_common(c, "nav_slam_run", (const nav_point *)frames[t], nullptr);
-    };
+    // NAV_RUN_INPUT_*; every non-zero value other than NAV_RUN_INPUT_MM means depth matrices
+    const InputKind kind = input_kind == NAV_RUN_INPUT_XYZ ? kInputCloud
+                           : input_kind == NAV_RUN_INPUT_MM ? kInputMm
+                                                            : kInputDepth;
+    auto prefetch = [&](int t) { return prefetch_common(c, "nav_slam_run", kind, frames[t]); };
+    // a frame that is not a cloud is found as the oldest prefetched one, never uploaded as a cloud
+    auto cloud_of = [&](int t) { return kind == kInputCloud ? (const nav_point *)frames[t] : nullptr; };
     for (auto &ps : c->pre) ps.pending = false;
     // the loop maps its own frames: a frame an earlier localization call left unmapped in a prefetch slot is
     // given up, so that the slot can be refilled
@@ -1322,7 +1340,7 @@ extern "C" int nav_slam_run(nav_ctx *c, const void *const *frames, int n_frames,
             // one launch: map of frame t-1 from its fitted pose (deferred from the previous iteration), match of
             // frame t, statistics dedupe, mailbox post (k_loop_step)
             const double t0 = c->trace ? now_us() : 0.0;
-            nav_ctx::PreSlot *ps = find_prefetched(c, depth_input ? nullptr : frames[t]);
+            nav_ctx::PreSlot *ps = find_prefetched(c, cloud_of(t));
             if (!ps) return fail("nav_slam_run: frame %d was not prefetched", t);
             order_after_async(c);
             const PoseBatch poses = pose_batch(c, &pred, &last);
@@ -1341,7 +1359,7 @@ extern "C" int nav_slam_run(nav_ctx *c, const void *const *frames, int n_frames,
             set_current_frame(c, ps);
             deferred = ps;
             if (c->trace) c->trace_us[1] += now_us() - t0;
-        } else if (loc_fast_launch(c, depth_input ? nullptr : (const nav_point *)frames[t], &pred, &last)) {
+        } else if (loc_fast_launch(c, cloud_of(t), &pred, &last)) {
             return 1;
         }
         const double tp = c->trace ? now_us() : 0.0;
@@ -1395,19 +1413,26 @@ extern "C" int nav_slam_mapping(nav_ctx *c, const nav_pos *pos, const nav_point 
 // the blocking front-end frame from a host cloud, or (distances != null) from a depth matrix: L5 ingest fused with
 // the frame (SURVEY 8f #3, device part) -- the depth matrix (4 B/pixel instead of the 24 B/pixel cloud) is uploaded,
 // converted on the device (a2) and fed straight to the frame kernel; the converted lidar-frame cloud is returned only
-// if the caller asks for it (cloud_out)
+// if the caller asks for it (cloud_out).  cloud_mm != null: integer-mm xyz (12 B/point), widened on the device into
+// the same cloud a double upload would have given
 static int frontend_frame(nav_ctx *c, const char *name, const nav_point *cloud, const int *distances,
-                          const nav_pos *pos_predict, const nav_pos *pos_last, const nav_pos *pos_final,
-                          nav_point *cloud_out, int *feature_out, int32_t *nn_idx_out, double *nn_dist_out,
-                          nav_point *global_out) {
-    if ((!cloud && !distances) || !pos_predict || !pos_last || !pos_final) return fail("%s: null argument", name);
+                          const int32_t *cloud_mm, const nav_pos *pos_predict, const nav_pos *pos_last,
+                          const nav_pos *pos_final, nav_point *cloud_out, int *feature_out, int32_t *nn_idx_out,
+                          double *nn_dist_out, nav_point *global_out) {
+    if ((!cloud && !distances && !cloud_mm) || !pos_predict || !pos_last || !pos_final)
+        return fail("%s: null argument", name);
     if (distances && c->n_seq != 1) return fail("%s: needs n_seq == 1", name);
     if (!c->have_map) return fail("%s: call nav_slam_init first", name);
-    if (c->stage.reserve(c->ntot * ((distances ? 4 : 0) + 24 + 24 + 4 + 4 + 8) + 4096, c->stream))
+    if (c->stage.reserve(c->ntot * ((distances ? 4 : 0) + (cloud_mm ? 12 : 0) + 24 + 24 + 4 + 4 + 8) + 4096, c->stream))
         return fail("%s: staging", name);
     if (distances) {
         if (c->stage.h2d(c->d_dist, distances, c->npx * 4, c->stream)) return fail("%s: H2D", name);
         launch_convert(c->d_dist, c->d_tan_col, c->d_tan_row, c->d_cloud, c->rows, c->cols, c->sm_count, c->stream);
+        c->launches++;
+    } else if (cloud_mm) {
+        if (!c->d_mm) CU(cudaMalloc((void **)&c->d_mm, c->ntot * 12));
+        if (c->stage.h2d(c->d_mm, cloud_mm, c->ntot * 12, c->stream)) return fail("%s: H2D", name);
+        launch_widen_mm(c->d_mm, c->d_cloud, (long long)c->ntot, c->sm_count, c->stream);
         c->launches++;
     } else if (upload_cloud(c, cloud, name)) {
         return 1;
@@ -1429,8 +1454,16 @@ extern "C" int nav_frontend_frame(nav_ctx *c, const nav_point *cloud, const nav_
                                   const nav_pos *pos_last, const nav_pos *pos_final, int *feature_out,
                                   int32_t *nn_idx_out, double *nn_dist_out, nav_point *global_out) {
     CTX_ENTER(c, "nav_frontend_frame");
-    return frontend_frame(c, "nav_frontend_frame", cloud, nullptr, pos_predict, pos_last, pos_final, nullptr, feature_out,
-                          nn_idx_out, nn_dist_out, global_out);
+    return frontend_frame(c, "nav_frontend_frame", cloud, nullptr, nullptr, pos_predict, pos_last, pos_final, nullptr,
+                          feature_out, nn_idx_out, nn_dist_out, global_out);
+}
+
+extern "C" int nav_frontend_frame_mm(nav_ctx *c, const int32_t *cloud_mm, const nav_pos *pos_predict,
+                                     const nav_pos *pos_last, const nav_pos *pos_final, int *feature_out,
+                                     int32_t *nn_idx_out, double *nn_dist_out, nav_point *global_out) {
+    CTX_ENTER(c, "nav_frontend_frame_mm");
+    return frontend_frame(c, "nav_frontend_frame_mm", nullptr, nullptr, cloud_mm, pos_predict, pos_last, pos_final,
+                          nullptr, feature_out, nn_idx_out, nn_dist_out, global_out);
 }
 
 extern "C" int nav_frontend_frame_depth(nav_ctx *c, const int *distances, const nav_pos *pos_predict,
@@ -1438,8 +1471,8 @@ extern "C" int nav_frontend_frame_depth(nav_ctx *c, const int *distances, const 
                                         int *feature_out, int32_t *nn_idx_out, double *nn_dist_out,
                                         nav_point *global_out) {
     CTX_ENTER(c, "nav_frontend_frame_depth");
-    return frontend_frame(c, "nav_frontend_frame_depth", nullptr, distances, pos_predict, pos_last, pos_final, cloud_out,
-                          feature_out, nn_idx_out, nn_dist_out, global_out);
+    return frontend_frame(c, "nav_frontend_frame_depth", nullptr, distances, nullptr, pos_predict, pos_last, pos_final,
+                          cloud_out, feature_out, nn_idx_out, nn_dist_out, global_out);
 }
 
 // ------------------------------------------------------------------ CSV rows on the device ---
@@ -1590,27 +1623,38 @@ static int async_setup(nav_ctx *c) {
     return 0;
 }
 
-extern "C" int nav_frontend_submit(nav_ctx *c, const nav_frame_io *io, const nav_pos *pos_predict,
-                                   const nav_pos *pos_last, const nav_pos *pos_final) {
-    CTX_ENTER(c, "nav_frontend_submit");
-    REFUSE_UNDER_REF_TIES(c, "nav_frontend_submit");
-    if (!io || !pos_predict || !pos_last || !pos_final) return fail("nav_frontend_submit: null argument");
-    if (!io->cloud == !io->distances) return fail("nav_frontend_submit: give exactly one of cloud and distances");
-    if (io->distances && c->n_seq != 1) return fail("nav_frontend_submit: depth input needs n_seq == 1");
-    if (io->cloud_out && !io->distances) return fail("nav_frontend_submit: cloud_out is the converted depth matrix; there is none");
-    if (!c->have_map) return fail("nav_frontend_submit: call nav_slam_init first");
+// nav_frontend_submit (cloud_mm == null: the input is io->cloud or io->distances) and nav_frontend_submit_mm (the input
+// is cloud_mm, io carries outputs only)
+static int frontend_submit(nav_ctx *c, const char *name, const int32_t *cloud_mm, const nav_frame_io *io,
+                           const nav_pos *pos_predict, const nav_pos *pos_last, const nav_pos *pos_final) {
+    if (!c) return fail("%s: null context", name);
+    CU(cudaSetDevice(c->device));
+    REFUSE_UNDER_REF_TIES(c, name);
+    if (!io || !pos_predict || !pos_last || !pos_final) return fail("%s: null argument", name);
+    if (cloud_mm) {
+        if (io->cloud || io->distances || io->cloud_out)
+            return fail("%s: the frame is cloud_mm; io->cloud, io->distances and io->cloud_out must be NULL", name);
+    } else {
+        if (!io->cloud == !io->distances) return fail("%s: give exactly one of cloud and distances", name);
+        if (io->distances && c->n_seq != 1) return fail("%s: depth input needs n_seq == 1", name);
+        if (io->cloud_out && !io->distances) return fail("%s: cloud_out is the converted depth matrix; there is none", name);
+    }
+    if (!c->have_map) return fail("%s: call nav_slam_init first", name);
     if (async_setup(c)) return 1;
-    const void *hp[] = {io->cloud, io->distances, io->cloud_out, io->feature_out, io->mask_out,
+    const void *hp[] = {cloud_mm, io->cloud, io->distances, io->cloud_out, io->feature_out, io->mask_out,
                         io->nn_idx_out, io->nn_dist_out, io->global_out};
     for (const void *p : hp)
         if (p && !Stager::is_pinned(p))
-            return fail("nav_frontend_submit: host buffers must be pinned (nav_host_alloc / cudaHostRegister)");
+            return fail("%s: host buffers must be pinned (nav_host_alloc / cudaHostRegister)", name);
     static_assert(nav_ctx::kSlots == 2, "slots pair up with the two map buffers (see nav_ctx)");
     nav_ctx::AsyncSlot &sl = c->slots[c->async_frames % nav_ctx::kSlots];
     const bool reused = c->async_frames >= (uint64_t)nav_ctx::kSlots;
     // copy-in: the slot's cloud was last read by the kernels of frame t-2
     if (reused) CU(cudaStreamWaitEvent(c->s_in, sl.compute_done, 0));
-    if (io->distances) {
+    if (cloud_mm) {
+        if (!sl.d_mm) CU(cudaMalloc((void **)&sl.d_mm, c->ntot * 12));
+        CU(cudaMemcpyAsync(sl.d_mm, cloud_mm, c->ntot * 12, cudaMemcpyHostToDevice, c->s_in));
+    } else if (io->distances) {
         if (!sl.d_depth) CU(cudaMalloc((void **)&sl.d_depth, c->npx * 4));
         CU(cudaMemcpyAsync(sl.d_depth, io->distances, c->npx * 4, cudaMemcpyHostToDevice, c->s_in));
     } else {
@@ -1620,7 +1664,10 @@ extern "C" int nav_frontend_submit(nav_ctx *c, const nav_frame_io *io, const nav
     // kernels: need the upload, and the slot's output buffers released by the downloads of frame t-2
     CU(cudaStreamWaitEvent(c->stream, sl.in_done, 0));
     if (reused) CU(cudaStreamWaitEvent(c->stream, sl.out_done, 0));
-    if (io->distances) {  // a2 on the device: 4 B/pixel crossed PCIe instead of 24
+    if (cloud_mm) {  // widened on the device: 12 B/point crossed PCIe instead of 24
+        launch_widen_mm(sl.d_mm, sl.d_cloud, (long long)c->ntot, c->sm_count, c->stream);
+        c->launches++;
+    } else if (io->distances) {  // a2 on the device: 4 B/pixel crossed PCIe instead of 24
         launch_convert(sl.d_depth, c->d_tan_col, c->d_tan_row, sl.d_cloud, c->rows, c->cols, c->sm_count, c->stream);
         c->launches++;
     }
@@ -1652,6 +1699,17 @@ extern "C" int nav_frontend_submit(nav_ctx *c, const nav_frame_io *io, const nav
     CU(cudaEventRecord(sl.out_done, c->s_out));
     c->async_frames++;
     return 0;
+}
+
+extern "C" int nav_frontend_submit(nav_ctx *c, const nav_frame_io *io, const nav_pos *pos_predict,
+                                   const nav_pos *pos_last, const nav_pos *pos_final) {
+    return frontend_submit(c, "nav_frontend_submit", nullptr, io, pos_predict, pos_last, pos_final);
+}
+
+extern "C" int nav_frontend_submit_mm(nav_ctx *c, const int32_t *cloud_mm, const nav_frame_io *io,
+                                      const nav_pos *pos_predict, const nav_pos *pos_last, const nav_pos *pos_final) {
+    if (!cloud_mm) return fail("nav_frontend_submit_mm: null argument");
+    return frontend_submit(c, "nav_frontend_submit_mm", cloud_mm, io, pos_predict, pos_last, pos_final);
 }
 
 extern "C" int nav_frontend_frame_async(nav_ctx *c, const nav_point *cloud, const nav_pos *pos_predict,

@@ -109,13 +109,16 @@ inline bool expect(const char *&p, const char *end, char c) {  // a literal in t
 
 }  // namespace
 
-extern "C" int nav_l9_csv_read(const char *path, int rows, int cols, size_t max_frames, nav_point *frames_out,
-                               int *timestamps_out, size_t *n_frames_out) {
-    if (!path || !frames_out || !n_frames_out || rows < 1 || cols < 1)
-        return nav_io_fail("nav_l9_csv_read: bad argument");
+namespace {
+
+// the record loop of both L9 readers.  store(i, v) puts the record's x y z into pixel i (frame-major) and returns the
+// index (0..2) of a value it cannot store, or -1; a refused value fails the call with its line and text.
+template <class Store>
+int l9_csv_parse(const char *fn, const char *path, int rows, int cols, size_t max_frames, int *timestamps_out,
+                 size_t *n_frames_out, Store store) {
     *n_frames_out = 0;
     FILE *fp = fopen(path, "rb");
-    if (!fp) return nav_io_fail("nav_l9_csv_read: cannot open %s: %s", path, strerror(errno));
+    if (!fp) return nav_io_fail("%s: cannot open %s: %s", fn, path, strerror(errno));
     std::string text;
     {
         char chunk[1 << 16];
@@ -138,12 +141,18 @@ extern "C" int nav_l9_csv_read(const char *path, int rows, int cols, size_t max_
     size_t count = 0;  // index of the frame being filled
     while (true) {
         int frame, row, col, conf;
-        double x, y, z;
+        double v[3];
+        const char *tok[3], *tok_end[3];  // where each of x y z was read (for the error of a refused value)
         const char *q = p;
+        auto coord = [&](int k) {
+            tok[k] = q;
+            const bool ok = parse_double(q, end, v[k]);
+            tok_end[k] = q;
+            return ok;
+        };
         if (!(parse_int(q, end, frame) && expect(q, end, ',') && parse_int(q, end, row) && expect(q, end, ',') &&
-              parse_int(q, end, col) && expect(q, end, ',') && parse_double(q, end, x) && expect(q, end, ',') &&
-              parse_double(q, end, y) && expect(q, end, ',') && parse_double(q, end, z) && expect(q, end, ',') &&
-              parse_int(q, end, conf)))
+              parse_int(q, end, col) && expect(q, end, ',') && coord(0) && expect(q, end, ',') && coord(1) &&
+              expect(q, end, ',') && coord(2) && expect(q, end, ',') && parse_int(q, end, conf)))
             break;
         p = q;
         if (row < 0 || row >= rows || col < 0 || col >= cols) continue;
@@ -151,19 +160,58 @@ extern "C" int nav_l9_csv_read(const char *path, int rows, int cols, size_t max_
             if (have_frame) ++count;
             if (count >= max_frames) {  // the reference overruns its lidarData[10] here; stop instead
                 *n_frames_out = max_frames;
-                return nav_io_fail("nav_l9_csv_read: more than %zu frames in %s", max_frames, path);
+                return nav_io_fail("%s: more than %zu frames in %s", fn, max_frames, path);
             }
             have_frame = true;
             current = frame;
             if (timestamps_out) timestamps_out[count] = frame;
         }
-        nav_point &dst = frames_out[count * npx + (size_t)row * cols + col];
-        dst.x = x;
-        dst.y = y;
-        dst.z = z;
+        const int bad = store(count * npx + (size_t)row * cols + col, v);
+        if (bad >= 0) {
+            const char *t = skip_ws(tok[bad], tok_end[bad]);
+            size_t line = 1;
+            for (const char *c = text.data(); c < t; ++c) line += *c == '\n';
+            return nav_io_fail("%s: line %zu of %s: %c = '%.*s' is not a whole number of millimetres that int32 holds "
+                               "with the same binary64 bits (fractions, |v| > 2^31-1, inf, nan and -0 are refused)",
+                               fn, line, path, "xyz"[bad], (int)(tok_end[bad] - t), t);
+        }
     }
     *n_frames_out = have_frame ? count + 1 : 0;
     return 0;
+}
+
+}  // namespace
+
+extern "C" int nav_l9_csv_read(const char *path, int rows, int cols, size_t max_frames, nav_point *frames_out,
+                               int *timestamps_out, size_t *n_frames_out) {
+    if (!path || !frames_out || !n_frames_out || rows < 1 || cols < 1)
+        return nav_io_fail("nav_l9_csv_read: bad argument");
+    return l9_csv_parse("nav_l9_csv_read", path, rows, cols, max_frames, timestamps_out, n_frames_out,
+                        [&](size_t i, const double v[3]) {
+                            frames_out[i].x = v[0];
+                            frames_out[i].y = v[1];
+                            frames_out[i].z = v[2];
+                            return -1;
+                        });
+}
+
+extern "C" int nav_l9_csv_read_mm(const char *path, int rows, int cols, size_t max_frames, int32_t *frames_out,
+                                  int *timestamps_out, size_t *n_frames_out) {
+    if (!path || !frames_out || !n_frames_out || rows < 1 || cols < 1)
+        return nav_io_fail("nav_l9_csv_read_mm: bad argument");
+    return l9_csv_parse("nav_l9_csv_read_mm", path, rows, cols, max_frames, timestamps_out, n_frames_out,
+                        [&](size_t i, const double v[3]) {
+                            for (int k = 0; k < 3; ++k) {
+                                // in range first (the conversion of anything else is undefined), then the
+                                // bits: this refuses fractions and -0.0, whose int32 widens to +0.0
+                                if (!(v[k] >= -2147483648.0 && v[k] <= 2147483647.0)) return k;
+                                const int32_t m = (int32_t)v[k];
+                                const double back = (double)m;
+                                if (memcmp(&back, &v[k], sizeof(double)) != 0) return k;
+                                frames_out[i * 3 + k] = m;
+                            }
+                            return -1;
+                        });
 }
 
 // ---------------------------------------------------------------------------------- writer -----

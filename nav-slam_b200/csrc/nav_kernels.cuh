@@ -9,6 +9,8 @@ void launch_labels(const double *cloud, int *labels, double *curv_or_null, long 
                    int sm_count, unsigned *n_exact, cudaStream_t stream);
 void launch_convert(const int *dist, const double *tan_col, const double *tan_row, double *out, int rows,
                     int cols, int sm_count, cudaStream_t stream);
+// int32 [n_points][3] (whole millimetres) -> double [n_points][3], exact
+void launch_widen_mm(const int *in, double *out, long long n_points, int sm_count, cudaStream_t stream);
 void launch_transform(const double *in, double *out, long long n, const PoseXf &pose, int sm_count,
                       cudaStream_t stream);
 

@@ -277,6 +277,33 @@ void launch_convert(const int *dist, const double *tan_col, const double *tan_ro
     k_convert<<<(unsigned)grid, 256, 0, stream>>>(dist, tan_col, tan_row, out, rows, cols);
 }
 
+// ---------------------------------------------------------------- integer-mm xyz -----------
+// L9 clouds in whole millimetres cross PCIe as int32 [n][3] (12 B/point instead of 24) and are widened here.  Every
+// int32 is exact in binary64, so the cloud equals the one the host would have uploaded as doubles, bit for bit.
+// The 3n values are one flat run: a 16-byte load of four ints and two 16-byte stores of four doubles per step, the
+// last (3n) % 4 values one at a time.  Both buffers come from cudaMalloc (16-byte aligned).
+__global__ void k_widen_mm(const int *__restrict__ in, double *__restrict__ out, long long n_vals) {
+    const long long n4 = n_vals >> 2, stride = (long long)gridDim.x * blockDim.x;
+    const long long t = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    const int4 *in4 = reinterpret_cast<const int4 *>(in);
+    double2 *out2 = reinterpret_cast<double2 *>(out);
+    for (long long i = t; i < n4; i += stride) {
+        const int4 v = __ldg(in4 + i);
+        out2[2 * i] = make_double2((double)v.x, (double)v.y);
+        out2[2 * i + 1] = make_double2((double)v.z, (double)v.w);
+    }
+    for (long long i = 4 * n4 + t; i < n_vals; i += stride) out[i] = (double)in[i];
+}
+
+void launch_widen_mm(const int *in, double *out, long long n_points, int sm_count, cudaStream_t stream) {
+    const long long n_vals = n_points * 3;
+    if (n_vals <= 0) return;
+    long long grid = (n_vals / 4 + 255) / 256;
+    if (grid < 1) grid = 1;
+    if (grid > sm_count * 8LL) grid = sm_count * 8LL;
+    k_widen_mm<<<(unsigned)grid, 256, 0, stream>>>(in, out, n_vals);
+}
+
 // ---------------------------------------------------------------- a7 ------------------------
 __global__ void k_transform(const double *__restrict__ in, double *__restrict__ out, long long n, PoseXf pose) {
     for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n;
