@@ -426,6 +426,42 @@ int nav_frontend_sequence_out_dev(nav_ctx *ctx, const void *dev_frames, size_t n
                                   const nav_pos *pos_predict, const nav_pos *pos_last, const nav_pos *pos_final,
                                   const nav_sequence_out *out);
 
+/* The closed loop of nav_slam_run on a recording resident in HBM, with pose feedback and no host in the loop, for
+ * one or up to NAV_MAX_SEQ sequences side by side.
+ *   - Inputs: dev_frames = xyz clouds [n_frames][n_seq][rows][cols][3] (laid out as for nav_frontend_sequence_dev);
+ *     deltas (host) [n_frames][n_seq]: the prediction of frame t is last + deltas[t] component by component, last =
+ *     the fitted pose of frame t-1 (pos_start[s] (host) [n_seq] for frame 0, the pose the map was built with).
+ *   - Outputs (device or managed pointers on the context's device, `error` and `fit_stats` optional), frame t of
+ *     sequence s in slot [t][s]: the fitted pose, the RMS residual (nav_slam_run's error_out) and the five totals the
+ *     fit used, {N, sum rx, sum ry, sum rz, sum |r|^2} (fit_stats[.][0] = nav_slam_run's n_corr_out).
+ *   - Results: for n_seq == 1 poses, error and fit_stats equal, bit for bit, what nav_slam_run(ctx, host copies of the
+ *     same frames, NAV_RUN_INPUT_XYZ, NULL, NULL, deltas, pos_start, ...) returns on a context in the same state, and
+ *     fit_stats slot t what nav_slam_fit_stats would report after its frame t.  For n_seq > 1 sequence s gets exactly
+ *     what that call returns on a single-sequence context replaying sequence s.  The fit runs on the device, from the
+ *     same source as the host's (nav_slam_fit_from_stats) and with the same bias tables: same bits (where a result
+ *     is NaN, as after a diverged prediction, it is NaN on both sides; its payload bits may differ).
+ *   - Asynchronous: everything is queued on the context's stream (n_frames + 1 kernel launches and one upload of
+ *     about 200 B per frame and sequence) and the call returns without synchronising -- except when its scratch
+ *     has to grow, or when the staging buffer of a call four calls back is still in flight.  deltas and pos_start
+ *     are consumed before the call returns.  The outputs are complete once the stream has passed the call.
+ *   - Afterwards the context is as after nav_slam_run: the map of the last frame is built at its fitted pose, and
+ *     nav_frame_results_dev gives the last frame's labels, nn_idx and nn_dist.  A following nav_slam_run or
+ *     nav_slam_localization_fast with pos_last = the last pose continues the trajectory.  One difference: the frames
+ *     are the caller's memory, so the context keeps no resident copy of the last one, and nav_slam_mapping(ctx, pos,
+ *     NULL, ...), which after nav_slam_run maps its last frame again, is refused until a call leaves a frame resident.  The host mailbox is not
+ *     written: nav_slam_fit_stats keeps reporting the last fit of a host-side call (use out->fit_stats instead).
+ *   - Refused (non-zero return, an error naming the cause, nothing queued, the context unchanged): under
+ *     NAV_TIE_REFERENCE; rows wider than 2048 columns; no map yet (nav_slam_init[_dev] not called); a null out,
+ *     out->poses, deltas, pos_start or dev_frames; dev_frames or an output that is not device or managed memory on the
+ *     context's device (the error names the field).  n_frames == 0 returns 0 and writes nothing. */
+typedef struct {
+    nav_pos *poses;    /* [n_frames][n_seq]     fitted pose of every frame (required)            */
+    double *error;     /* [n_frames][n_seq]     RMS residual, as nav_slam_run's error_out        */
+    double *fit_stats; /* [n_frames][n_seq][5]  totals the fit used; [0] = correspondence count  */
+} nav_run_dev_out;
+int nav_slam_run_dev(nav_ctx *ctx, const void *dev_frames, int n_frames, const nav_pos *deltas,
+                     const nav_pos *pos_start, const nav_run_dev_out *out);
+
 /* copy out the map the context holds for one (sequence,row): the labelled global points of the
  * frame mapped last, compacted in column order (= the flattenedPoints array of src/slam.c:170-171),
  * and the column each came from.  pts_out needs room for cols points; col_out may be NULL. */

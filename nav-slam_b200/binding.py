@@ -37,6 +37,11 @@ class NavSequenceOut(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in ("label_mask", "nn_idx", "nn_dist", "fit_stats")]
 
 
+class NavRunDevOut(C.Structure):
+    """nav_run_dev_out of include/navslam_b200.h (device pointers; error / fit_stats may be None)."""
+    _fields_ = [(n, C.c_void_p) for n in ("poses", "error", "fit_stats")]
+
+
 class NavError(RuntimeError):
     pass
 
@@ -65,6 +70,7 @@ EXPORTS = [
     "nav_peer_create", "nav_peer_connect", "nav_kdtree_nn_allgather_dev", "nav_kdtree_nn_sharded_map_dev", "nav_peer_check",
     "nav_peer_destroy", "nav_shard_range", "nav_shard_owner",
     "nav_frontend_frame_mm", "nav_frontend_submit_mm", "nav_slam_prefetch_mm", "nav_l9_csv_read_mm",
+    "nav_slam_run_dev",
 ]
 
 
@@ -144,6 +150,7 @@ def load_library(build_if_missing: bool = True):
                                                  vp, vp, vp, vp, vp]
     L.nav_slam_run.argtypes = [vp, C.POINTER(C.c_void_p), C.c_int, C.c_int, vp, vp, C.POINTER(NavPos),
                                C.POINTER(NavPos), C.POINTER(NavPos), C.POINTER(C.c_double), C.POINTER(C.c_size_t)]
+    L.nav_slam_run_dev.argtypes = [vp, vp, C.c_int, C.POINTER(NavPos), C.POINTER(NavPos), C.POINTER(NavRunDevOut)]
     L.nav_peer_create.restype = C.c_void_p
     L.nav_peer_create.argtypes = [C.c_int, C.c_size_t, C.c_char_p]
     L.nav_peer_connect.argtypes = [vp, C.c_int, C.c_int, C.c_char_p]
@@ -512,6 +519,18 @@ class Context:
         out = None if all(v is None for v in fields) else C.byref(NavSequenceOut(*fields))
         _check(self.L.nav_frontend_sequence_out_dev(self.h, dev_frames_ptr, n_frames, _pos_array(pos_predict, n),
                                                     _pos_array(pos_last, n), _pos_array(pos_final, n), out), self.L)
+
+    def slam_run_dev(self, dev_frames_ptr, n_frames, deltas, pos_start, poses_ptr, error_ptr=None, stats_ptr=None):
+        """nav_slam_run_dev: the closed loop over n_frames device-resident xyz frames [n_frames][n_seq][rows][cols][3]
+        with the pose fit on the GPU.  deltas [n_frames][n_seq][6] (prediction = last pose + deltas[t]), pos_start
+        [n_seq][6]; the outputs are device buffers (ints): poses nav_pos [n_frames][n_seq], error double
+        [n_frames][n_seq] and stats double [n_frames][n_seq][5] (None = not wanted).  Queued on the context's stream;
+        the outputs are complete after synchronize()."""
+        n = n_frames * self.n_seq
+        d = _pos_array(deltas, n) if n > 0 else (NavPos * 1)()
+        out = NavRunDevOut(poses_ptr, error_ptr, stats_ptr)
+        _check(self.L.nav_slam_run_dev(self.h, dev_frames_ptr, n_frames, d, _pos_array(pos_start, self.n_seq),
+                                       C.byref(out)), self.L)
 
     def frame_results_dev(self) -> NavFrameResults:
         r = NavFrameResults()

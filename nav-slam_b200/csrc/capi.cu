@@ -284,6 +284,14 @@ struct nav_ctx {
     // per-frame partials of the fit statistics of nav_frontend_sequence_out_dev (grows like d_pose)
     double *d_seq_part = nullptr;
     size_t d_seq_part_cap = 0;
+    // the device closed loop (nav_slam_run_dev): pose records [2][n_seq] around the host tables [n_frames][n_seq]
+    // (grows like d_pose), per-sequence tickets, and the second slot of the label ring (the first is d_labels)
+    void *d_loop = nullptr;
+    size_t d_loop_cap = 0;
+    unsigned *d_loop_ticket = nullptr;
+    int *d_labels_alt = nullptr;
+    bool fit_tables_queued = false;  // the fit's bias tables were uploaded on the context's stream (nav_set_stream
+                                     // synchronises the old stream, so a later stream finds them in place)
     // NAV_RUN_TRACE=1: nav_slam_run prints where the host side of the closed loop spends its time
     // [prefetch call, launches of match + dedupe, wait for the statistics, fit, mapping call]
     bool trace = false;
@@ -398,6 +406,8 @@ extern "C" void nav_destroy(nav_ctx *c) {
     }
     if (c->d_pose) cudaFree(c->d_pose);
     if (c->d_seq_part) cudaFree(c->d_seq_part);
+    for (void *p : {c->d_loop, (void *)c->d_loop_ticket, (void *)c->d_labels_alt})
+        if (p) cudaFree(p);
     if (c->d_fit_ticket) cudaFree(c->d_fit_ticket);
     if (c->s_in) cudaStreamDestroy(c->s_in);
     if (c->s_out) cudaStreamDestroy(c->s_out);
@@ -1165,42 +1175,34 @@ static int wait_fit_mail(nav_ctx *c, const char *name) {
     return 0;
 }
 
-// the O(1)-per-iteration Adam loop on the five totals (also exported as nav_slam_fit_from_stats); bias corrections 1 - beta^t from tables computed once
-// with the same pow() calls the loop used to make
-static void fit_from_stats(const double st[5], const nav_pos *pos_predict, const nav_pos *pos_last, nav_pos *pos_out,
-                           double *error_out, size_t *n_corr_out) {
-    static double c1_tab[200], c2_tab[200];
+// the bias corrections 1 - beta^t of the fit, tables computed once with the same pow() calls the loop used to make;
+// the device loop (nav_slam_run_dev) gets a copy of these very values
+static void fit_bias_tables(const double **c1, const double **c2) {
+    static double c1_tab[kFitIters], c2_tab[kFitIters];
     static bool have_tab = false;
-    const double lr = 0.1, tol = 1e-6, b1 = 0.9, b2 = 0.999, eps = 1e-8;
     if (!have_tab) {
-        for (int i = 0; i < 200; ++i) {
-            c1_tab[i] = 1 - pow(b1, i + 1);
-            c2_tab[i] = 1 - pow(b2, i + 1);
+        for (int i = 0; i < kFitIters; ++i) {
+            c1_tab[i] = 1 - pow(0.9, i + 1);
+            c2_tab[i] = 1 - pow(0.999, i + 1);
         }
         __atomic_thread_fence(__ATOMIC_RELEASE);
         have_tab = true;
     }
-    const double N = st[0], S[3] = {st[1], st[2], st[3]}, Q = st[4];
+    *c1 = c1_tab;
+    *c2 = c2_tab;
+}
+
+// the O(1)-per-iteration Adam loop on the five totals (fit_translation, also exported as nav_slam_fit_from_stats)
+static void fit_from_stats(const double st[5], const nav_pos *pos_predict, const nav_pos *pos_last, nav_pos *pos_out,
+                           double *error_out, size_t *n_corr_out) {
+    const double *c1, *c2;
+    fit_bias_tables(&c1, &c2);
     double t[6] = {pos_predict->x - pos_last->x,       pos_predict->y - pos_last->y,
                    pos_predict->z - pos_last->z,       pos_predict->roll - pos_last->roll,
                    pos_predict->pitch - pos_last->pitch, pos_predict->yaw - pos_last->yaw};
-    double m[3] = {0, 0, 0}, v[3] = {0, 0, 0}, prev = 0, total = 0;
-    for (int iter = 0; iter < 200; ++iter) {
-        total = Q - 2.0 * (t[0] * S[0] + t[1] * S[1] + t[2] * S[2]) + N * (t[0] * t[0] + t[1] * t[1] + t[2] * t[2]);
-        if (N == 0) total = 0;
-        if (fabs(total - prev) < tol) break;
-        prev = total;
-        const double c1 = c1_tab[iter], c2 = c2_tab[iter];
-        for (int j = 0; j < 3; ++j) {
-            const double g = N > 0 ? -(S[j] - N * t[j]) / N : 0.0;
-            m[j] = b1 * m[j] + (1 - b1) * g;
-            v[j] = b2 * v[j] + (1 - b2) * g * g;
-            const double mh = m[j] / c1, vh = v[j] / c2;
-            t[j] -= lr * mh / (sqrt(vh) + eps);
-        }
-    }
-    if (error_out) *error_out = N > 0 ? sqrt(fmax(total, 0.0) / N) : 0.0;
-    if (n_corr_out) *n_corr_out = (size_t)N;
+    const double err = fit_translation(st, t, c1, c2);
+    if (error_out) *error_out = err;
+    if (n_corr_out) *n_corr_out = (size_t)st[0];
     pos_out->x = pos_last->x + t[0];
     pos_out->y = pos_last->y + t[1];
     pos_out->z = pos_last->z + t[2];
@@ -1381,6 +1383,134 @@ extern "C" int nav_slam_run(nav_ctx *c, const void *const *frames, int n_frames,
                 c->trace_us[1] / n_frames, c->trace_us[2] / n_frames, c->trace_us[3] / n_frames, c->trace_us[4] / n_frames);
         c->trace = false;
     }
+    return 0;
+}
+
+static bool on_ctx_device(const nav_ctx *c, const void *p);
+
+// The closed loop of nav_slam_run on frames resident in HBM, with no host in the loop: launch t (k_loop_step<true>)
+// maps frame t-1 from its fitted pose, matches frame t from its predicted pose -- both read from the device pose
+// record -- and the last CTA of each sequence fits the pose and writes the record of frame t+1; one more launch maps
+// the last frame.  Only the translation depends on the fit, so every rotation (and the fitted roll / pitch / yaw)
+// is formed here up front with the host libm, exactly as make_pose forms it in nav_slam_run.
+extern "C" int nav_slam_run_dev(nav_ctx *c, const void *dev_frames, int n_frames, const nav_pos *deltas,
+                                const nav_pos *pos_start, const nav_run_dev_out *out) {
+    static const char *name = "nav_slam_run_dev";
+    CTX_ENTER(c, "nav_slam_run_dev");
+    REFUSE_UNDER_REF_TIES(c, "nav_slam_run_dev");
+    if (!dev_frames || !deltas || !pos_start || !out || !out->poses)
+        return fail("%s: null argument (dev_frames, deltas, pos_start, out and out->poses are required)", name);
+    if (n_frames < 0) return fail("%s: n_frames = %d is negative", name, n_frames);
+    if (!row_cluster_supported(c->cols))
+        return fail("%s: rows of %d columns are wider than one thread-block cluster (2048 columns at most)", name,
+                    c->cols);
+    if (!c->have_map) return fail("%s: call nav_slam_init or nav_slam_init_dev first", name);
+    const std::pair<const void *, const char *> fields[] = {
+        {dev_frames, "dev_frames"}, {out->poses, "out->poses"}, {out->error, "out->error"}, {out->fit_stats, "out->fit_stats"}};
+    for (const auto &fd : fields)
+        if (fd.first && !on_ctx_device(c, fd.first))
+            return fail("%s: %s is not device or managed memory on device %d", name, fd.second, c->device);
+    if (n_frames == 0) return 0;
+    const int ns = c->n_seq;
+    const size_t n_tab = (size_t)n_frames * ns;
+    const size_t rec_bytes = (size_t)ns * sizeof(LoopRec), bytes = rec_bytes + n_tab * sizeof(LoopTab);
+    // one-time set-up and growth of the scratch (these may synchronise)
+    if (!c->fit_tables_queued) {
+        const double *c1, *c2;
+        fit_bias_tables(&c1, &c2);
+        CU((cudaError_t)upload_fit_tables(c1, c2, c->stream));
+        c->fit_tables_queued = true;
+    }
+    if (!c->d_loop_ticket) {
+        CU(cudaMalloc((void **)&c->d_loop_ticket, NAV_MAX_SEQ * sizeof(unsigned)));
+        CU(cudaMemsetAsync(c->d_loop_ticket, 0, NAV_MAX_SEQ * sizeof(unsigned), c->stream));
+    }
+    if (!c->d_labels_alt) CU(cudaMalloc((void **)&c->d_labels_alt, c->ntot * 4));
+    if (c->d_loop_cap < bytes + rec_bytes) {
+        CU(cudaStreamSynchronize(c->stream));
+        if (c->d_loop) cudaFree(c->d_loop);
+        c->d_loop = nullptr;
+        c->d_loop_cap = 0;
+        CU(cudaMalloc(&c->d_loop, bytes + rec_bytes));
+        c->d_loop_cap = bytes + rec_bytes;
+    }
+    nav_ctx::PoseRing &pr = c->pose_ring[c->pose_ring_next];
+    c->pose_ring_next = (c->pose_ring_next + 1) % nav_ctx::kPoseRing;
+    if (pr.done) CU(cudaEventSynchronize(pr.done));  // the staging buffer's previous upload (several calls ago)
+    if (pr.cap < bytes) {
+        if (pr.host) cudaFreeHost(pr.host);
+        pr.host = nullptr;
+        pr.cap = 0;
+        CU(cudaHostAlloc((void **)&pr.host, bytes, cudaHostAllocDefault));
+        pr.cap = bytes;
+    }
+    if (!pr.done) CU(cudaEventCreateWithFlags(&pr.done, cudaEventDisableTiming));
+    // staging: the records of frame 0, then the tables; on the device the records of frame 1 follow the tables
+    LoopRec *rec0 = (LoopRec *)pr.host;
+    LoopTab *tab = (LoopTab *)((unsigned char *)pr.host + rec_bytes);
+    for (int s = 0; s < ns; ++s) {
+        const nav_pos &st = pos_start[s], &d = deltas[s];
+        const nav_pos pred = {st.x + d.x, st.y + d.y, st.z + d.z, st.roll + d.roll, st.pitch + d.pitch, st.yaw + d.yaw};
+        rec0[s].loc = make_pose(&pred, &st);
+        rec0[s].map = make_pose(&st, nullptr);
+        nav_pos last = st;
+        for (int t = 0; t < n_frames; ++t) {
+            const nav_pos &dt = deltas[(size_t)t * ns + s];
+            nav_pos p = last, f = last;  // prediction and fitted pose; only roll / pitch / yaw are used here
+            p.roll = last.roll + dt.roll;
+            p.pitch = last.pitch + dt.pitch;
+            p.yaw = last.yaw + dt.yaw;
+            f.roll = last.roll + (p.roll - last.roll);  // fit_from_stats: pos_last + (pos_predict - pos_last)
+            f.pitch = last.pitch + (p.pitch - last.pitch);
+            f.yaw = last.yaw + (p.yaw - last.yaw);
+            LoopTab &tb = tab[(size_t)t * ns + s];
+            rotation_from_pos(&p, tb.Rq);
+            rotation_from_pos(&f, tb.Rm);
+            tb.rpy[0] = f.roll;
+            tb.rpy[1] = f.pitch;
+            tb.rpy[2] = f.yaw;
+            tb.d[0] = dt.x;
+            tb.d[1] = dt.y;
+            tb.d[2] = dt.z;
+            last = f;
+        }
+    }
+    unsigned char *dl_base = (unsigned char *)c->d_loop;
+    LoopRec *d_rec[2] = {(LoopRec *)dl_base, (LoopRec *)(dl_base + bytes)};
+    const LoopTab *d_tab = (const LoopTab *)(dl_base + rec_bytes);
+    order_after_async(c);
+    CU(cudaMemcpyAsync(c->d_loop, pr.host, bytes, cudaMemcpyHostToDevice, c->stream));
+    CU(cudaEventRecord(pr.done, c->stream));
+    // the label ring: frame t's labels go where the launch of frame t+1 maps them from; the last frame's land in
+    // d_labels, as nav_frame_results_dev reports them
+    auto labels_of = [&](int t) { return ((n_frames - 1 - t) & 1) ? c->d_labels_alt : c->d_labels; };
+    const double *frames = (const double *)dev_frames;
+    const long long stride = (long long)c->ntot * 3;
+    const MatchOut mo = {c->d_nn_idx, c->d_nn_dist, c->d_corr_rows, c->d_corr_row_count};
+    for (int t = 0; t <= n_frames; ++t) {  // t == n_frames: the last frame's map
+        const bool match = t < n_frames;
+        const DevLoop dl = {t, n_frames, ns, match ? 1 : 0, match ? labels_of(t) : nullptr, d_rec[t & 1],
+                            d_rec[(t + 1) & 1], d_tab, c->d_loop_ticket, c->d_n_exact, (nav_pos *)out->poses,
+                            out->error, out->fit_stats};
+        CU((cudaError_t)launch_loop_step_dev(dl, match ? frames + t * stride : nullptr,
+                                             t > 0 ? frames + (t - 1) * stride : nullptr, t > 0 ? labels_of(t - 1) : nullptr,
+                                             t > 0, c->map, mo, ns, c->rows, c->cols, c->d_tile_stats, c->stream));
+        c->launches++;
+    }
+    c->cloud_resident = false;
+    CU(cudaGetLastError());
+    return 0;
+}
+
+// test seam: the device fit (fit_translation with the uploaded tables) on n stat vectors, one thread each
+extern "C" int nav_debug_fit_from_stats_dev(const double *dev_stats, const nav_pos *dev_pred, const nav_pos *dev_last,
+                                            size_t n, nav_pos *dev_pose_out, double *dev_err_out, void *stream) {
+    if (!dev_stats || !dev_pred || !dev_last || !dev_pose_out) return fail("nav_debug_fit_from_stats_dev: null argument");
+    const double *c1, *c2;
+    fit_bias_tables(&c1, &c2);
+    CU((cudaError_t)upload_fit_tables(c1, c2, (cudaStream_t)stream));
+    launch_fit_debug(dev_stats, dev_pred, dev_last, n, dev_pose_out, dev_err_out, (cudaStream_t)stream);
+    CU(cudaGetLastError());
     return 0;
 }
 

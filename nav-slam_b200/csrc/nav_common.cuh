@@ -92,6 +92,34 @@ __device__ __forceinline__ float box_lower_bound32(const float4 lo, const float4
     return __fmul_rd(s, 0.99999905f);
 }
 
+// The closed loop's translation fit (src/slam.c:341-370 on five sufficient statistics): 200 Adam iterations on
+// st = {N, sum rx, sum ry, sum rz, sum |r|^2}, starting from t[0..2] = pred - last; t is updated in place and the
+// RMS residual returned.  c1[i] / c2[i] = 1 - beta1^(i+1) / 1 - beta2^(i+1), tables the host forms once with its
+// pow() (the only libm call of the loop).  One source for the host (nav_slam_fit_from_stats, the host closed loop)
+// and the device (nav_slam_run_dev): the rest is + - * /, sqrt, fabs and fmax, device code is built with
+// -fmad=false and host code with -ffp-contract=off, so both sides give the same bits.
+constexpr int kFitIters = 200;
+__host__ __device__ inline double fit_translation(const double st[5], double t[3], const double *c1, const double *c2) {
+    const double lr = 0.1, tol = 1e-6, b1 = 0.9, b2 = 0.999, eps = 1e-8;
+    const double N = st[0], S[3] = {st[1], st[2], st[3]}, Q = st[4];
+    double m[3] = {0, 0, 0}, v[3] = {0, 0, 0}, prev = 0, total = 0;
+    for (int iter = 0; iter < kFitIters; ++iter) {
+        total = Q - 2.0 * (t[0] * S[0] + t[1] * S[1] + t[2] * S[2]) + N * (t[0] * t[0] + t[1] * t[1] + t[2] * t[2]);
+        if (N == 0) total = 0;
+        if (fabs(total - prev) < tol) break;
+        prev = total;
+        const double k1 = c1[iter], k2 = c2[iter];
+        for (int j = 0; j < 3; ++j) {
+            const double g = N > 0 ? -(S[j] - N * t[j]) / N : 0.0;
+            m[j] = b1 * m[j] + (1 - b1) * g;
+            v[j] = b2 * v[j] + (1 - b2) * g * g;
+            const double mh = m[j] / k1, vh = v[j] / k2;
+            t[j] -= lr * mh / (sqrt(vh) + eps);
+        }
+    }
+    return N > 0 ? sqrt(fmax(total, 0.0) / N) : 0.0;
+}
+
 constexpr int kChunk = 16;       // map points per leaf box
 constexpr int kChunksPerSuper = 16;
 

@@ -106,6 +106,43 @@ int launch_loop_step(const double *cloud, const int *labels, const RowMap &map, 
                      const PoseBatch &poses, int n_seq, int rows, int cols, cudaStream_t stream,
                      const double *prev_cloud, const int *prev_labels, const PoseBatch &prev_poses, bool do_map,
                      double *part, const FitMailbox &mail);
+
+// The closed loop on device-resident frames (nav_slam_run_dev): the same k_loop_step, its poses read from a device
+// record per sequence that the previous launch's fit wrote.  What the host knows up front, per frame and sequence:
+struct LoopTab {
+    double Rq[9];   // rotation of the prediction (query pose)
+    double Rm[9];   // rotation of the fitted pose (map pose)
+    double rpy[3];  // roll, pitch, yaw of the fitted pose: last + (pred - last), the fit never moves them
+    double d[3];    // deltas[t].xyz: pred.xyz = last.xyz + d
+};
+// the device pose record of one sequence: this frame's query pose (R from the table, t = pred.xyz, shift =
+// pred.xyz - last.xyz, as make_pose forms it) and the previous frame's map pose (t = last.xyz, shift 0)
+struct LoopRec {
+    PoseXf loc, map;
+};
+struct DevLoop {
+    int t, n_frames, n_seq;
+    int do_match;              // 0: the launch after the last frame, which only maps it
+    int *labels_out;           // this frame's labels (the next launch maps the frame with them)
+    const LoopRec *rec_in;     // [n_seq] poses of frame t
+    LoopRec *rec_out;          // [n_seq] poses of frame t+1, written by the fit (a different buffer)
+    const LoopTab *tab;        // [n_frames][n_seq]
+    unsigned *ticket;          // [n_seq] finished CTAs of each sequence (zero between launches)
+    unsigned *n_exact;
+    nav_pos *poses;            // [n_frames][n_seq]
+    double *error;             // [n_frames][n_seq] or null
+    double *fit_stats;         // [n_frames][n_seq][5] or null
+};
+// launch t of the device loop: cloud = frame t, prev_cloud / prev_labels = frame t-1 (do_map); part: the CTA partials
+// [n_seq*rows*tiles][5].  Needs row_cluster_supported(cols) and the fit tables (upload_fit_tables).
+int launch_loop_step_dev(const DevLoop &dl, const double *cloud, const double *prev_cloud, const int *prev_labels,
+                         bool do_map, const RowMap &map, const MatchOut &out, int n_seq, int rows, int cols,
+                         double *part, cudaStream_t stream);
+// the fit's bias tables (1 - beta^t, formed on the host) into the device's constant memory, queued on `stream`
+int upload_fit_tables(const double *c1, const double *c2, cudaStream_t stream);
+// fit_translation on the device, one thread per stat vector (nav_debug_fit_from_stats_dev)
+void launch_fit_debug(const double *stats, const nav_pos *pred, const nav_pos *last, size_t n, nav_pos *pose_out,
+                      double *err_out, cudaStream_t stream);
 void launch_gather_corr(const nav_corr *corr_rows, const int *corr_row_count, nav_corr *corr_out,
                         int *corr_total, int n_seq, int rows, int cols, cudaStream_t stream);
 void launch_flatten_row(const double *row_pts, const int *row_feature, const unsigned *row_mask, double *out,

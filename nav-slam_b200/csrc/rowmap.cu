@@ -1034,24 +1034,123 @@ k_dedupe_stats(const double *__restrict__ cloud, const int *__restrict__ labels,
 //   2. the match of this frame (labels already computed by the prefetch) exactly as k_frame_match;
 //   3. the statistics dedupe of k_dedupe_stats on the results still in registers, and the mailbox post.
 // The serial chain of a frame is then: fit -> this launch -> the host sees the totals.
+//
+// The pose source is a compile-time choice.  kDevLoop = false (nav_slam_run): the poses of this frame and of the
+// previous one are kernel parameters (LoopPoses<false>), the labels were computed by the prefetch, and the last CTA
+// posts the totals to the host mailbox.  kDevLoop = true (nav_slam_run_dev, frames resident in HBM): the poses are the
+// device record of the sequence (LoopRec), which the previous launch's fit wrote; the tile's labels are computed here
+// from the staged tile, as k_frame_seq does, and stored for the next launch's map; the tickets count per sequence, and
+// the last CTA of a sequence adds that sequence's partials, runs the fit (fit_translation) and writes the frame's
+// pose, error and totals and the next frame's record.  With do_match = 0 the launch only maps the previous frame.
+#ifdef NAV_SEQ_TIMING
+// developer instrumentation (profiles/prof_slam_run_dev.py): thread 0 of the last CTA of every sequence stamps
+// %globaltimer before the partials are added, before the fit and after the outputs are written
+__device__ unsigned long long *g_loop_stamps;  // [frames][n_seq][4]
+extern "C" int nav_debug_set_loop_stamps(void *dev_ptr) {
+    return (int)cudaMemcpyToSymbol(g_loop_stamps, &dev_ptr, sizeof(void *));
+}
+#define NAV_LOOP_STAMP(k)                                                                                         \
+    do {                                                                                                          \
+        if (threadIdx.x == 0 && g_loop_stamps) {                                                                  \
+            unsigned long long t_;                                                                                \
+            asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t_));                                               \
+            g_loop_stamps[((long long)ps.t * ps.n_seq + seq) * 4 + (k)] = t_;                                     \
+        }                                                                                                         \
+    } while (0)
+#else
+#define NAV_LOOP_STAMP(k)
+#endif
+
+// the fit's bias corrections 1 - beta1^t, 1 - beta2^t (upload_fit_tables: the host's pow() values)
+__constant__ double c_fit_bias[2][kFitIters];
+
+template <bool kDevLoop>
+struct LoopPoses {
+    PoseBatch cur, prev;  // this frame's query poses, the previous frame's map poses
+};
+template <>
+struct LoopPoses<true> : DevLoop {};
+
+// the fit tail of the device loop, by thread 0 of the last CTA of sequence `seq` once st = its totals:
+// outputs of frame dl.t and the pose record of frame dl.t + 1
+__device__ __forceinline__ void loop_fit_tail(const DevLoop &dl, int seq, const LoopRec &rec, const double *st) {
+    const long long fs = (long long)dl.t * dl.n_seq + seq;
+    const LoopTab &tb = dl.tab[fs];
+    double tr[3] = {rec.loc.shift[0], rec.loc.shift[1], rec.loc.shift[2]};  // pred - last, as make_pose forms it
+    double s[5];
+#pragma unroll
+    for (int k = 0; k < 5; ++k) s[k] = st[k];
+    const double err = fit_translation(s, tr, c_fit_bias[0], c_fit_bias[1]);
+    const double *last = rec.map.t;
+    nav_pos p;
+    p.x = last[0] + tr[0];
+    p.y = last[1] + tr[1];
+    p.z = last[2] + tr[2];
+    p.roll = tb.rpy[0];
+    p.pitch = tb.rpy[1];
+    p.yaw = tb.rpy[2];
+    dl.poses[fs] = p;
+    if (dl.error) dl.error[fs] = err;
+    if (dl.fit_stats)
+#pragma unroll
+        for (int k = 0; k < 5; ++k) dl.fit_stats[fs * 5 + k] = s[k];
+    LoopRec &nx = dl.rec_out[seq];
+    const double pt[3] = {p.x, p.y, p.z};
+#pragma unroll
+    for (int k = 0; k < 9; ++k) nx.map.R[k] = tb.Rm[k];
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        nx.map.t[k] = pt[k];
+        nx.map.shift[k] = 0.0;
+    }
+    if (dl.t + 1 < dl.n_frames) {  // pred = last + deltas[t+1] (nav_slam_run's prediction), shift = pred - last
+        const LoopTab &tn = dl.tab[fs + dl.n_seq];
+#pragma unroll
+        for (int k = 0; k < 9; ++k) nx.loc.R[k] = tn.Rq[k];
+#pragma unroll
+        for (int k = 0; k < 3; ++k) {
+            nx.loc.t[k] = pt[k] + tn.d[k];
+            nx.loc.shift[k] = nx.loc.t[k] - pt[k];
+        }
+    }
+}
+
+template <bool kDevLoop>
 __global__ void __launch_bounds__(kTile, NAV_MATCH_MIN_CTAS)
 k_loop_step(const double *__restrict__ cloud, const int *__restrict__ labels, RowMap map, MatchOut out,
-            const __grid_constant__ PoseBatch poses, int rows, int cols, int tiles_per_row,
-            const double *__restrict__ prev_cloud, const int *__restrict__ prev_labels,
-            const __grid_constant__ PoseBatch prev_poses, int do_map, double *__restrict__ part, FitMailbox mail) {
+            const __grid_constant__ LoopPoses<kDevLoop> ps, int rows, int cols, int tiles_per_row,
+            const double *__restrict__ prev_cloud, const int *__restrict__ prev_labels, int do_map,
+            double *__restrict__ part, FitMailbox mail) {
     __shared__ int s_warp[65];
     __shared__ int s_qcol[kTile];
     __shared__ MapSmem sm;
     __shared__ unsigned long long s_best[kTile];
     __shared__ int s_win[kTile];
     __shared__ StatsSmem ss;
+    // kDevLoop only: the sequence's pose record, the staged tile of this frame and the label filter's taps
+    __shared__ LoopRec s_rec;
+    __shared__ __align__(16) double s_pts[kTilePts * 3];
+    __shared__ float s_f1[kTile + kHalo], s_f2[kTile + kHalo];
+    __shared__ double s_st[5];
     const int rid = blockIdx.x / tiles_per_row;
     const int tile = blockIdx.x % tiles_per_row;
     const int seq = rid / rows, row = rid % rows;
     const long long base = (long long)rid * cols;
     const int c0 = tile * kTile;
     const int c = c0 + threadIdx.x;
-    const int label = c < cols ? labels[base + c] : 0;
+    int label = 0;
+    if constexpr (kDevLoop) {
+        if (ps.do_match) {
+            tile_stage_async(s_pts, cloud + base * 3, c0, cols);
+            cp_async_commit();
+        }
+        constexpr int kRecWords = (int)(sizeof(LoopRec) / sizeof(double));
+        static_assert(kRecWords <= kTile, "one word of the record per thread");
+        if ((int)threadIdx.x < kRecWords) ((double *)&s_rec)[threadIdx.x] = ((const double *)(ps.rec_in + seq))[threadIdx.x];
+        __syncthreads();
+    } else {
+        label = c < cols ? labels[base + c] : 0;
+    }
     if (do_map) {
         __shared__ float4 s_lo[kChunksPerSuper], s_hi[kChunksPerSuper];
         bool lab = false;
@@ -1060,17 +1159,66 @@ k_loop_step(const double *__restrict__ cloud, const int *__restrict__ labels, Ro
             lab = prev_labels[base + c] == 1;
             p = load_p3(prev_cloud + (base + c) * 3);
         }
-        map_tile(lab, c < cols, p, prev_poses.p[seq], map, rid, tile, c, base, s_lo, s_hi);
-        cluster_sync_all();  // release / acquire: the row's new map is visible to all CTAs of its cluster
+        if constexpr (kDevLoop)
+            map_tile(lab, c < cols, p, s_rec.map, map, rid, tile, c, base, s_lo, s_hi);
+        else
+            map_tile(lab, c < cols, p, ps.prev.p[seq], map, rid, tile, c, base, s_lo, s_hi);
+        if constexpr (kDevLoop) {
+            if (!ps.do_match) return;  // the last frame's map: nothing reads it in this launch
+        }
+        // release / acquire: the row's new map is visible to all CTAs of its cluster.  The device loop computes the
+        // tile's labels between the arrive and the wait (they need nothing from the other tiles).
+        cluster_arrive_all();
     }
+    if constexpr (kDevLoop) {
+        cp_async_wait_all();
+        __syncthreads();
+        label = tile_labels_filtered(s_pts, s_f1, s_f2, c0, cols, ps.n_exact);
+        if (c < cols) ps.labels_out[base + c] = label;
+    }
+    if (do_map) cluster_wait_all();
     const RowView rv = row_view(map, rid, base, tile);
     prefetch_neighbourhood<true>(sm, rv, cols);
     cp_async_wait_all();
-    const TileQuery m = match_tile<true, false>(sm, rv, s_warp, s_qcol, label,
-                                                [&](int t) { return load_p3(cloud + (base + (c0 + t)) * 3); },
-                                                [&]() -> const PoseXf & { return poses.p[seq]; }, out, base, row, cols, c0,
-                                                TieList{nullptr, nullptr});
+    auto point_at = [&](int t) {  // the lidar-frame point of column-in-tile t
+        if constexpr (kDevLoop) {
+            const double *sp = s_pts + (t + kHalo) * 3;
+            return P3{sp[0], sp[1], sp[2]};
+        } else {
+            return load_p3(cloud + (base + (c0 + t)) * 3);
+        }
+    };
+    const TileQuery m = match_tile<true, false>(sm, rv, s_warp, s_qcol, label, point_at,
+                                                [&]() -> const PoseXf & {
+                                                    if constexpr (kDevLoop)
+                                                        return s_rec.loc;
+                                                    else
+                                                        return ps.cur.p[seq];
+                                                },
+                                                out, base, row, cols, c0, TieList{nullptr, nullptr});
     tile_fit_stats(m, [&](int) { return m.ori; }, map.pts, base, c0, sm, s_qcol, s_best, s_win, ss, part, mail);
+    if constexpr (kDevLoop) {
+        // the per-sequence ticket (block_post_stats without a mailbox has written this CTA's partial)
+        const unsigned n_cta = (unsigned)(rows * tiles_per_row);
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            __threadfence();  // cumulative: publishes the partial (ordered before it by the barrier)
+            ss.last = atomicAdd(ps.ticket + seq, 1u) == n_cta - 1;
+        }
+        __syncthreads();
+        if (!ss.last) return;
+        __threadfence();
+        NAV_LOOP_STAMP(0);
+        // the sequence's rows*tiles partials in the order k_seq_fit_totals and the mailbox post use
+        sum_fit_partials<kTile>(part + (long long)seq * n_cta * 5, (int)n_cta, ss.tot, s_st);
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            NAV_LOOP_STAMP(1);
+            loop_fit_tail(ps, seq, s_rec, s_st);
+            ps.ticket[seq] = 0u;
+            NAV_LOOP_STAMP(2);
+        }
+    }
 }
 
 bool row_cluster_supported(int cols) { return div_up(cols, kTile) <= 8; }  // portable cluster size
@@ -1105,9 +1253,61 @@ int launch_loop_step(const double *cloud, const int *labels, const RowMap &map, 
                      const double *prev_cloud, const int *prev_labels, const PoseBatch &prev_poses, bool do_map,
                      double *part, const FitMailbox &mail) {
     const int tiles = div_up(cols, kTile);
-    return launch_row_clusters(k_loop_step, dim3((unsigned)(n_seq * rows * tiles)), tiles, stream, cloud, labels, map,
-                               out, poses, rows, cols, tiles, prev_cloud, prev_labels, prev_poses, do_map ? 1 : 0, part,
-                               mail);
+    LoopPoses<false> ps;
+    ps.cur = poses;
+    ps.prev = prev_poses;
+    return launch_row_clusters(k_loop_step<false>, dim3((unsigned)(n_seq * rows * tiles)), tiles, stream, cloud, labels,
+                               map, out, ps, rows, cols, tiles, prev_cloud, prev_labels, do_map ? 1 : 0, part, mail);
+}
+
+int launch_loop_step_dev(const DevLoop &dl, const double *cloud, const double *prev_cloud, const int *prev_labels,
+                         bool do_map, const RowMap &map, const MatchOut &out, int n_seq, int rows, int cols,
+                         double *part, cudaStream_t stream) {
+    const int tiles = div_up(cols, kTile);
+    LoopPoses<true> ps;
+    static_cast<DevLoop &>(ps) = dl;
+    const FitMailbox no_mail = {nullptr, nullptr, 0ull};
+    return launch_row_clusters(k_loop_step<true>, dim3((unsigned)(n_seq * rows * tiles)), tiles, stream, cloud,
+                               (const int *)nullptr, map, out, ps, rows, cols, tiles, prev_cloud, prev_labels,
+                               do_map ? 1 : 0, part, no_mail);
+}
+
+// queued on `stream`, in front of the kernels that read the tables; c1 / c2 must stay valid (the host's static tables).
+// A second upload by another context rewrites the same values, so it never changes what a running kernel reads.
+int upload_fit_tables(const double *c1, const double *c2, cudaStream_t stream) {
+    const size_t bytes = kFitIters * sizeof(double);
+    cudaError_t e = cudaMemcpyToSymbolAsync(c_fit_bias, c1, bytes, 0, cudaMemcpyHostToDevice, stream);
+    if (e == cudaSuccess) e = cudaMemcpyToSymbolAsync(c_fit_bias, c2, bytes, bytes, cudaMemcpyHostToDevice, stream);
+    return (int)e;
+}
+
+// fit_translation on n stat vectors, one thread each: the pose last + (pred - last) with the fitted translation, as
+// nav_slam_fit_from_stats forms it
+__global__ void k_fit_debug(const double *__restrict__ stats, const nav_pos *__restrict__ pred,
+                            const nav_pos *__restrict__ last, size_t n, nav_pos *__restrict__ pose_out,
+                            double *__restrict__ err_out) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const nav_pos a = pred[i], b = last[i];
+    double st[5];
+    for (int k = 0; k < 5; ++k) st[k] = stats[i * 5 + k];
+    double t[6] = {a.x - b.x, a.y - b.y, a.z - b.z, a.roll - b.roll, a.pitch - b.pitch, a.yaw - b.yaw};
+    const double err = fit_translation(st, t, c_fit_bias[0], c_fit_bias[1]);
+    nav_pos p;
+    p.x = b.x + t[0];
+    p.y = b.y + t[1];
+    p.z = b.z + t[2];
+    p.roll = b.roll + t[3];
+    p.pitch = b.pitch + t[4];
+    p.yaw = b.yaw + t[5];
+    pose_out[i] = p;
+    if (err_out) err_out[i] = err;
+}
+
+void launch_fit_debug(const double *stats, const nav_pos *pred, const nav_pos *last, size_t n, nav_pos *pose_out,
+                      double *err_out, cudaStream_t stream) {
+    if (n == 0) return;
+    k_fit_debug<<<(unsigned)((n + 127) / 128), 128, 0, stream>>>(stats, pred, last, n, pose_out, err_out);
 }
 
 // ---------------------------------------------------------------------------------------------
