@@ -281,6 +281,7 @@ struct nav_ctx {
     int pose_ring_next = 0;
     void *d_pose = nullptr;
     size_t d_pose_cap = 0;
+    int seq_path = -1;  // how the last sequence replay ran (nav_debug_sequence_path)
     // per-frame partials of the fit statistics of nav_frontend_sequence_out_dev (grows like d_pose)
     double *d_seq_part = nullptr;
     size_t d_seq_part_cap = 0;
@@ -1502,6 +1503,11 @@ extern "C" int nav_slam_run_dev(nav_ctx *c, const void *dev_frames, int n_frames
     return 0;
 }
 
+// test seam: how the last nav_frontend_sequence_dev / nav_frontend_sequence_out_dev of the context ran -- 0: one
+// launch per frame, 1: one k_frame_seq launch staging with cp.async, 2: one k_frame_seq launch staging with bulk
+// copies; -1 before the first replay
+extern "C" int nav_debug_sequence_path(const nav_ctx *c) { return c ? c->seq_path : -1; }
+
 // test seam: the device fit (fit_translation with the uploaded tables) on n stat vectors, one thread each
 extern "C" int nav_debug_fit_from_stats_dev(const double *dev_stats, const nav_pos *dev_pred, const nav_pos *dev_last,
                                             size_t n, nav_pos *dev_pose_out, double *dev_err_out, void *stream) {
@@ -1969,7 +1975,9 @@ static int frontend_sequence(nav_ctx *c, const char *name, const void *dev_frame
     }
     const SeqOut seq_out = {so ? (unsigned *)so->label_mask : nullptr, so ? (int *)so->nn_idx : nullptr,
                             so ? (double *)so->nn_dist : nullptr, part};
+    c->seq_path = 0;
     if (fused) {
+        bool bulk = false;
         const size_t n_pose = n_frames * (size_t)c->n_seq, bytes = n_pose * 2 * sizeof(PoseXf);
         const MatchOut out = {c->d_nn_idx, c->d_nn_dist, c->d_corr_rows, c->d_corr_row_count};
         if ((int)n_frames <= frame_seq_inline_frames()) {  // short sequence: poses as kernel parameters
@@ -1982,7 +1990,7 @@ static int frontend_sequence(nav_ctx *c, const char *name, const void *dev_frame
             }
             CU((cudaError_t)launch_frame_seq(base, (long long)c->ntot * 3, (int)n_frames, c->d_labels, c->map, c->map_alt, out,
                                              nullptr, nullptr, c->n_seq, c->rows, c->cols, c->d_n_exact, c->stream, loc, fin,
-                                             so ? &seq_out : nullptr));
+                                             so ? &seq_out : nullptr, &bulk));
         } else {
             nav_ctx::PoseRing &pr = c->pose_ring[c->pose_ring_next];
             c->pose_ring_next = (c->pose_ring_next + 1) % nav_ctx::kPoseRing;
@@ -2012,8 +2020,9 @@ static int frontend_sequence(nav_ctx *c, const char *name, const void *dev_frame
             CU(cudaEventRecord(pr.done, c->stream));
             CU((cudaError_t)launch_frame_seq(base, (long long)c->ntot * 3, (int)n_frames, c->d_labels, c->map, c->map_alt, out,
                                              (const PoseXf *)c->d_pose, (const PoseXf *)c->d_pose + n_pose, c->n_seq, c->rows,
-                                             c->cols, c->d_n_exact, c->stream, nullptr, nullptr, so ? &seq_out : nullptr));
+                                             c->cols, c->d_n_exact, c->stream, nullptr, nullptr, so ? &seq_out : nullptr, &bulk));
         }
+        c->seq_path = bulk ? 2 : 1;
         c->launches++;
         if (n_frames & 1) std::swap(c->map, c->map_alt);
     } else {

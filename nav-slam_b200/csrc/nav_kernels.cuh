@@ -57,7 +57,7 @@ int launch_frame_seq(const double *frames, long long frame_stride, int n_frames,
                      const RowMap &map1, const MatchOut &out, const PoseXf *d_pose_loc, const PoseXf *d_pose_fin,
                      int n_seq, int rows, int cols, unsigned *n_exact, cudaStream_t stream,
                      const PoseXf *h_pose_loc = nullptr, const PoseXf *h_pose_fin = nullptr,
-                     const SeqOut *seq_out = nullptr);
+                     const SeqOut *seq_out = nullptr, bool *bulk_out = nullptr);  // *bulk_out: staged by bulk copies
 // fit totals stats[f][s][0..4] of the partials part[f][s][n_part][5], in the closed loop's summation order:
 // row_partials = false for tile partials (k_frame_seq, k_dedupe_stats), true for row totals (k_dedupe_rows)
 void launch_seq_fit_totals(const double *part, bool row_partials, int n_part, int n_frames, int n_seq, double *stats,

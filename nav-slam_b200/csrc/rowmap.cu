@@ -27,10 +27,13 @@
 //   k_export_row / k_flatten_row : stable row compaction (a4) for the API and the shim
 #include <limits.h>
 #include <math.h>
+#include <stddef.h>
+#include <stdint.h>
 #include <stdlib.h>
 
 #include <utility>
 
+#include "nav_bulk.cuh"
 #include "nav_kernels.cuh"
 #include "stencil_tile.cuh"
 
@@ -175,6 +178,25 @@ __device__ __forceinline__ int block_excl_count(bool pred, int *s_warp, int &tot
     return s_warp[32 + warp] + in_warp;
 }
 
+// block_excl_count with one barrier instead of three: every thread adds up the warp counts itself.  s_warp is
+// written without a barrier in front, so two uses must be separated by a barrier of the caller's (match_tile is
+// called once per kernel, or once per frame of k_frame_seq with the frame's other barriers in between).
+__device__ __forceinline__ int block_excl_count_once(bool pred, int *s_warp, int &total) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const unsigned m = __ballot_sync(kFull, pred);
+    if (lane == 0) s_warp[warp] = __popc(m);
+    __syncthreads();
+    int before = 0, all = 0;
+#pragma unroll
+    for (int w = 0; w < kTile / 32; ++w) {
+        const int v = s_warp[w];
+        before += w < warp ? v : 0;
+        all += v;
+    }
+    total = all;
+    return before + __popc(m & ((1u << lane) - 1u));
+}
+
 // scan the labelled points of one 16-column block of the map row.  `pts` points at column col0 of
 // the block (shared-memory copy for the CTA's own neighbourhood, global memory otherwise).  Four
 // candidates are loaded before any arithmetic so that their load latencies overlap; a short last
@@ -260,8 +282,12 @@ struct MapSmem {
     float4 box[kNbLeaves * 2];
     float4 sbox[kMaxSuperSmem * 2];
     float4 rbox[kMaxRowLeafSmem * 2];
-    unsigned mask[kNbLeaves];
+    // mask[j]: leaf leaf0 + j.  k_frame_seq's bulk copy moves the row's mask words in whole 16-byte groups, from
+    // the group that holds leaf0 (= 16 * tile - 1, i.e. 3 mod 4): up to three words in front, three behind.
+    unsigned mask_lead[3];
+    unsigned mask[kNbLeaves + 3];
 };
+static_assert(offsetof(MapSmem, mask) % 16 == 12 && sizeof(MapSmem) % 16 == 0, "mask word leaf0 + 1 on a 16-byte boundary");
 
 // one row of the map as the search sees it
 struct RowView {
@@ -308,6 +334,40 @@ __device__ __forceinline__ void prefetch_neighbourhood(MapSmem &sm, const RowVie
     // every leaf box of the row: a query near the edge of its tile (or far from its neighbour) tests
     // the leaves of other super blocks too, and sixteen dependent global loads made those warps the tail
     if (n_leaf <= kMaxRowLeafSmem && (int)threadIdx.x < 2 * n_leaf) cp_async16(&sm.rbox[threadIdx.x], rv.box + threadIdx.x);
+}
+
+// ---- bulk staging (k_frame_seq<kBulk = true>): one thread issues one cp.async.bulk per contiguous range and
+// every consumer waits on the range's mbarrier.  Taken when the rules of the copies hold for every range
+// (frame_seq_bulk_ok): an even number of columns (a row, and every span of it starting at an even column, is then
+// 16-byte aligned and a multiple of 48 bytes long), a mask row of a multiple of four words, 16-byte aligned base
+// pointers, and a row whose leaf boxes fit sm.rbox.
+
+// columns [max(c0-2, 0), min(c0+kTile+2, cols)) of one row (row_ptr = its column 0) into pts, laid out as
+// tile_stage_async does; the slots of columns outside the row are not written (k_frame_seq zeroes them once)
+__device__ __forceinline__ void tile_stage_bulk(double *pts, const double *row_ptr, int c0, int cols,
+                                                unsigned long long *bar) {
+    const int first = c0 - kHalo, lo = max(first, 0), hi = min(first + kTilePts, cols);
+    const unsigned bytes = (unsigned)(hi - lo) * 24u;
+    mbar_expect_tx(bar, bytes);
+    bulk_g2s(pts + (lo - first) * 3, row_ptr + (long long)lo * 3, bytes, bar);
+}
+
+// the neighbourhood of prefetch_neighbourhood, clamped to the row: the points of its leaves, the leaf boxes of
+// the row (rbox), the super boxes and the mask words.  sm.box is not staged: search_row reads it only for rows
+// wider than kMaxRowLeafSmem leaves.  The mask words go in whole 16-byte groups of the row (MapSmem); words of
+// leaves outside the row are never written (k_frame_seq zeroes them once).
+__device__ __forceinline__ void stage_neighbourhood_bulk(MapSmem &sm, const RowView &rv, int cols,
+                                                         unsigned long long *bar) {
+    const int leaf0 = rv.leaf0, lf_lo = max(leaf0, 0), lf_hi = min(leaf0 + kNbLeaves, rv.n_leaf);
+    const int col_lo = lf_lo * kChunk, col_hi = min(lf_hi * kChunk, cols);
+    const int w_lo = lf_lo & ~3, w_hi = min((lf_hi + 3) & ~3, rv.n_leaf);
+    const unsigned pts_b = (unsigned)(col_hi - col_lo) * 24u, row_b = (unsigned)rv.n_leaf * 32u,
+                   sup_b = (unsigned)rv.n_sup * 32u, mask_b = (unsigned)(w_hi - w_lo) * 4u;
+    mbar_expect_tx(bar, pts_b + row_b + sup_b + mask_b);
+    bulk_g2s(sm.pts + (lf_lo - leaf0) * kChunk * 3, rv.pts + (long long)col_lo * 3, pts_b, bar);
+    bulk_g2s(sm.rbox, rv.box, row_b, bar);
+    bulk_g2s(sm.sbox, rv.sbox, sup_b, bar);
+    bulk_g2s(sm.mask + (w_lo - leaf0), rv.mask + w_lo, mask_b, bar);
 }
 
 // exact nearest labelled map point of the row for query q of column qc: seed leaf, its neighbours, then the
@@ -512,7 +572,7 @@ __device__ __forceinline__ TileQuery match_tile(const MapSmem &sm, const RowView
         out.nn_dist[base + c] = -1.0;
     }
     int nq;
-    const int slot = block_excl_count(label == 1, s_warp, nq);  // its barriers also publish the prefetch
+    const int slot = block_excl_count_once(label == 1, s_warp, nq);  // its barrier also publishes a cp.async prefetch
     if (label == 1) s_qcol[slot] = threadIdx.x;
     __syncthreads();
     TileQuery m = {-1, -1, 0ull, {0, 0, 0}};
@@ -1360,7 +1420,11 @@ struct SeqInlinePoses {
 };
 static_assert(sizeof(SeqInlinePoses) + 256 < 32764, "inline poses must fit the kernel parameter space");
 
-template <bool kInline, bool kOut>
+// kBulk (frame_seq_bulk_ok): the frame's tile and the map neighbourhood arrive by bulk copies, one thread issues
+// them and every thread waits on an mbarrier -- s_bar[slot] for the tile in that slot, s_bar[2] for the
+// neighbourhood.  Otherwise every thread issues its share of 8- and 16-byte cp.async and waits for its own groups,
+// and a CTA barrier publishes them.
+template <bool kInline, bool kOut, bool kBulk>
 __global__ void __launch_bounds__(kTile, NAV_MATCH_MIN_CTAS)
 k_frame_seq(SeqArgs a, int *__restrict__ labels, RowMap map0, RowMap map1, MatchOut out, int rows, int cols,
             unsigned *__restrict__ n_exact, const __grid_constant__ SeqInlinePoses ip, SeqOut o) {
@@ -1377,30 +1441,77 @@ k_frame_seq(SeqArgs a, int *__restrict__ labels, RowMap map0, RowMap map1, Match
     const int c = c0 + threadIdx.x;
     // ring slots: per frame n_seq*rows rows of cols pixels / n_chunks mask words / `tiles` CTA partials
     const long long px_frame = (long long)a.n_seq * rows * cols, cta_frame = (long long)a.n_seq * rows * gridDim.x;
-    tile_stage_async(s_pts[0], a.frames + base * 3, c0, cols);
-    cp_async_commit();
+    __shared__ __align__(8) unsigned long long s_bar[3];
+    if constexpr (kBulk) {
+        // the copies only ever write the slots of columns inside the row and the mask words of leaves inside it;
+        // the rest reads as zero, as the cp.async path leaves it
+        for (int i = threadIdx.x; i < kTilePts * 3; i += kTile) {
+            const int col = c0 - kHalo + i / 3;
+            if (col < 0 || col >= cols) s_pts[0][i] = s_pts[1][i] = 0.0;
+        }
+        if (threadIdx.x < 3) sm.mask_lead[threadIdx.x] = 0u;
+        if (threadIdx.x < kNbLeaves + 3) sm.mask[threadIdx.x] = 0u;
+        if (threadIdx.x == 0) {
+            for (int i = 0; i < 3; ++i) mbar_init(&s_bar[i], 1);
+            asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        }
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // the zeros above before the copies
+            tile_stage_bulk(s_pts[0], a.frames + base * 3, c0, cols, &s_bar[0]);
+        }
+    } else {
+        tile_stage_async(s_pts[0], a.frames + base * 3, c0, cols);
+        cp_async_commit();
+    }
     for (int f = 0; f < a.n_frames; ++f) {
         NAV_STAMP(0);
         const double *pts = s_pts[f & 1];
         const RowMap &map = (f & 1) ? map1 : map0;
         const RowMap &map_next = (f & 1) ? map0 : map1;
         const RowView rv = row_view(map, rid, base, tile);
-        cp_async_wait_group<0>();  // this frame's tile has landed
-        __syncthreads();
+        // this frame's tile has landed
+        if constexpr (kBulk) {
+            mbar_wait(&s_bar[f & 1], (unsigned)(f >> 1) & 1u);  // phase f / 2 of its slot's barrier
+        } else {
+            cp_async_wait_group<0>();
+            __syncthreads();
+        }
         NAV_STAMP(1);
         // the labels need nothing from the row's other tiles: they are computed BEFORE waiting for the cluster
         // (the barrier was only signalled at the end of the previous frame), which turns the wait for the row's
         // slowest tile into useful time
         const int label = tile_labels_filtered(pts, s_f1, s_f2, c0, cols, n_exact);
+        // the next frame's tile starts its way from HBM now and has the whole search to arrive.  Its slot was last
+        // read in frame f-1; the barrier that ends the labels is behind those reads (cp.async path: the cluster wait).
+        // Nothing but generic reads touched the slot since its last copy, so the refill needs no proxy fence.
+        if constexpr (kBulk) {
+            if (threadIdx.x == 0 && f + 1 < a.n_frames)
+                tile_stage_bulk(s_pts[(f + 1) & 1], a.frames + (long long)(f + 1) * a.frame_stride + base * 3, c0, cols,
+                                &s_bar[(f + 1) & 1]);
+        }
         NAV_STAMP(2);
         if (f > 0) cluster_wait_all();  // the row's map of the previous frame is complete (also a CTA barrier)
         NAV_STAMP(3);
-        prefetch_neighbourhood<true>(sm, rv, cols);
-        cp_async_commit();
-        // the next frame's tile starts its way from HBM now and has the whole search to arrive
-        if (f + 1 < a.n_frames)
-            tile_stage_async(s_pts[(f + 1) & 1], a.frames + (long long)(f + 1) * a.frame_stride + base * 3, c0, cols);
-        cp_async_commit();
+        if constexpr (kBulk) {
+            if (threadIdx.x == 0) {
+                // The row's map was written by the CTAs of the cluster with generic stores, ordered before this
+                // thread by the release / acquire of the cluster barrier; the async proxy of the copies below is
+                // ordered behind it by this thread's proxy fence, which is enough as the copies are issued by this
+                // thread after the fence.  (Frame 0 reads a map of an earlier launch.)  The same for shared memory:
+                // the generic reads and writes of sm (search, statistics dedupe) precede the CTA barrier above, the
+                // async writes of the copies follow the fence.
+                asm volatile("fence.proxy.async.global;" ::: "memory");
+                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+                stage_neighbourhood_bulk(sm, rv, cols, &s_bar[2]);
+            }
+        } else {
+            prefetch_neighbourhood<true>(sm, rv, cols);
+            cp_async_commit();
+            if (f + 1 < a.n_frames)
+                tile_stage_async(s_pts[(f + 1) & 1], a.frames + (long long)(f + 1) * a.frame_stride + base * 3, c0, cols);
+            cp_async_commit();
+        }
         if (c < cols) {
             labels[base + c] = label;
             if (kOut && label != 1) {
@@ -1421,7 +1532,11 @@ k_frame_seq(SeqArgs a, int *__restrict__ labels, RowMap map0, RowMap map1, Match
                      tile, c, base, s_lo, s_hi, mask_out);
         }
         NAV_STAMP(4);
-        cp_async_wait_group<1>();  // the neighbourhood of the map; the next tile may still be in flight
+        // the neighbourhood of the map; the next tile may still be in flight
+        if constexpr (kBulk)
+            mbar_wait(&s_bar[2], (unsigned)f & 1u);
+        else
+            cp_async_wait_group<1>();
         NAV_STAMP(5);
         const TileQuery m = match_tile<true, false>(sm, rv, s_warp, s_qcol, label, point_at, [&]() -> const PoseXf & { return pose; }, out, base, row, cols,
                                                     c0, TieList{nullptr, nullptr});
@@ -1449,12 +1564,23 @@ k_frame_seq(SeqArgs a, int *__restrict__ labels, RowMap map0, RowMap map1, Match
 
 int frame_seq_inline_frames() { return kSeqInlineFrames; }
 
-// h_pose_loc / h_pose_fin != null (n_seq == 1, n_frames <= frame_seq_inline_frames()): the poses are passed as
-// kernel parameters and the device arrays are not read.  seq_out != null: the output mode of k_frame_seq.
-int launch_frame_seq(const double *frames, long long frame_stride, int n_frames, int *labels, const RowMap &map0,
-                     const RowMap &map1, const MatchOut &out, const PoseXf *d_pose_loc, const PoseXf *d_pose_fin,
-                     int n_seq, int rows, int cols, unsigned *n_exact, cudaStream_t stream, const PoseXf *h_pose_loc,
-                     const PoseXf *h_pose_fin, const SeqOut *seq_out) {
+// Whether k_frame_seq can stage with bulk copies (kBulk): every range it copies must start on a 16-byte boundary and
+// be a multiple of 16 bytes long.  Rows of an even number of columns up to 2048 whose mask rows are a multiple of
+// four words -- 64x2048 and every width that is a multiple of 64 -- take the bulk path; odd widths (e.g. 257) and
+// even ones with a ragged mask row (e.g. 1800: 113 words) keep the cp.async path.
+static bool frame_seq_bulk_ok(const double *frames, long long frame_stride, const RowMap &m0, const RowMap &m1, int cols) {
+    auto al16 = [](const void *p) { return ((uintptr_t)p & 15u) == 0; };
+    auto map_ok = [&](const RowMap &m) { return al16(m.pts) && al16(m.mask) && al16(m.box) && al16(m.sbox); };
+    return cols % 2 == 0 && cols <= kMaxRowLeafSmem * kChunk && div_up(cols, kChunk) % 4 == 0 && frame_stride % 2 == 0 &&
+           al16(frames) && map_ok(m0) && map_ok(m1);
+}
+
+template <bool kBulk>
+static int launch_frame_seq_variant(const double *frames, long long frame_stride, int n_frames, int *labels,
+                                    const RowMap &map0, const RowMap &map1, const MatchOut &out,
+                                    const PoseXf *d_pose_loc, const PoseXf *d_pose_fin, int n_seq, int rows, int cols,
+                                    unsigned *n_exact, cudaStream_t stream, const PoseXf *h_pose_loc,
+                                    const PoseXf *h_pose_fin, const SeqOut *seq_out) {
     const int tiles = div_up(cols, kTile);
     const SeqArgs a = {frames, frame_stride, n_frames, n_seq, d_pose_loc, d_pose_fin};
     const bool inl = h_pose_loc && h_pose_fin && n_seq == 1 && n_frames <= kSeqInlineFrames;
@@ -1468,17 +1594,33 @@ int launch_frame_seq(const double *frames, long long frame_stride, int n_frames,
         }
         for (int f = n_frames; f < kSeqInlineFrames; ++f) ip.loc[f] = ip.fin[f] = h_pose_loc[0];
         if (seq_out)
-            return launch_row_clusters(k_frame_seq<true, true>, grid, tiles, stream, a, labels, map0, map1, out, rows,
+            return launch_row_clusters(k_frame_seq<true, true, kBulk>, grid, tiles, stream, a, labels, map0, map1, out, rows,
                                        cols, n_exact, ip, *seq_out);
-        return launch_row_clusters(k_frame_seq<true, false>, grid, tiles, stream, a, labels, map0, map1, out, rows, cols,
+        return launch_row_clusters(k_frame_seq<true, false, kBulk>, grid, tiles, stream, a, labels, map0, map1, out, rows, cols,
                                    n_exact, ip, no_out);
     }
     static const SeqInlinePoses none = {};
     if (seq_out)
-        return launch_row_clusters(k_frame_seq<false, true>, grid, tiles, stream, a, labels, map0, map1, out, rows, cols,
+        return launch_row_clusters(k_frame_seq<false, true, kBulk>, grid, tiles, stream, a, labels, map0, map1, out, rows, cols,
                                    n_exact, none, *seq_out);
-    return launch_row_clusters(k_frame_seq<false, false>, grid, tiles, stream, a, labels, map0, map1, out, rows, cols,
+    return launch_row_clusters(k_frame_seq<false, false, kBulk>, grid, tiles, stream, a, labels, map0, map1, out, rows, cols,
                                n_exact, none, no_out);
+}
+
+// h_pose_loc / h_pose_fin != null (n_seq == 1, n_frames <= frame_seq_inline_frames()): the poses are passed as
+// kernel parameters and the device arrays are not read.  seq_out != null: the output mode of k_frame_seq.
+int launch_frame_seq(const double *frames, long long frame_stride, int n_frames, int *labels, const RowMap &map0,
+                     const RowMap &map1, const MatchOut &out, const PoseXf *d_pose_loc, const PoseXf *d_pose_fin,
+                     int n_seq, int rows, int cols, unsigned *n_exact, cudaStream_t stream, const PoseXf *h_pose_loc,
+                     const PoseXf *h_pose_fin, const SeqOut *seq_out, bool *bulk_out) {
+    const bool bulk = frame_seq_bulk_ok(frames, frame_stride, map0, map1, cols);
+    if (bulk_out) *bulk_out = bulk;
+    return bulk ? launch_frame_seq_variant<true>(frames, frame_stride, n_frames, labels, map0, map1, out, d_pose_loc,
+                                                 d_pose_fin, n_seq, rows, cols, n_exact, stream, h_pose_loc, h_pose_fin,
+                                                 seq_out)
+                : launch_frame_seq_variant<false>(frames, frame_stride, n_frames, labels, map0, map1, out, d_pose_loc,
+                                                  d_pose_fin, n_seq, rows, cols, n_exact, stream, h_pose_loc,
+                                                  h_pose_fin, seq_out);
 }
 
 // Fit totals of frame blockIdx.x, sequence blockIdx.y: part = [n_frames][n_seq][n_part][5] partials, stats =

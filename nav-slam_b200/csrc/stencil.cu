@@ -14,6 +14,7 @@
 // reference evaluates 8).  Algorithmic traffic: 24 B read + 4 B written per point (SURVEY 8d).
 #include <stdlib.h>
 
+#include "nav_bulk.cuh"
 #include "nav_kernels.cuh"
 #include "stencil_tile.cuh"
 
@@ -62,44 +63,6 @@ constexpr int kTileOut = kWarps * kWarpOut;  // 240 output points per tile
 constexpr int kTileIn = kTileOut + 2 * kHalo;
 constexpr int kTileInBytes = kTileIn * 24;
 static_assert(kTileInBytes % 16 == 0 && (kTileOut * 24) % 16 == 0, "bulk copies move multiples of 16 bytes");
-
-__device__ __forceinline__ unsigned smem_u32(const void *p) { return (unsigned)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(unsigned long long *bar, unsigned count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(unsigned long long *bar, unsigned bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(unsigned long long *bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(unsigned long long *bar, unsigned parity) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "WAIT_%=:\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1, %2;\n\t"
-        "@p bra DONE_%=;\n\t"
-        "bra WAIT_%=;\n\t"
-        "DONE_%=:\n\t}" ::"r"(smem_u32(bar)), "r"(parity), "r"(0x989680u) : "memory");  // suspend-time hint
-}
-__device__ __forceinline__ void mbar_wait_addr(unsigned bar_addr, unsigned parity) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "WAIT_%=:\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1, %2;\n\t"
-        "@p bra DONE_%=;\n\t"
-        "bra WAIT_%=;\n\t"
-        "DONE_%=:\n\t}" ::"r"(bar_addr), "r"(parity), "r"(0x989680u) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_addr(unsigned bar_addr) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar_addr) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(void *dst, const void *src, unsigned bytes, unsigned long long *bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                     smem_u32(dst)),
-                 "l"(src), "r"(bytes), "r"(smem_u32(bar))
-                 : "memory");
-}
 
 // Measured on the 1000-image batch (share of the measured HBM peak): 6 CTAs/SM (40 registers, spills)
 // 66.8 %, 5 CTAs/SM (48 registers) 72.5 %, 4 CTAs/SM (54 registers) 73.8 %; the same ring with the
