@@ -462,6 +462,37 @@ typedef struct {
 int nav_slam_run_dev(nav_ctx *ctx, const void *dev_frames, int n_frames, const nav_pos *deltas,
                      const nav_pos *pos_start, const nav_run_dev_out *out);
 
+/* ---- device-resident recordings in the sensors' own formats ----------------------------------------------------
+ * The _ex forms of nav_slam_init_dev, nav_frontend_sequence_dev / nav_frontend_sequence_out_dev and nav_slam_run_dev
+ * take the frames as the two sensors give them, so that a recording needs no widening to xyz doubles in HBM
+ * (a 64x2048 frame is 512 KB as depth and 1.5 MB as integer mm against 3 MB as xyz).  input_kind:
+ *   - NAV_RUN_INPUT_XYZ: nav_point [n_frames][n_seq][rows][cols], the xyz calls themselves;
+ *   - NAV_RUN_INPUT_DEPTH: int32 [n_frames][n_seq][rows][cols] in the reference's `distances` units, converted as
+ *     nav_convert_to_pointcloud converts them (utils/pointcloud.c; d <= 0 becomes (0, 0, 0)), for every n_seq;
+ *   - NAV_RUN_INPUT_MM: int32 [n_frames][n_seq][rows][cols][3] whole millimetres, widened exactly to doubles.
+ * Contract: each call returns, bit for bit, what its xyz form returns on the clouds the frames stand for -- every ring
+ * of nav_sequence_out, the poses, errors and fit totals of nav_run_dev_out, and the context state afterwards.
+ * The conversion runs inside the kernels where one sequence of rows up to 2048 columns is replayed in one launch
+ * (each tile staged raw and converted where it is read) and in the closed loop (still n_frames + 1 launches).  The
+ * per-frame replay (n_seq > 1, rows wider than 2048 columns, NAV_SEQ_LAUNCHES, the profiler, n_frames == 1) converts
+ * each frame into a context buffer of two frames first: two launches per frame (conversion, frame kernel), plus the
+ * copies and dedupe of nav_frontend_sequence_out_dev, without the overlap of consecutive frame kernels that xyz frames
+ * get; the buffer (48 B per pixel of a frame) is allocated by the first such call.
+ * Refused (non-zero return, an error naming the cause, nothing queued, the context unchanged): an input_kind other
+ * than 0, 1 or 2 (unlike nav_slam_run, which takes every non-zero value other than NAV_RUN_INPUT_MM for depth); a
+ * frame pointer off its element's alignment (4 bytes for int32, 8 for xyz); and everything the xyz forms refuse. */
+/* nav_slam_init_dev on a frame of input_kind: the frame is converted into the context's cloud buffer, then labelled
+ * and mapped. */
+int nav_slam_init_dev_ex(nav_ctx *ctx, const void *dev_frame, int input_kind, const nav_pos *pos);
+/* nav_frontend_sequence_out_dev (out may be NULL: nav_frontend_sequence_dev) on frames of input_kind. */
+int nav_frontend_sequence_dev_ex(nav_ctx *ctx, const void *dev_frames, int input_kind, size_t n_frames,
+                                 const nav_pos *pos_predict, const nav_pos *pos_last, const nav_pos *pos_final,
+                                 const nav_sequence_out *out);
+/* nav_slam_run_dev on frames of input_kind: for n_seq == 1 the results equal nav_slam_run(ctx, host copies of the
+ * same frames, NAV_RUN_INPUT_DEPTH / NAV_RUN_INPUT_MM, ...) bit for bit. */
+int nav_slam_run_dev_ex(nav_ctx *ctx, const void *dev_frames, int input_kind, int n_frames, const nav_pos *deltas,
+                        const nav_pos *pos_start, const nav_run_dev_out *out);
+
 /* copy out the map the context holds for one (sequence,row): the labelled global points of the
  * frame mapped last, compacted in column order (= the flattenedPoints array of src/slam.c:170-171),
  * and the column each came from.  pts_out needs room for cols points; col_out may be NULL. */

@@ -70,7 +70,7 @@ EXPORTS = [
     "nav_peer_create", "nav_peer_connect", "nav_kdtree_nn_allgather_dev", "nav_kdtree_nn_sharded_map_dev", "nav_peer_check",
     "nav_peer_destroy", "nav_shard_range", "nav_shard_owner",
     "nav_frontend_frame_mm", "nav_frontend_submit_mm", "nav_slam_prefetch_mm", "nav_l9_csv_read_mm",
-    "nav_slam_run_dev",
+    "nav_slam_run_dev", "nav_slam_init_dev_ex", "nav_frontend_sequence_dev_ex", "nav_slam_run_dev_ex",
 ]
 
 
@@ -151,6 +151,11 @@ def load_library(build_if_missing: bool = True):
     L.nav_slam_run.argtypes = [vp, C.POINTER(C.c_void_p), C.c_int, C.c_int, vp, vp, C.POINTER(NavPos),
                                C.POINTER(NavPos), C.POINTER(NavPos), C.POINTER(C.c_double), C.POINTER(C.c_size_t)]
     L.nav_slam_run_dev.argtypes = [vp, vp, C.c_int, C.POINTER(NavPos), C.POINTER(NavPos), C.POINTER(NavRunDevOut)]
+    L.nav_slam_init_dev_ex.argtypes = [vp, vp, C.c_int, C.POINTER(NavPos)]
+    L.nav_frontend_sequence_dev_ex.argtypes = [vp, vp, C.c_int, C.c_size_t, C.POINTER(NavPos), C.POINTER(NavPos),
+                                               C.POINTER(NavPos), C.POINTER(NavSequenceOut)]
+    L.nav_slam_run_dev_ex.argtypes = [vp, vp, C.c_int, C.c_int, C.POINTER(NavPos), C.POINTER(NavPos),
+                                      C.POINTER(NavRunDevOut)]
     L.nav_peer_create.restype = C.c_void_p
     L.nav_peer_create.argtypes = [C.c_int, C.c_size_t, C.c_char_p]
     L.nav_peer_connect.argtypes = [vp, C.c_int, C.c_int, C.c_char_p]
@@ -462,13 +467,16 @@ class Context:
 
     RUN_INPUT_XYZ, RUN_INPUT_DEPTH, RUN_INPUT_MM = 0, 1, 2  # NAV_RUN_INPUT_* of include/navslam_b200.h
 
+    def _input_kind(self, name, depth_input, mm_input):
+        if depth_input and mm_input:
+            raise ValueError(f"{name}: depth_input and mm_input exclude each other")
+        return self.RUN_INPUT_DEPTH if depth_input else self.RUN_INPUT_MM if mm_input else self.RUN_INPUT_XYZ
+
     def slam_run(self, frame_ptrs, deltas, pos_start, depth_input=False, mm_input=False):
         """nav_slam_run: the closed loop over pinned host frames (raw pointers) with dead-reckoning increments
         deltas[t] (prediction = last pose + deltas[t]).  Frames are clouds, depth matrices (depth_input) or int32
         integer-mm clouds (mm_input).  Returns (poses [n,6], rms [n], n_corr [n])."""
-        if depth_input and mm_input:
-            raise ValueError("slam_run: depth_input and mm_input exclude each other")
-        kind = self.RUN_INPUT_DEPTH if depth_input else self.RUN_INPUT_MM if mm_input else self.RUN_INPUT_XYZ
+        kind = self._input_kind("slam_run", depth_input, mm_input)
         n = len(frame_ptrs)
         ptrs = (C.c_void_p * n)(*[int(p) for p in frame_ptrs])
         d = (NavPos * n)(*[NavPos(*[float(v) for v in row]) for row in np.asarray(deltas, dtype=np.float64).reshape(n, 6)])
@@ -497,40 +505,65 @@ class Context:
     def extract_feature_batch_dev(self, dev_clouds_ptr, n_images, dev_labels_ptr):
         _check(self.L.nav_extract_feature_batch_dev(self.h, dev_clouds_ptr, n_images, dev_labels_ptr), self.L)
 
-    def slam_init_dev(self, dev_cloud_ptr, pos):
-        _check(self.L.nav_slam_init_dev(self.h, dev_cloud_ptr, _pos_array(pos, self.n_seq)), self.L)
+    def slam_init_dev(self, dev_cloud_ptr, pos, depth_input=False, mm_input=False):
+        """nav_slam_init_dev_ex: the map of one device-resident frame -- an xyz cloud, int32 depth matrices
+        (depth_input) or an int32 integer-mm cloud (mm_input)."""
+        kind = self._input_kind("slam_init_dev", depth_input, mm_input)
+        pos = _pos_array(pos, self.n_seq)
+        if kind == self.RUN_INPUT_XYZ:
+            _check(self.L.nav_slam_init_dev(self.h, dev_cloud_ptr, pos), self.L)
+        else:
+            _check(self.L.nav_slam_init_dev_ex(self.h, dev_cloud_ptr, kind, pos), self.L)
 
     def frontend_frame_dev(self, dev_cloud_ptr, pos_predict, pos_last, pos_final):
         n = self.n_seq
         _check(self.L.nav_frontend_frame_dev(self.h, dev_cloud_ptr, _pos_array(pos_predict, n),
                                              _pos_array(pos_last, n), _pos_array(pos_final, n)), self.L)
 
-    def frontend_sequence_dev(self, dev_frames_ptr, n_frames, pos_predict, pos_last, pos_final):
+    def frontend_sequence_dev(self, dev_frames_ptr, n_frames, pos_predict, pos_last, pos_final, depth_input=False,
+                              mm_input=False):
+        """nav_frontend_sequence_dev[_ex] (out = NULL): the replay of n_frames device-resident frames -- xyz clouds,
+        int32 depth matrices (depth_input) or int32 integer-mm clouds (mm_input)."""
+        kind = self._input_kind("frontend_sequence_dev", depth_input, mm_input)
         n = n_frames * self.n_seq
-        _check(self.L.nav_frontend_sequence_dev(self.h, dev_frames_ptr, n_frames, _pos_array(pos_predict, n),
-                                                _pos_array(pos_last, n), _pos_array(pos_final, n)), self.L)
+        poses = (_pos_array(pos_predict, n), _pos_array(pos_last, n), _pos_array(pos_final, n))
+        if kind == self.RUN_INPUT_XYZ:
+            _check(self.L.nav_frontend_sequence_dev(self.h, dev_frames_ptr, n_frames, *poses), self.L)
+        else:
+            _check(self.L.nav_frontend_sequence_dev_ex(self.h, dev_frames_ptr, kind, n_frames, *poses, None), self.L)
 
     def frontend_sequence_out_dev(self, dev_frames_ptr, n_frames, pos_predict, pos_last, pos_final, label_mask=None,
-                                  nn_idx=None, nn_dist=None, fit_stats=None):
-        """nav_frontend_sequence_out_dev: the replay of frontend_sequence_dev keeping every frame's results in the
-        given device buffers (ints; None = not wanted).  With all four None the call passes out = NULL."""
+                                  nn_idx=None, nn_dist=None, fit_stats=None, depth_input=False, mm_input=False):
+        """nav_frontend_sequence_out_dev / nav_frontend_sequence_dev_ex: the replay of frontend_sequence_dev keeping
+        every frame's results in the given device buffers (ints; None = not wanted).  With all four None the call
+        passes out = NULL."""
+        kind = self._input_kind("frontend_sequence_out_dev", depth_input, mm_input)
         n = n_frames * self.n_seq
         fields = (label_mask, nn_idx, nn_dist, fit_stats)
         out = None if all(v is None for v in fields) else C.byref(NavSequenceOut(*fields))
-        _check(self.L.nav_frontend_sequence_out_dev(self.h, dev_frames_ptr, n_frames, _pos_array(pos_predict, n),
-                                                    _pos_array(pos_last, n), _pos_array(pos_final, n), out), self.L)
+        poses = (_pos_array(pos_predict, n), _pos_array(pos_last, n), _pos_array(pos_final, n))
+        if kind == self.RUN_INPUT_XYZ:
+            _check(self.L.nav_frontend_sequence_out_dev(self.h, dev_frames_ptr, n_frames, *poses, out), self.L)
+        else:
+            _check(self.L.nav_frontend_sequence_dev_ex(self.h, dev_frames_ptr, kind, n_frames, *poses, out), self.L)
 
-    def slam_run_dev(self, dev_frames_ptr, n_frames, deltas, pos_start, poses_ptr, error_ptr=None, stats_ptr=None):
-        """nav_slam_run_dev: the closed loop over n_frames device-resident xyz frames [n_frames][n_seq][rows][cols][3]
-        with the pose fit on the GPU.  deltas [n_frames][n_seq][6] (prediction = last pose + deltas[t]), pos_start
-        [n_seq][6]; the outputs are device buffers (ints): poses nav_pos [n_frames][n_seq], error double
-        [n_frames][n_seq] and stats double [n_frames][n_seq][5] (None = not wanted).  Queued on the context's stream;
-        the outputs are complete after synchronize()."""
+    def slam_run_dev(self, dev_frames_ptr, n_frames, deltas, pos_start, poses_ptr, error_ptr=None, stats_ptr=None,
+                     depth_input=False, mm_input=False):
+        """nav_slam_run_dev_ex: the closed loop over n_frames device-resident frames [n_frames][n_seq][rows][cols] --
+        xyz clouds, int32 depth matrices (depth_input) or int32 integer-mm clouds (mm_input) -- with the pose fit on
+        the GPU.  deltas [n_frames][n_seq][6] (prediction = last pose + deltas[t]), pos_start [n_seq][6]; the outputs
+        are device buffers (ints): poses nav_pos [n_frames][n_seq], error double [n_frames][n_seq] and stats double
+        [n_frames][n_seq][5] (None = not wanted).  Queued on the context's stream; the outputs are complete after
+        synchronize()."""
+        kind = self._input_kind("slam_run_dev", depth_input, mm_input)
         n = n_frames * self.n_seq
         d = _pos_array(deltas, n) if n > 0 else (NavPos * 1)()
         out = NavRunDevOut(poses_ptr, error_ptr, stats_ptr)
-        _check(self.L.nav_slam_run_dev(self.h, dev_frames_ptr, n_frames, d, _pos_array(pos_start, self.n_seq),
-                                       C.byref(out)), self.L)
+        start = _pos_array(pos_start, self.n_seq)
+        if kind == self.RUN_INPUT_XYZ:
+            _check(self.L.nav_slam_run_dev(self.h, dev_frames_ptr, n_frames, d, start, C.byref(out)), self.L)
+        else:
+            _check(self.L.nav_slam_run_dev_ex(self.h, dev_frames_ptr, kind, n_frames, d, start, C.byref(out)), self.L)
 
     def frame_results_dev(self) -> NavFrameResults:
         r = NavFrameResults()

@@ -291,6 +291,9 @@ struct nav_ctx {
     size_t d_loop_cap = 0;
     unsigned *d_loop_ticket = nullptr;
     int *d_labels_alt = nullptr;
+    // depth / integer-mm frames of a per-frame replay, converted to xyz: two frame slots, so that a conversion never
+    // overwrites the frame a kernel still in flight reads (lazy)
+    double *d_conv = nullptr;
     bool fit_tables_queued = false;  // the fit's bias tables were uploaded on the context's stream (nav_set_stream
                                      // synchronises the old stream, so a later stream finds them in place)
     // NAV_RUN_TRACE=1: nav_slam_run prints where the host side of the closed loop spends its time
@@ -407,7 +410,7 @@ extern "C" void nav_destroy(nav_ctx *c) {
     }
     if (c->d_pose) cudaFree(c->d_pose);
     if (c->d_seq_part) cudaFree(c->d_seq_part);
-    for (void *p : {c->d_loop, (void *)c->d_loop_ticket, (void *)c->d_labels_alt})
+    for (void *p : {c->d_loop, (void *)c->d_loop_ticket, (void *)c->d_labels_alt, (void *)c->d_conv})
         if (p) cudaFree(p);
     if (c->d_fit_ticket) cudaFree(c->d_fit_ticket);
     if (c->s_in) cudaStreamDestroy(c->s_in);
@@ -857,7 +860,7 @@ extern "C" int nav_convert_to_pointcloud(nav_ctx *c, const int *distances, nav_p
     if (!distances || !cloud_out) return fail("nav_convert_to_pointcloud: null argument");
     if (c->stage.reserve(c->npx * 28 + 512, c->stream)) return fail("nav_convert_to_pointcloud: staging");
     if (c->stage.h2d(c->d_dist, distances, c->npx * 4, c->stream)) return fail("nav_convert_to_pointcloud: H2D");
-    launch_convert(c->d_dist, c->d_tan_col, c->d_tan_row, c->d_cloud, c->rows, c->cols, c->sm_count, c->stream);
+    launch_convert(c->d_dist, c->d_tan_col, c->d_tan_row, c->d_cloud, c->rows, c->cols, 1, c->sm_count, c->stream);
     c->launches++;
     c->cloud_resident = false;
     if (c->stage.d2h(cloud_out, c->d_cloud, c->npx * 24, c->stream)) return fail("nav_convert_to_pointcloud: D2H");
@@ -960,15 +963,60 @@ extern "C" int nav_slam_init(nav_ctx *c, const nav_pos *pos, const nav_point *cl
     return finish_call(c, "nav_slam_init");
 }
 
-extern "C" int nav_slam_init_dev(nav_ctx *c, const void *dev_cloud, const nav_pos *pos) {
-    CTX_ENTER(c, "nav_slam_init_dev");
-    if (!pos || !dev_cloud) return fail("nav_slam_init_dev: null argument");
+// The frame formats of the device-resident calls (NAV_RUN_INPUT_*): a kind other than the three, or a frame pointer
+// off its element's alignment (8 bytes for xyz doubles, 4 for int32), is refused before anything is queued.
+static int check_frame_input(const char *name, const void *frames, int kind) {
+    if (kind != NAV_RUN_INPUT_XYZ && kind != NAV_RUN_INPUT_DEPTH && kind != NAV_RUN_INPUT_MM)
+        return fail("%s: input_kind %d is none of NAV_RUN_INPUT_XYZ (0), NAV_RUN_INPUT_DEPTH (1), NAV_RUN_INPUT_MM (2)",
+                    name, kind);
+    const unsigned align = kind == NAV_RUN_INPUT_XYZ ? 8u : 4u;
+    if (((uintptr_t)frames & (align - 1u)) != 0)
+        return fail("%s: the frame pointer %p is not %u-byte aligned", name, frames, align);
+    return 0;
+}
+
+// elements between consecutive frames of a device-resident recording: doubles for xyz, int32 otherwise
+static long long frame_stride_elems(const nav_ctx *c, int kind) {
+    return (long long)c->ntot * (kind == NAV_RUN_INPUT_DEPTH ? 1 : 3);
+}
+
+// one depth or integer-mm frame (n_seq images) -> xyz doubles at dst, on the context's stream: k_convert (a2) or
+// k_widen_mm, the arithmetic the in-kernel conversion of k_frame_seq / k_loop_step shares
+static void convert_frame(nav_ctx *c, const void *src, int kind, double *dst) {
+    if (kind == NAV_RUN_INPUT_DEPTH)
+        launch_convert((const int *)src, c->d_tan_col, c->d_tan_row, dst, c->rows, c->cols, c->n_seq, c->sm_count,
+                       c->stream);
+    else
+        launch_widen_mm((const int *)src, dst, (long long)c->ntot, c->sm_count, c->stream);
+    c->launches++;
+}
+
+// nav_slam_init_dev (xyz) and nav_slam_init_dev_ex; `name` is the entry point the caller used
+static int slam_init_dev(nav_ctx *c, const char *name, const void *dev_frame, int kind, const nav_pos *pos) {
+    if (!pos || !dev_frame) return fail("%s: null argument", name);
+    if (check_frame_input(name, dev_frame, kind)) return 1;
     for (auto &ps : c->pre) ps.pending = false;
-    run_labels(c, (const double *)dev_cloud, c->d_labels, nullptr, c->n_seq);
-    run_map(c, (const double *)dev_cloud, c->d_labels, pose_batch(c, pos, nullptr));
+    const double *cloud = (const double *)dev_frame;
+    if (kind != NAV_RUN_INPUT_XYZ) {  // converted into the context's cloud buffer, then labelled and mapped as xyz
+        order_after_async(c);
+        convert_frame(c, dev_frame, kind, c->d_cloud);
+        cloud = c->d_cloud;
+    }
+    run_labels(c, cloud, c->d_labels, nullptr, c->n_seq);
+    run_map(c, cloud, c->d_labels, pose_batch(c, pos, nullptr));
     c->cloud_resident = false;
     CU(cudaGetLastError());
     return 0;
+}
+
+extern "C" int nav_slam_init_dev(nav_ctx *c, const void *dev_cloud, const nav_pos *pos) {
+    CTX_ENTER(c, "nav_slam_init_dev");
+    return slam_init_dev(c, "nav_slam_init_dev", dev_cloud, NAV_RUN_INPUT_XYZ, pos);
+}
+
+extern "C" int nav_slam_init_dev_ex(nav_ctx *c, const void *dev_frame, int input_kind, const nav_pos *pos) {
+    CTX_ENTER(c, "nav_slam_init_dev_ex");
+    return slam_init_dev(c, "nav_slam_init_dev_ex", dev_frame, input_kind, pos);
 }
 
 extern "C" int nav_slam_match(nav_ctx *c, const nav_point *cloud, const nav_pos *pos_predict,
@@ -1106,7 +1154,7 @@ static int prefetch_common(nav_ctx *c, const char *name, InputKind kind, const v
     if (kind == kInputDepth) {
         if (!ps.d_depth) CU(cudaMalloc((void **)&ps.d_depth, c->npx * 4));
         CU(cudaMemcpyAsync(ps.d_depth, src, c->npx * 4, cudaMemcpyHostToDevice, c->s_in));
-        launch_convert(ps.d_depth, c->d_tan_col, c->d_tan_row, ps.d_cloud, c->rows, c->cols, c->sm_count, c->s_in);
+        launch_convert(ps.d_depth, c->d_tan_col, c->d_tan_row, ps.d_cloud, c->rows, c->cols, 1, c->sm_count, c->s_in);
         c->launches++;
     } else if (kind == kInputMm) {
         if (!ps.d_mm) CU(cudaMalloc((void **)&ps.d_mm, c->ntot * 12));
@@ -1394,13 +1442,14 @@ static bool on_ctx_device(const nav_ctx *c, const void *p);
 // record -- and the last CTA of each sequence fits the pose and writes the record of frame t+1; one more launch maps
 // the last frame.  Only the translation depends on the fit, so every rotation (and the fitted roll / pitch / yaw)
 // is formed here up front with the host libm, exactly as make_pose forms it in nav_slam_run.
-extern "C" int nav_slam_run_dev(nav_ctx *c, const void *dev_frames, int n_frames, const nav_pos *deltas,
-                                const nav_pos *pos_start, const nav_run_dev_out *out) {
-    static const char *name = "nav_slam_run_dev";
-    CTX_ENTER(c, "nav_slam_run_dev");
-    REFUSE_UNDER_REF_TIES(c, "nav_slam_run_dev");
+// Depth and integer-mm frames are read raw by the same kernel (k_loop_step<true, kind>), converted where the tile is
+// staged and where the previous frame is mapped: still n_frames + 1 launches.  `name`: the entry point the caller used.
+static int slam_run_dev(nav_ctx *c, const char *name, const void *dev_frames, int kind, int n_frames,
+                        const nav_pos *deltas, const nav_pos *pos_start, const nav_run_dev_out *out) {
+    REFUSE_UNDER_REF_TIES(c, name);
     if (!dev_frames || !deltas || !pos_start || !out || !out->poses)
         return fail("%s: null argument (dev_frames, deltas, pos_start, out and out->poses are required)", name);
+    if (check_frame_input(name, dev_frames, kind)) return 1;
     if (n_frames < 0) return fail("%s: n_frames = %d is negative", name, n_frames);
     if (!row_cluster_supported(c->cols))
         return fail("%s: rows of %d columns are wider than one thread-block cluster (2048 columns at most)", name,
@@ -1485,22 +1534,36 @@ extern "C" int nav_slam_run_dev(nav_ctx *c, const void *dev_frames, int n_frames
     // the label ring: frame t's labels go where the launch of frame t+1 maps them from; the last frame's land in
     // d_labels, as nav_frame_results_dev reports them
     auto labels_of = [&](int t) { return ((n_frames - 1 - t) & 1) ? c->d_labels_alt : c->d_labels; };
-    const double *frames = (const double *)dev_frames;
-    const long long stride = (long long)c->ntot * 3;
+    const size_t elem = kind == NAV_RUN_INPUT_XYZ ? sizeof(double) : sizeof(int);
+    const long long stride = frame_stride_elems(c, kind);
+    auto frame = [&](int t) { return (const void *)((const unsigned char *)dev_frames + (size_t)t * stride * elem); };
     const MatchOut mo = {c->d_nn_idx, c->d_nn_dist, c->d_corr_rows, c->d_corr_row_count};
+    const TanTables tan = {c->d_tan_col, c->d_tan_row};
     for (int t = 0; t <= n_frames; ++t) {  // t == n_frames: the last frame's map
         const bool match = t < n_frames;
         const DevLoop dl = {t, n_frames, ns, match ? 1 : 0, match ? labels_of(t) : nullptr, d_rec[t & 1],
                             d_rec[(t + 1) & 1], d_tab, c->d_loop_ticket, c->d_n_exact, (nav_pos *)out->poses,
                             out->error, out->fit_stats};
-        CU((cudaError_t)launch_loop_step_dev(dl, match ? frames + t * stride : nullptr,
-                                             t > 0 ? frames + (t - 1) * stride : nullptr, t > 0 ? labels_of(t - 1) : nullptr,
-                                             t > 0, c->map, mo, ns, c->rows, c->cols, c->d_tile_stats, c->stream));
+        CU((cudaError_t)launch_loop_step_dev(kind, dl, match ? frame(t) : nullptr, t > 0 ? frame(t - 1) : nullptr,
+                                             t > 0 ? labels_of(t - 1) : nullptr, t > 0, c->map, mo, ns, c->rows, c->cols,
+                                             c->d_tile_stats, c->stream, tan));
         c->launches++;
     }
     c->cloud_resident = false;
     CU(cudaGetLastError());
     return 0;
+}
+
+extern "C" int nav_slam_run_dev(nav_ctx *c, const void *dev_frames, int n_frames, const nav_pos *deltas,
+                                const nav_pos *pos_start, const nav_run_dev_out *out) {
+    CTX_ENTER(c, "nav_slam_run_dev");
+    return slam_run_dev(c, "nav_slam_run_dev", dev_frames, NAV_RUN_INPUT_XYZ, n_frames, deltas, pos_start, out);
+}
+
+extern "C" int nav_slam_run_dev_ex(nav_ctx *c, const void *dev_frames, int input_kind, int n_frames,
+                                   const nav_pos *deltas, const nav_pos *pos_start, const nav_run_dev_out *out) {
+    CTX_ENTER(c, "nav_slam_run_dev_ex");
+    return slam_run_dev(c, "nav_slam_run_dev_ex", dev_frames, input_kind, n_frames, deltas, pos_start, out);
 }
 
 // test seam: how the last nav_frontend_sequence_dev / nav_frontend_sequence_out_dev of the context ran -- 0: one
@@ -1563,7 +1626,7 @@ static int frontend_frame(nav_ctx *c, const char *name, const nav_point *cloud, 
         return fail("%s: staging", name);
     if (distances) {
         if (c->stage.h2d(c->d_dist, distances, c->npx * 4, c->stream)) return fail("%s: H2D", name);
-        launch_convert(c->d_dist, c->d_tan_col, c->d_tan_row, c->d_cloud, c->rows, c->cols, c->sm_count, c->stream);
+        launch_convert(c->d_dist, c->d_tan_col, c->d_tan_row, c->d_cloud, c->rows, c->cols, 1, c->sm_count, c->stream);
         c->launches++;
     } else if (cloud_mm) {
         if (!c->d_mm) CU(cudaMalloc((void **)&c->d_mm, c->ntot * 12));
@@ -1804,7 +1867,7 @@ static int frontend_submit(nav_ctx *c, const char *name, const int32_t *cloud_mm
         launch_widen_mm(sl.d_mm, sl.d_cloud, (long long)c->ntot, c->sm_count, c->stream);
         c->launches++;
     } else if (io->distances) {  // a2 on the device: 4 B/pixel crossed PCIe instead of 24
-        launch_convert(sl.d_depth, c->d_tan_col, c->d_tan_row, sl.d_cloud, c->rows, c->cols, c->sm_count, c->stream);
+        launch_convert(sl.d_depth, c->d_tan_col, c->d_tan_row, sl.d_cloud, c->rows, c->cols, 1, c->sm_count, c->stream);
         c->launches++;
     }
     if (run_frame_fused(c, sl.d_cloud, sl.d_labels, sl.d_nn_idx, sl.d_nn_dist, pos_predict, pos_last, pos_final)) return 1;
@@ -1930,11 +1993,14 @@ static bool on_ctx_device(const nav_ctx *c, const void *p) {
     return (a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged) && a.device == c->device;
 }
 
-// nav_frontend_sequence_dev, and with per-frame outputs (so != null) nav_frontend_sequence_out_dev
-static int frontend_sequence(nav_ctx *c, const char *name, const void *dev_frames, size_t n_frames,
+// nav_frontend_sequence_dev, and with per-frame outputs (so != null) nav_frontend_sequence_out_dev; their _ex forms
+// with a frame kind (NAV_RUN_INPUT_*).  `name`: the entry point the caller used.
+static int frontend_sequence(nav_ctx *c, const char *name, const void *dev_frames, int kind, size_t n_frames,
                              const nav_pos *pos_predict, const nav_pos *pos_last, const nav_pos *pos_final,
                              const nav_sequence_out *so) {
+    REFUSE_UNDER_REF_TIES(c, name);
     if (!dev_frames || !pos_predict || !pos_last || !pos_final) return fail("%s: null argument", name);
+    if (check_frame_input(name, dev_frames, kind)) return 1;
     if (!c->have_map) return fail("%s: call nav_slam_init_dev first", name);
     if (so) {
         const std::pair<const void *, const char *> fields[] = {
@@ -1944,7 +2010,8 @@ static int frontend_sequence(nav_ctx *c, const char *name, const void *dev_frame
                 return fail("%s: out->%s is not device or managed memory on device %d", name, fd.second, c->device);
         if (!so->label_mask && !so->nn_idx && !so->nn_dist && !so->fit_stats) so = nullptr;
     }
-    const double *base = (const double *)dev_frames;
+    const bool raw = kind != NAV_RUN_INPUT_XYZ;
+    const long long stride = frame_stride_elems(c, kind);
     order_after_async(c);
     // One launch for the whole sequence (k_frame_seq: a thread-block cluster per image row walks through the
     // frames with a cluster barrier per frame) when a row's tiles fit a cluster; NAV_SEQ_LAUNCHES=1 keeps one
@@ -1975,6 +2042,9 @@ static int frontend_sequence(nav_ctx *c, const char *name, const void *dev_frame
     }
     const SeqOut seq_out = {so ? (unsigned *)so->label_mask : nullptr, so ? (int *)so->nn_idx : nullptr,
                             so ? (double *)so->nn_dist : nullptr, part};
+    const TanTables tan = {c->d_tan_col, c->d_tan_row};
+    // the per-frame path converts depth / integer-mm frames into two context-owned frame slots first
+    if (!fused && raw && n_frames > 0 && !c->d_conv) CU(cudaMalloc((void **)&c->d_conv, c->ntot * 24 * 2));
     c->seq_path = 0;
     if (fused) {
         bool bulk = false;
@@ -1988,9 +2058,9 @@ static int frontend_sequence(nav_ctx *c, const char *name, const void *dev_frame
                 loc[i] = make_pose(&pos_predict[i], &pos_last[i]);
                 fin[i] = make_pose(&pos_final[i], nullptr);
             }
-            CU((cudaError_t)launch_frame_seq(base, (long long)c->ntot * 3, (int)n_frames, c->d_labels, c->map, c->map_alt, out,
+            CU((cudaError_t)launch_frame_seq(kind, dev_frames, stride, (int)n_frames, c->d_labels, c->map, c->map_alt, out,
                                              nullptr, nullptr, c->n_seq, c->rows, c->cols, c->d_n_exact, c->stream, loc, fin,
-                                             so ? &seq_out : nullptr, &bulk));
+                                             so ? &seq_out : nullptr, &bulk, tan));
         } else {
             nav_ctx::PoseRing &pr = c->pose_ring[c->pose_ring_next];
             c->pose_ring_next = (c->pose_ring_next + 1) % nav_ctx::kPoseRing;
@@ -2018,9 +2088,10 @@ static int frontend_sequence(nav_ctx *c, const char *name, const void *dev_frame
             }
             CU(cudaMemcpyAsync(c->d_pose, pr.host, bytes, cudaMemcpyHostToDevice, c->stream));
             CU(cudaEventRecord(pr.done, c->stream));
-            CU((cudaError_t)launch_frame_seq(base, (long long)c->ntot * 3, (int)n_frames, c->d_labels, c->map, c->map_alt, out,
+            CU((cudaError_t)launch_frame_seq(kind, dev_frames, stride, (int)n_frames, c->d_labels, c->map, c->map_alt, out,
                                              (const PoseXf *)c->d_pose, (const PoseXf *)c->d_pose + n_pose, c->n_seq, c->rows,
-                                             c->cols, c->d_n_exact, c->stream, nullptr, nullptr, so ? &seq_out : nullptr, &bulk));
+                                             c->cols, c->d_n_exact, c->stream, nullptr, nullptr, so ? &seq_out : nullptr, &bulk,
+                                             tan));
         }
         c->seq_path = bulk ? 2 : 1;
         c->launches++;
@@ -2028,13 +2099,18 @@ static int frontend_sequence(nav_ctx *c, const char *name, const void *dev_frame
     } else {
         const size_t n_chunks = (size_t)c->map.n_chunks;
         for (size_t f = 0; f < n_frames; ++f) {
-            const double *cl = base + f * c->ntot * 3;
+            const double *cl = (const double *)dev_frames + f * c->ntot * 3;
+            if (raw) {  // frame f into slot f % 2: the kernels of frame f-1 read the other slot
+                cl = c->d_conv + (f & 1) * c->ntot * 3;
+                convert_frame(c, (const int *)dev_frames + f * stride, kind, (double *)cl);
+            }
             const size_t o = f * (size_t)c->n_seq;
             // consecutive launches overlap (programmatic dependent launch): frame f+1 computes its labels
             // while frame f finishes its searches.  With per-frame outputs the copies and the dedupe of frame f
-            // come between them, and the launches are ordinary.
+            // come between them, and the launches are ordinary; so they are with a conversion between them, whose
+            // output the frame kernel reads in front of its dependency wait.
             if (run_frame_fused(c, cl, c->d_labels, c->d_nn_idx, c->d_nn_dist, pos_predict + o, pos_last + o, pos_final + o,
-                                /*pdl=*/!so))
+                                /*pdl=*/!so && !raw))
                 return 1;
             if (!so) continue;
             // frame f's results while the context holds them: the map just built carries its label masks, and
@@ -2076,18 +2152,24 @@ extern "C" int nav_frontend_sequence_dev(nav_ctx *c, const void *dev_frames, siz
                                          const nav_pos *pos_predict, const nav_pos *pos_last,
                                          const nav_pos *pos_final) {
     CTX_ENTER(c, "nav_frontend_sequence_dev");
-    REFUSE_UNDER_REF_TIES(c, "nav_frontend_sequence_dev");
-    return frontend_sequence(c, "nav_frontend_sequence_dev", dev_frames, n_frames, pos_predict, pos_last, pos_final,
-                             nullptr);
+    return frontend_sequence(c, "nav_frontend_sequence_dev", dev_frames, NAV_RUN_INPUT_XYZ, n_frames, pos_predict,
+                             pos_last, pos_final, nullptr);
 }
 
 extern "C" int nav_frontend_sequence_out_dev(nav_ctx *c, const void *dev_frames, size_t n_frames,
                                              const nav_pos *pos_predict, const nav_pos *pos_last,
                                              const nav_pos *pos_final, const nav_sequence_out *out) {
     CTX_ENTER(c, "nav_frontend_sequence_out_dev");
-    REFUSE_UNDER_REF_TIES(c, "nav_frontend_sequence_out_dev");
-    return frontend_sequence(c, "nav_frontend_sequence_out_dev", dev_frames, n_frames, pos_predict, pos_last, pos_final,
-                             out);
+    return frontend_sequence(c, "nav_frontend_sequence_out_dev", dev_frames, NAV_RUN_INPUT_XYZ, n_frames, pos_predict,
+                             pos_last, pos_final, out);
+}
+
+extern "C" int nav_frontend_sequence_dev_ex(nav_ctx *c, const void *dev_frames, int input_kind, size_t n_frames,
+                                            const nav_pos *pos_predict, const nav_pos *pos_last,
+                                            const nav_pos *pos_final, const nav_sequence_out *out) {
+    CTX_ENTER(c, "nav_frontend_sequence_dev_ex");
+    return frontend_sequence(c, "nav_frontend_sequence_dev_ex", dev_frames, input_kind, n_frames, pos_predict, pos_last,
+                             pos_final, out);
 }
 
 extern "C" int nav_frame_results_dev(nav_ctx *c, nav_frame_results *out) {

@@ -7,8 +7,9 @@ namespace nav {
 // ---- stencil.cu
 void launch_labels(const double *cloud, int *labels, double *curv_or_null, long long n_rows, int cols,
                    int sm_count, unsigned *n_exact, cudaStream_t stream);
+// depth matrices of n_img images [n_img][rows][cols] -> xyz clouds (a2)
 void launch_convert(const int *dist, const double *tan_col, const double *tan_row, double *out, int rows,
-                    int cols, int sm_count, cudaStream_t stream);
+                    int cols, int n_img, int sm_count, cudaStream_t stream);
 // int32 [n_points][3] (whole millimetres) -> double [n_points][3], exact
 void launch_widen_mm(const int *in, double *out, long long n_points, int sm_count, cudaStream_t stream);
 void launch_transform(const double *in, double *out, long long n, const PoseXf &pose, int sm_count,
@@ -46,18 +47,24 @@ struct FitMailbox {
 // d_pose_loc / d_pose_fin: device arrays [n_frames][n_seq].  Needs row_cluster_supported(cols).
 // seq_out (optional): per-frame outputs -- slot f of every non-null ring receives frame f (nav_sequence_out), and
 // part != null adds the statistics dedupe, CTA partials [n_frames][n_seq*rows*tiles][5] for launch_seq_fit_totals.
+// kind (NAV_RUN_INPUT_*): frames of xyz doubles, frame_stride in doubles; or depth matrices / integer-mm clouds
+// (int32, 1 or 3 per pixel), frame_stride in int32, converted inside the kernel (depth with the context's tan tables).
 int frame_seq_inline_frames();  // sequences up to this length (one sequence) carry their poses as kernel parameters
+// the context's tan tables of a2 (device memory: tan of every column, of every image row), for depth frames
+struct TanTables {
+    const double *col, *row;
+};
 struct SeqOut {
     unsigned *mask;   // [n_frames][n_seq*rows][n_chunks]
     int *nn_idx;      // [n_frames][n_seq*rows][cols]
     double *nn_dist;  // [n_frames][n_seq*rows][cols]
     double *part;     // [n_frames][n_seq*rows*tiles][5]
 };
-int launch_frame_seq(const double *frames, long long frame_stride, int n_frames, int *labels, const RowMap &map0,
+int launch_frame_seq(int kind, const void *frames, long long frame_stride, int n_frames, int *labels, const RowMap &map0,
                      const RowMap &map1, const MatchOut &out, const PoseXf *d_pose_loc, const PoseXf *d_pose_fin,
-                     int n_seq, int rows, int cols, unsigned *n_exact, cudaStream_t stream,
-                     const PoseXf *h_pose_loc = nullptr, const PoseXf *h_pose_fin = nullptr,
-                     const SeqOut *seq_out = nullptr, bool *bulk_out = nullptr);  // *bulk_out: staged by bulk copies
+                     int n_seq, int rows, int cols, unsigned *n_exact, cudaStream_t stream, const PoseXf *h_pose_loc,
+                     const PoseXf *h_pose_fin, const SeqOut *seq_out, bool *bulk_out,  // *bulk_out: staged by bulk copies
+                     const TanTables &tan);
 // fit totals stats[f][s][0..4] of the partials part[f][s][n_part][5], in the closed loop's summation order:
 // row_partials = false for tile partials (k_frame_seq, k_dedupe_stats), true for row totals (k_dedupe_rows)
 void launch_seq_fit_totals(const double *part, bool row_partials, int n_part, int n_frames, int n_seq, double *stats,
@@ -135,9 +142,10 @@ struct DevLoop {
 };
 // launch t of the device loop: cloud = frame t, prev_cloud / prev_labels = frame t-1 (do_map); part: the CTA partials
 // [n_seq*rows*tiles][5].  Needs row_cluster_supported(cols) and the fit tables (upload_fit_tables).
-int launch_loop_step_dev(const DevLoop &dl, const double *cloud, const double *prev_cloud, const int *prev_labels,
+// kind (NAV_RUN_INPUT_*): cloud / prev_cloud are xyz doubles, or depth / integer-mm int32 converted in the kernel.
+int launch_loop_step_dev(int kind, const DevLoop &dl, const void *cloud, const void *prev_cloud, const int *prev_labels,
                          bool do_map, const RowMap &map, const MatchOut &out, int n_seq, int rows, int cols,
-                         double *part, cudaStream_t stream);
+                         double *part, cudaStream_t stream, const TanTables &tan);
 // the fit's bias tables (1 - beta^t, formed on the host) into the device's constant memory, queued on `stream`
 int upload_fit_tables(const double *c1, const double *c2, cudaStream_t stream);
 // fit_translation on the device, one thread per stat vector (nav_debug_fit_from_stats_dev)

@@ -247,6 +247,11 @@ __device__ __forceinline__ void cp_async8(void *smem_dst, const void *gmem_src) 
                  "l"(gmem_src)
                  : "memory");
 }
+__device__ __forceinline__ void cp_async4(void *smem_dst, const void *gmem_src) {
+    asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"((unsigned)__cvta_generic_to_shared(smem_dst)),
+                 "l"(gmem_src)
+                 : "memory");
+}
 __device__ __forceinline__ void cp_async16(void *smem_dst, const void *gmem_src) {
     asm volatile("cp.async.ca.shared.global [%0], [%1], 16;" ::"r"((unsigned)__cvta_generic_to_shared(smem_dst)),
                  "l"(gmem_src)
@@ -350,6 +355,53 @@ __device__ __forceinline__ void tile_stage_bulk(double *pts, const double *row_p
     const unsigned bytes = (unsigned)(hi - lo) * 24u;
     mbar_expect_tx(bar, bytes);
     bulk_g2s(pts + (lo - first) * 3, row_ptr + (long long)lo * 3, bytes, bar);
+}
+
+// ---- raw tiles of depth (kE = 1) and integer-mm (kE = 3) frames: kE int32 per column, columns [c0-4, c0+kTile+4)
+// of the row.  The span is rounded out to whole groups of four columns, so that for rows of a multiple of four
+// columns it starts on a 16-byte boundary and is a multiple of 16 bytes long (16 B per 4 depth values, 48 B per 4 mm
+// points).  Element li of the RawTile view (column c0 - kHalo + li) is element li + kRawLead - kHalo of the buffer.
+constexpr int kRawLead = 4;
+constexpr int kRawPts = kTile + 2 * kRawLead;  // 264 staged columns
+template <int kKind>
+constexpr int kRawElems = kKind == kKindMm ? 3 : 1;  // int32 per point
+
+// the 4-byte cp.async form (any 4-byte aligned row): slots of columns outside the row are zeroed
+template <int kE>
+__device__ __forceinline__ void raw_stage_async(int *raw, const int *__restrict__ row_ptr, int c0, int cols) {
+    const int first = c0 - kRawLead;
+    for (int i = threadIdx.x; i < kRawPts * kE; i += kTile) {
+        const int col = first + i / kE;
+        if (col >= 0 && col < cols)
+            cp_async4(&raw[i], row_ptr + (long long)first * kE + i);
+        else
+            raw[i] = 0;
+    }
+}
+// the bulk form (rows of a multiple of four columns, 16-byte aligned): one copy of the columns inside the row; the
+// other slots are not written (k_frame_seq zeroes them once)
+template <int kE>
+__device__ __forceinline__ void raw_stage_bulk(int *raw, const int *row_ptr, int c0, int cols, unsigned long long *bar) {
+    const int first = c0 - kRawLead, lo = max(first, 0), hi = min(first + kRawPts, cols);
+    const unsigned bytes = (unsigned)(hi - lo) * 4u * kE;
+    mbar_expect_tx(bar, bytes);
+    bulk_g2s(raw + (lo - first) * kE, row_ptr + (long long)lo * kE, bytes, bar);
+}
+// the tans of the staged columns (depth only; zero outside the row), read once per launch: they do not change from
+// frame to frame.  Complete after the caller's next CTA barrier.
+__device__ __forceinline__ void stage_tan_cols(double *s_tan, const double *__restrict__ tan_col, int c0, int cols) {
+    for (int i = threadIdx.x; i < kRawPts; i += kTile) {
+        const int col = c0 - kRawLead + i;
+        s_tan[i] = col >= 0 && col < cols ? tan_col[col] : 0.0;
+    }
+}
+// the RawTile view of a raw buffer
+template <int kKind>
+__device__ __forceinline__ RawTile<kKind> raw_view(const int *raw, const double *s_tan, double tan_r) {
+    if constexpr (kKind == kKindDepth)
+        return RawTile<kKindDepth>{raw + (kRawLead - kHalo), s_tan + (kRawLead - kHalo), tan_r};
+    else
+        return RawTile<kKindMm>{raw + (kRawLead - kHalo) * 3};
 }
 
 // the neighbourhood of prefetch_neighbourhood, clamped to the row: the points of its leaves, the leaf boxes of
@@ -1175,12 +1227,20 @@ __device__ __forceinline__ void loop_fit_tail(const DevLoop &dl, int seq, const 
     }
 }
 
-template <bool kDevLoop>
+// kKind (kDevLoop only, NAV_RUN_INPUT_*): depth and integer-mm frames are read raw, as k_frame_seq reads them -- this
+// frame's tile staged with 4-byte cp.async and converted on read, the previous frame's column converted as it is
+// loaded for its map; cloud / prev_cloud then point at int32.
+template <bool kDevLoop, int kKind = kKindXyz>
 __global__ void __launch_bounds__(kTile, NAV_MATCH_MIN_CTAS)
 k_loop_step(const double *__restrict__ cloud, const int *__restrict__ labels, RowMap map, MatchOut out,
             const __grid_constant__ LoopPoses<kDevLoop> ps, int rows, int cols, int tiles_per_row,
             const double *__restrict__ prev_cloud, const int *__restrict__ prev_labels, int do_map,
-            double *__restrict__ part, FitMailbox mail) {
+            double *__restrict__ part, FitMailbox mail, TanTables tan) {
+    static_assert(kDevLoop || kKind == kKindXyz, "the host loop converts its frames in the prefetch");
+    constexpr bool kRaw = kKind != kKindXyz;
+    constexpr int kE = kRawElems<kKind>;
+    __shared__ __align__(16) int s_raw[kRawPts * kE];  // kRaw: this frame's tile, raw
+    __shared__ double s_tan[kRawPts];                  // depth: the tans of the staged columns
     __shared__ int s_warp[65];
     __shared__ int s_qcol[kTile];
     __shared__ MapSmem sm;
@@ -1199,9 +1259,17 @@ k_loop_step(const double *__restrict__ cloud, const int *__restrict__ labels, Ro
     const int c0 = tile * kTile;
     const int c = c0 + threadIdx.x;
     int label = 0;
+    double tan_r = 0.0;
+    if constexpr (kKind == kKindDepth) {
+        stage_tan_cols(s_tan, tan.col, c0, cols);  // published by the barrier below
+        tan_r = tan.row[row];
+    }
     if constexpr (kDevLoop) {
         if (ps.do_match) {
-            tile_stage_async(s_pts, cloud + base * 3, c0, cols);
+            if constexpr (kRaw)
+                raw_stage_async<kE>(s_raw, (const int *)cloud + base * kE, c0, cols);
+            else
+                tile_stage_async(s_pts, cloud + base * 3, c0, cols);
             cp_async_commit();
         }
         constexpr int kRecWords = (int)(sizeof(LoopRec) / sizeof(double));
@@ -1217,7 +1285,12 @@ k_loop_step(const double *__restrict__ cloud, const int *__restrict__ labels, Ro
         P3 p = {0, 0, 0};
         if (c < cols) {
             lab = prev_labels[base + c] == 1;
-            p = load_p3(prev_cloud + (base + c) * 3);
+            if constexpr (kKind == kKindDepth)
+                p = depth_point(((const int *)prev_cloud)[base + c], s_tan[threadIdx.x + kRawLead], tan_r);
+            else if constexpr (kKind == kKindMm)
+                p = RawTile<kKindMm>{(const int *)prev_cloud + (base + c) * 3}.at(0);
+            else
+                p = load_p3(prev_cloud + (base + c) * 3);
         }
         if constexpr (kDevLoop)
             map_tile(lab, c < cols, p, s_rec.map, map, rid, tile, c, base, s_lo, s_hi);
@@ -1233,7 +1306,10 @@ k_loop_step(const double *__restrict__ cloud, const int *__restrict__ labels, Ro
     if constexpr (kDevLoop) {
         cp_async_wait_all();
         __syncthreads();
-        label = tile_labels_filtered(s_pts, s_f1, s_f2, c0, cols, ps.n_exact);
+        if constexpr (kRaw)
+            label = tile_labels_filtered(raw_view<kKind>(s_raw, s_tan, tan_r), s_f1, s_f2, c0, cols, ps.n_exact);
+        else
+            label = tile_labels_filtered(s_pts, s_f1, s_f2, c0, cols, ps.n_exact);
         if (c < cols) ps.labels_out[base + c] = label;
     }
     if (do_map) cluster_wait_all();
@@ -1241,7 +1317,9 @@ k_loop_step(const double *__restrict__ cloud, const int *__restrict__ labels, Ro
     prefetch_neighbourhood<true>(sm, rv, cols);
     cp_async_wait_all();
     auto point_at = [&](int t) {  // the lidar-frame point of column-in-tile t
-        if constexpr (kDevLoop) {
+        if constexpr (kRaw) {
+            return raw_view<kKind>(s_raw, s_tan, tan_r).at(t + kHalo);
+        } else if constexpr (kDevLoop) {
             const double *sp = s_pts + (t + kHalo) * 3;
             return P3{sp[0], sp[1], sp[2]};
         } else {
@@ -1316,20 +1394,25 @@ int launch_loop_step(const double *cloud, const int *labels, const RowMap &map, 
     LoopPoses<false> ps;
     ps.cur = poses;
     ps.prev = prev_poses;
+    const TanTables no_tan = {nullptr, nullptr};
     return launch_row_clusters(k_loop_step<false>, dim3((unsigned)(n_seq * rows * tiles)), tiles, stream, cloud, labels,
-                               map, out, ps, rows, cols, tiles, prev_cloud, prev_labels, do_map ? 1 : 0, part, mail);
+                               map, out, ps, rows, cols, tiles, prev_cloud, prev_labels, do_map ? 1 : 0, part, mail,
+                               no_tan);
 }
 
-int launch_loop_step_dev(const DevLoop &dl, const double *cloud, const double *prev_cloud, const int *prev_labels,
+int launch_loop_step_dev(int kind, const DevLoop &dl, const void *cloud, const void *prev_cloud, const int *prev_labels,
                          bool do_map, const RowMap &map, const MatchOut &out, int n_seq, int rows, int cols,
-                         double *part, cudaStream_t stream) {
+                         double *part, cudaStream_t stream, const TanTables &tan) {
     const int tiles = div_up(cols, kTile);
     LoopPoses<true> ps;
     static_cast<DevLoop &>(ps) = dl;
     const FitMailbox no_mail = {nullptr, nullptr, 0ull};
-    return launch_row_clusters(k_loop_step<true>, dim3((unsigned)(n_seq * rows * tiles)), tiles, stream, cloud,
-                               (const int *)nullptr, map, out, ps, rows, cols, tiles, prev_cloud, prev_labels,
-                               do_map ? 1 : 0, part, no_mail);
+    auto kernel = kind == kKindDepth ? k_loop_step<true, kKindDepth>
+                  : kind == kKindMm  ? k_loop_step<true, kKindMm>
+                                     : k_loop_step<true, kKindXyz>;
+    return launch_row_clusters(kernel, dim3((unsigned)(n_seq * rows * tiles)), tiles, stream, (const double *)cloud,
+                               (const int *)nullptr, map, out, ps, rows, cols, tiles, (const double *)prev_cloud,
+                               prev_labels, do_map ? 1 : 0, part, no_mail, tan);
 }
 
 // queued on `stream`, in front of the kernels that read the tables; c1 / c2 must stay valid (the host's static tables).
@@ -1424,11 +1507,18 @@ static_assert(sizeof(SeqInlinePoses) + 256 < 32764, "inline poses must fit the k
 // them and every thread waits on an mbarrier -- s_bar[slot] for the tile in that slot, s_bar[2] for the
 // neighbourhood.  Otherwise every thread issues its share of 8- and 16-byte cp.async and waits for its own groups,
 // and a CTA barrier publishes them.
-template <bool kInline, bool kOut, bool kBulk>
+// kKind (NAV_RUN_INPUT_*): xyz frames are staged as doubles; depth and integer-mm frames are staged raw, 4 or 12 B per
+// point, into s_raw and converted where they are read (RawTile: depth_point / mm_coord, the arithmetic of k_convert and
+// k_widen_mm) -- no conversion pass, so no CTA barrier is added per frame.  a.frames / a.frame_stride then count int32.
+template <bool kInline, bool kOut, bool kBulk, int kKind = kKindXyz>
 __global__ void __launch_bounds__(kTile, NAV_MATCH_MIN_CTAS)
 k_frame_seq(SeqArgs a, int *__restrict__ labels, RowMap map0, RowMap map1, MatchOut out, int rows, int cols,
-            unsigned *__restrict__ n_exact, const __grid_constant__ SeqInlinePoses ip, SeqOut o) {
+            unsigned *__restrict__ n_exact, const __grid_constant__ SeqInlinePoses ip, SeqOut o, TanTables tan) {
+    constexpr bool kRaw = kKind != kKindXyz;
+    constexpr int kE = kRawElems<kKind>;
     __shared__ __align__(16) double s_pts[2][kTilePts * 3];  // the tile of this frame / of the next one (in flight)
+    __shared__ __align__(16) int s_raw[2][kRawPts * kE];     // kRaw: the same, raw
+    __shared__ double s_tan[kRawPts];                        // depth: the tans of the staged columns
     __shared__ float s_f1[kTile + kHalo], s_f2[kTile + kHalo];
     __shared__ int s_warp[65];
     __shared__ int s_qcol[kTile];
@@ -1442,12 +1532,28 @@ k_frame_seq(SeqArgs a, int *__restrict__ labels, RowMap map0, RowMap map1, Match
     // ring slots: per frame n_seq*rows rows of cols pixels / n_chunks mask words / `tiles` CTA partials
     const long long px_frame = (long long)a.n_seq * rows * cols, cta_frame = (long long)a.n_seq * rows * gridDim.x;
     __shared__ __align__(8) unsigned long long s_bar[3];
+    // kRaw: the frames as int32, the tile of slot `slot` as points, and where frame f's row starts
+    const int *raw_frames = (const int *)a.frames;
+    double tan_r = 0.0;
+    if constexpr (kKind == kKindDepth) {
+        stage_tan_cols(s_tan, tan.col, c0, cols);  // published by the barrier in front of the first labels
+        tan_r = tan.row[row];
+    }
+    auto raw_tile = [&](auto slot) { return raw_view<kKind>(s_raw[slot], s_tan, tan_r); };  // kRaw only
+    auto raw_row = [&](int f) { return raw_frames + (long long)f * a.frame_stride + base * kE; };
     if constexpr (kBulk) {
         // the copies only ever write the slots of columns inside the row and the mask words of leaves inside it;
         // the rest reads as zero, as the cp.async path leaves it
-        for (int i = threadIdx.x; i < kTilePts * 3; i += kTile) {
-            const int col = c0 - kHalo + i / 3;
-            if (col < 0 || col >= cols) s_pts[0][i] = s_pts[1][i] = 0.0;
+        if constexpr (kRaw) {
+            for (int i = threadIdx.x; i < kRawPts * kE; i += kTile) {
+                const int col = c0 - kRawLead + i / kE;
+                if (col < 0 || col >= cols) s_raw[0][i] = s_raw[1][i] = 0;
+            }
+        } else {
+            for (int i = threadIdx.x; i < kTilePts * 3; i += kTile) {
+                const int col = c0 - kHalo + i / 3;
+                if (col < 0 || col >= cols) s_pts[0][i] = s_pts[1][i] = 0.0;
+            }
         }
         if (threadIdx.x < 3) sm.mask_lead[threadIdx.x] = 0u;
         if (threadIdx.x < kNbLeaves + 3) sm.mask[threadIdx.x] = 0u;
@@ -1458,10 +1564,16 @@ k_frame_seq(SeqArgs a, int *__restrict__ labels, RowMap map0, RowMap map1, Match
         __syncthreads();
         if (threadIdx.x == 0) {
             asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // the zeros above before the copies
-            tile_stage_bulk(s_pts[0], a.frames + base * 3, c0, cols, &s_bar[0]);
+            if constexpr (kRaw)
+                raw_stage_bulk<kE>(s_raw[0], raw_row(0), c0, cols, &s_bar[0]);
+            else
+                tile_stage_bulk(s_pts[0], a.frames + base * 3, c0, cols, &s_bar[0]);
         }
     } else {
-        tile_stage_async(s_pts[0], a.frames + base * 3, c0, cols);
+        if constexpr (kRaw)
+            raw_stage_async<kE>(s_raw[0], raw_row(0), c0, cols);
+        else
+            tile_stage_async(s_pts[0], a.frames + base * 3, c0, cols);
         cp_async_commit();
     }
     for (int f = 0; f < a.n_frames; ++f) {
@@ -1481,14 +1593,22 @@ k_frame_seq(SeqArgs a, int *__restrict__ labels, RowMap map0, RowMap map1, Match
         // the labels need nothing from the row's other tiles: they are computed BEFORE waiting for the cluster
         // (the barrier was only signalled at the end of the previous frame), which turns the wait for the row's
         // slowest tile into useful time
-        const int label = tile_labels_filtered(pts, s_f1, s_f2, c0, cols, n_exact);
+        int label;
+        if constexpr (kRaw)
+            label = tile_labels_filtered(raw_tile(f & 1), s_f1, s_f2, c0, cols, n_exact);
+        else
+            label = tile_labels_filtered(pts, s_f1, s_f2, c0, cols, n_exact);
         // the next frame's tile starts its way from HBM now and has the whole search to arrive.  Its slot was last
         // read in frame f-1; the barrier that ends the labels is behind those reads (cp.async path: the cluster wait).
         // Nothing but generic reads touched the slot since its last copy, so the refill needs no proxy fence.
         if constexpr (kBulk) {
-            if (threadIdx.x == 0 && f + 1 < a.n_frames)
-                tile_stage_bulk(s_pts[(f + 1) & 1], a.frames + (long long)(f + 1) * a.frame_stride + base * 3, c0, cols,
-                                &s_bar[(f + 1) & 1]);
+            if (threadIdx.x == 0 && f + 1 < a.n_frames) {
+                if constexpr (kRaw)
+                    raw_stage_bulk<kE>(s_raw[(f + 1) & 1], raw_row(f + 1), c0, cols, &s_bar[(f + 1) & 1]);
+                else
+                    tile_stage_bulk(s_pts[(f + 1) & 1], a.frames + (long long)(f + 1) * a.frame_stride + base * 3, c0,
+                                    cols, &s_bar[(f + 1) & 1]);
+            }
         }
         NAV_STAMP(2);
         if (f > 0) cluster_wait_all();  // the row's map of the previous frame is complete (also a CTA barrier)
@@ -1508,8 +1628,13 @@ k_frame_seq(SeqArgs a, int *__restrict__ labels, RowMap map0, RowMap map1, Match
         } else {
             prefetch_neighbourhood<true>(sm, rv, cols);
             cp_async_commit();
-            if (f + 1 < a.n_frames)
-                tile_stage_async(s_pts[(f + 1) & 1], a.frames + (long long)(f + 1) * a.frame_stride + base * 3, c0, cols);
+            if (f + 1 < a.n_frames) {
+                if constexpr (kRaw)
+                    raw_stage_async<kE>(s_raw[(f + 1) & 1], raw_row(f + 1), c0, cols);
+                else
+                    tile_stage_async(s_pts[(f + 1) & 1], a.frames + (long long)(f + 1) * a.frame_stride + base * 3, c0,
+                                     cols);
+            }
             cp_async_commit();
         }
         if (c < cols) {
@@ -1521,8 +1646,12 @@ k_frame_seq(SeqArgs a, int *__restrict__ labels, RowMap map0, RowMap map1, Match
         }
         const PoseXf &pose = kInline ? ip.loc[f] : a.pose_loc[(long long)f * a.n_seq + seq];
         auto point_at = [&](int t) {  // the lidar-frame point of column-in-tile t
-            const double *sp = pts + (t + kHalo) * 3;
-            return P3{sp[0], sp[1], sp[2]};
+            if constexpr (kRaw) {
+                return raw_tile(f & 1).at(t + kHalo);
+            } else {
+                const double *sp = pts + (t + kHalo) * 3;
+                return P3{sp[0], sp[1], sp[2]};
+            }
         };
         {
             const P3 own = c < cols ? point_at(threadIdx.x) : P3{0, 0, 0};
@@ -1565,24 +1694,29 @@ k_frame_seq(SeqArgs a, int *__restrict__ labels, RowMap map0, RowMap map1, Match
 int frame_seq_inline_frames() { return kSeqInlineFrames; }
 
 // Whether k_frame_seq can stage with bulk copies (kBulk): every range it copies must start on a 16-byte boundary and
-// be a multiple of 16 bytes long.  Rows of an even number of columns up to 2048 whose mask rows are a multiple of
+// be a multiple of 16 bytes long.  xyz: rows of an even number of columns up to 2048 whose mask rows are a multiple of
 // four words -- 64x2048 and every width that is a multiple of 64 -- take the bulk path; odd widths (e.g. 257) and
-// even ones with a ragged mask row (e.g. 1800: 113 words) keep the cp.async path.
-static bool frame_seq_bulk_ok(const double *frames, long long frame_stride, const RowMap &m0, const RowMap &m1, int cols) {
+// even ones with a ragged mask row (e.g. 1800: 113 words) keep the cp.async path.  Depth and integer-mm frames (raw
+// spans of whole groups of four columns): rows of a multiple of four columns, frames and frame stride on 16 bytes, and
+// the same mask-row and map conditions; any other shape stages with 4-byte cp.async.
+static bool frame_seq_bulk_ok(int kind, const void *frames, long long frame_stride, const RowMap &m0, const RowMap &m1,
+                              int cols) {
     auto al16 = [](const void *p) { return ((uintptr_t)p & 15u) == 0; };
     auto map_ok = [&](const RowMap &m) { return al16(m.pts) && al16(m.mask) && al16(m.box) && al16(m.sbox); };
-    return cols % 2 == 0 && cols <= kMaxRowLeafSmem * kChunk && div_up(cols, kChunk) % 4 == 0 && frame_stride % 2 == 0 &&
-           al16(frames) && map_ok(m0) && map_ok(m1);
+    const bool maps = cols <= kMaxRowLeafSmem * kChunk && div_up(cols, kChunk) % 4 == 0 && al16(frames) && map_ok(m0) &&
+                      map_ok(m1);
+    if (kind == kKindXyz) return cols % 2 == 0 && frame_stride % 2 == 0 && maps;
+    return cols % 4 == 0 && frame_stride % 4 == 0 && maps;
 }
 
-template <bool kBulk>
-static int launch_frame_seq_variant(const double *frames, long long frame_stride, int n_frames, int *labels,
+template <bool kBulk, int kKind>
+static int launch_frame_seq_variant(const void *frames, long long frame_stride, int n_frames, int *labels,
                                     const RowMap &map0, const RowMap &map1, const MatchOut &out,
                                     const PoseXf *d_pose_loc, const PoseXf *d_pose_fin, int n_seq, int rows, int cols,
                                     unsigned *n_exact, cudaStream_t stream, const PoseXf *h_pose_loc,
-                                    const PoseXf *h_pose_fin, const SeqOut *seq_out) {
+                                    const PoseXf *h_pose_fin, const SeqOut *seq_out, const TanTables &tan) {
     const int tiles = div_up(cols, kTile);
-    const SeqArgs a = {frames, frame_stride, n_frames, n_seq, d_pose_loc, d_pose_fin};
+    const SeqArgs a = {(const double *)frames, frame_stride, n_frames, n_seq, d_pose_loc, d_pose_fin};
     const bool inl = h_pose_loc && h_pose_fin && n_seq == 1 && n_frames <= kSeqInlineFrames;
     const dim3 grid((unsigned)tiles, (unsigned)rows, (unsigned)n_seq);
     const SeqOut no_out = {nullptr, nullptr, nullptr, nullptr};
@@ -1594,33 +1728,52 @@ static int launch_frame_seq_variant(const double *frames, long long frame_stride
         }
         for (int f = n_frames; f < kSeqInlineFrames; ++f) ip.loc[f] = ip.fin[f] = h_pose_loc[0];
         if (seq_out)
-            return launch_row_clusters(k_frame_seq<true, true, kBulk>, grid, tiles, stream, a, labels, map0, map1, out, rows,
-                                       cols, n_exact, ip, *seq_out);
-        return launch_row_clusters(k_frame_seq<true, false, kBulk>, grid, tiles, stream, a, labels, map0, map1, out, rows, cols,
-                                   n_exact, ip, no_out);
+            return launch_row_clusters(k_frame_seq<true, true, kBulk, kKind>, grid, tiles, stream, a, labels, map0, map1, out,
+                                       rows, cols, n_exact, ip, *seq_out, tan);
+        return launch_row_clusters(k_frame_seq<true, false, kBulk, kKind>, grid, tiles, stream, a, labels, map0, map1, out,
+                                   rows, cols, n_exact, ip, no_out, tan);
     }
     static const SeqInlinePoses none = {};
     if (seq_out)
-        return launch_row_clusters(k_frame_seq<false, true, kBulk>, grid, tiles, stream, a, labels, map0, map1, out, rows, cols,
-                                   n_exact, none, *seq_out);
-    return launch_row_clusters(k_frame_seq<false, false, kBulk>, grid, tiles, stream, a, labels, map0, map1, out, rows, cols,
-                               n_exact, none, no_out);
+        return launch_row_clusters(k_frame_seq<false, true, kBulk, kKind>, grid, tiles, stream, a, labels, map0, map1, out,
+                                   rows, cols, n_exact, none, *seq_out, tan);
+    return launch_row_clusters(k_frame_seq<false, false, kBulk, kKind>, grid, tiles, stream, a, labels, map0, map1, out,
+                               rows, cols, n_exact, none, no_out, tan);
+}
+
+template <int kKind>
+static int launch_frame_seq_kind(bool bulk, const void *frames, long long frame_stride, int n_frames, int *labels,
+                                 const RowMap &map0, const RowMap &map1, const MatchOut &out, const PoseXf *d_pose_loc,
+                                 const PoseXf *d_pose_fin, int n_seq, int rows, int cols, unsigned *n_exact,
+                                 cudaStream_t stream, const PoseXf *h_pose_loc, const PoseXf *h_pose_fin,
+                                 const SeqOut *seq_out, const TanTables &tan) {
+    return bulk ? launch_frame_seq_variant<true, kKind>(frames, frame_stride, n_frames, labels, map0, map1, out, d_pose_loc,
+                                                        d_pose_fin, n_seq, rows, cols, n_exact, stream, h_pose_loc,
+                                                        h_pose_fin, seq_out, tan)
+                : launch_frame_seq_variant<false, kKind>(frames, frame_stride, n_frames, labels, map0, map1, out,
+                                                         d_pose_loc, d_pose_fin, n_seq, rows, cols, n_exact, stream,
+                                                         h_pose_loc, h_pose_fin, seq_out, tan);
 }
 
 // h_pose_loc / h_pose_fin != null (n_seq == 1, n_frames <= frame_seq_inline_frames()): the poses are passed as
 // kernel parameters and the device arrays are not read.  seq_out != null: the output mode of k_frame_seq.
-int launch_frame_seq(const double *frames, long long frame_stride, int n_frames, int *labels, const RowMap &map0,
+int launch_frame_seq(int kind, const void *frames, long long frame_stride, int n_frames, int *labels, const RowMap &map0,
                      const RowMap &map1, const MatchOut &out, const PoseXf *d_pose_loc, const PoseXf *d_pose_fin,
                      int n_seq, int rows, int cols, unsigned *n_exact, cudaStream_t stream, const PoseXf *h_pose_loc,
-                     const PoseXf *h_pose_fin, const SeqOut *seq_out, bool *bulk_out) {
-    const bool bulk = frame_seq_bulk_ok(frames, frame_stride, map0, map1, cols);
+                     const PoseXf *h_pose_fin, const SeqOut *seq_out, bool *bulk_out, const TanTables &tan) {
+    const bool bulk = frame_seq_bulk_ok(kind, frames, frame_stride, map0, map1, cols);
     if (bulk_out) *bulk_out = bulk;
-    return bulk ? launch_frame_seq_variant<true>(frames, frame_stride, n_frames, labels, map0, map1, out, d_pose_loc,
+    if (kind == kKindDepth)
+        return launch_frame_seq_kind<kKindDepth>(bulk, frames, frame_stride, n_frames, labels, map0, map1, out, d_pose_loc,
                                                  d_pose_fin, n_seq, rows, cols, n_exact, stream, h_pose_loc, h_pose_fin,
-                                                 seq_out)
-                : launch_frame_seq_variant<false>(frames, frame_stride, n_frames, labels, map0, map1, out, d_pose_loc,
-                                                  d_pose_fin, n_seq, rows, cols, n_exact, stream, h_pose_loc,
-                                                  h_pose_fin, seq_out);
+                                                 seq_out, tan);
+    if (kind == kKindMm)
+        return launch_frame_seq_kind<kKindMm>(bulk, frames, frame_stride, n_frames, labels, map0, map1, out, d_pose_loc,
+                                              d_pose_fin, n_seq, rows, cols, n_exact, stream, h_pose_loc, h_pose_fin,
+                                              seq_out, tan);
+    return launch_frame_seq_kind<kKindXyz>(bulk, frames, frame_stride, n_frames, labels, map0, map1, out, d_pose_loc,
+                                           d_pose_fin, n_seq, rows, cols, n_exact, stream, h_pose_loc, h_pose_fin, seq_out,
+                                           tan);
 }
 
 // Fit totals of frame blockIdx.x, sequence blockIdx.y: part = [n_frames][n_seq][n_part][5] partials, stats =

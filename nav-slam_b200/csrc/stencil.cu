@@ -211,60 +211,56 @@ void launch_labels(const double *cloud, int *labels, double *curv_or_null, long 
 
 // ---------------------------------------------------------------- a2 ------------------------
 // utils/pointcloud.c:18-47.  tan(theta_col) / tan(phi_row) come from the host's libm (the
-// reference's own tan), uploaded once per context; y = (-d) * tan is one rounded multiply.
+// reference's own tan), uploaded once per context; y = (-d) * tan is one rounded multiply (depth_point).
+// n_img images of `rows` rows back to back: tan_row is indexed by the row within its image.
 __global__ void k_convert(const int *__restrict__ dist, const double *__restrict__ tan_col,
-                          const double *__restrict__ tan_row, double *__restrict__ out, int rows, int cols) {
-    const long long n = (long long)rows * cols;
+                          const double *__restrict__ tan_row, double *__restrict__ out, int rows, int cols, int n_img) {
+    const long long n = (long long)n_img * rows * cols;
     for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n;
          i += (long long)gridDim.x * blockDim.x) {
-        const int r = (int)(i / cols), c = (int)(i % cols);
-        const double d = (double)dist[i];
-        double x = 0.0, y = 0.0, z = 0.0;
-        if (!(d <= 0.0)) {
-            x = d;
-            y = dmul(-d, tan_col[c]);
-            z = dmul(-d, tan_row[r]);
-        }
-        out[i * 3 + 0] = x;
-        out[i * 3 + 1] = y;
-        out[i * 3 + 2] = z;
+        const int r = (int)((i / cols) % rows), c = (int)(i % cols);
+        const P3 p = depth_point(dist[i], tan_col[c], tan_row[r]);
+        out[i * 3 + 0] = p.x;
+        out[i * 3 + 1] = p.y;
+        out[i * 3 + 2] = p.z;
     }
 }
 
 void launch_convert(const int *dist, const double *tan_col, const double *tan_row, double *out, int rows,
-                    int cols, int sm_count, cudaStream_t stream) {
-    const long long n = (long long)rows * cols;
+                    int cols, int n_img, int sm_count, cudaStream_t stream) {
+    const long long n = (long long)n_img * rows * cols;
     if (n <= 0) return;
     long long grid = (n + 255) / 256;
     if (grid > sm_count * 8LL) grid = sm_count * 8LL;
-    k_convert<<<(unsigned)grid, 256, 0, stream>>>(dist, tan_col, tan_row, out, rows, cols);
+    k_convert<<<(unsigned)grid, 256, 0, stream>>>(dist, tan_col, tan_row, out, rows, cols, n_img);
 }
 
 // ---------------------------------------------------------------- integer-mm xyz -----------
 // L9 clouds in whole millimetres cross PCIe as int32 [n][3] (12 B/point instead of 24) and are widened here.  Every
 // int32 is exact in binary64, so the cloud equals the one the host would have uploaded as doubles, bit for bit.
-// The 3n values are one flat run: a 16-byte load of four ints and two 16-byte stores of four doubles per step, the
-// last (3n) % 4 values one at a time.  Both buffers come from cudaMalloc (16-byte aligned).
-__global__ void k_widen_mm(const int *__restrict__ in, double *__restrict__ out, long long n_vals) {
-    const long long n4 = n_vals >> 2, stride = (long long)gridDim.x * blockDim.x;
+// The 3n values are one flat run: a 16-byte load of four ints and two 16-byte stores of four doubles per step for the
+// first n4 groups of four, the rest one at a time.  n4 = 0 unless both buffers are 16-byte aligned (a frame of a
+// device-resident recording may start on any 4-byte boundary).
+__global__ void k_widen_mm(const int *__restrict__ in, double *__restrict__ out, long long n_vals, long long n4) {
+    const long long stride = (long long)gridDim.x * blockDim.x;
     const long long t = blockIdx.x * (long long)blockDim.x + threadIdx.x;
     const int4 *in4 = reinterpret_cast<const int4 *>(in);
     double2 *out2 = reinterpret_cast<double2 *>(out);
     for (long long i = t; i < n4; i += stride) {
         const int4 v = __ldg(in4 + i);
-        out2[2 * i] = make_double2((double)v.x, (double)v.y);
-        out2[2 * i + 1] = make_double2((double)v.z, (double)v.w);
+        out2[2 * i] = make_double2(mm_coord(v.x), mm_coord(v.y));
+        out2[2 * i + 1] = make_double2(mm_coord(v.z), mm_coord(v.w));
     }
-    for (long long i = 4 * n4 + t; i < n_vals; i += stride) out[i] = (double)in[i];
+    for (long long i = 4 * n4 + t; i < n_vals; i += stride) out[i] = mm_coord(in[i]);
 }
 
 void launch_widen_mm(const int *in, double *out, long long n_points, int sm_count, cudaStream_t stream) {
     const long long n_vals = n_points * 3;
     if (n_vals <= 0) return;
-    long long grid = (n_vals / 4 + 255) / 256;
-    if (grid < 1) grid = 1;
+    const bool vec = (((uintptr_t)in | (uintptr_t)out) & 15u) == 0;
+    long long grid = (vec ? n_vals / 4 : n_vals) / 256 + 1;
     if (grid > sm_count * 8LL) grid = sm_count * 8LL;
-    k_widen_mm<<<(unsigned)grid, 256, 0, stream>>>(in, out, n_vals);
+    k_widen_mm<<<(unsigned)grid, 256, 0, stream>>>(in, out, n_vals, vec ? n_vals >> 2 : 0);
 }
 
 // ---------------------------------------------------------------- a7 ------------------------

@@ -73,6 +73,46 @@ __device__ __forceinline__ void tile_stage(StencilSmem &s, const double *__restr
     }
 }
 
+// ---- the narrow frame formats (NAV_RUN_INPUT_DEPTH / _MM), converted point by point where they are read.  One
+// definition for the conversion kernels (k_convert, k_widen_mm) and for the kernels that stage raw tiles, so the
+// bits cannot drift between them.
+constexpr int kKindXyz = 0, kKindDepth = 1, kKindMm = 2;  // NAV_RUN_INPUT_*
+
+// a2 of one pixel, utils/pointcloud.c:18-47: tan(theta_col) / tan(phi_row) are the host libm's values, y = (-d) * tan
+// is one rounded multiply; d <= 0 is no return, (0, 0, 0)
+__device__ __forceinline__ P3 depth_point(int dist, double tan_c, double tan_r) {
+    const double d = (double)dist;
+    P3 p = {0.0, 0.0, 0.0};
+    if (!(d <= 0.0)) {
+        p.x = d;
+        p.y = dmul(-d, tan_c);
+        p.z = dmul(-d, tan_r);
+    }
+    return p;
+}
+// whole millimetres: every int32 is exact in binary64
+__device__ __forceinline__ double mm_coord(int v) { return (double)v; }
+
+// A tile of a depth or integer-mm row staged raw in shared memory: element li is column c0 - kHalo + li, as in the
+// xyz tile.  Columns outside the row hold zeros, which both conversions turn into (0, 0, 0), the xyz tile's padding.
+template <int kKind>
+struct RawTile;
+template <>
+struct RawTile<kKindDepth> {
+    const int *d;         // depth of element li at d[li]
+    const double *tan_c;  // tan of its column at tan_c[li]
+    double tan_r;         // tan of the image row
+    __device__ __forceinline__ P3 at(int li) const { return depth_point(d[li], tan_c[li], tan_r); }
+};
+template <>
+struct RawTile<kKindMm> {
+    const int *v;  // x, y, z of element li at v[3 li ..]
+    __device__ __forceinline__ P3 at(int li) const {
+        const int *p = v + li * 3;
+        return P3{mm_coord(p[0]), mm_coord(p[1]), mm_coord(p[2])};
+    }
+};
+
 __device__ __forceinline__ double curvature_from_taps(double dm2, double dm1, double dp1, double dp2) {
     const double sum = dadd(dadd(dadd(dm2, dm1), dp1), dp2);
     const double avg = dmul(sum, 0.25);  // sum / 4: exact scaling
@@ -95,6 +135,12 @@ __device__ __forceinline__ double curvature_from_taps(double dm2, double dm1, do
 __device__ __forceinline__ double tile_dist(const double *pts, int a, int b) {
     const double *p = pts + a * 3, *q = pts + b * 3;
     return __dsqrt_rn(dsq3(dsub(p[0], q[0]), dsub(p[1], q[1]), dsub(p[2], q[2])));
+}
+
+template <int kKind>
+__device__ __forceinline__ double tile_dist(const RawTile<kKind> &t, int a, int b) {
+    const P3 p = t.at(a), q = t.at(b);
+    return __dsqrt_rn(dsq3(dsub(p.x, q.x), dsub(p.y, q.y), dsub(p.z, q.z)));
 }
 
 // exact curvature of the thread's own column; needs tile_stage + __syncthreads before.
@@ -131,6 +177,13 @@ __device__ __forceinline__ float tile_dist32(const double *pts, int a, int b) {
     return sqrt_approx(__fmaf_rn(dx, dx, __fmaf_rn(dy, dy, dz * dz)));
 }
 
+template <int kKind>
+__device__ __forceinline__ float tile_dist32(const RawTile<kKind> &t, int a, int b) {
+    const P3 p = t.at(a), q = t.at(b);
+    const float dx = (float)dsub(p.x, q.x), dy = (float)dsub(p.y, q.y), dz = (float)dsub(p.z, q.z);
+    return sqrt_approx(__fmaf_rn(dx, dx, __fmaf_rn(dy, dy, dz * dz)));
+}
+
 // the reference's exact binary64 label of staged point li (rare path: kept out of line so that its
 // sqrt/div sequences do not inflate the register budget of the streaming kernels)
 static __device__ __noinline__ int label_exact_at(const double *pts, int li) {
@@ -138,11 +191,19 @@ static __device__ __noinline__ int label_exact_at(const double *pts, int li) {
                                             tile_dist(pts, li, li + 1), tile_dist(pts, li, li + 2));
     return curv > 0.1 ? 1 : 0;
 }
+template <int kKind>
+static __device__ __noinline__ int label_exact_at(RawTile<kKind> t, int li) {
+    const double curv = curvature_from_taps(tile_dist(t, li, li - 2), tile_dist(t, li, li - 1), tile_dist(t, li, li + 1),
+                                            tile_dist(t, li, li + 2));
+    return curv > 0.1 ? 1 : 0;
+}
 
 // decide one label from the four fp32 tap distances, falling back to the reference's binary64
-// expression (evaluated from the staged points around local index li) when fp32 cannot decide
-__device__ __forceinline__ int label_from_taps32(float dm2, float dm1, float dp1, float dp2, const double *pts,
-                                                 int li, unsigned *n_exact) {
+// expression (evaluated from the staged points around local index li) when fp32 cannot decide.
+// Pts: the staged xyz tile (const double *) or a RawTile
+template <typename Pts>
+__device__ __forceinline__ int label_from_taps32(float dm2, float dm1, float dp1, float dp2, Pts pts, int li,
+                                                 unsigned *n_exact) {
     const float avg = 0.25f * (((dm2 + dm1) + dp1) + dp2);
     const float e0 = dm2 - avg, e1 = dm1 - avg, e2 = dp1 - avg, e3 = dp2 - avg;
     const float var = __fmaf_rn(e3, e3, __fmaf_rn(e2, e2, __fmaf_rn(e1, e1, e0 * e0)));
@@ -161,7 +222,8 @@ __device__ __forceinline__ int label_from_taps32(float dm2, float dm1, float dp1
 
 // label (0/1) of the thread's own column; needs tile_stage + __syncthreads before.
 // Contains two __syncthreads: call from all kTile threads.  *n_exact counts exact re-evaluations.
-__device__ __forceinline__ int tile_labels_filtered(const double *pts, float *f1, float *f2, int c0, int cols,
+template <typename Pts>
+__device__ __forceinline__ int tile_labels_filtered(Pts pts, float *f1, float *f2, int c0, int cols,
                                                     unsigned *n_exact) {
     for (int i = threadIdx.x; i < kTile + kHalo; i += kTile) {
         f1[i] = tile_dist32(pts, i, i + 1);
@@ -176,7 +238,7 @@ __device__ __forceinline__ int tile_labels_filtered(const double *pts, float *f1
     return label;
 }
 __device__ __forceinline__ int tile_labels_filtered(StencilSmem &s, int c0, int cols, unsigned *n_exact) {
-    return tile_labels_filtered(s.pts, s.fl.f1, s.fl.f2, c0, cols, n_exact);
+    return tile_labels_filtered((const double *)s.pts, s.fl.f1, s.fl.f2, c0, cols, n_exact);
 }
 
 }  // namespace nav
