@@ -224,8 +224,9 @@ struct nav_ctx {
     RowMap map_alt = {};  // second buffer: the fused frame kernel builds the next map here, then they swap
     nav_corr *d_corr_rows = nullptr, *d_corr = nullptr;
     int *d_corr_row_count = nullptr, *d_corr_total = nullptr;
-    int *d_dist = nullptr;
-    int *d_mm = nullptr;  // integer-mm cloud of the blocking call, int32 [ntot][3] (lazy)
+    // the raw frames of the blocking calls, before they become xyz (raw_buf): [0] depth (allocated by nav_create,
+    // one image), [1] integer mm.  Each async slot and prefetch slot holds its own pair.
+    int *raw[2] = {nullptr, nullptr};
     double *d_tan_col = nullptr, *d_tan_row = nullptr;
     double *d_flat = nullptr;
     int *d_flat_count = nullptr;
@@ -243,7 +244,8 @@ struct nav_ctx {
     static constexpr int kSlots = 2;
     struct AsyncSlot {
         double *d_cloud = nullptr, *d_nn_dist = nullptr;
-        int *d_labels = nullptr, *d_nn_idx = nullptr, *d_depth = nullptr, *d_mm = nullptr;
+        int *d_labels = nullptr, *d_nn_idx = nullptr;
+        int *raw[2] = {nullptr, nullptr};
         cudaEvent_t in_done = nullptr, compute_done = nullptr, out_done = nullptr;
     } slots[kSlots];
     cudaStream_t s_in = nullptr, s_out = nullptr;
@@ -253,7 +255,8 @@ struct nav_ctx {
     // stream while the current one is matched and fitted
     struct PreSlot {
         double *d_cloud = nullptr;
-        int *d_labels = nullptr, *d_depth = nullptr, *d_mm = nullptr;
+        int *d_labels = nullptr;
+        int *raw[2] = {nullptr, nullptr};
         cudaEvent_t ready = nullptr, released = nullptr;
         const void *host_src = nullptr;  // identity of the prefetched frame
         bool pending = false;
@@ -382,21 +385,21 @@ extern "C" void nav_destroy(nav_ctx *c) {
     void *ptrs[] = {c->d_cloud, c->d_global, c->d_curv, c->d_nn_dist, c->d_labels, c->d_nn_idx, c->map.pts,
                     c->map.mask, c->d_n_exact, c->map.box, c->map.sbox, c->map_alt.pts, c->map_alt.mask,
                     c->map_alt.box, c->map_alt.sbox, c->d_corr_rows, c->d_corr,
-                    c->d_corr_row_count, c->d_corr_total, c->d_dist, c->d_tan_col, c->d_tan_row, c->d_flat,
-                    c->d_flat_count, c->d_tie_rec, c->d_tie_count, c->d_tie_fix, c->d_mm};
+                    c->d_corr_row_count, c->d_corr_total, c->raw[0], c->raw[1], c->d_tan_col, c->d_tan_row, c->d_flat,
+                    c->d_flat_count, c->d_tie_rec, c->d_tie_count, c->d_tie_fix};
     for (void *p : ptrs)
         if (p) cudaFree(p);
     if (c->h_small) cudaFreeHost(c->h_small);
     if (c->d_csv) cudaFree(c->d_csv);
     if (c->d_csv_scratch) cudaFree(c->d_csv_scratch);
     for (auto &sl : c->slots) {
-        for (void *p : {(void *)sl.d_cloud, (void *)sl.d_labels, (void *)sl.d_depth, (void *)sl.d_mm})  // the other outputs live inside d_labels
+        for (void *p : {(void *)sl.d_cloud, (void *)sl.d_labels, (void *)sl.raw[0], (void *)sl.raw[1]})  // the other outputs live inside d_labels
             if (p) cudaFree(p);
         for (cudaEvent_t e : {sl.in_done, sl.compute_done, sl.out_done})
             if (e) cudaEventDestroy(e);
     }
     for (auto &ps : c->pre) {
-        for (void *p : {(void *)ps.d_cloud, (void *)ps.d_labels, (void *)ps.d_depth, (void *)ps.d_mm})
+        for (void *p : {(void *)ps.d_cloud, (void *)ps.d_labels, (void *)ps.raw[0], (void *)ps.raw[1]})
             if (p) cudaFree(p);
         for (cudaEvent_t e : {ps.ready, ps.released})
             if (e) cudaEventDestroy(e);
@@ -492,7 +495,7 @@ extern "C" nav_ctx *nav_create(int rows, int cols, int device, int n_seq) {
     ALLOC(c->d_corr, nt * sizeof(nav_corr));
     ALLOC(c->d_corr_row_count, nr * 4);
     ALLOC(c->d_corr_total, (size_t)n_seq * 4);
-    ALLOC(c->d_dist, c->npx * 4);
+    ALLOC(c->raw[0], c->npx * 4);
     ALLOC(c->d_tan_col, (size_t)cols * 8);
     ALLOC(c->d_tan_row, (size_t)rows * 8);
     ALLOC(c->d_flat, (size_t)cols * 24 * 2 + (size_t)cols * 8);
@@ -854,14 +857,59 @@ static PoseBatch pose_batch(const nav_ctx *c, const nav_pos *pos, const nav_pos 
     return b;
 }
 
+// ------------------------------------------------------------------ frame formats -----------
+// A frame (n_seq images) comes as xyz doubles (NAV_RUN_INPUT_XYZ, 24 B/point), a depth matrix (NAV_RUN_INPUT_DEPTH,
+// int32, 4 B/pixel) or integer-mm xyz (NAV_RUN_INPUT_MM, int32 x 3, 12 B/point).  The int32 formats cross PCIe raw and
+// become xyz on the device (to_xyz), or are read raw by the sequence and device-loop kernels.
+
+// bytes of one element (a double of xyz, an int32 otherwise) and of one frame of `kind`
+static size_t elem_bytes(int kind) { return kind == NAV_RUN_INPUT_XYZ ? sizeof(double) : sizeof(int); }
+static size_t frame_bytes(const nav_ctx *c, int kind) {
+    return c->ntot * elem_bytes(kind) * (kind == NAV_RUN_INPUT_DEPTH ? 1 : 3);
+}
+
+// frame f of a device-resident recording (frames back to back)
+static const void *frame_at(const nav_ctx *c, const void *frames, int kind, size_t f) {
+    return (const unsigned char *)frames + f * frame_bytes(c, kind);
+}
+
+// The frame formats of the device-resident calls: a kind other than the three, or a frame pointer off its element's
+// alignment (8 bytes for xyz doubles, 4 for int32), is refused before anything is queued.
+static int check_frame_input(const char *name, const void *frames, int kind) {
+    if (kind != NAV_RUN_INPUT_XYZ && kind != NAV_RUN_INPUT_DEPTH && kind != NAV_RUN_INPUT_MM)
+        return fail("%s: input_kind %d is none of NAV_RUN_INPUT_XYZ (0), NAV_RUN_INPUT_DEPTH (1), NAV_RUN_INPUT_MM (2)",
+                    name, kind);
+    const unsigned align = (unsigned)elem_bytes(kind);
+    if (((uintptr_t)frames & (align - 1u)) != 0)
+        return fail("%s: the frame pointer %p is not %u-byte aligned", name, frames, align);
+    return 0;
+}
+
+// where a raw frame of `kind` is uploaded: slot [0] (depth) or [1] (integer mm) of its holder's pair, allocated at
+// frame_bytes on first use.  NULL, with the error set, if that allocation fails.
+static int *raw_buf(const nav_ctx *c, int *(&raw)[2], int kind) {
+    int *&p = raw[kind == NAV_RUN_INPUT_MM];
+    if (!p) CUP(cudaMalloc((void **)&p, frame_bytes(c, kind)));
+    return p;
+}
+
+// n_img images of depth or integer-mm xyz at `raw` -> xyz doubles, on `stream`: k_convert (a2) or k_widen_mm, the
+// arithmetic the in-kernel conversion of k_frame_seq / k_loop_step shares.  The caller orders `stream`.
+static void to_xyz(nav_ctx *c, int kind, const int *raw, double *xyz, int n_img, cudaStream_t stream) {
+    if (kind == NAV_RUN_INPUT_DEPTH)
+        launch_convert(raw, c->d_tan_col, c->d_tan_row, xyz, c->rows, c->cols, n_img, c->sm_count, stream);
+    else
+        launch_widen_mm(raw, xyz, (long long)(n_img * c->npx), c->sm_count, stream);
+    c->launches++;
+}
+
 // ------------------------------------------------------------------ function level ----------
 extern "C" int nav_convert_to_pointcloud(nav_ctx *c, const int *distances, nav_point *cloud_out) {
     CTX_ENTER(c, "nav_convert_to_pointcloud");
     if (!distances || !cloud_out) return fail("nav_convert_to_pointcloud: null argument");
     if (c->stage.reserve(c->npx * 28 + 512, c->stream)) return fail("nav_convert_to_pointcloud: staging");
-    if (c->stage.h2d(c->d_dist, distances, c->npx * 4, c->stream)) return fail("nav_convert_to_pointcloud: H2D");
-    launch_convert(c->d_dist, c->d_tan_col, c->d_tan_row, c->d_cloud, c->rows, c->cols, 1, c->sm_count, c->stream);
-    c->launches++;
+    if (c->stage.h2d(c->raw[0], distances, c->npx * 4, c->stream)) return fail("nav_convert_to_pointcloud: H2D");
+    to_xyz(c, NAV_RUN_INPUT_DEPTH, c->raw[0], c->d_cloud, 1, c->stream);  // one image, whatever n_seq
     c->cloud_resident = false;
     if (c->stage.d2h(cloud_out, c->d_cloud, c->npx * 24, c->stream)) return fail("nav_convert_to_pointcloud: D2H");
     return finish_call(c, "nav_convert_to_pointcloud");
@@ -963,34 +1011,6 @@ extern "C" int nav_slam_init(nav_ctx *c, const nav_pos *pos, const nav_point *cl
     return finish_call(c, "nav_slam_init");
 }
 
-// The frame formats of the device-resident calls (NAV_RUN_INPUT_*): a kind other than the three, or a frame pointer
-// off its element's alignment (8 bytes for xyz doubles, 4 for int32), is refused before anything is queued.
-static int check_frame_input(const char *name, const void *frames, int kind) {
-    if (kind != NAV_RUN_INPUT_XYZ && kind != NAV_RUN_INPUT_DEPTH && kind != NAV_RUN_INPUT_MM)
-        return fail("%s: input_kind %d is none of NAV_RUN_INPUT_XYZ (0), NAV_RUN_INPUT_DEPTH (1), NAV_RUN_INPUT_MM (2)",
-                    name, kind);
-    const unsigned align = kind == NAV_RUN_INPUT_XYZ ? 8u : 4u;
-    if (((uintptr_t)frames & (align - 1u)) != 0)
-        return fail("%s: the frame pointer %p is not %u-byte aligned", name, frames, align);
-    return 0;
-}
-
-// elements between consecutive frames of a device-resident recording: doubles for xyz, int32 otherwise
-static long long frame_stride_elems(const nav_ctx *c, int kind) {
-    return (long long)c->ntot * (kind == NAV_RUN_INPUT_DEPTH ? 1 : 3);
-}
-
-// one depth or integer-mm frame (n_seq images) -> xyz doubles at dst, on the context's stream: k_convert (a2) or
-// k_widen_mm, the arithmetic the in-kernel conversion of k_frame_seq / k_loop_step shares
-static void convert_frame(nav_ctx *c, const void *src, int kind, double *dst) {
-    if (kind == NAV_RUN_INPUT_DEPTH)
-        launch_convert((const int *)src, c->d_tan_col, c->d_tan_row, dst, c->rows, c->cols, c->n_seq, c->sm_count,
-                       c->stream);
-    else
-        launch_widen_mm((const int *)src, dst, (long long)c->ntot, c->sm_count, c->stream);
-    c->launches++;
-}
-
 // nav_slam_init_dev (xyz) and nav_slam_init_dev_ex; `name` is the entry point the caller used
 static int slam_init_dev(nav_ctx *c, const char *name, const void *dev_frame, int kind, const nav_pos *pos) {
     if (!pos || !dev_frame) return fail("%s: null argument", name);
@@ -999,7 +1019,7 @@ static int slam_init_dev(nav_ctx *c, const char *name, const void *dev_frame, in
     const double *cloud = (const double *)dev_frame;
     if (kind != NAV_RUN_INPUT_XYZ) {  // converted into the context's cloud buffer, then labelled and mapped as xyz
         order_after_async(c);
-        convert_frame(c, dev_frame, kind, c->d_cloud);
+        to_xyz(c, kind, (const int *)dev_frame, c->d_cloud, c->n_seq, c->stream);
         cloud = c->d_cloud;
     }
     run_labels(c, cloud, c->d_labels, nullptr, c->n_seq);
@@ -1115,10 +1135,6 @@ extern "C" int nav_slam_localization(nav_ctx *c, const nav_point *cloud, const n
 // nav_slam_prefetch queues both on the copy-in stream, so they run under frame t's match, download and
 // host fit; nav_slam_localization_fast then finds the frame resident and labelled.
 
-// What a host frame holds: the cloud itself (nav_point, 24 B/point), the L5 depth matrix (int mm per pixel, converted
-// on the device, n_seq == 1) or integer-mm xyz (int32 [n][3], widened on the device).
-enum InputKind { kInputCloud, kInputDepth, kInputMm };
-
 static int pre_setup(nav_ctx *c) {
     if (c->pre[0].d_cloud) return 0;
     if (!c->s_in) CU(cudaStreamCreateWithFlags(&c->s_in, cudaStreamNonBlocking));
@@ -1131,9 +1147,10 @@ static int pre_setup(nav_ctx *c) {
     return 0;
 }
 
-static int prefetch_common(nav_ctx *c, const char *name, InputKind kind, const void *src) {
+// src: a host frame of `kind` (NAV_RUN_INPUT_*; depth needs n_seq == 1)
+static int prefetch_common(nav_ctx *c, const char *name, int kind, const void *src) {
     if (!src) return fail("%s: null argument", name);
-    if (kind == kInputDepth && c->n_seq != 1) return fail("%s: depth input needs n_seq == 1", name);
+    if (kind == NAV_RUN_INPUT_DEPTH && c->n_seq != 1) return fail("%s: depth input needs n_seq == 1", name);
     if (!Stager::is_pinned(src)) return fail("%s: the host buffer must be pinned (nav_host_alloc / cudaHostRegister)", name);
     if (pre_setup(c)) return 1;
     nav_ctx::PreSlot &ps = c->pre[c->pre_next];
@@ -1151,19 +1168,10 @@ static int prefetch_common(nav_ctx *c, const char *name, InputKind kind, const v
     if (!ps.release_recorded) CU(cudaEventRecord(ps.released, c->stream));
     ps.release_recorded = false;
     CU(cudaStreamWaitEvent(c->s_in, ps.released, 0));
-    if (kind == kInputDepth) {
-        if (!ps.d_depth) CU(cudaMalloc((void **)&ps.d_depth, c->npx * 4));
-        CU(cudaMemcpyAsync(ps.d_depth, src, c->npx * 4, cudaMemcpyHostToDevice, c->s_in));
-        launch_convert(ps.d_depth, c->d_tan_col, c->d_tan_row, ps.d_cloud, c->rows, c->cols, 1, c->sm_count, c->s_in);
-        c->launches++;
-    } else if (kind == kInputMm) {
-        if (!ps.d_mm) CU(cudaMalloc((void **)&ps.d_mm, c->ntot * 12));
-        CU(cudaMemcpyAsync(ps.d_mm, src, c->ntot * 12, cudaMemcpyHostToDevice, c->s_in));
-        launch_widen_mm(ps.d_mm, ps.d_cloud, (long long)c->ntot, c->sm_count, c->s_in);
-        c->launches++;
-    } else {
-        CU(cudaMemcpyAsync(ps.d_cloud, src, c->ntot * 24, cudaMemcpyHostToDevice, c->s_in));
-    }
+    int *raw = nullptr;
+    if (kind != NAV_RUN_INPUT_XYZ && !(raw = raw_buf(c, ps.raw, kind))) return 1;
+    CU(cudaMemcpyAsync(raw ? (void *)raw : ps.d_cloud, src, frame_bytes(c, kind), cudaMemcpyHostToDevice, c->s_in));
+    if (raw) to_xyz(c, kind, raw, ps.d_cloud, c->n_seq, c->s_in);
     launch_labels(ps.d_cloud, ps.d_labels, nullptr, (long long)c->n_seq * c->rows, c->cols, c->sm_count, c->d_n_exact,
                   c->s_in);
     c->launches++;
@@ -1176,17 +1184,17 @@ static int prefetch_common(nav_ctx *c, const char *name, InputKind kind, const v
 
 extern "C" int nav_slam_prefetch(nav_ctx *c, const nav_point *cloud) {
     CTX_ENTER(c, "nav_slam_prefetch");
-    return prefetch_common(c, "nav_slam_prefetch", kInputCloud, cloud);
+    return prefetch_common(c, "nav_slam_prefetch", NAV_RUN_INPUT_XYZ, cloud);
 }
 
 extern "C" int nav_slam_prefetch_depth(nav_ctx *c, const int *distances) {
     CTX_ENTER(c, "nav_slam_prefetch_depth");
-    return prefetch_common(c, "nav_slam_prefetch_depth", kInputDepth, distances);
+    return prefetch_common(c, "nav_slam_prefetch_depth", NAV_RUN_INPUT_DEPTH, distances);
 }
 
 extern "C" int nav_slam_prefetch_mm(nav_ctx *c, const int32_t *cloud_mm) {
     CTX_ENTER(c, "nav_slam_prefetch_mm");
-    return prefetch_common(c, "nav_slam_prefetch_mm", kInputMm, cloud_mm);
+    return prefetch_common(c, "nav_slam_prefetch_mm", NAV_RUN_INPUT_MM, cloud_mm);
 }
 
 // slam_localization with the fit driven by five sufficient statistics reduced on the device
@@ -1352,13 +1360,11 @@ extern "C" int nav_slam_run(nav_ctx *c, const void *const *frames, int n_frames,
     if (c->n_seq != 1) return fail("nav_slam_run: needs n_seq == 1");
     if (!c->have_map) return fail("nav_slam_run: call nav_slam_init first");
     nav_pos last = *pos_start;
-    // NAV_RUN_INPUT_*; every non-zero value other than NAV_RUN_INPUT_MM means depth matrices
-    const InputKind kind = input_kind == NAV_RUN_INPUT_XYZ ? kInputCloud
-                           : input_kind == NAV_RUN_INPUT_MM ? kInputMm
-                                                            : kInputDepth;
+    // every non-zero value other than NAV_RUN_INPUT_MM means depth matrices
+    const int kind = input_kind == NAV_RUN_INPUT_XYZ || input_kind == NAV_RUN_INPUT_MM ? input_kind : NAV_RUN_INPUT_DEPTH;
     auto prefetch = [&](int t) { return prefetch_common(c, "nav_slam_run", kind, frames[t]); };
     // a frame that is not a cloud is found as the oldest prefetched one, never uploaded as a cloud
-    auto cloud_of = [&](int t) { return kind == kInputCloud ? (const nav_point *)frames[t] : nullptr; };
+    auto cloud_of = [&](int t) { return kind == NAV_RUN_INPUT_XYZ ? (const nav_point *)frames[t] : nullptr; };
     for (auto &ps : c->pre) ps.pending = false;
     // the loop maps its own frames: a frame an earlier localization call left unmapped in a prefetch slot is
     // given up, so that the slot can be refilled
@@ -1534,9 +1540,7 @@ static int slam_run_dev(nav_ctx *c, const char *name, const void *dev_frames, in
     // the label ring: frame t's labels go where the launch of frame t+1 maps them from; the last frame's land in
     // d_labels, as nav_frame_results_dev reports them
     auto labels_of = [&](int t) { return ((n_frames - 1 - t) & 1) ? c->d_labels_alt : c->d_labels; };
-    const size_t elem = kind == NAV_RUN_INPUT_XYZ ? sizeof(double) : sizeof(int);
-    const long long stride = frame_stride_elems(c, kind);
-    auto frame = [&](int t) { return (const void *)((const unsigned char *)dev_frames + (size_t)t * stride * elem); };
+    auto frame = [&](int t) { return frame_at(c, dev_frames, kind, (size_t)t); };
     const MatchOut mo = {c->d_nn_idx, c->d_nn_dist, c->d_corr_rows, c->d_corr_row_count};
     const TanTables tan = {c->d_tan_col, c->d_tan_row};
     for (int t = 0; t <= n_frames; ++t) {  // t == n_frames: the last frame's map
@@ -1609,32 +1613,25 @@ extern "C" int nav_slam_mapping(nav_ctx *c, const nav_pos *pos, const nav_point 
     return finish_call(c, "nav_slam_mapping");
 }
 
-// the blocking front-end frame from a host cloud, or (distances != null) from a depth matrix: L5 ingest fused with
-// the frame (SURVEY 8f #3, device part) -- the depth matrix (4 B/pixel instead of the 24 B/pixel cloud) is uploaded,
-// converted on the device (a2) and fed straight to the frame kernel; the converted lidar-frame cloud is returned only
-// if the caller asks for it (cloud_out).  cloud_mm != null: integer-mm xyz (12 B/point), widened on the device into
-// the same cloud a double upload would have given
-static int frontend_frame(nav_ctx *c, const char *name, const nav_point *cloud, const int *distances,
-                          const int32_t *cloud_mm, const nav_pos *pos_predict, const nav_pos *pos_last,
-                          const nav_pos *pos_final, nav_point *cloud_out, int *feature_out, int32_t *nn_idx_out,
-                          double *nn_dist_out, nav_point *global_out) {
-    if ((!cloud && !distances && !cloud_mm) || !pos_predict || !pos_last || !pos_final)
-        return fail("%s: null argument", name);
-    if (distances && c->n_seq != 1) return fail("%s: needs n_seq == 1", name);
+// the blocking front-end frame from a host frame of `kind` (NAV_RUN_INPUT_*).  A depth matrix (4 B/pixel instead of
+// the 24 B/pixel cloud; L5 ingest fused with the frame, SURVEY 8f #3, device part) or integer-mm xyz (12 B/point) is
+// uploaded, made xyz on the device and fed straight to the frame kernel; the converted lidar-frame cloud is returned
+// only if the caller asks for it (cloud_out)
+static int frontend_frame(nav_ctx *c, const char *name, int kind, const void *src, const nav_pos *pos_predict,
+                          const nav_pos *pos_last, const nav_pos *pos_final, nav_point *cloud_out, int *feature_out,
+                          int32_t *nn_idx_out, double *nn_dist_out, nav_point *global_out) {
+    if (!src || !pos_predict || !pos_last || !pos_final) return fail("%s: null argument", name);
+    if (kind == NAV_RUN_INPUT_DEPTH && c->n_seq != 1) return fail("%s: needs n_seq == 1", name);
     if (!c->have_map) return fail("%s: call nav_slam_init first", name);
-    if (c->stage.reserve(c->ntot * ((distances ? 4 : 0) + (cloud_mm ? 12 : 0) + 24 + 24 + 4 + 4 + 8) + 4096, c->stream))
-        return fail("%s: staging", name);
-    if (distances) {
-        if (c->stage.h2d(c->d_dist, distances, c->npx * 4, c->stream)) return fail("%s: H2D", name);
-        launch_convert(c->d_dist, c->d_tan_col, c->d_tan_row, c->d_cloud, c->rows, c->cols, 1, c->sm_count, c->stream);
-        c->launches++;
-    } else if (cloud_mm) {
-        if (!c->d_mm) CU(cudaMalloc((void **)&c->d_mm, c->ntot * 12));
-        if (c->stage.h2d(c->d_mm, cloud_mm, c->ntot * 12, c->stream)) return fail("%s: H2D", name);
-        launch_widen_mm(c->d_mm, c->d_cloud, (long long)c->ntot, c->sm_count, c->stream);
-        c->launches++;
-    } else if (upload_cloud(c, cloud, name)) {
-        return 1;
+    const size_t raw_bytes = kind == NAV_RUN_INPUT_XYZ ? 0 : frame_bytes(c, kind);
+    if (c->stage.reserve(raw_bytes + c->ntot * (24 + 24 + 4 + 4 + 8) + 4096, c->stream)) return fail("%s: staging", name);
+    if (kind == NAV_RUN_INPUT_XYZ) {
+        if (upload_cloud(c, (const nav_point *)src, name)) return 1;
+    } else {
+        int *raw = raw_buf(c, c->raw, kind);
+        if (!raw) return 1;
+        if (c->stage.h2d(raw, src, raw_bytes, c->stream)) return fail("%s: H2D", name);
+        to_xyz(c, kind, raw, c->d_cloud, c->n_seq, c->stream);
     }
     order_after_async(c);
     if (run_frame_fused(c, c->d_cloud, c->d_labels, c->d_nn_idx, c->d_nn_dist, pos_predict, pos_last, pos_final, false,
@@ -1653,7 +1650,7 @@ extern "C" int nav_frontend_frame(nav_ctx *c, const nav_point *cloud, const nav_
                                   const nav_pos *pos_last, const nav_pos *pos_final, int *feature_out,
                                   int32_t *nn_idx_out, double *nn_dist_out, nav_point *global_out) {
     CTX_ENTER(c, "nav_frontend_frame");
-    return frontend_frame(c, "nav_frontend_frame", cloud, nullptr, nullptr, pos_predict, pos_last, pos_final, nullptr,
+    return frontend_frame(c, "nav_frontend_frame", NAV_RUN_INPUT_XYZ, cloud, pos_predict, pos_last, pos_final, nullptr,
                           feature_out, nn_idx_out, nn_dist_out, global_out);
 }
 
@@ -1661,7 +1658,7 @@ extern "C" int nav_frontend_frame_mm(nav_ctx *c, const int32_t *cloud_mm, const 
                                      const nav_pos *pos_last, const nav_pos *pos_final, int *feature_out,
                                      int32_t *nn_idx_out, double *nn_dist_out, nav_point *global_out) {
     CTX_ENTER(c, "nav_frontend_frame_mm");
-    return frontend_frame(c, "nav_frontend_frame_mm", nullptr, nullptr, cloud_mm, pos_predict, pos_last, pos_final,
+    return frontend_frame(c, "nav_frontend_frame_mm", NAV_RUN_INPUT_MM, cloud_mm, pos_predict, pos_last, pos_final,
                           nullptr, feature_out, nn_idx_out, nn_dist_out, global_out);
 }
 
@@ -1670,8 +1667,8 @@ extern "C" int nav_frontend_frame_depth(nav_ctx *c, const int *distances, const 
                                         int *feature_out, int32_t *nn_idx_out, double *nn_dist_out,
                                         nav_point *global_out) {
     CTX_ENTER(c, "nav_frontend_frame_depth");
-    return frontend_frame(c, "nav_frontend_frame_depth", nullptr, distances, nullptr, pos_predict, pos_last, pos_final,
-                          cloud_out, feature_out, nn_idx_out, nn_dist_out, global_out);
+    return frontend_frame(c, "nav_frontend_frame_depth", NAV_RUN_INPUT_DEPTH, distances, pos_predict, pos_last,
+                          pos_final, cloud_out, feature_out, nn_idx_out, nn_dist_out, global_out);
 }
 
 // ------------------------------------------------------------------ CSV rows on the device ---
@@ -1746,9 +1743,9 @@ extern "C" int nav_csv_format_frame_gpu(nav_ctx *c, unsigned long long timestamp
         if (c->stage.h2d(c->d_global, global_cloud, c->npx * 24, c->stream)) return fail("nav_csv_format_frame_gpu: H2D");
         d_cloud = c->d_global;
     }
-    if (distances && c->stage.h2d(c->d_dist, distances, c->npx * 4, c->stream)) return fail("nav_csv_format_frame_gpu: H2D");
+    if (distances && c->stage.h2d(c->raw[0], distances, c->npx * 4, c->stream)) return fail("nav_csv_format_frame_gpu: H2D");
     CsvJob job;
-    int rc = csv_job(c, "nav_csv_format_frame_gpu", timestamp, d_cloud, distances ? c->d_dist : nullptr, imu, lidar_pos,
+    int rc = csv_job(c, "nav_csv_format_frame_gpu", timestamp, d_cloud, distances ? c->raw[0] : nullptr, imu, lidar_pos,
                      ekf_pos, job);
     if (rc > 0) return rc;
     bool host_format = rc < 0;
@@ -1838,10 +1835,12 @@ static int frontend_submit(nav_ctx *c, const char *name, const int32_t *cloud_mm
         if (io->distances && c->n_seq != 1) return fail("%s: depth input needs n_seq == 1", name);
         if (io->cloud_out && !io->distances) return fail("%s: cloud_out is the converted depth matrix; there is none", name);
     }
+    const int kind = cloud_mm ? NAV_RUN_INPUT_MM : io->distances ? NAV_RUN_INPUT_DEPTH : NAV_RUN_INPUT_XYZ;
+    const void *src = cloud_mm ? (const void *)cloud_mm : io->distances ? (const void *)io->distances : io->cloud;
     if (!c->have_map) return fail("%s: call nav_slam_init first", name);
     if (async_setup(c)) return 1;
-    const void *hp[] = {cloud_mm, io->cloud, io->distances, io->cloud_out, io->feature_out, io->mask_out,
-                        io->nn_idx_out, io->nn_dist_out, io->global_out};
+    const void *hp[] = {src, io->cloud_out, io->feature_out, io->mask_out, io->nn_idx_out, io->nn_dist_out,
+                        io->global_out};
     for (const void *p : hp)
         if (p && !Stager::is_pinned(p))
             return fail("%s: host buffers must be pinned (nav_host_alloc / cudaHostRegister)", name);
@@ -1850,26 +1849,14 @@ static int frontend_submit(nav_ctx *c, const char *name, const int32_t *cloud_mm
     const bool reused = c->async_frames >= (uint64_t)nav_ctx::kSlots;
     // copy-in: the slot's cloud was last read by the kernels of frame t-2
     if (reused) CU(cudaStreamWaitEvent(c->s_in, sl.compute_done, 0));
-    if (cloud_mm) {
-        if (!sl.d_mm) CU(cudaMalloc((void **)&sl.d_mm, c->ntot * 12));
-        CU(cudaMemcpyAsync(sl.d_mm, cloud_mm, c->ntot * 12, cudaMemcpyHostToDevice, c->s_in));
-    } else if (io->distances) {
-        if (!sl.d_depth) CU(cudaMalloc((void **)&sl.d_depth, c->npx * 4));
-        CU(cudaMemcpyAsync(sl.d_depth, io->distances, c->npx * 4, cudaMemcpyHostToDevice, c->s_in));
-    } else {
-        CU(cudaMemcpyAsync(sl.d_cloud, io->cloud, c->ntot * 24, cudaMemcpyHostToDevice, c->s_in));
-    }
+    int *raw = nullptr;
+    if (kind != NAV_RUN_INPUT_XYZ && !(raw = raw_buf(c, sl.raw, kind))) return 1;
+    CU(cudaMemcpyAsync(raw ? (void *)raw : sl.d_cloud, src, frame_bytes(c, kind), cudaMemcpyHostToDevice, c->s_in));
     CU(cudaEventRecord(sl.in_done, c->s_in));
     // kernels: need the upload, and the slot's output buffers released by the downloads of frame t-2
     CU(cudaStreamWaitEvent(c->stream, sl.in_done, 0));
     if (reused) CU(cudaStreamWaitEvent(c->stream, sl.out_done, 0));
-    if (cloud_mm) {  // widened on the device: 12 B/point crossed PCIe instead of 24
-        launch_widen_mm(sl.d_mm, sl.d_cloud, (long long)c->ntot, c->sm_count, c->stream);
-        c->launches++;
-    } else if (io->distances) {  // a2 on the device: 4 B/pixel crossed PCIe instead of 24
-        launch_convert(sl.d_depth, c->d_tan_col, c->d_tan_row, sl.d_cloud, c->rows, c->cols, 1, c->sm_count, c->stream);
-        c->launches++;
-    }
+    if (raw) to_xyz(c, kind, raw, sl.d_cloud, c->n_seq, c->stream);  // 4 or 12 B/point crossed PCIe instead of 24
     if (run_frame_fused(c, sl.d_cloud, sl.d_labels, sl.d_nn_idx, sl.d_nn_dist, pos_predict, pos_last, pos_final)) return 1;
     CU(cudaEventRecord(sl.compute_done, c->stream));
     c->cloud_resident = false;
@@ -2011,7 +1998,7 @@ static int frontend_sequence(nav_ctx *c, const char *name, const void *dev_frame
         if (!so->label_mask && !so->nn_idx && !so->nn_dist && !so->fit_stats) so = nullptr;
     }
     const bool raw = kind != NAV_RUN_INPUT_XYZ;
-    const long long stride = frame_stride_elems(c, kind);
+    const long long stride = (long long)(frame_bytes(c, kind) / elem_bytes(kind));  // in elements, for k_frame_seq
     order_after_async(c);
     // One launch for the whole sequence (k_frame_seq: a thread-block cluster per image row walks through the
     // frames with a cluster barrier per frame) when a row's tiles fit a cluster; NAV_SEQ_LAUNCHES=1 keeps one
@@ -2099,10 +2086,11 @@ static int frontend_sequence(nav_ctx *c, const char *name, const void *dev_frame
     } else {
         const size_t n_chunks = (size_t)c->map.n_chunks;
         for (size_t f = 0; f < n_frames; ++f) {
-            const double *cl = (const double *)dev_frames + f * c->ntot * 3;
+            const void *frame = frame_at(c, dev_frames, kind, f);
+            const double *cl = (const double *)frame;
             if (raw) {  // frame f into slot f % 2: the kernels of frame f-1 read the other slot
                 cl = c->d_conv + (f & 1) * c->ntot * 3;
-                convert_frame(c, (const int *)dev_frames + f * stride, kind, (double *)cl);
+                to_xyz(c, kind, (const int *)frame, (double *)cl, c->n_seq, c->stream);
             }
             const size_t o = f * (size_t)c->n_seq;
             // consecutive launches overlap (programmatic dependent launch): frame f+1 computes its labels

@@ -31,6 +31,7 @@
 #include <stdint.h>
 #include <stdlib.h>
 
+#include <type_traits>
 #include <utility>
 
 #include "nav_bulk.cuh"
@@ -1378,6 +1379,19 @@ static int launch_row_clusters(void (*kernel)(Params...), dim3 grid, int tiles, 
     return (int)cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
 }
 
+// f(std::integral_constant<int, K>) for the frame kind K == kind (NAV_RUN_INPUT_*), and f(std::bool_constant<b>):
+// a run-time choice turned into the template argument of a kernel
+template <typename F>
+static int with_kind(int kind, F &&f) {
+    if (kind == kKindDepth) return f(std::integral_constant<int, kKindDepth>{});
+    if (kind == kKindMm) return f(std::integral_constant<int, kKindMm>{});
+    return f(std::integral_constant<int, kKindXyz>{});
+}
+template <typename F>
+static int with_flag(bool b, F &&f) {
+    return b ? f(std::true_type{}) : f(std::false_type{});
+}
+
 int launch_dedupe_stats(const double *cloud, const int *labels, const RowMap &map, const MatchOut &out,
                         const PoseBatch &poses, int n_seq, int rows, int cols, cudaStream_t stream, double *part,
                         const FitMailbox &mail) {
@@ -1407,12 +1421,11 @@ int launch_loop_step_dev(int kind, const DevLoop &dl, const void *cloud, const v
     LoopPoses<true> ps;
     static_cast<DevLoop &>(ps) = dl;
     const FitMailbox no_mail = {nullptr, nullptr, 0ull};
-    auto kernel = kind == kKindDepth ? k_loop_step<true, kKindDepth>
-                  : kind == kKindMm  ? k_loop_step<true, kKindMm>
-                                     : k_loop_step<true, kKindXyz>;
-    return launch_row_clusters(kernel, dim3((unsigned)(n_seq * rows * tiles)), tiles, stream, (const double *)cloud,
-                               (const int *)nullptr, map, out, ps, rows, cols, tiles, (const double *)prev_cloud,
-                               prev_labels, do_map ? 1 : 0, part, no_mail, tan);
+    return with_kind(kind, [&](auto k) {
+        return launch_row_clusters(k_loop_step<true, k>, dim3((unsigned)(n_seq * rows * tiles)), tiles, stream,
+                                   (const double *)cloud, (const int *)nullptr, map, out, ps, rows, cols, tiles,
+                                   (const double *)prev_cloud, prev_labels, do_map ? 1 : 0, part, no_mail, tan);
+    });
 }
 
 // queued on `stream`, in front of the kernels that read the tables; c1 / c2 must stay valid (the host's static tables).
@@ -1709,52 +1722,6 @@ static bool frame_seq_bulk_ok(int kind, const void *frames, long long frame_stri
     return cols % 4 == 0 && frame_stride % 4 == 0 && maps;
 }
 
-template <bool kBulk, int kKind>
-static int launch_frame_seq_variant(const void *frames, long long frame_stride, int n_frames, int *labels,
-                                    const RowMap &map0, const RowMap &map1, const MatchOut &out,
-                                    const PoseXf *d_pose_loc, const PoseXf *d_pose_fin, int n_seq, int rows, int cols,
-                                    unsigned *n_exact, cudaStream_t stream, const PoseXf *h_pose_loc,
-                                    const PoseXf *h_pose_fin, const SeqOut *seq_out, const TanTables &tan) {
-    const int tiles = div_up(cols, kTile);
-    const SeqArgs a = {(const double *)frames, frame_stride, n_frames, n_seq, d_pose_loc, d_pose_fin};
-    const bool inl = h_pose_loc && h_pose_fin && n_seq == 1 && n_frames <= kSeqInlineFrames;
-    const dim3 grid((unsigned)tiles, (unsigned)rows, (unsigned)n_seq);
-    const SeqOut no_out = {nullptr, nullptr, nullptr, nullptr};
-    if (inl) {
-        SeqInlinePoses ip;  // the launch copies its parameters at the call
-        for (int f = 0; f < n_frames; ++f) {
-            ip.loc[f] = h_pose_loc[f];
-            ip.fin[f] = h_pose_fin[f];
-        }
-        for (int f = n_frames; f < kSeqInlineFrames; ++f) ip.loc[f] = ip.fin[f] = h_pose_loc[0];
-        if (seq_out)
-            return launch_row_clusters(k_frame_seq<true, true, kBulk, kKind>, grid, tiles, stream, a, labels, map0, map1, out,
-                                       rows, cols, n_exact, ip, *seq_out, tan);
-        return launch_row_clusters(k_frame_seq<true, false, kBulk, kKind>, grid, tiles, stream, a, labels, map0, map1, out,
-                                   rows, cols, n_exact, ip, no_out, tan);
-    }
-    static const SeqInlinePoses none = {};
-    if (seq_out)
-        return launch_row_clusters(k_frame_seq<false, true, kBulk, kKind>, grid, tiles, stream, a, labels, map0, map1, out,
-                                   rows, cols, n_exact, none, *seq_out, tan);
-    return launch_row_clusters(k_frame_seq<false, false, kBulk, kKind>, grid, tiles, stream, a, labels, map0, map1, out,
-                               rows, cols, n_exact, none, no_out, tan);
-}
-
-template <int kKind>
-static int launch_frame_seq_kind(bool bulk, const void *frames, long long frame_stride, int n_frames, int *labels,
-                                 const RowMap &map0, const RowMap &map1, const MatchOut &out, const PoseXf *d_pose_loc,
-                                 const PoseXf *d_pose_fin, int n_seq, int rows, int cols, unsigned *n_exact,
-                                 cudaStream_t stream, const PoseXf *h_pose_loc, const PoseXf *h_pose_fin,
-                                 const SeqOut *seq_out, const TanTables &tan) {
-    return bulk ? launch_frame_seq_variant<true, kKind>(frames, frame_stride, n_frames, labels, map0, map1, out, d_pose_loc,
-                                                        d_pose_fin, n_seq, rows, cols, n_exact, stream, h_pose_loc,
-                                                        h_pose_fin, seq_out, tan)
-                : launch_frame_seq_variant<false, kKind>(frames, frame_stride, n_frames, labels, map0, map1, out,
-                                                         d_pose_loc, d_pose_fin, n_seq, rows, cols, n_exact, stream,
-                                                         h_pose_loc, h_pose_fin, seq_out, tan);
-}
-
 // h_pose_loc / h_pose_fin != null (n_seq == 1, n_frames <= frame_seq_inline_frames()): the poses are passed as
 // kernel parameters and the device arrays are not read.  seq_out != null: the output mode of k_frame_seq.
 int launch_frame_seq(int kind, const void *frames, long long frame_stride, int n_frames, int *labels, const RowMap &map0,
@@ -1763,17 +1730,30 @@ int launch_frame_seq(int kind, const void *frames, long long frame_stride, int n
                      const PoseXf *h_pose_fin, const SeqOut *seq_out, bool *bulk_out, const TanTables &tan) {
     const bool bulk = frame_seq_bulk_ok(kind, frames, frame_stride, map0, map1, cols);
     if (bulk_out) *bulk_out = bulk;
-    if (kind == kKindDepth)
-        return launch_frame_seq_kind<kKindDepth>(bulk, frames, frame_stride, n_frames, labels, map0, map1, out, d_pose_loc,
-                                                 d_pose_fin, n_seq, rows, cols, n_exact, stream, h_pose_loc, h_pose_fin,
-                                                 seq_out, tan);
-    if (kind == kKindMm)
-        return launch_frame_seq_kind<kKindMm>(bulk, frames, frame_stride, n_frames, labels, map0, map1, out, d_pose_loc,
-                                              d_pose_fin, n_seq, rows, cols, n_exact, stream, h_pose_loc, h_pose_fin,
-                                              seq_out, tan);
-    return launch_frame_seq_kind<kKindXyz>(bulk, frames, frame_stride, n_frames, labels, map0, map1, out, d_pose_loc,
-                                           d_pose_fin, n_seq, rows, cols, n_exact, stream, h_pose_loc, h_pose_fin, seq_out,
-                                           tan);
+    const int tiles = div_up(cols, kTile);
+    const SeqArgs a = {(const double *)frames, frame_stride, n_frames, n_seq, d_pose_loc, d_pose_fin};
+    const bool inl = h_pose_loc && h_pose_fin && n_seq == 1 && n_frames <= kSeqInlineFrames;
+    const dim3 grid((unsigned)tiles, (unsigned)rows, (unsigned)n_seq);
+    const SeqOut no_out = {nullptr, nullptr, nullptr, nullptr};
+    static const SeqInlinePoses none = {};
+    SeqInlinePoses ip;  // the launch copies its parameters at the call
+    if (inl) {
+        for (int f = 0; f < n_frames; ++f) {
+            ip.loc[f] = h_pose_loc[f];
+            ip.fin[f] = h_pose_fin[f];
+        }
+        for (int f = n_frames; f < kSeqInlineFrames; ++f) ip.loc[f] = ip.fin[f] = h_pose_loc[0];
+    }
+    return with_kind(kind, [&](auto k) {
+        return with_flag(bulk, [&](auto b) {
+            return with_flag(inl, [&](auto i) {
+                return with_flag(seq_out != nullptr, [&](auto o) {
+                    return launch_row_clusters(k_frame_seq<i, o, b, k>, grid, tiles, stream, a, labels, map0, map1, out,
+                                               rows, cols, n_exact, inl ? ip : none, seq_out ? *seq_out : no_out, tan);
+                });
+            });
+        });
+    });
 }
 
 // Fit totals of frame blockIdx.x, sequence blockIdx.y: part = [n_frames][n_seq][n_part][5] partials, stats =

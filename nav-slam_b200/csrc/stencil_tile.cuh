@@ -76,7 +76,7 @@ __device__ __forceinline__ void tile_stage(StencilSmem &s, const double *__restr
 // ---- the narrow frame formats (NAV_RUN_INPUT_DEPTH / _MM), converted point by point where they are read.  One
 // definition for the conversion kernels (k_convert, k_widen_mm) and for the kernels that stage raw tiles, so the
 // bits cannot drift between them.
-constexpr int kKindXyz = 0, kKindDepth = 1, kKindMm = 2;  // NAV_RUN_INPUT_*
+constexpr int kKindXyz = NAV_RUN_INPUT_XYZ, kKindDepth = NAV_RUN_INPUT_DEPTH, kKindMm = NAV_RUN_INPUT_MM;
 
 // a2 of one pixel, utils/pointcloud.c:18-47: tan(theta_col) / tan(phi_row) are the host libm's values, y = (-d) * tan
 // is one rounded multiply; d <= 0 is no return, (0, 0, 0)

@@ -3,7 +3,7 @@
 and the `-Xptxas -v` lines (registers, spills, shared memory) of each entry function.  A kernel of the new dump is
 matched with the old one of the same name once a trailing template argument 0 and a trailing TanTables parameter are
 dropped (the xyz instantiations of the kernels that gained a frame-kind parameter).
-usage: sass_diff.py old.sass new.sass [new_ptxas.txt]"""
+usage: sass_diff.py old.sass new.sass [new_ptxas.txt [old_ptxas.txt]]"""
 import re
 import subprocess
 import sys
@@ -60,11 +60,19 @@ def main():
         else:
             print(f"DIFFERS  {name.split('(')[0]}: {len(old[name])} -> {len(got[0])} instructions")
     print(f"{same} of {len(old)} kernels of the old dump compile to the same instructions")
-    added = [n for n in new if old_name(n) not in old]
+    added = [n for n in new if n not in old and old_name(n) not in old]
     info = ptxas_lines(sys.argv[3]) if len(sys.argv) > 3 else {}
     print(f"{len(added)} new kernels:")
     for n in sorted(added):
         print(f"  {n.split('(')[0]}: {info.get(n, '')}")
+    if len(sys.argv) > 4:  # the -Xptxas -v lines of every function of both builds, file-hash prefixes dropped
+        strip = lambda d: {re.sub(r"_INTERNAL_[0-9a-f]+_", "_INTERNAL_", k): v for k, v in d.items()}
+        old_info, new_info = strip(ptxas_lines(sys.argv[4])), strip(info)
+        differ = sorted(k for k in old_info.keys() | new_info.keys() if old_info.get(k) != new_info.get(k))
+        print(f"-Xptxas -v: {len(old_info) - len(differ)} of {len(old_info)} functions of the old build report the same"
+              f" registers, stack, spills and shared memory; {len(new_info)} functions in the new build")
+        for k in differ:
+            print(f"  {k.split('(')[0]}: {old_info.get(k)} -> {new_info.get(k)}")
 
 
 if __name__ == "__main__":
